@@ -10,8 +10,9 @@ from .hypergraph_pb2 import (EvaluationMetrics, ExperimentalResult, Hypergraph,
 from .hypergraph_util import (AddNodeToEdge, CompressRange, IsEmpty, Relabel, ToCsrMatrix,
                               ToEdgeCsrMatrix)
 from .algebraic_distance import EmbedAlgebraicDistance
-from .hg2v_sample import (AlgebraicDistanceSamples, AlgebraicDistanceSamplesCsr, BooleanSamples,
-                          BooleanSamplesCsr,
+from .hg2v_sample import (AlgebraicDistanceSamples, AlgebraicDistanceSamplesCsr,
+                          AlgebraicDistanceSamplesDevice, BooleanSamples, BooleanSamplesCsr,
+                          BooleanSamplesDevice,
                           SampleColumns, SamplesToModelInput, SimilarityRecord,
                           SparseWeightedJaccard, WeightedJaccardSamples)
 from .hg2v_model import BooleanModel, KerasModelToEmbedding, UnweightedFloatModel
@@ -26,7 +27,8 @@ __all__ = [
     "Hypergraph", "HypergraphEmbedding", "EvaluationMetrics", "ExperimentalResult",
     "AddNodeToEdge", "CompressRange", "IsEmpty", "Relabel", "ToCsrMatrix", "ToEdgeCsrMatrix",
     "EmbedAlgebraicDistance",
-    "AlgebraicDistanceSamples", "AlgebraicDistanceSamplesCsr", "BooleanSamples", "BooleanSamplesCsr",
+    "AlgebraicDistanceSamples", "AlgebraicDistanceSamplesCsr", "AlgebraicDistanceSamplesDevice",
+    "BooleanSamples", "BooleanSamplesCsr", "BooleanSamplesDevice",
     "SampleColumns",
     "SamplesToModelInput", "SimilarityRecord", "SparseWeightedJaccard", "WeightedJaccardSamples",
     "BooleanModel", "UnweightedFloatModel", "KerasModelToEmbedding", "EMBEDDING_OPTIONS",

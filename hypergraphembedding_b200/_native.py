@@ -150,6 +150,14 @@ SIGNATURES = {
     "hge_embedding_arrays": (ctypes.c_int, [c_vp] * 7),
     "hge_sample_neighbors": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, ctypes.c_int64,
                                             ctypes.c_int, c_vp, c_vp, c_vp]),
+    "hge_sample_pairs_device": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int32,
+                                               ctypes.c_int32, c_vp, ctypes.c_int, ctypes.c_uint64,
+                                               ctypes.c_uint32, ctypes.c_int64, c_vp, c_vp,
+                                               ctypes.c_int64, ctypes.POINTER(ctypes.c_int64),
+                                               ctypes.c_int]),
+    "hge_sample_neighbors_device": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, ctypes.c_int64, ctypes.c_int,
+                                                   ctypes.c_uint64, ctypes.c_uint32, ctypes.c_int64,
+                                                   c_vp, c_vp, ctypes.c_int]),
 }
 
 
@@ -708,6 +716,51 @@ def sample_neighbors(n2e, e2n, nodes, edges, k, state):
   if rc == HGE_ERR_INVALID and "cannot be empty" in last_error():
     raise ValueError("'a' cannot be empty unless no samples are taken")
   check(rc, "hge_sample_neighbors")
+  return nbr_e, nbr_n
+
+
+# ---------------------------------------------------------------------------------------------
+# device sampling (Philox streams, csrc/hge_device_sampler.cu)
+# ---------------------------------------------------------------------------------------------
+
+# phase constants of csrc/hge_philox.cuh (HgePhase)
+PHASE_NN, PHASE_EE, PHASE_NE, PHASE_EN, PHASE_NEIGHBORS = 1, 2, 3, 4, 5
+PHASE_NEG_NN, PHASE_NEG_EE, PHASE_NEG_EE_AGAIN, PHASE_NEG_NE, PHASE_NEG_EN = 6, 7, 8, 9, 10
+PHASE_NEG_NEIGHBORS = 11
+
+
+def sample_pairs_device(ctx, inc, side, factors, row0, samples, seed, phase, negative=False,
+                        workspace_mb=0):
+  """hge_sample_pairs_device over rows [row0, row0 + len(samples)): (row, col) int32 CUDA tensors."""
+  import torch
+  dev = torch.device("cuda", ctx.device)
+  k = torch.as_tensor(_as_i32(samples)).to(dev)
+  cap = int(np.asarray(samples, dtype=np.int64).clip(min=0).sum())
+  out_row = torch.empty(max(cap, 1), dtype=torch.int32, device=dev)
+  out_col = torch.empty(max(cap, 1), dtype=torch.int32, device=dev)
+  count = ctypes.c_int64(0)
+  check(ctx.lib.hge_sample_pairs_device(ctx.handle, inc.handle, int(side), int(factors), int(row0),
+                                        int(row0) + len(k), ptr(k), 1 if negative else 0,
+                                        int(seed) & 0xFFFFFFFFFFFFFFFF, int(phase), int(workspace_mb),
+                                        ptr(out_row), ptr(out_col), cap, ctypes.byref(count), MEM_DEVICE),
+        "hge_sample_pairs_device")
+  return out_row[:count.value], out_col[:count.value]
+
+
+def sample_neighbors_device(ctx, inc, nodes, edges, k, seed, phase, first_index):
+  """hge_sample_neighbors_device on int32 CUDA tensors: ([m, k] edges of the nodes, [m, k] nodes
+  of the edges) as CUDA tensors."""
+  import torch
+  m = int(nodes.shape[0])
+  nbr_e = torch.empty((m, int(k)), dtype=torch.int32, device=nodes.device)
+  nbr_n = torch.empty((m, int(k)), dtype=torch.int32, device=nodes.device)
+  rc = ctx.lib.hge_sample_neighbors_device(ctx.handle, inc.handle, ptr(nodes.contiguous()),
+                                           ptr(edges.contiguous()), m, int(k),
+                                           int(seed) & 0xFFFFFFFFFFFFFFFF, int(phase), int(first_index),
+                                           ptr(nbr_e), ptr(nbr_n), MEM_DEVICE)
+  if rc == HGE_ERR_INVALID and "cannot be empty" in last_error():
+    raise ValueError("'a' cannot be empty unless no samples are taken")
+  check(rc, "hge_sample_neighbors_device")
   return nbr_e, nbr_n
 
 

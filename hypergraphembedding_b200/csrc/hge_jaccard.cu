@@ -30,6 +30,7 @@
 #include <vector>
 
 #include "hge_common.cuh"
+#include "hge_expand.cuh"
 #include "hge_staged.cuh"
 
 namespace {
@@ -147,12 +148,6 @@ __global__ void __launch_bounds__(kBlock) k_expand(
   }
 }
 
-__global__ void k_run_heads(int64_t n, const uint64_t* __restrict__ keys, int64_t* __restrict__ head) {
-  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n;
-       i += (int64_t)gridDim.x * blockDim.x)
-    head[i] = (i == 0 || keys[i] != keys[i - 1]) ? 1 : 0;
-}
-
 // head of a run: the members' values added in member order, then one division by the group size
 // (targets2features[rows].sum(axis=0) / len(rows), hg2v_sample.py:293)
 __global__ void k_run_sums(int64_t n, int64_t g0, const uint64_t* __restrict__ keys,
@@ -172,28 +167,6 @@ __global__ void k_run_sums(int64_t n, int64_t g0, const uint64_t* __restrict__ k
   }
 }
 
-// cptr[g] for g in [g0, g1]: compressed position of the first run of group g (+ rows before this batch)
-__global__ void k_centroid_ptr(int64_t g0, int64_t g1, int64_t n, int64_t n_runs, int64_t rows_before,
-                               const uint64_t* __restrict__ keys, const int64_t* __restrict__ pos,
-                               int64_t* __restrict__ cptr, bool last_batch) {
-  const int64_t count = g1 - g0 + (last_batch ? 1 : 0);
-  for (int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; k < count;
-       k += (int64_t)gridDim.x * blockDim.x) {
-    const uint64_t want = (uint64_t)k << 32;
-    int64_t lo = 0, hi = n;
-    while (lo < hi) {
-      const int64_t mid = (lo + hi) >> 1;
-      if (keys[mid] < want) lo = mid + 1; else hi = mid;
-    }
-    cptr[g0 + k] = rows_before + (lo < n ? pos[lo] : n_runs);
-  }
-}
-
-int grid_for(const hge_ctx* ctx, int64_t work, int per_block = kBlock) {
-  const int64_t want = std::max<int64_t>(1, (work + per_block - 1) / per_block);
-  return (int)std::min<int64_t>(want, (int64_t)ctx->num_sms * 16);
-}
-
 struct FeatureMatrix {
   Staged<int64_t> ptr;
   Staged<int32_t> idx;
@@ -205,13 +178,6 @@ struct FeatureMatrix {
     return HGE_OK;
   }
 };
-
-template <typename T>
-int read_back(hge_ctx* ctx, const T* dev, T* host, size_t n) {
-  HGE_CUDA(cudaMemcpyAsync(host, dev, n * sizeof(T), cudaMemcpyDeviceToHost, ctx->stream));
-  HGE_CUDA(cudaStreamSynchronize(ctx->stream));
-  return HGE_OK;
-}
 
 // Centroid rows of the groups named by pg[0 .. num_pairs): CSR over ALL groups (rows of the
 // groups no pair names are empty).  Everything on ctx->stream; the arrays are the caller's to free.
@@ -270,8 +236,8 @@ int build_centroids(hge_ctx* ctx, const int64_t* gptr, const int32_t* gidx, int6
     const bool last = g1 == groups;
     if (n == 0) {
       // no pair names any of these groups: empty rows
-      k_centroid_ptr<<<grid_for(ctx, g1 - g0 + 1), kBlock, 0, ctx->stream>>>(g0, g1, 0, 0, rows_before, nullptr,
-                                                                           nullptr, out->ptr, last);
+      k_run_starts<<<grid_for(ctx, g1 - g0 + 1), kBlock, 0, ctx->stream>>>(g0, g1, 0, 0, rows_before, nullptr,
+                                                                         nullptr, out->ptr, last);
       HGE_CHECK_LAUNCH(ctx);
       g0 = g1;
       continue;
@@ -315,8 +281,8 @@ int build_centroids(hge_ctx* ctx, const int64_t* gptr, const int32_t* gidx, int6
       HGE_TRY(hge_dev_alloc(ctx, &part.val, (size_t)std::max<int64_t>(1, part.n)));
       k_run_sums<<<grid_for(ctx, n), kBlock, 0, ctx->stream>>>(n, g0, keys2, vals2, pos, gptr, part.idx, part.val);
       HGE_CHECK_LAUNCH(ctx);
-      k_centroid_ptr<<<grid_for(ctx, g1 - g0 + 1), kBlock, 0, ctx->stream>>>(g0, g1, n, part.n, rows_before, keys2,
-                                                                           pos, out->ptr, last);
+      k_run_starts<<<grid_for(ctx, g1 - g0 + 1), kBlock, 0, ctx->stream>>>(g0, g1, n, part.n, rows_before, keys2,
+                                                                         pos, out->ptr, last);
       HGE_CHECK_LAUNCH(ctx);
       return HGE_OK;
     };

@@ -390,6 +390,122 @@ def BooleanSamplesCsr(incidence, num_neighbors, num_samples, neg_samples=0, node
 
 
 ################################################################################
+# Device sampling from seeded Philox streams                                   #
+################################################################################
+
+
+class _DeviceSampler(object):
+  """Pair and neighbour draws of csrc/hge_device_sampler.cu over a device incidence, in row chunks
+  of `chunk_rows` (0 = one call per block).  Every row and every record owns its Philox stream
+  (csrc/hge_philox.cuh), so the chunking does not change the result.  `spent` receives the seconds
+  of the pair ("pairs") and neighbour ("neighbours") calls; both end in a device synchronise."""
+
+  def __init__(self, g, ctx, inc, k, seed, chunk_rows, workspace_mb=0):
+    assert np.array_equal(g.node_rows, np.arange(g.num_nodes)) and \
+        np.array_equal(g.edge_rows, np.arange(g.num_edges)), \
+        "the device sampler emits rows in ascending id order"
+    self.ctx, self.inc, self.k, self.seed = ctx, inc, int(k), int(seed)
+    self.chunk_rows, self.workspace_mb = int(chunk_rows), int(workspace_mb)
+    self.spent = {"pairs": 0.0, "neighbours": 0.0}
+
+  def _timed(self, kind, fn, *args, **kw):
+    import time
+    t = time.perf_counter()
+    out = fn(*args, **kw)
+    self.spent[kind] += time.perf_counter() - t
+    return out
+
+  def pairs(self, side, factors, samples, phase, negative=False):
+    """(row, col) CUDA tensors, chunk by chunk, rows ascending."""
+    samples = np.asarray(samples, dtype=np.int32)
+    step = len(samples) if not self.chunk_rows else self.chunk_rows
+    for lo in range(0, len(samples), max(step, 1)):
+      yield self._timed("pairs", _native.sample_pairs_device, self.ctx, self.inc, side, factors, lo,
+                        samples[lo:lo + step], self.seed, phase, negative=negative,
+                        workspace_mb=self.workspace_mb)
+
+  def node_edge(self, node_s, edge_s, factors, phases, negative=False):
+    """(nodes, edges, neighbour nodes, neighbour edges) CUDA tensors of the node-edge block: node
+    rows, then edge rows; the neighbour streams are numbered by record inside the block."""
+    ne, en, nbr = phases
+    first = 0
+    for side, samples, phase in ((0, node_s, ne), (1, edge_s, en)):
+      for r, c in self.pairs(side, factors, samples, phase, negative):
+        nodes, edges = (r, c) if side == 0 else (c, r)
+        nbr_e, nbr_n = self._timed("neighbours", _native.sample_neighbors_device, self.ctx, self.inc,
+                                   nodes, edges, self.k, self.seed, nbr, first)
+        first += int(nodes.shape[0])
+        yield nodes, edges, nbr_n, nbr_e
+
+
+def _host(t):
+  return t.cpu().numpy()
+
+
+def _per_row(weights, count, base):
+  if weights is None:
+    return np.full(count, int(base), dtype=np.int32)
+  return np.asarray([int(w * base) for w in weights], dtype=np.int32)
+
+
+def BooleanSamplesDevice(incidence, num_neighbors, num_samples, neg_samples=0, node_weights=None,
+                         edge_weights=None, seed=0, chunk_rows=0, stream=False):
+  """BooleanSamplesCsr drawn on the GPU from seeded Philox streams instead of numpy's global
+  MT19937 (which is neither read nor advanced).  Same distribution of every record as the
+  reference's FOBE sampler, same blocks in the same order (node-node, edge-edge, node-edge rows,
+  edge-node rows; with negatives their negative blocks, the edge-edge one twice as in the
+  reference), same columns; not the reference's stream.  The result depends only on the graph,
+  the counts and `seed`, not on `chunk_rows`.  With ``stream=True`` returns an iterator of
+  SampleColumns chunks of about `chunk_rows` rows; otherwise one SampleColumns."""
+  assert num_neighbors >= 0
+  assert num_samples >= 0
+  assert neg_samples >= 0
+  g = incidence if isinstance(incidence, _Graph) else _Graph.from_csr(incidence)
+  node_s = _per_row(node_weights, g.num_nodes, num_samples)
+  edge_s = _per_row(edge_weights, g.num_edges, num_samples)
+  assert node_s.min(initial=0) >= 0 and edge_s.min(initial=0) >= 0
+  k = num_neighbors
+  ones = lambda m: np.broadcast_to(np.float32(1.0), (m,))
+
+  def chunks():
+    ctx = _native.default_context()
+    inc = g.incidence(ctx)
+    s = _DeviceSampler(g, ctx, inc, k, seed, chunk_rows)
+    try:
+      blocks = [(0, node_s, _native.PHASE_NN, "left_node", "right_node", "nn_prob", False),
+                (1, edge_s, _native.PHASE_EE, "left_edge", "right_edge", "ee_prob", False)]
+      for side, samples, phase, left, right, prob, neg in blocks:
+        for r, c in s.pairs(side, 2, samples, phase, negative=neg):
+          cols = {left: _host(r), right: _host(c), prob: ones(int(r.shape[0]))}
+          yield SampleColumns.build(k, int(r.shape[0]), **cols)
+      phases = (_native.PHASE_NE, _native.PHASE_EN, _native.PHASE_NEIGHBORS)
+      for nodes, edges, nbr_n, nbr_e in s.node_edge(node_s, edge_s, 1, phases):
+        m = int(nodes.shape[0])
+        yield SampleColumns.build(k, m, left_node=_host(nodes), right_edge=_host(edges),
+                                  neigh_node=_host(nbr_n), neigh_edge=_host(nbr_e), ne_prob=ones(m))
+      if neg_samples > 0:
+        neg_n = _per_row(node_weights, g.num_nodes, neg_samples)
+        neg_e = _per_row(edge_weights, g.num_edges, neg_samples)
+        for side, samples, phase, left, right in (
+            (0, neg_n, _native.PHASE_NEG_NN, "left_node", "right_node"),
+            (1, neg_e, _native.PHASE_NEG_EE, "left_edge", "right_edge"),
+            (1, neg_e, _native.PHASE_NEG_EE_AGAIN, "left_edge", "right_edge")):   # sic, :215-221
+          for r, c in s.pairs(side, 2, samples, phase, negative=True):
+            yield SampleColumns.build(k, int(r.shape[0]), **{left: _host(r), right: _host(c)})
+        phases = (_native.PHASE_NEG_NE, _native.PHASE_NEG_EN, _native.PHASE_NEG_NEIGHBORS)
+        for nodes, edges, nbr_n, nbr_e in s.node_edge(neg_n, neg_e, 1, phases, negative=True):
+          yield SampleColumns.build(k, int(nodes.shape[0]), left_node=_host(nodes),
+                                    right_edge=_host(edges), neigh_node=_host(nbr_n),
+                                    neigh_edge=_host(nbr_e))
+    finally:
+      inc.close()
+
+  if stream:
+    return chunks()
+  return SampleColumns.concatenate(list(chunks()))
+
+
+################################################################################
 # WeightedJaccard Samples - helper and sampler                                 #
 ################################################################################
 
@@ -664,6 +780,64 @@ def _hobe_samples(g, xn, xe, k, num_samples, timings=None):
   if timings is not None:
     timings.update(spent)
   return SampleColumns.concatenate(parts)
+
+
+def AlgebraicDistanceSamplesDevice(incidence, xn, xe, num_neighbors, num_samples, seed=0,
+                                   chunk_rows=0, stream=False, timings=None):
+  """AlgebraicDistanceSamplesCsr with the pairs and neighbour arrays drawn on the GPU from seeded
+  Philox streams (see BooleanSamplesDevice) instead of numpy's global MT19937, which is neither
+  read nor advanced.  The pairs stay on the device and go straight into the probability kernels.
+  Same blocks, columns and probabilities as the reference's HOBE sampler; not its stream.  With
+  ``stream=True`` returns an iterator of SampleColumns chunks of about `chunk_rows` rows.
+  `timings` (a dict) receives the seconds spent drawing pairs ("pairs") and neighbour arrays
+  ("neighbours") and computing the incidence weights and probabilities ("probabilities"); it is
+  filled when the result is complete."""
+  import time
+  assert num_neighbors >= 0
+  assert num_samples >= 0
+  g = incidence if isinstance(incidence, _Graph) else _Graph.from_csr(incidence)
+  xn = np.ascontiguousarray(xn, dtype=np.float32)
+  xe = np.ascontiguousarray(xe, dtype=np.float32)
+  assert xn.shape[0] == g.num_nodes and xe.shape[0] == g.num_edges and xn.shape[1] == xe.shape[1]
+  k = num_neighbors
+  per_node = _per_row(None, g.num_nodes, num_samples)
+  per_edge = _per_row(None, g.num_edges, num_samples)
+
+  def chunks():
+    spent = {"probabilities": 0.0}
+
+    def prob(fn, *args):
+      t = time.perf_counter()
+      out = _host(fn(*args))
+      spent["probabilities"] += time.perf_counter() - t
+      return out
+
+    t = time.perf_counter()
+    weights = _HobeWeights(g, xn, xe)
+    spent["probabilities"] += time.perf_counter() - t
+    ctx, inc = weights.ctx, weights.inc
+    s = _DeviceSampler(g, ctx, inc, k, seed, chunk_rows)
+    try:
+      for side, samples, phase, left, right, field, w in (
+          (0, per_node, _native.PHASE_NN, "left_node", "right_node", "nn_prob", weights.w_n2e),
+          (1, per_edge, _native.PHASE_EE, "left_edge", "right_edge", "ee_prob", weights.w_e2n)):
+        for r, c in s.pairs(side, 2, samples, phase):
+          p = prob(_native.same_type_prob, ctx, inc, side, w, r, c)
+          yield SampleColumns.build(k, len(p), **{left: _host(r), right: _host(c), field: p})
+      phases = (_native.PHASE_NE, _native.PHASE_EN, _native.PHASE_NEIGHBORS)
+      for nodes, edges, nbr_n, nbr_e in s.node_edge(per_node, per_edge, 3, phases):
+        p = prob(_native.diff_type_prob, ctx, inc, weights.w_e2n, nodes, edges)
+        yield SampleColumns.build(k, len(p), left_node=_host(nodes), right_edge=_host(edges),
+                                  neigh_node=_host(nbr_n), neigh_edge=_host(nbr_e), ne_prob=p)
+    finally:
+      weights.close()
+    if timings is not None:
+      timings.update(s.spent)
+      timings.update(spent)
+
+  if stream:
+    return chunks()
+  return SampleColumns.concatenate(list(chunks()))
 
 
 def SameTypeDistanceSample(indices, idx2target=None, source_half_emb=None, target_half_emb=None,

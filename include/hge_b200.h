@@ -322,6 +322,37 @@ int hge_sample_neighbors(const int64_t* n2e_ptr, const int32_t* n2e_idx, const i
                          int64_t num_samples, int k, uint32_t* state625, int32_t* out_nbr_edges,
                          int32_t* out_nbr_nodes);
 
+/* ---- device sampling from a seeded counter-based generator -------------------------------
+ * The distribution of _sample_adj_matrix / _sample_neighbors (hg2v_sample.py:49-86), drawn on the
+ * GPU from Philox4x32-10 word streams instead of numpy's MT19937 (csrc/hge_philox.cuh documents the
+ * key / counter layout and the phase constants; oracle/device_sampler_ref.py restates it).  Every
+ * row (pairs) and every record (neighbours) owns its stream, so results do not depend on how a
+ * caller splits rows or records into calls, nor on the workspace budget.  The bit-exact replay
+ * of the reference's stream is hge_sample_adj_rows above.  `mem` applies to every array argument.
+ *
+ * Pairs: rows [row0, row1) of P = M1 (factors 1), M1 * M2 (2) or (M1 * M2) * M3 (3), with
+ * M1 = M3 = the node -> edge CSR and M2 = the edge -> node CSR for side 0 (node rows), the other
+ * way round for side 1 (edge rows).  Positive (negative == 0): row r emits min(k_r, n_r) distinct
+ * columns, uniform among the subsets of that size of its n_r distinct candidates, ascending; rows
+ * without candidates emit nothing.  Negative: row r emits k_r columns uniform on [0, columns of
+ * P), with replacement, in draw order.  Rows come out in ascending order as (out_row, out_col);
+ * samples_per_row holds k_r for the row1 - row0 rows; capacity >= sum(k_r) always suffices.
+ * Candidate rows are built in batches of rows whose expansion fits workspace_mb megabytes
+ * (0 = 2048); a row that needs more than the device holds is HGE_ERR_NOMEM.  A negative k_r is
+ * HGE_ERR_INVALID.  Needs an incidence made by hge_incidence_create (not a shard). */
+int hge_sample_pairs_device(hge_ctx* ctx, hge_incidence* inc, int side, int factors, int32_t row0,
+                            int32_t row1, const int32_t* samples_per_row, int negative, uint64_t seed,
+                            uint32_t phase, int64_t workspace_mb, int32_t* out_row, int32_t* out_col,
+                            int64_t capacity, int64_t* out_count, int mem);
+
+/* Neighbour arrays of `count` (node, edge) records, record i being number first_index + i of its
+ * block: k draws with replacement from the node's edges, then k from the edge's nodes.  Outputs
+ * are [count, k].  A draw from an empty list is HGE_ERR_INVALID ("cannot be empty"). */
+int hge_sample_neighbors_device(hge_ctx* ctx, hge_incidence* inc, const int32_t* nodes,
+                                const int32_t* edges, int64_t count, int k, uint64_t seed,
+                                uint32_t phase, int64_t first_index, int32_t* out_nbr_edges,
+                                int32_t* out_nbr_nodes, int mem);
+
 /* ---- hypergraph2vec training (hg2v_model.py:51-203, fit loop embedding.py:269-305) ---------
  * The consumer of the sample columns.  Two embedding tables [rows, dim] fp32 whose row 0 is the
  * trained padding row (Embedding(input_dim = max id + 2)); outputs

@@ -12,11 +12,12 @@ from .hypergraph_util import (AddNodeToEdge, CompressRange, IsEmpty, Relabel, To
 from .algebraic_distance import EmbedAlgebraicDistance
 from .hg2v_sample import (AlgebraicDistanceSamples, AlgebraicDistanceSamplesCsr,
                           AlgebraicDistanceSamplesDevice, BooleanSamples, BooleanSamplesCsr,
-                          BooleanSamplesDevice,
+                          BooleanSamplesDevice, DeviceSampleColumns,
                           SampleColumns, SamplesToModelInput, SimilarityRecord,
                           SparseWeightedJaccard, WeightedJaccardSamples)
 from .hg2v_model import BooleanModel, KerasModelToEmbedding, UnweightedFloatModel
-from .embedding import (EMBEDDING_OPTIONS, EmbedHg2vAdjJaccard, EmbedHg2vAlgDist, EmbedHg2vBoolean,
+from .embedding import (EMBEDDING_OPTIONS, EmbedHg2vAdjJaccard, EmbedHg2vAlgDist,
+                        EmbedHg2vAlgDistDevice, EmbedHg2vBoolean, EmbedHg2vBooleanDevice,
                         EmbedHg2vNeighborhoodWeightedJaccard)
 from .hg2v_weighting import (AlphaScaleValues, ComputeSpans, DictToSparseRow, OneMinusValues,
                              UniformWeight, WeightByAlgebraicSpan, WeightByDistance,
@@ -29,11 +30,11 @@ __all__ = [
     "EmbedAlgebraicDistance",
     "AlgebraicDistanceSamples", "AlgebraicDistanceSamplesCsr", "AlgebraicDistanceSamplesDevice",
     "BooleanSamples", "BooleanSamplesCsr", "BooleanSamplesDevice",
-    "SampleColumns",
+    "DeviceSampleColumns", "SampleColumns",
     "SamplesToModelInput", "SimilarityRecord", "SparseWeightedJaccard", "WeightedJaccardSamples",
     "BooleanModel", "UnweightedFloatModel", "KerasModelToEmbedding", "EMBEDDING_OPTIONS",
     "EmbedHg2vBoolean", "EmbedHg2vAdjJaccard", "EmbedHg2vNeighborhoodWeightedJaccard",
-    "EmbedHg2vAlgDist",
+    "EmbedHg2vAlgDist", "EmbedHg2vBooleanDevice", "EmbedHg2vAlgDistDevice",
     "AlphaScaleValues", "ComputeSpans", "DictToSparseRow", "OneMinusValues", "UniformWeight",
     "WeightByAlgebraicSpan", "WeightByDistance", "WeightByDistanceCluster", "WeightByNeighborhood",
     "WeightBySameTypeDistance", "ZeroOneScaleValues",

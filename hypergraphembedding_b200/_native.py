@@ -123,6 +123,14 @@ SIGNATURES = {
                                           ctypes.POINTER(ctypes.c_double)]),
     "hge_hg2v_get_weights": (ctypes.c_int, [c_vp, c_vp, c_vp, ctypes.c_int]),
     "hge_hg2v_last_clusters": (ctypes.c_int, [c_vp]),
+    "hge_hg2v_create_seeded": (ctypes.c_int, [c_vp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int, ctypes.c_int,
+                                              ctypes.c_int, ctypes.c_int, ctypes.c_uint64, ctypes.POINTER(c_vp)]),
+    "hge_hg2v_reserve_samples": (ctypes.c_int, [c_vp, ctypes.c_int64]),
+    "hge_hg2v_append_samples": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, ctypes.c_int,
+                                               ctypes.c_float, ctypes.c_int64]),
+    "hge_hg2v_get_samples": (ctypes.c_int, [c_vp, c_vp, c_vp, ctypes.c_int]),
+    "hge_shuffle_order": (ctypes.c_int, [c_vp, ctypes.c_uint64, ctypes.c_uint32, ctypes.c_int64, c_vp,
+                                         ctypes.c_int]),
     "hge_mt19937_random_raw": (ctypes.c_int, [c_vp, ctypes.c_int64, c_vp]),
     "hge_mt19937_interval": (ctypes.c_int, [c_vp, ctypes.c_uint32, ctypes.c_int64, c_vp]),
     "hge_spgemm_rows": (ctypes.c_int, [ctypes.c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
@@ -727,6 +735,7 @@ def sample_neighbors(n2e, e2n, nodes, edges, k, state):
 PHASE_NN, PHASE_EE, PHASE_NE, PHASE_EN, PHASE_NEIGHBORS = 1, 2, 3, 4, 5
 PHASE_NEG_NN, PHASE_NEG_EE, PHASE_NEG_EE_AGAIN, PHASE_NEG_NE, PHASE_NEG_EN = 6, 7, 8, 9, 10
 PHASE_NEG_NEIGHBORS = 11
+PHASE_SHUFFLE, PHASE_INIT_NODES, PHASE_INIT_EDGES = 12, 13, 14
 
 
 def sample_pairs_device(ctx, inc, side, factors, row0, samples, seed, phase, negative=False,
@@ -762,6 +771,18 @@ def sample_neighbors_device(ctx, inc, nodes, edges, k, seed, phase, first_index)
     raise ValueError("'a' cannot be empty unless no samples are taken")
   check(rc, "hge_sample_neighbors_device")
   return nbr_e, nbr_n
+
+
+def shuffle_order(ctx, seed, epoch, n, out=None):
+  """hge_shuffle_order: the seeded permutation of [0, n) of one epoch as an int32 CUDA tensor
+  (written into `out` when given)."""
+  import torch
+  if out is None:
+    out = torch.empty(max(int(n), 1), dtype=torch.int32, device=torch.device("cuda", ctx.device))[:int(n)]
+  assert out.dtype == torch.int32 and out.is_cuda and int(out.shape[0]) == int(n)
+  check(ctx.lib.hge_shuffle_order(ctx.handle, int(seed) & 0xFFFFFFFFFFFFFFFF, int(epoch), int(n), ptr(out),
+                                  MEM_DEVICE), "hge_shuffle_order")
+  return out
 
 
 class PeerArena(object):

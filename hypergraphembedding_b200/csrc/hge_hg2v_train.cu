@@ -25,12 +25,21 @@
 // B200), a sample per warp again, and the two per-batch barriers become cluster barrier ->
 // one arrival per cluster on a global counter -> cluster barrier.  The one-cluster launch keeps
 // the pure hardware barrier.
+//
+// The sample buffer can also be filled on the device (hge_hg2v_reserve_samples, then
+// hge_hg2v_append_samples per block of sampler output: k_hg2v_append packs and range-checks one
+// record per thread), the epoch order drawn on the device (hge_shuffle_order: Philox keys, stable
+// radix sort) and the tables initialised on the device (hge_hg2v_create_seeded).
 #include <cooperative_groups.h>
+#include <cub/device/device_radix_sort.cuh>
 
 #include <algorithm>
+#include <cfloat>
 #include <new>
 
 #include "hge_common.cuh"
+#include "hge_expand.cuh"
+#include "hge_philox.cuh"
 #include "hge_staged.cuh"
 
 namespace cg = cooperative_groups;
@@ -50,6 +59,9 @@ struct hge_hg2v_model {
   unsigned int* grid_bar = nullptr;   // arrival counter of the inter-cluster batch barrier
   int max_clusters = 0;               // co-resident clusters of k_hg2v_epoch (0: not asked yet)
   int last_clusters = 0;              // clusters of the last epoch's launch
+  bool reserved = false;              // feat / target come from hge_hg2v_reserve_samples ...
+  int64_t filled = 0;                 // ... and hold this many appended records
+  unsigned long long* bad = nullptr;  // first bad (record << 5 | column) of the last append
 };
 
 namespace {
@@ -379,6 +391,162 @@ int upload(hge_ctx* ctx, T** dst, const T* src, size_t count, int mem) {
   return HGE_OK;
 }
 
+// ---- the sample buffer filled on the device ---------------------------------------------------
+
+struct AppendArgs {
+  const int32_t *ln, *le, *rn, *re;    // [count] each, NULL = padding index 0
+  const int32_t *nbr_n, *nbr_e;        // [count, k] row-major, NULL = padding index 0
+  const float* prob;                   // [count], NULL = prob_value
+  int prob_slot;                       // target slot of prob, -1 = none
+  float prob_value;
+  int64_t count, at, M;
+  int k;
+  int32_t node_rows, edge_rows;
+  int32_t* feat;
+  float* target;
+  unsigned long long* bad;
+};
+
+// np.nan_to_num(x, nan=0.0) in fp32
+__device__ __forceinline__ float nan_to_num(float x) {
+  if (isnan(x)) return 0.0f;
+  if (isinf(x)) return x > 0.0f ? FLT_MAX : -FLT_MAX;
+  return x;
+}
+
+// _columns_to_model_input(..., weighted=False) for one block of records at record `at` of the
+// buffer, one thread per record.  Every index written is checked against its table; the first
+// bad one (lowest record, then column) is kept in *bad.
+__global__ void k_hg2v_append(const AppendArgs a) {
+  const int cols = 4 + 2 * a.k;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < a.count;
+       i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t o = a.at + i;
+    unsigned long long bad = ~0ull;
+    for (int c = 0; c < cols; ++c) {
+      const int32_t* src = c == 0 ? a.ln : c == 1 ? a.le : c == 2 ? a.rn : c == 3 ? a.re
+                           : c < 4 + a.k ? a.nbr_n : a.nbr_e;
+      const int64_t j = c < 4 ? i : i * a.k + (c < 4 + a.k ? c - 4 : c - 4 - a.k);
+      const int64_t v = src ? (int64_t)src[j] + 1 : 0;
+      const bool node = c == 0 || c == 2 || (c >= 4 && c < 4 + a.k);
+      if (v < 0 || v >= (node ? a.node_rows : a.edge_rows))
+        bad = min(bad, ((unsigned long long)i << 5) | (unsigned long long)c);
+      a.feat[(size_t)c * a.M + o] = (int32_t)v;
+    }
+    if (bad != ~0ull) atomicMin(a.bad, bad);
+    const float p = nan_to_num(a.prob ? a.prob[i] : a.prob_value);
+    for (int s = 0; s < 3; ++s) a.target[(size_t)s * a.M + o] = s == a.prob_slot ? p : 0.0f;
+  }
+}
+
+// ---- seeded epoch order and tables ------------------------------------------------------------
+
+// key of item i in epoch e: words 2e, 2e + 1 of its HGE_PHASE_SHUFFLE stream (high, low)
+__global__ void k_shuffle_keys(int64_t n, uint64_t seed, uint32_t epoch, uint64_t* __restrict__ keys,
+                               int32_t* __restrict__ idx) {
+  const int w = (int)(epoch & 1u) * 2;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n;
+       i += (int64_t)gridDim.x * blockDim.x) {
+    const HgeWords4 r = hge_philox4x32_10(epoch >> 1, (uint32_t)i, (uint32_t)((uint64_t)i >> 32),
+                                          HGE_PHASE_SHUFFLE, (uint32_t)seed, (uint32_t)(seed >> 32));
+    keys[i] = ((uint64_t)r.v[w] << 32) | r.v[w + 1];
+    idx[i] = (int32_t)i;
+  }
+}
+
+// element (r, c) = -0.05 + 0.1 * ((word c of the stream of row r) >> 8) * 2^-24, each operation
+// rounded on its own (no contraction), so that the float32 numpy restatement gives the same bits
+__global__ void k_init_table(int64_t rows, int dim, uint64_t seed, uint32_t phase, float* __restrict__ t) {
+  const int blocks = (dim + 3) / 4;
+  for (int64_t g = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; g < rows * blocks;
+       g += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = g / blocks;
+    const int b = (int)(g - r * blocks);
+    const HgeWords4 w = hge_philox4x32_10((uint32_t)b, (uint32_t)r, (uint32_t)((uint64_t)r >> 32), phase,
+                                          (uint32_t)seed, (uint32_t)(seed >> 32));
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int c = 4 * b + j;
+      if (c < dim) {
+        const float u = __fmul_rn(__uint2float_rn(w.v[j] >> 8), 0x1p-24f);
+        t[(size_t)r * dim + c] = __fadd_rn(-0.05f, __fmul_rn(0.1f, u));
+      }
+    }
+  }
+}
+
+// hge_hg2v_create and hge_hg2v_create_seeded: tables uploaded from node_init / edge_init, or
+// (seed != NULL) drawn on the device
+int create_model(hge_ctx* ctx, int32_t node_rows, int32_t edge_rows, int dim, int num_neighbors,
+                 int activation, int loss, const float* node_init, const float* edge_init, int mem,
+                 const uint64_t* seed, hge_hg2v_model** out, const char* what) {
+  HGE_REQUIRE(node_rows >= 1 && edge_rows >= 1, "%s: empty embedding table", what);
+  HGE_REQUIRE(dim >= 1 && dim <= kMaxDim, "%s: dimension %d not in [1, %d]", what, dim, kMaxDim);
+  HGE_REQUIRE(num_neighbors >= 0 && 4 + 2 * num_neighbors <= 32,
+              "%s: num_neighbors %d not in [0, 14]", what, num_neighbors);
+  HGE_REQUIRE((activation == 0 || activation == 1) && (loss == 0 || loss == 1),
+              "%s: activation / loss must be 0 or 1", what);
+  HGE_REQUIRE(mem == HGE_MEM_HOST || mem == HGE_MEM_DEVICE, "%s: bad mem %d", what, mem);
+  HGE_CUDA(cudaSetDevice(ctx->device));
+  hge_hg2v_model* m = new (std::nothrow) hge_hg2v_model();
+  if (!m) return HGE_ERR_NOMEM;
+  m->ctx = ctx;
+  m->node_rows = node_rows;
+  m->edge_rows = edge_rows;
+  m->dim = dim;
+  m->k = num_neighbors;
+  m->activation = activation;
+  m->loss = loss;
+  const size_t nn = (size_t)node_rows * dim, ne = (size_t)edge_rows * dim;
+  int rc = HGE_OK;
+  if (seed) {
+    rc = hge_dev_alloc(ctx, &m->N, nn);
+    if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &m->E, ne);
+    if (rc == HGE_OK) {
+      const int blocks = (dim + 3) / 4;
+      k_init_table<<<grid_for(ctx, (int64_t)node_rows * blocks), kExpandBlock, 0, ctx->stream>>>(
+          node_rows, dim, *seed, HGE_PHASE_INIT_NODES, m->N);
+      k_init_table<<<grid_for(ctx, (int64_t)edge_rows * blocks), kExpandBlock, 0, ctx->stream>>>(
+          edge_rows, dim, *seed, HGE_PHASE_INIT_EDGES, m->E);
+      ctx->launches += 2;
+      const cudaError_t e = cudaGetLastError();
+      if (e != cudaSuccess) {
+        hge_set_error("%s: init launch failed: %s", what, cudaGetErrorString(e));
+        rc = HGE_ERR_CUDA;
+      }
+    }
+  } else {
+    rc = upload(ctx, &m->N, node_init, nn, mem);
+    if (rc == HGE_OK) rc = upload(ctx, &m->E, edge_init, ne, mem);
+  }
+  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &m->accN, nn);
+  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &m->accE, ne);
+  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &m->gN, nn);
+  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &m->gE, ne);
+  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &m->claimN, (size_t)node_rows);
+  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &m->claimE, (size_t)edge_rows);
+  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &m->d_loss, 1);
+  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &m->grid_bar, 1);
+  if (rc == HGE_OK) {
+    cudaError_t e = cudaMemsetAsync(m->accN, 0, nn * 4, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(m->accE, 0, ne * 4, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(m->gN, 0, nn * 4, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(m->gE, 0, ne * 4, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(m->claimN, 0xff, (size_t)node_rows * 4, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(m->claimE, 0xff, (size_t)edge_rows * 4, ctx->stream);
+    if (e != cudaSuccess) {
+      hge_set_error("%s: memset failed: %s", what, cudaGetErrorString(e));
+      rc = HGE_ERR_CUDA;
+    }
+  }
+  if (rc != HGE_OK) {
+    hge_hg2v_destroy(m);
+    return rc;
+  }
+  *out = m;
+  return HGE_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -400,6 +568,7 @@ int hge_hg2v_destroy(hge_hg2v_model* m) {
   hge_dev_free(ctx, m->order);
   hge_dev_free(ctx, m->d_loss);
   hge_dev_free(ctx, m->grid_bar);
+  hge_dev_free(ctx, m->bad);
   delete m;
   return HGE_OK;
 }
@@ -409,52 +578,16 @@ int hge_hg2v_create(hge_ctx* ctx, int32_t node_rows, int32_t edge_rows, int dim,
                     int mem, hge_hg2v_model** out) {
   HGE_REQUIRE(ctx && out && node_init && edge_init, "hge_hg2v_create: NULL argument");
   *out = nullptr;
-  HGE_REQUIRE(node_rows >= 1 && edge_rows >= 1, "hge_hg2v_create: empty embedding table");
-  HGE_REQUIRE(dim >= 1 && dim <= kMaxDim, "hge_hg2v_create: dimension %d not in [1, %d]", dim, kMaxDim);
-  HGE_REQUIRE(num_neighbors >= 0 && 4 + 2 * num_neighbors <= 32,
-              "hge_hg2v_create: num_neighbors %d not in [0, 14]", num_neighbors);
-  HGE_REQUIRE((activation == 0 || activation == 1) && (loss == 0 || loss == 1),
-              "hge_hg2v_create: activation / loss must be 0 or 1");
-  HGE_REQUIRE(mem == HGE_MEM_HOST || mem == HGE_MEM_DEVICE, "hge_hg2v_create: bad mem %d", mem);
-  HGE_CUDA(cudaSetDevice(ctx->device));
-  hge_hg2v_model* m = new (std::nothrow) hge_hg2v_model();
-  if (!m) return HGE_ERR_NOMEM;
-  m->ctx = ctx;
-  m->node_rows = node_rows;
-  m->edge_rows = edge_rows;
-  m->dim = dim;
-  m->k = num_neighbors;
-  m->activation = activation;
-  m->loss = loss;
-  const size_t nn = (size_t)node_rows * dim, ne = (size_t)edge_rows * dim;
-  int rc = upload(ctx, &m->N, node_init, nn, mem);
-  if (rc == HGE_OK) rc = upload(ctx, &m->E, edge_init, ne, mem);
-  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &m->accN, nn);
-  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &m->accE, ne);
-  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &m->gN, nn);
-  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &m->gE, ne);
-  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &m->claimN, (size_t)node_rows);
-  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &m->claimE, (size_t)edge_rows);
-  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &m->d_loss, 1);
-  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &m->grid_bar, 1);
-  if (rc == HGE_OK) {
-    cudaError_t e = cudaMemsetAsync(m->accN, 0, nn * 4, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(m->accE, 0, ne * 4, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(m->gN, 0, nn * 4, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(m->gE, 0, ne * 4, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(m->claimN, 0xff, (size_t)node_rows * 4, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(m->claimE, 0xff, (size_t)edge_rows * 4, ctx->stream);
-    if (e != cudaSuccess) {
-      hge_set_error("hge_hg2v_create: memset failed: %s", cudaGetErrorString(e));
-      rc = HGE_ERR_CUDA;
-    }
-  }
-  if (rc != HGE_OK) {
-    hge_hg2v_destroy(m);
-    return rc;
-  }
-  *out = m;
-  return HGE_OK;
+  return create_model(ctx, node_rows, edge_rows, dim, num_neighbors, activation, loss, node_init, edge_init,
+                      mem, nullptr, out, "hge_hg2v_create");
+}
+
+int hge_hg2v_create_seeded(hge_ctx* ctx, int32_t node_rows, int32_t edge_rows, int dim, int num_neighbors,
+                           int activation, int loss, uint64_t seed, hge_hg2v_model** out) {
+  HGE_REQUIRE(ctx && out, "hge_hg2v_create_seeded: NULL argument");
+  *out = nullptr;
+  return create_model(ctx, node_rows, edge_rows, dim, num_neighbors, activation, loss, nullptr, nullptr,
+                      HGE_MEM_DEVICE, &seed, out, "hge_hg2v_create_seeded");
 }
 
 int hge_hg2v_set_samples(hge_hg2v_model* m, const int32_t* features, const float* targets,
@@ -467,6 +600,7 @@ int hge_hg2v_set_samples(hge_hg2v_model* m, const int32_t* features, const float
   hge_dev_free(ctx, m->feat);
   hge_dev_free(ctx, m->target);
   hge_dev_free(ctx, m->order);
+  m->reserved = false;
   m->M = num_samples;
   const size_t cols = 4 + 2 * (size_t)m->k;
   HGE_TRY(upload(ctx, &m->feat, features, cols * (size_t)num_samples, mem));
@@ -492,6 +626,9 @@ int hge_hg2v_fit_epoch(hge_hg2v_model* m, const int32_t* order, int batch_size, 
   HGE_REQUIRE(m && epoch_loss && batch_size >= 1, "hge_hg2v_fit_epoch: bad argument");
   HGE_REQUIRE(m->M > 0 && order, "hge_hg2v_fit_epoch: no samples (hge_hg2v_set_samples) or no order");
   HGE_REQUIRE(mem == HGE_MEM_HOST || mem == HGE_MEM_DEVICE, "hge_hg2v_fit_epoch: bad mem %d", mem);
+  HGE_REQUIRE(!m->reserved || m->filled == m->M,
+              "hge_hg2v_fit_epoch: %lld of the %lld reserved samples are filled (hge_hg2v_append_samples)",
+              (long long)m->filled, (long long)m->M);
   hge_ctx* ctx = m->ctx;
   HGE_CUDA(cudaSetDevice(ctx->device));
   if (mem == HGE_MEM_HOST)
@@ -580,6 +717,127 @@ int hge_hg2v_get_weights(hge_hg2v_model* m, float* node, float* edge, int mem) {
   HGE_CUDA(cudaMemcpyAsync(edge, m->E, (size_t)m->edge_rows * m->dim * 4, kind, ctx->stream));
   HGE_CUDA(cudaStreamSynchronize(ctx->stream));
   return HGE_OK;
+}
+
+int hge_hg2v_reserve_samples(hge_hg2v_model* m, int64_t num_samples) {
+  HGE_REQUIRE(m, "hge_hg2v_reserve_samples: NULL model");
+  HGE_REQUIRE(num_samples >= 0 && num_samples < ((int64_t)1 << 31),
+              "hge_hg2v_reserve_samples: %lld samples not in [0, 2^31) (the order is int32)",
+              (long long)num_samples);
+  hge_ctx* ctx = m->ctx;
+  HGE_CUDA(cudaSetDevice(ctx->device));
+  hge_dev_free(ctx, m->feat);
+  hge_dev_free(ctx, m->target);
+  hge_dev_free(ctx, m->order);
+  m->M = 0;
+  m->reserved = false;
+  m->filled = 0;
+  const size_t cols = 4 + 2 * (size_t)m->k;
+  HGE_TRY(hge_dev_alloc(ctx, &m->feat, cols * (size_t)num_samples));
+  HGE_TRY(hge_dev_alloc(ctx, &m->target, 3 * (size_t)num_samples));
+  HGE_TRY(hge_dev_alloc(ctx, &m->order, (size_t)num_samples));
+  if (!m->bad) HGE_TRY(hge_dev_alloc(ctx, &m->bad, 1));
+  m->M = num_samples;
+  m->reserved = true;
+  return HGE_OK;
+}
+
+int hge_hg2v_append_samples(hge_hg2v_model* m, const int32_t* left_node, const int32_t* left_edge,
+                            const int32_t* right_node, const int32_t* right_edge, const int32_t* nbr_nodes,
+                            const int32_t* nbr_edges, const float* prob, int prob_slot, float prob_value,
+                            int64_t count) {
+  HGE_REQUIRE(m, "hge_hg2v_append_samples: NULL model");
+  HGE_REQUIRE(m->reserved, "hge_hg2v_append_samples: no buffer (hge_hg2v_reserve_samples)");
+  HGE_REQUIRE(count >= 0 && count <= m->M - m->filled,
+              "hge_hg2v_append_samples: %lld records do not fit: %lld of %lld reserved are filled",
+              (long long)count, (long long)m->filled, (long long)m->M);
+  HGE_REQUIRE(prob_slot >= -1 && prob_slot <= 2, "hge_hg2v_append_samples: prob_slot %d not in [-1, 2]",
+              prob_slot);
+  if (count == 0) return HGE_OK;
+  hge_ctx* ctx = m->ctx;
+  HGE_CUDA(cudaSetDevice(ctx->device));
+  AppendArgs a;
+  a.ln = left_node; a.le = left_edge; a.rn = right_node; a.re = right_edge;
+  a.nbr_n = nbr_nodes; a.nbr_e = nbr_edges;
+  a.prob = prob; a.prob_slot = prob_slot; a.prob_value = prob_value;
+  a.count = count; a.at = m->filled; a.M = m->M; a.k = m->k;
+  a.node_rows = m->node_rows; a.edge_rows = m->edge_rows;
+  a.feat = m->feat; a.target = m->target; a.bad = m->bad;
+  HGE_CUDA(cudaMemsetAsync(m->bad, 0xff, sizeof(unsigned long long), ctx->stream));
+  k_hg2v_append<<<grid_for(ctx, count), kExpandBlock, 0, ctx->stream>>>(a);
+  HGE_CHECK_LAUNCH(ctx);
+  unsigned long long bad = 0;
+  HGE_TRY(read_back(ctx, m->bad, &bad, 1));
+  if (bad != ~0ull) {
+    const int c = (int)(bad & 31u);
+    const bool node = c == 0 || c == 2 || (c >= 4 && c < 4 + m->k);
+    hge_set_error("hge_hg2v_append_samples: feature column %d, record %lld of the block: index outside its "
+                  "table of %d rows", c, (long long)(bad >> 5), node ? m->node_rows : m->edge_rows);
+    return HGE_ERR_INVALID;
+  }
+  m->filled += count;
+  return HGE_OK;
+}
+
+int hge_hg2v_get_samples(hge_hg2v_model* m, int32_t* features, float* targets, int mem) {
+  HGE_REQUIRE(m && (m->M == 0 || (features && targets)), "hge_hg2v_get_samples: NULL argument");
+  HGE_REQUIRE(mem == HGE_MEM_HOST || mem == HGE_MEM_DEVICE, "hge_hg2v_get_samples: bad mem %d", mem);
+  if (m->M == 0) return HGE_OK;
+  hge_ctx* ctx = m->ctx;
+  HGE_CUDA(cudaSetDevice(ctx->device));
+  const cudaMemcpyKind kind = mem == HGE_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+  HGE_CUDA(cudaMemcpyAsync(features, m->feat, (4 + 2 * (size_t)m->k) * (size_t)m->M * 4, kind, ctx->stream));
+  HGE_CUDA(cudaMemcpyAsync(targets, m->target, 3 * (size_t)m->M * 4, kind, ctx->stream));
+  HGE_CUDA(cudaStreamSynchronize(ctx->stream));
+  return HGE_OK;
+}
+
+int hge_shuffle_order(hge_ctx* ctx, uint64_t seed, uint32_t epoch, int64_t n, int32_t* order, int mem) {
+  HGE_REQUIRE(ctx, "hge_shuffle_order: NULL context");
+  HGE_REQUIRE(n >= 0 && n < ((int64_t)1 << 31), "hge_shuffle_order: n = %lld not in [0, 2^31)", (long long)n);
+  HGE_REQUIRE(n == 0 || order, "hge_shuffle_order: NULL order");
+  HGE_REQUIRE(mem == HGE_MEM_HOST || mem == HGE_MEM_DEVICE, "hge_shuffle_order: bad mem %d", mem);
+  if (n == 0) return HGE_OK;
+  HGE_CUDA(cudaSetDevice(ctx->device));
+  Staged<int32_t> out;
+  HGE_TRY(out.init(ctx, order, (size_t)n, mem, false, true));
+  uint64_t *k0 = nullptr, *k1 = nullptr;
+  int32_t* v1 = nullptr;
+  char* temp = nullptr;
+  int rc = hge_dev_alloc(ctx, &k0, (size_t)n);
+  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &k1, (size_t)n);
+  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &v1, (size_t)n);
+  cub::DoubleBuffer<uint64_t> keys(k0, k1);
+  cub::DoubleBuffer<int32_t> vals(out.dev, v1);
+  size_t bytes = 0;
+  if (rc == HGE_OK) {
+    k_shuffle_keys<<<grid_for(ctx, n), kExpandBlock, 0, ctx->stream>>>(n, seed, epoch, k0, out.dev);
+    ctx->launches++;
+    cudaError_t e = cudaGetLastError();
+    // LSD radix sort: stable, so equal keys keep ascending item order
+    if (e == cudaSuccess) e = cub::DeviceRadixSort::SortPairs(nullptr, bytes, keys, vals, n, 0, 64, ctx->stream);
+    if (e != cudaSuccess) {
+      hge_set_error("hge_shuffle_order: %s", cudaGetErrorString(e));
+      rc = HGE_ERR_CUDA;
+    }
+  }
+  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &temp, bytes);
+  if (rc == HGE_OK) {
+    cudaError_t e = cub::DeviceRadixSort::SortPairs(temp, bytes, keys, vals, n, 0, 64, ctx->stream);
+    ctx->launches++;
+    if (e == cudaSuccess && vals.Current() != out.dev)
+      e = cudaMemcpyAsync(out.dev, vals.Current(), (size_t)n * 4, cudaMemcpyDeviceToDevice, ctx->stream);
+    if (e != cudaSuccess) {
+      hge_set_error("hge_shuffle_order: %s", cudaGetErrorString(e));
+      rc = HGE_ERR_CUDA;
+    }
+  }
+  hge_dev_free(ctx, temp);
+  hge_dev_free(ctx, k0);
+  hge_dev_free(ctx, k1);
+  hge_dev_free(ctx, v1);
+  HGE_TRY(rc);
+  return out.finish();
 }
 
 }  // extern "C"

@@ -1,6 +1,7 @@
 // Philox4x32-10 (Salmon et al., "Parallel random numbers: as easy as 1, 2, 3", SC'11) and the
 // word-stream layout of the device sampler (csrc/hge_device_sampler.cu).  oracle/
-// device_sampler_ref.py restates everything in this file in numpy.
+// device_sampler_ref.py restates everything in this file in numpy; oracle/seeded_training_ref.py
+// restates the training phases (epoch order, initial tables).
 //
 // Layout.  Every item owns one stream of 32-bit words:
 //   key     = { (uint32)seed, (uint32)(seed >> 32) }
@@ -33,6 +34,12 @@ enum HgePhase : uint32_t {
   HGE_PHASE_NEG_NE = 9,
   HGE_PHASE_NEG_EN = 10,
   HGE_PHASE_NEG_NEIGHBORS = 11,
+  // hypergraph2vec training (csrc/hge_hg2v_train.cu): item = sample index, epoch e reads words
+  // 2e and 2e + 1 as its 64-bit sort key
+  HGE_PHASE_SHUFFLE = 12,
+  // initial embedding tables: item = row, word c is column c
+  HGE_PHASE_INIT_NODES = 13,
+  HGE_PHASE_INIT_EDGES = 14,
 };
 
 #ifdef __CUDACC__

@@ -9,12 +9,17 @@ ids with the reference's ``method_name``).  Sampling and training run in libhge_
 """
 import logging
 
+import numpy as np
+
+from . import _native
 from .algebraic_distance import EmbedAlgebraicDistance
-from .hg2v_model import (BooleanModel, EarlyStopping, KerasModelToEmbedding, UnweightedFloatModel)
-from .hg2v_sample import (AlgebraicDistanceSamples, BooleanSamples, PlotDistributions,
-                          SamplesToModelInput, WeightedJaccardSamples)
+from .hg2v_model import (BooleanModel, EarlyStopping, Hg2vModel, KerasModelToEmbedding,
+                         UnweightedFloatModel)
+from .hg2v_sample import (AlgebraicDistanceSamples, AlgebraicDistanceSamplesDevice, BooleanSamples,
+                          BooleanSamplesDevice, PlotDistributions, SamplesToModelInput,
+                          WeightedJaccardSamples, _Graph)
 from .hg2v_weighting import UniformWeight, WeightByNeighborhood
-from .hypergraph_util import CompressRange
+from .hypergraph_util import CompressRange, ToCsrMatrix, ToEdgeCsrMatrix
 
 log = logging.getLogger()
 
@@ -110,6 +115,69 @@ def EmbedHg2vAlgDist(hypergraph, dimension, alpha=0, num_neighbors=5, num_sample
   model_fn = lambda hg: UnweightedFloatModel(hg, dimension=dimension, num_neighbors=num_neighbors)
   embedding = _hypergraph2vec_skeleton(hypergraph, dimension, num_neighbors, sampler_fn, model_fn,
                                        batch_size, epochs, debug_summary_path, disable_pbar)
+  embedding.method_name = "HG2V_ALG_DIST"
+  return embedding
+
+
+def _hypergraph2vec_device(hypergraph, dimension, num_neighbors, sampler_fn, activation, loss,
+                           batch_size, epochs, seed):
+  """_hypergraph2vec_skeleton with the samples kept on the device: CompressRange, sampler_fn(the
+  compressed graph's _Graph) -> DeviceSampleColumns, Hg2vModel.seeded, fit_device,
+  KerasModelToEmbedding.  Sampling, tables and epoch orders all derive from `seed`."""
+  compressed_hg, inv_node_map, inv_edge_map = CompressRange(hypergraph)
+  g = _Graph.from_csr(ToCsrMatrix(compressed_hg), ToEdgeCsrMatrix(compressed_hg))
+  log.info("Sampling on the device")
+  samples = sampler_fn(g, compressed_hg)
+  model = Hg2vModel.seeded(g.num_nodes, g.num_edges, dimension, num_neighbors, activation, loss, seed)
+  stopper = EarlyStopping(monitor="loss", min_delta=1e-3)
+  try:
+    model.fit_device(samples, batch_size=batch_size, epochs=epochs, seed=seed, callbacks=[stopper])
+    log.info("Recording embeddings.")
+    return KerasModelToEmbedding(compressed_hg, model, inv_node_map, inv_edge_map)
+  finally:
+    model.close()
+
+
+def EmbedHg2vBooleanDevice(hypergraph, dimension, num_neighbors=5, num_samples=200, batch_size=256,
+                           epochs=10, neg_samples=0, seed=0, chunk_rows=0):
+  """EmbedHg2vBoolean (FOBE) as a seeded pipeline whose samples never leave the GPU:
+  BooleanSamplesDevice (per-row counts from the node / edge weights, as BooleanSamples), a
+  BooleanModel with seeded tables, and per-epoch orders from hge_shuffle_order.  The result
+  depends on `seed`, not on numpy's global RNG, which is neither read nor advanced."""
+
+  def sampler_fn(g, hg):
+    nw = [hg.node[i].weight for i in range(g.num_nodes)]
+    ew = [hg.edge[i].weight for i in range(g.num_edges)]
+    return BooleanSamplesDevice(g, num_neighbors, num_samples, neg_samples=neg_samples, node_weights=nw,
+                                edge_weights=ew, seed=seed, chunk_rows=chunk_rows, keep_on_device=True)
+
+  embedding = _hypergraph2vec_device(hypergraph, dimension, num_neighbors, sampler_fn, "sigmoid",
+                                     "kullback_leibler_divergence", batch_size, epochs, seed)
+  embedding.method_name = "HG2V_BOOLEAN"
+  return embedding
+
+
+def EmbedHg2vAlgDistDevice(hypergraph, dimension, num_neighbors=5, num_samples=200, batch_size=256,
+                           epochs=10, seed=0, chunk_rows=0):
+  """EmbedHg2vAlgDist (HOBE) as a seeded pipeline whose samples never leave the GPU: the
+  algebraic-distance relaxation (dimension 10, 20 sweeps, initial vectors from a private
+  RandomState seeded by `seed`), AlgebraicDistanceSamplesDevice, an UnweightedFloatModel with
+  seeded tables, per-epoch orders from hge_shuffle_order.  numpy's global RNG is neither read
+  nor advanced."""
+
+  def sampler_fn(g, hg):
+    del hg
+    log.info("Embedding weighted by algebraic distance.")
+    rng = np.random.RandomState(seed & 0xFFFFFFFF)
+    xn = rng.random_sample((g.num_nodes, 10)).astype(np.float32)
+    xe = rng.random_sample((g.num_edges, 10)).astype(np.float32)
+    _native.algdist_run_csr(_native.default_context(), g.num_nodes, g.num_edges, g.a.ptr, g.a.idx, xn, xe,
+                            20, e2n_ptr=g.b.ptr, e2n_idx=g.b.idx)
+    return AlgebraicDistanceSamplesDevice(g, xn, xe, num_neighbors, num_samples, seed=seed,
+                                          chunk_rows=chunk_rows, keep_on_device=True)
+
+  embedding = _hypergraph2vec_device(hypergraph, dimension, num_neighbors, sampler_fn, "relu",
+                                     "mean_squared_error", batch_size, epochs, seed)
   embedding.method_name = "HG2V_ALG_DIST"
   return embedding
 

@@ -107,6 +107,29 @@ class Hg2vModel(object):
                     "edge_embedding": _EmbeddingLayer(self, 1, "edge_embedding")}
     self.stop_training = False
 
+  @classmethod
+  def seeded(cls, num_nodes, num_edges, dimension, num_neighbors, activation, loss, seed, ctx=None):
+    """The model for `num_nodes` / `num_edges` compressed ids (num + 1 table rows, as
+    Embedding(input_dim = max id + 2) gives), its tables drawn on the device from U(-0.05, 0.05)
+    by seeded Philox streams (hge_hg2v_create_seeded).  numpy's global RNG is neither read nor
+    advanced."""
+    self = cls.__new__(cls)
+    self.dimension, self.num_neighbors = int(dimension), int(num_neighbors)
+    self.activation, self.loss = activation, loss
+    self.ctx = ctx or _native.default_context()
+    self.node_rows, self.edge_rows = int(num_nodes) + 1, int(num_edges) + 1
+    handle = _native.c_vp()
+    _native.check(self.ctx.lib.hge_hg2v_create_seeded(self.ctx.handle, self.node_rows, self.edge_rows,
+                                                      self.dimension, self.num_neighbors,
+                                                      ACTIVATIONS[activation], LOSSES[loss],
+                                                      int(seed) & 0xFFFFFFFFFFFFFFFF, ctypes.byref(handle)),
+                  "hge_hg2v_create_seeded")
+    self.handle = handle
+    self._layers = {"node_embedding": _EmbeddingLayer(self, 0, "node_embedding"),
+                    "edge_embedding": _EmbeddingLayer(self, 1, "edge_embedding")}
+    self.stop_training = False
+    return self
+
   def get_layer(self, name):
     return self._layers[name]
 
@@ -138,6 +161,62 @@ class Hg2vModel(object):
                                                   _native.MEM_HOST, ctypes.byref(loss)),
                   "hge_hg2v_fit_epoch")
     return loss.value
+
+  def set_device_samples(self, samples):
+    """Packs a DeviceSampleColumns into the model's sample buffer on the device, as
+    SamplesToModelInput(samples.to_host(), k, weighted=False) would, then releases the blocks and
+    the memory torch cached for them.  Every index is range-checked on the device."""
+    import torch
+    assert samples.num_neighbors == self.num_neighbors, \
+        "samples have %d neighbours, the model %d" % (samples.num_neighbors, self.num_neighbors)
+    lib = self.ctx.lib
+    self.num_samples = len(samples)
+    _native.check(lib.hge_hg2v_reserve_samples(self.handle, self.num_samples), "hge_hg2v_reserve_samples")
+    for b in samples.blocks:
+      c = b.cols
+      _native.check(lib.hge_hg2v_append_samples(
+          self.handle, _native.ptr(c["left_node"]), _native.ptr(c["left_edge"]), _native.ptr(c["right_node"]),
+          _native.ptr(c["right_edge"]), _native.ptr(c["neigh_node"]), _native.ptr(c["neigh_edge"]),
+          _native.ptr(b.prob), b.prob_slot, b.prob_value, b.count),
+                    "hge_hg2v_append_samples")
+    samples.release()
+    torch.cuda.empty_cache()
+
+  def samples(self):
+    """The packed sample buffer as SamplesToModelInput's (features, targets) lists."""
+    cols = 4 + 2 * self.num_neighbors
+    feats = np.empty((cols, self.num_samples), np.int32)
+    targets = np.empty((3, self.num_samples), np.float32)
+    _native.check(self.ctx.lib.hge_hg2v_get_samples(self.handle, _native.ptr(feats), _native.ptr(targets),
+                                                    _native.MEM_HOST), "hge_hg2v_get_samples")
+    return list(feats), list(targets)
+
+  def fit_device(self, samples, batch_size=32, epochs=1, seed=0, callbacks=None, verbose=1):
+    """fit() on a DeviceSampleColumns without a host round trip: the blocks are packed into the
+    model's buffer on the device and then released (the caller's `samples` is empty afterwards),
+    and epoch e trains in the order hge_shuffle_order(seed, e) draws on the device.  Callbacks and
+    the returned history are those of fit(); numpy's global RNG is neither read nor advanced."""
+    import torch
+    self.set_device_samples(samples)
+    order = torch.empty(max(self.num_samples, 1), dtype=torch.int32,
+                        device=torch.device("cuda", self.ctx.device))[:self.num_samples]
+    history = History()
+    stoppers = [c for c in (callbacks or []) if isinstance(c, EarlyStopping)]
+    for c in stoppers:
+      c.on_train_begin()
+    for epoch in range(int(epochs)):
+      _native.shuffle_order(self.ctx, seed, epoch, self.num_samples, out=order)
+      loss = ctypes.c_double(0.0)
+      _native.check(self.ctx.lib.hge_hg2v_fit_epoch(self.handle, _native.ptr(order), int(batch_size),
+                                                    _native.MEM_DEVICE, ctypes.byref(loss)),
+                    "hge_hg2v_fit_epoch")
+      history.epoch.append(epoch)
+      history.history["loss"].append(loss.value)
+      if verbose:
+        log.info("Epoch %d/%d - loss: %.6f", epoch + 1, epochs, loss.value)
+      if any([c.on_epoch_end(epoch, loss.value) for c in stoppers]):
+        break
+    return history
 
   @property
   def last_clusters(self):

@@ -448,15 +448,89 @@ def _per_row(weights, count, base):
   return np.asarray([int(w * base) for w in weights], dtype=np.int32)
 
 
+class _DeviceBlock(object):
+  """One block of device sampler output: int32 CUDA tensors of the index columns it has ([m, k]
+  for the neighbour arrays), and the one probability column it fills, `prob_field`, as an fp32
+  CUDA tensor `prob` or the constant `prob_value`."""
+
+  INDEX = ("left_node", "left_edge", "right_node", "right_edge", "neigh_node", "neigh_edge")
+  PROB_SLOT = {"nn_prob": 0, "ee_prob": 1, "ne_prob": 2}
+
+  def __init__(self, count, prob_field=None, prob=None, prob_value=1.0, **cols):
+    assert set(cols) <= set(self.INDEX)
+    self.count = int(count)
+    self.cols = {name: cols.get(name) for name in self.INDEX}
+    self.prob_field, self.prob, self.prob_value = prob_field, prob, float(prob_value)
+
+  @property
+  def prob_slot(self):
+    """Target slot of the probability column (hge_hg2v_append_samples), -1 for none."""
+    return self.PROB_SLOT.get(self.prob_field, -1)
+
+  def compact(self):
+    """Copies every column that is a view of a larger buffer (the sampler's output buffers are
+    sized for sum(k_r) records) into one of its own, so a kept block holds only its records."""
+    def own(t):
+      return t if t is None or t.untyped_storage().nbytes() == t.nbytes else t.clone()
+    self.cols = {name: own(t) for name, t in self.cols.items()}
+    self.prob = own(self.prob)
+    return self
+
+  def to_host(self, k):
+    cols = {name: _host(t) for name, t in self.cols.items() if t is not None}
+    if self.prob_field is not None:
+      cols[self.prob_field] = (_host(self.prob) if self.prob is not None else
+                               np.broadcast_to(np.float32(self.prob_value), (self.count,)))
+    return SampleColumns.build(k, self.count, **cols)
+
+
+class DeviceSampleColumns(object):
+  """Output of BooleanSamplesDevice / AlgebraicDistanceSamplesDevice with ``keep_on_device=True``:
+  the sampler's blocks in record order, each a set of CUDA tensors (``blocks[i].cols``,
+  ``.prob``) with its record count.  ``to_host()`` is the SampleColumns the default call returns;
+  ``Hg2vModel.fit_device`` packs the blocks into the model's sample buffer on the device."""
+
+  def __init__(self, num_neighbors, blocks):
+    self.num_neighbors = int(num_neighbors)
+    self.blocks = list(blocks)
+
+  @property
+  def counts(self):
+    return [b.count for b in self.blocks]
+
+  def __len__(self):
+    return sum(self.counts)
+
+  def to_host(self):
+    assert self.blocks, "the device blocks were released"
+    return SampleColumns.concatenate([b.to_host(self.num_neighbors) for b in self.blocks])
+
+  def release(self):
+    """Drops the device tensors (the caller frees the cached memory, e.g. torch.cuda.empty_cache)."""
+    self.blocks = []
+
+
+def _device_result(blocks, k, stream, keep_on_device):
+  """The three forms of a device sampler's result from its generator of _DeviceBlock."""
+  if keep_on_device:
+    assert not stream, "keep_on_device=True holds every block on the device; it does not stream"
+    return DeviceSampleColumns(k, (b.compact() for b in blocks))
+  chunks = (b.to_host(k) for b in blocks)
+  if stream:
+    return chunks
+  return SampleColumns.concatenate(list(chunks))
+
+
 def BooleanSamplesDevice(incidence, num_neighbors, num_samples, neg_samples=0, node_weights=None,
-                         edge_weights=None, seed=0, chunk_rows=0, stream=False):
+                         edge_weights=None, seed=0, chunk_rows=0, stream=False, keep_on_device=False):
   """BooleanSamplesCsr drawn on the GPU from seeded Philox streams instead of numpy's global
   MT19937 (which is neither read nor advanced).  Same distribution of every record as the
   reference's FOBE sampler, same blocks in the same order (node-node, edge-edge, node-edge rows,
   edge-node rows; with negatives their negative blocks, the edge-edge one twice as in the
   reference), same columns; not the reference's stream.  The result depends only on the graph,
   the counts and `seed`, not on `chunk_rows`.  With ``stream=True`` returns an iterator of
-  SampleColumns chunks of about `chunk_rows` rows; otherwise one SampleColumns."""
+  SampleColumns chunks of about `chunk_rows` rows; with ``keep_on_device=True`` a
+  DeviceSampleColumns whose blocks stay on the GPU; otherwise one SampleColumns."""
   assert num_neighbors >= 0
   assert num_samples >= 0
   assert neg_samples >= 0
@@ -465,24 +539,21 @@ def BooleanSamplesDevice(incidence, num_neighbors, num_samples, neg_samples=0, n
   edge_s = _per_row(edge_weights, g.num_edges, num_samples)
   assert node_s.min(initial=0) >= 0 and edge_s.min(initial=0) >= 0
   k = num_neighbors
-  ones = lambda m: np.broadcast_to(np.float32(1.0), (m,))
 
-  def chunks():
+  def blocks():
     ctx = _native.default_context()
     inc = g.incidence(ctx)
     s = _DeviceSampler(g, ctx, inc, k, seed, chunk_rows)
     try:
-      blocks = [(0, node_s, _native.PHASE_NN, "left_node", "right_node", "nn_prob", False),
-                (1, edge_s, _native.PHASE_EE, "left_edge", "right_edge", "ee_prob", False)]
-      for side, samples, phase, left, right, prob, neg in blocks:
-        for r, c in s.pairs(side, 2, samples, phase, negative=neg):
-          cols = {left: _host(r), right: _host(c), prob: ones(int(r.shape[0]))}
-          yield SampleColumns.build(k, int(r.shape[0]), **cols)
+      for side, samples, phase, left, right, prob in (
+          (0, node_s, _native.PHASE_NN, "left_node", "right_node", "nn_prob"),
+          (1, edge_s, _native.PHASE_EE, "left_edge", "right_edge", "ee_prob")):
+        for r, c in s.pairs(side, 2, samples, phase):
+          yield _DeviceBlock(r.shape[0], prob, **{left: r, right: c})
       phases = (_native.PHASE_NE, _native.PHASE_EN, _native.PHASE_NEIGHBORS)
       for nodes, edges, nbr_n, nbr_e in s.node_edge(node_s, edge_s, 1, phases):
-        m = int(nodes.shape[0])
-        yield SampleColumns.build(k, m, left_node=_host(nodes), right_edge=_host(edges),
-                                  neigh_node=_host(nbr_n), neigh_edge=_host(nbr_e), ne_prob=ones(m))
+        yield _DeviceBlock(nodes.shape[0], "ne_prob", left_node=nodes, right_edge=edges, neigh_node=nbr_n,
+                           neigh_edge=nbr_e)
       if neg_samples > 0:
         neg_n = _per_row(node_weights, g.num_nodes, neg_samples)
         neg_e = _per_row(edge_weights, g.num_edges, neg_samples)
@@ -491,18 +562,15 @@ def BooleanSamplesDevice(incidence, num_neighbors, num_samples, neg_samples=0, n
             (1, neg_e, _native.PHASE_NEG_EE, "left_edge", "right_edge"),
             (1, neg_e, _native.PHASE_NEG_EE_AGAIN, "left_edge", "right_edge")):   # sic, :215-221
           for r, c in s.pairs(side, 2, samples, phase, negative=True):
-            yield SampleColumns.build(k, int(r.shape[0]), **{left: _host(r), right: _host(c)})
+            yield _DeviceBlock(r.shape[0], **{left: r, right: c})
         phases = (_native.PHASE_NEG_NE, _native.PHASE_NEG_EN, _native.PHASE_NEG_NEIGHBORS)
         for nodes, edges, nbr_n, nbr_e in s.node_edge(neg_n, neg_e, 1, phases, negative=True):
-          yield SampleColumns.build(k, int(nodes.shape[0]), left_node=_host(nodes),
-                                    right_edge=_host(edges), neigh_node=_host(nbr_n),
-                                    neigh_edge=_host(nbr_e))
+          yield _DeviceBlock(nodes.shape[0], left_node=nodes, right_edge=edges, neigh_node=nbr_n,
+                             neigh_edge=nbr_e)
     finally:
       inc.close()
 
-  if stream:
-    return chunks()
-  return SampleColumns.concatenate(list(chunks()))
+  return _device_result(blocks(), k, stream, keep_on_device)
 
 
 ################################################################################
@@ -783,12 +851,13 @@ def _hobe_samples(g, xn, xe, k, num_samples, timings=None):
 
 
 def AlgebraicDistanceSamplesDevice(incidence, xn, xe, num_neighbors, num_samples, seed=0,
-                                   chunk_rows=0, stream=False, timings=None):
+                                   chunk_rows=0, stream=False, timings=None, keep_on_device=False):
   """AlgebraicDistanceSamplesCsr with the pairs and neighbour arrays drawn on the GPU from seeded
   Philox streams (see BooleanSamplesDevice) instead of numpy's global MT19937, which is neither
   read nor advanced.  The pairs stay on the device and go straight into the probability kernels.
   Same blocks, columns and probabilities as the reference's HOBE sampler; not its stream.  With
-  ``stream=True`` returns an iterator of SampleColumns chunks of about `chunk_rows` rows.
+  ``stream=True`` returns an iterator of SampleColumns chunks of about `chunk_rows` rows, with
+  ``keep_on_device=True`` a DeviceSampleColumns (see BooleanSamplesDevice).
   `timings` (a dict) receives the seconds spent drawing pairs ("pairs") and neighbour arrays
   ("neighbours") and computing the incidence weights and probabilities ("probabilities"); it is
   filled when the result is complete."""
@@ -803,19 +872,20 @@ def AlgebraicDistanceSamplesDevice(incidence, xn, xe, num_neighbors, num_samples
   per_node = _per_row(None, g.num_nodes, num_samples)
   per_edge = _per_row(None, g.num_edges, num_samples)
 
-  def chunks():
+  def blocks():
     spent = {"probabilities": 0.0}
-
-    def prob(fn, *args):
-      t = time.perf_counter()
-      out = _host(fn(*args))
-      spent["probabilities"] += time.perf_counter() - t
-      return out
-
     t = time.perf_counter()
     weights = _HobeWeights(g, xn, xe)
     spent["probabilities"] += time.perf_counter() - t
     ctx, inc = weights.ctx, weights.inc
+
+    def prob(fn, *args):
+      t = time.perf_counter()
+      out = fn(*args)
+      ctx.sync()
+      spent["probabilities"] += time.perf_counter() - t
+      return out
+
     s = _DeviceSampler(g, ctx, inc, k, seed, chunk_rows)
     try:
       for side, samples, phase, left, right, field, w in (
@@ -823,21 +893,19 @@ def AlgebraicDistanceSamplesDevice(incidence, xn, xe, num_neighbors, num_samples
           (1, per_edge, _native.PHASE_EE, "left_edge", "right_edge", "ee_prob", weights.w_e2n)):
         for r, c in s.pairs(side, 2, samples, phase):
           p = prob(_native.same_type_prob, ctx, inc, side, w, r, c)
-          yield SampleColumns.build(k, len(p), **{left: _host(r), right: _host(c), field: p})
+          yield _DeviceBlock(p.shape[0], field, p, **{left: r, right: c})
       phases = (_native.PHASE_NE, _native.PHASE_EN, _native.PHASE_NEIGHBORS)
       for nodes, edges, nbr_n, nbr_e in s.node_edge(per_node, per_edge, 3, phases):
         p = prob(_native.diff_type_prob, ctx, inc, weights.w_e2n, nodes, edges)
-        yield SampleColumns.build(k, len(p), left_node=_host(nodes), right_edge=_host(edges),
-                                  neigh_node=_host(nbr_n), neigh_edge=_host(nbr_e), ne_prob=p)
+        yield _DeviceBlock(p.shape[0], "ne_prob", p, left_node=nodes, right_edge=edges, neigh_node=nbr_n,
+                           neigh_edge=nbr_e)
     finally:
       weights.close()
     if timings is not None:
       timings.update(s.spent)
       timings.update(spent)
 
-  if stream:
-    return chunks()
-  return SampleColumns.concatenate(list(chunks()))
+  return _device_result(blocks(), k, stream, keep_on_device)
 
 
 def SameTypeDistanceSample(indices, idx2target=None, source_half_emb=None, target_half_emb=None,

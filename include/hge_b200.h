@@ -383,6 +383,38 @@ int hge_hg2v_fit_epoch(hge_hg2v_model* m, const int32_t* order, int batch_size, 
 int hge_hg2v_last_clusters(const hge_hg2v_model* m);
 int hge_hg2v_get_weights(hge_hg2v_model* m, float* node, float* edge, int mem);
 
+/* Seeded sample -> train pipeline on the device (Hg2vModel.seeded / fit_device).
+ *
+ * hge_hg2v_create_seeded: hge_hg2v_create with the tables drawn on the device from U(-0.05, 0.05),
+ * the range of Keras' 'uniform' initializer (hg2v_model.py:75-84): element (r, c) =
+ * -0.05 + 0.1 * ((w >> 8) * 2^-24) in fp32, each operation rounded on its own, w = word c of the
+ * Philox stream of item r (csrc/hge_philox.cuh), phase HGE_PHASE_INIT_NODES (13) for the node
+ * table and HGE_PHASE_INIT_EDGES (14) for the edge table. */
+int hge_hg2v_create_seeded(hge_ctx* ctx, int32_t node_rows, int32_t edge_rows, int dim, int num_neighbors,
+                           int activation, int loss, uint64_t seed, hge_hg2v_model** out);
+/* Allocates the model's own sample buffer (features [4 + 2k][num_samples] int32, targets
+ * [3][num_samples] fp32) and sets its append cursor to 0; num_samples < 2^31.  Until every
+ * record is appended hge_hg2v_fit_epoch refuses the model. */
+int hge_hg2v_reserve_samples(hge_hg2v_model* m, int64_t num_samples);
+/* Writes `count` records of sampler output at the cursor, as SamplesToModelInput(..., weighted =
+ * False) (hg2v_sample.py:751-797) packs them: indices + 1, a NULL column is the padding index 0,
+ * nbr_nodes / nbr_edges are [count, k] row-major and go to the k neighbour-node then the k
+ * neighbour-edge columns; target slot prob_slot (0 node-node, 1 edge-edge, 2 node-edge) is prob[i]
+ * (NaN -> 0), or prob_value when prob is NULL, every other slot 0 (prob_slot = -1: all three 0).
+ * All pointers are device pointers.  Every index written is checked against its table on the
+ * device; a bad one, or records past the reservation, is HGE_ERR_INVALID and leaves the cursor. */
+int hge_hg2v_append_samples(hge_hg2v_model* m, const int32_t* left_node, const int32_t* left_edge,
+                            const int32_t* right_node, const int32_t* right_edge, const int32_t* nbr_nodes,
+                            const int32_t* nbr_edges, const float* prob, int prob_slot, float prob_value,
+                            int64_t count);
+/* Copies the sample buffer out, in the layout of hge_hg2v_set_samples. */
+int hge_hg2v_get_samples(hge_hg2v_model* m, int32_t* features, float* targets, int mem);
+/* A uniform random permutation of [0, n), n < 2^31, for epoch `epoch` (Keras: np.random.shuffle
+ * per epoch, training_arrays.py).  Item i's 64-bit key is (word 2e << 32) | word 2e + 1 of its
+ * Philox stream in phase HGE_PHASE_SHUFFLE (12); items are stably sorted by key, so ties go by
+ * index.  The result is hge_hg2v_fit_epoch's order. */
+int hge_shuffle_order(hge_ctx* ctx, uint64_t seed, uint32_t epoch, int64_t n, int32_t* order, int mem);
+
 /* ---- hypergraph.proto wire format (host code; all pointers are host pointers) --------------
  * The data formats either side of the path: a serialized Hypergraph (hypergraph.proto:6-23) is
  * read straight into arrays, replacing the per-incidence Python loops of ToCsrMatrix /

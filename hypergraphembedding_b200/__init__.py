@@ -14,11 +14,13 @@ from .hg2v_sample import (AlgebraicDistanceSamples, AlgebraicDistanceSamplesCsr,
                           AlgebraicDistanceSamplesDevice, BooleanSamples, BooleanSamplesCsr,
                           BooleanSamplesDevice, DeviceSampleColumns,
                           SampleColumns, SamplesToModelInput, SimilarityRecord,
-                          SparseWeightedJaccard, WeightedJaccardSamples)
+                          SparseWeightedJaccard, WeightedJaccardSamples,
+                          WeightedJaccardSamplesDevice)
 from .hg2v_model import BooleanModel, KerasModelToEmbedding, UnweightedFloatModel
-from .embedding import (EMBEDDING_OPTIONS, EmbedHg2vAdjJaccard, EmbedHg2vAlgDist,
-                        EmbedHg2vAlgDistDevice, EmbedHg2vBoolean, EmbedHg2vBooleanDevice,
-                        EmbedHg2vNeighborhoodWeightedJaccard)
+from .embedding import (EMBEDDING_OPTIONS, EmbedHg2vAdjJaccard, EmbedHg2vAdjJaccardDevice,
+                        EmbedHg2vAlgDist, EmbedHg2vAlgDistDevice, EmbedHg2vBoolean,
+                        EmbedHg2vBooleanDevice, EmbedHg2vNeighborhoodWeightedJaccard,
+                        EmbedHg2vNeighborhoodWeightedJaccardDevice)
 from .hg2v_weighting import (AlphaScaleValues, ComputeSpans, DictToSparseRow, OneMinusValues,
                              UniformWeight, WeightByAlgebraicSpan, WeightByDistance,
                              WeightByDistanceCluster, WeightByNeighborhood,
@@ -32,9 +34,11 @@ __all__ = [
     "BooleanSamples", "BooleanSamplesCsr", "BooleanSamplesDevice",
     "DeviceSampleColumns", "SampleColumns",
     "SamplesToModelInput", "SimilarityRecord", "SparseWeightedJaccard", "WeightedJaccardSamples",
+    "WeightedJaccardSamplesDevice",
     "BooleanModel", "UnweightedFloatModel", "KerasModelToEmbedding", "EMBEDDING_OPTIONS",
     "EmbedHg2vBoolean", "EmbedHg2vAdjJaccard", "EmbedHg2vNeighborhoodWeightedJaccard",
     "EmbedHg2vAlgDist", "EmbedHg2vBooleanDevice", "EmbedHg2vAlgDistDevice",
+    "EmbedHg2vAdjJaccardDevice", "EmbedHg2vNeighborhoodWeightedJaccardDevice",
     "AlphaScaleValues", "ComputeSpans", "DictToSparseRow", "OneMinusValues", "UniformWeight",
     "WeightByAlgebraicSpan", "WeightByDistance", "WeightByDistanceCluster", "WeightByNeighborhood",
     "WeightBySameTypeDistance", "ZeroOneScaleValues",

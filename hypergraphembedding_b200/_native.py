@@ -114,6 +114,10 @@ SIGNATURES = {
                                             c_vp, c_vp, ctypes.c_int64, ctypes.c_int64, c_vp, c_vp,
                                             c_vp, ctypes.c_int64, ctypes.c_int64, c_vp, c_vp,
                                             ctypes.c_int64, c_vp, ctypes.c_int]),
+    "hge_jaccard_centroid_grouped": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int, c_vp, c_vp, c_vp, ctypes.c_int64,
+                                                    ctypes.c_int64, c_vp, c_vp, c_vp, ctypes.c_int64,
+                                                    ctypes.c_int64, c_vp, c_vp, ctypes.c_int64, ctypes.c_int64,
+                                                    c_vp]),
     "hge_hg2v_create": (ctypes.c_int, [c_vp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int, ctypes.c_int,
                                        ctypes.c_int, ctypes.c_int, c_vp, c_vp, ctypes.c_int,
                                        ctypes.POINTER(c_vp)]),
@@ -602,14 +606,25 @@ class FeatureCsr(object):
     self.idx = np.ascontiguousarray(m.indices, dtype=np.int32)
     self.val = np.ascontiguousarray(m.data, dtype=np.float32)
 
+  def to_device(self, device):
+    """The same matrix with its three arrays uploaded as CUDA tensors to `device`."""
+    import torch
+    d = FeatureCsr.__new__(FeatureCsr)
+    d.shape = self.shape
+    d.ptr, d.idx, d.val = (torch.from_numpy(a).to(device) for a in (self.ptr, self.idx, self.val))
+    return d
+
 
 def jaccard_rows(ctx, feat, pi, pj):
-  """J(F[pi], F[pj]) for host index arrays; returns a numpy fp32 array."""
-  pi, pj = _as_i32(pi), _as_i32(pj)
-  out = np.empty(len(pi), dtype=np.float32)
+  """J(F[pi], F[pj]): a numpy fp32 array for host index arrays, a CUDA tensor for int32 CUDA
+  tensors (then `feat` must be FeatureCsr.to_device)."""
+  if not is_device(pi):
+    pi, pj = _as_i32(pi), _as_i32(pj)
+  n = int(pi.shape[0])
+  out = _new_like(pi, n)
   check(ctx.lib.hge_jaccard_rows(ctx.handle, ptr(feat.ptr), ptr(feat.idx), ptr(feat.val),
-                                 feat.shape[0], len(feat.idx), ptr(pi), ptr(pj), len(pi), ptr(out),
-                                 MEM_HOST), "hge_jaccard_rows")
+                                 feat.shape[0], int(feat.idx.shape[0]), ptr(pi), ptr(pj), n, ptr(out),
+                                 _mem(feat.ptr, pi, pj)), "hge_jaccard_rows")
   return out
 
 
@@ -628,6 +643,23 @@ def jaccard_centroid(ctx, x, groups, feat, px, pg):
       ptr(groups.idx), groups.shape[0], len(groups.idx), ptr(feat.ptr), ptr(feat.idx), ptr(feat.val),
       feat.shape[0], len(feat.idx), ptr(px), ptr(pg), len(px), ptr(out), MEM_HOST),
         "hge_jaccard_centroid")
+  return out
+
+
+def jaccard_centroid_grouped(ctx, inc, group_side, x, feat, px, pg, workspace_mb=0):
+  """hge_jaccard_centroid_grouped: J(X[px], mean of F over the members of group pg) with the groups
+  taken from the incidence (group_side 1: edges and their nodes, 0: nodes and their edges).  x and
+  feat are FeatureCsr.to_device, px / pg int32 CUDA tensors; returns an fp32 CUDA tensor."""
+  import torch
+  n = int(px.shape[0])
+  assert int(pg.shape[0]) == n
+  assert x.shape[1] == feat.shape[1]
+  out = torch.empty(max(n, 1), dtype=torch.float32, device=px.device)[:n]
+  check(ctx.lib.hge_jaccard_centroid_grouped(
+      ctx.handle, inc.handle, int(group_side), ptr(x.ptr), ptr(x.idx), ptr(x.val), x.shape[0],
+      int(x.idx.shape[0]), ptr(feat.ptr), ptr(feat.idx), ptr(feat.val), feat.shape[0],
+      int(feat.idx.shape[0]), ptr(px.contiguous()), ptr(pg.contiguous()), n, int(workspace_mb), ptr(out)),
+        "hge_jaccard_centroid_grouped")
   return out
 
 

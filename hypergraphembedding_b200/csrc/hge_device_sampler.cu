@@ -39,19 +39,6 @@ constexpr int64_t kBytesPerEntry = 40;
 
 enum : int { kBadCount = 1, kEmptyList = 2 };
 
-// device buffer released when it goes out of scope (stream-ordered)
-template <typename T>
-struct DevBuf {
-  const hge_ctx* ctx;
-  T* p = nullptr;
-  explicit DevBuf(const hge_ctx* c) : ctx(c) {}
-  ~DevBuf() { hge_dev_free(ctx, p); }
-  int alloc(size_t n) {
-    hge_dev_free(ctx, p);
-    return hge_dev_alloc(ctx, &p, n);
-  }
-};
-
 int exclusive_sum(hge_ctx* ctx, const int64_t* in, int64_t* out, int64_t n) {
   size_t bytes = 0;
   HGE_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, bytes, in, out, n, ctx->stream));

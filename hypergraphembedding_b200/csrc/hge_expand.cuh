@@ -17,6 +17,19 @@ int grid_for(const hge_ctx* ctx, int64_t work, int per_block = kExpandBlock) {
   return (int)std::min<int64_t>(want, (int64_t)ctx->num_sms * 16);
 }
 
+// device buffer released when it goes out of scope (stream-ordered)
+template <typename T>
+struct DevBuf {
+  const hge_ctx* ctx;
+  T* p = nullptr;
+  explicit DevBuf(const hge_ctx* c) : ctx(c) {}
+  ~DevBuf() { hge_dev_free(ctx, p); }
+  int alloc(size_t n) {
+    hge_dev_free(ctx, p);
+    return hge_dev_alloc(ctx, &p, n);
+  }
+};
+
 template <typename T>
 int read_back(hge_ctx* ctx, const T* dev, T* host, size_t n) {
   HGE_CUDA(cudaMemcpyAsync(host, dev, n * sizeof(T), cudaMemcpyDeviceToHost, ctx->stream));

@@ -23,6 +23,9 @@
 //               expand (group, column, value) triples in member order, stable radix sort by
 //               (group, column), one sequential sum per run -- the classic expand / sort /
 //               compress product, batched so that the expansion stays inside a memory budget.
+//               hge_jaccard_centroid keeps every named centroid row resident until its merge;
+//               hge_jaccard_centroid_grouped sorts the pairs by group and builds, merges and
+//               frees the rows batch by batch, so its peak is the budget plus O(pairs).
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
@@ -31,6 +34,7 @@
 
 #include "hge_common.cuh"
 #include "hge_expand.cuh"
+#include "hge_incidence.cuh"
 #include "hge_staged.cuh"
 
 namespace {
@@ -51,8 +55,35 @@ __device__ __forceinline__ void jaccard_step(float x, float y, float& num, float
   }
 }
 
-// out[p] = J(A[pa[p]], B[pb[p]]), one thread per pair, union walked in ascending column order.
-// skip_empty_b: a pair whose B row is marked empty (bptr[r] < 0 never happens; see b_count) gives 0.
+// J(A[ra], B[rb]): the union of the two sorted rows walked in ascending column order
+__device__ __forceinline__ float jaccard_pair(const int64_t* __restrict__ aptr, const int32_t* __restrict__ aidx,
+                                              const float* __restrict__ aval, int64_t ra,
+                                              const int64_t* __restrict__ bptr, const int32_t* __restrict__ bidx,
+                                              const float* __restrict__ bval, int64_t rb) {
+  int64_t i = aptr[ra], j = bptr[rb];
+  const int64_t ie = aptr[ra + 1], je = bptr[rb + 1];
+  float num = 0.f, den = 0.f;
+  int32_t ci = i < ie ? aidx[i] : INT32_MAX, cj = j < je ? bidx[j] : INT32_MAX;
+  while (i < ie || j < je) {
+    float x = 0.f, y = 0.f;
+    const bool take_a = ci <= cj, take_b = cj <= ci;
+    if (take_a) {
+      x = aval[i];
+      ++i;
+    }
+    if (take_b) {
+      y = bval[j];
+      ++j;
+    }
+    if (take_a) ci = i < ie ? aidx[i] : INT32_MAX;
+    if (take_b) cj = j < je ? bidx[j] : INT32_MAX;
+    jaccard_step(x, y, num, den);
+  }
+  return den == 0.f ? 0.f : __fdiv_rn(num, den);
+}
+
+// out[p] = J(A[pa[p]], B[pb[p]]), one thread per pair.
+// b_members (optional): a pair whose group rb has no members gives 0.
 __global__ void __launch_bounds__(kBlock) k_jaccard_merge(
     int64_t num_pairs, const int64_t* __restrict__ aptr, const int32_t* __restrict__ aidx,
     const float* __restrict__ aval, const int64_t* __restrict__ bptr, const int32_t* __restrict__ bidx,
@@ -65,26 +96,7 @@ __global__ void __launch_bounds__(kBlock) k_jaccard_merge(
       out[p] = 0.f;
       continue;
     }
-    int64_t i = aptr[ra], j = bptr[rb];
-    const int64_t ie = aptr[ra + 1], je = bptr[rb + 1];
-    float num = 0.f, den = 0.f;
-    int32_t ci = i < ie ? aidx[i] : INT32_MAX, cj = j < je ? bidx[j] : INT32_MAX;
-    while (i < ie || j < je) {
-      float x = 0.f, y = 0.f;
-      const bool take_a = ci <= cj, take_b = cj <= ci;
-      if (take_a) {
-        x = aval[i];
-        ++i;
-      }
-      if (take_b) {
-        y = bval[j];
-        ++j;
-      }
-      if (take_a) ci = i < ie ? aidx[i] : INT32_MAX;
-      if (take_b) cj = j < je ? bidx[j] : INT32_MAX;
-      jaccard_step(x, y, num, den);
-    }
-    out[p] = den == 0.f ? 0.f : __fdiv_rn(num, den);
+    out[p] = jaccard_pair(aptr, aidx, aval, ra, bptr, bidx, bval, rb);
   }
 }
 
@@ -149,18 +161,19 @@ __global__ void __launch_bounds__(kBlock) k_expand(
 }
 
 // head of a run: the members' values added in member order, then one division by the group size
-// (targets2features[rows].sum(axis=0) / len(rows), hg2v_sample.py:293)
-__global__ void k_run_sums(int64_t n, int64_t g0, const uint64_t* __restrict__ keys,
-                           const float* __restrict__ vals, const int64_t* __restrict__ pos,
-                           const int64_t* __restrict__ gptr, int32_t* __restrict__ cidx,
-                           float* __restrict__ cval) {
+// (targets2features[rows].sum(axis=0) / len(rows), hg2v_sample.py:293).  Local group l is group
+// gid[l] of the group CSR, or g0 + l when gid is NULL.
+__global__ void k_run_sums(int64_t n, int64_t g0, const int32_t* __restrict__ gid,
+                           const uint64_t* __restrict__ keys, const float* __restrict__ vals,
+                           const int64_t* __restrict__ pos, const int64_t* __restrict__ gptr,
+                           int32_t* __restrict__ cidx, float* __restrict__ cval) {
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n;
        i += (int64_t)gridDim.x * blockDim.x) {
     const uint64_t key = keys[i];
     if (i > 0 && keys[i - 1] == key) continue;
     float s = 0.f;
     for (int64_t k = i; k < n && keys[k] == key; ++k) s = __fadd_rn(s, vals[k]);
-    const int64_t g = g0 + (int64_t)(key >> 32);
+    const int64_t l = (int64_t)(key >> 32), g = gid ? (int64_t)gid[l] : g0 + l;
     const int64_t o = pos[i];
     cidx[o] = (int32_t)(uint32_t)key;
     cval[o] = __fdiv_rn(s, (float)(gptr[g + 1] - gptr[g]));
@@ -186,6 +199,52 @@ struct CentroidRows {
   int32_t* idx = nullptr;
   float* val = nullptr;
 };
+
+// Centroid rows of one batch of L groups from its expansion: keys ((local group << 32) | column)
+// and vals, n > 0 entries in member order.  Stable radix sort by key (inside a (group, column) run
+// the members stay in ascending order), run heads, then one sequential fp32 sum per run.  Local
+// group l is group gid[l] of the group CSR (g0 + l when gid is NULL).  The rows' start offsets go to
+// start[s0 + l] = rows_before + first run of l (and start[s0 + L] when last); the n_runs column ids
+// and values to *cidx / *cval, which the caller frees.  keys / vals are used as sort buffers.
+int centroid_batch(hge_ctx* ctx, int64_t n, int64_t L, int64_t g0, const int32_t* gid, const int64_t* gptr,
+                   DevBuf<uint64_t>& keys, DevBuf<float>& vals, int64_t* start, int64_t s0, int64_t rows_before,
+                   bool last, int32_t** cidx, float** cval, int64_t* n_runs) {
+  DevBuf<uint64_t> keys2(ctx);
+  DevBuf<float> vals2(ctx);
+  DevBuf<int64_t> head(ctx), pos(ctx);
+  DevBuf<char> temp(ctx);
+  HGE_TRY(keys2.alloc((size_t)n));
+  HGE_TRY(vals2.alloc((size_t)n));
+  int group_bits = 1;
+  while ((1ll << group_bits) < L) ++group_bits;
+  cub::DoubleBuffer<uint64_t> dk(keys.p, keys2.p);
+  cub::DoubleBuffer<float> dv(vals.p, vals2.p);
+  size_t bytes = 0;
+  HGE_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, bytes, dk, dv, n, 0, 32 + group_bits, ctx->stream));
+  HGE_TRY(temp.alloc(bytes));
+  HGE_CUDA(cub::DeviceRadixSort::SortPairs(temp.p, bytes, dk, dv, n, 0, 32 + group_bits, ctx->stream));
+  ctx->launches++;
+  const uint64_t* sk = dk.Current();
+  const float* sv = dv.Current();
+  HGE_TRY(head.alloc((size_t)n + 1));
+  HGE_TRY(pos.alloc((size_t)n + 1));
+  k_run_heads<<<grid_for(ctx, n), kBlock, 0, ctx->stream>>>(n, sk, head.p);
+  HGE_CHECK_LAUNCH(ctx);
+  HGE_CUDA(cudaMemsetAsync(head.p + n, 0, sizeof(int64_t), ctx->stream));
+  HGE_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, bytes, head.p, pos.p, n + 1, ctx->stream));
+  HGE_TRY(temp.alloc(bytes));
+  HGE_CUDA(cub::DeviceScan::ExclusiveSum(temp.p, bytes, head.p, pos.p, n + 1, ctx->stream));
+  ctx->launches++;
+  HGE_TRY(read_back(ctx, pos.p + n, n_runs, 1));
+  HGE_TRY(hge_dev_alloc(ctx, cidx, (size_t)std::max<int64_t>(1, *n_runs)));
+  HGE_TRY(hge_dev_alloc(ctx, cval, (size_t)std::max<int64_t>(1, *n_runs)));
+  k_run_sums<<<grid_for(ctx, n), kBlock, 0, ctx->stream>>>(n, g0, gid, sk, sv, pos.p, gptr, *cidx, *cval);
+  HGE_CHECK_LAUNCH(ctx);
+  k_run_starts<<<grid_for(ctx, L + 1), kBlock, 0, ctx->stream>>>(s0, s0 + L, n, *n_runs, rows_before, sk, pos.p,
+                                                               start, last);
+  HGE_CHECK_LAUNCH(ctx);
+  return HGE_OK;
+}
 
 int build_centroids(hge_ctx* ctx, const int64_t* gptr, const int32_t* gidx, int64_t groups, int64_t gnnz,
                     const FeatureMatrix& f, const int32_t* pg, int64_t num_pairs, CentroidRows* out) {
@@ -242,58 +301,20 @@ int build_centroids(hge_ctx* ctx, const int64_t* gptr, const int32_t* gidx, int6
       g0 = g1;
       continue;
     }
-    uint64_t *keys = nullptr, *keys2 = nullptr;
-    float *vals = nullptr, *vals2 = nullptr;
-    int64_t *head = nullptr, *pos = nullptr;
-    char* temp = nullptr;
+    DevBuf<uint64_t> keys(ctx);
+    DevBuf<float> vals(ctx);
     Part part = {nullptr, nullptr, 0};
     auto batch = [&]() -> int {
-      HGE_TRY(hge_dev_alloc(ctx, &keys, (size_t)n));
-      HGE_TRY(hge_dev_alloc(ctx, &keys2, (size_t)n));
-      HGE_TRY(hge_dev_alloc(ctx, &vals, (size_t)n));
-      HGE_TRY(hge_dev_alloc(ctx, &vals2, (size_t)n));
+      HGE_TRY(keys.alloc((size_t)n));
+      HGE_TRY(vals.alloc((size_t)n));
       k_expand<<<grid_for(ctx, h_gptr[(size_t)g1] - h_gptr[(size_t)g0], kBlock / 32), kBlock, 0, ctx->stream>>>(
           h_gptr[(size_t)g0], h_gptr[(size_t)g1], g0, g1, h_goff[(size_t)g0], gptr, gidx, off, w, f.ptr.dev,
-          f.idx.dev, f.val.dev, keys, vals);
+          f.idx.dev, f.val.dev, keys.p, vals.p);
       HGE_CHECK_LAUNCH(ctx);
-      int group_bits = 1;
-      while ((1ll << group_bits) < g1 - g0) ++group_bits;
-      size_t bytes = 0;
-      HGE_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, bytes, keys, keys2, vals, vals2, n, 0, 32 + group_bits,
-                                               ctx->stream));
-      HGE_TRY(hge_dev_alloc(ctx, &temp, bytes));
-      // radix sort is stable: inside a (group, column) run the members stay in ascending order
-      HGE_CUDA(cub::DeviceRadixSort::SortPairs(temp, bytes, keys, keys2, vals, vals2, n, 0, 32 + group_bits,
-                                               ctx->stream));
-      ctx->launches++;
-      hge_dev_free(ctx, temp);
-      HGE_TRY(hge_dev_alloc(ctx, &head, (size_t)n + 1));
-      HGE_TRY(hge_dev_alloc(ctx, &pos, (size_t)n + 1));
-      k_run_heads<<<grid_for(ctx, n), kBlock, 0, ctx->stream>>>(n, keys2, head);
-      HGE_CHECK_LAUNCH(ctx);
-      HGE_CUDA(cudaMemsetAsync(head + n, 0, sizeof(int64_t), ctx->stream));
-      HGE_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, bytes, head, pos, n + 1, ctx->stream));
-      HGE_TRY(hge_dev_alloc(ctx, &temp, bytes));
-      HGE_CUDA(cub::DeviceScan::ExclusiveSum(temp, bytes, head, pos, n + 1, ctx->stream));
-      ctx->launches++;
-      HGE_TRY(read_back(ctx, pos + n, &part.n, 1));
-      HGE_TRY(hge_dev_alloc(ctx, &part.idx, (size_t)std::max<int64_t>(1, part.n)));
-      HGE_TRY(hge_dev_alloc(ctx, &part.val, (size_t)std::max<int64_t>(1, part.n)));
-      k_run_sums<<<grid_for(ctx, n), kBlock, 0, ctx->stream>>>(n, g0, keys2, vals2, pos, gptr, part.idx, part.val);
-      HGE_CHECK_LAUNCH(ctx);
-      k_run_starts<<<grid_for(ctx, g1 - g0 + 1), kBlock, 0, ctx->stream>>>(g0, g1, n, part.n, rows_before, keys2,
-                                                                         pos, out->ptr, last);
-      HGE_CHECK_LAUNCH(ctx);
-      return HGE_OK;
+      return centroid_batch(ctx, n, g1 - g0, g0, nullptr, gptr, keys, vals, out->ptr, g0, rows_before, last,
+                            &part.idx, &part.val, &part.n);
     };
     rc = batch();
-    hge_dev_free(ctx, keys);
-    hge_dev_free(ctx, keys2);
-    hge_dev_free(ctx, vals);
-    hge_dev_free(ctx, vals2);
-    hge_dev_free(ctx, head);
-    hge_dev_free(ctx, pos);
-    hge_dev_free(ctx, temp);
     if (rc == HGE_OK) {
       parts.push_back(part);
       rows_before += part.n;
@@ -335,6 +356,130 @@ int build_centroids(hge_ctx* ctx, const int64_t* gptr, const int32_t* gidx, int6
     hge_dev_free(ctx, out->val);
   }
   return rc;
+}
+
+// ---- centroid rows of the named groups, batch by batch (hge_jaccard_centroid_grouped) ----------
+
+constexpr int64_t kDefaultWorkspaceMb = 2048;
+// workspace bytes per expanded entry of a batch: keys and their sort buffer (16), values and theirs
+// (8), run heads and their scan (16), the centroid entry (8)
+constexpr int64_t kBytesPerEntry = 48;
+
+enum : int { kBadX = 1, kBadGroup = 2 };
+
+// sort input of the pairs: key = group, value = pair index; out-of-range ids are flagged
+__global__ void k_pair_keys(int64_t num_pairs, const int32_t* __restrict__ px, int64_t xrows,
+                            const int32_t* __restrict__ pg, int64_t groups, uint32_t* __restrict__ key,
+                            int32_t* __restrict__ idx, int* __restrict__ status) {
+  for (int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; p < num_pairs;
+       p += (int64_t)gridDim.x * blockDim.x) {
+    const int32_t x = px[p], g = pg[p];
+    if (x < 0 || x >= xrows) atomicOr(status, kBadX);
+    const bool bad_g = g < 0 || g >= groups;
+    if (bad_g) atomicOr(status, kBadGroup);
+    key[p] = bad_g ? 0u : (uint32_t)g;
+    idx[p] = (int32_t)p;
+  }
+}
+
+// head[i] = 1 where the run of pairs of one group starts (sorted group ids)
+__global__ void k_pair_heads(int64_t n, const uint32_t* __restrict__ sg, int32_t* __restrict__ head) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+    head[i] = (i == 0 || sg[i] != sg[i - 1]) ? 1 : 0;
+}
+
+// named group u = run u of the sorted pairs (u = rank[i] - 1, rank = inclusive scan of the heads):
+// ug[u] its group id, ustart[u] its first sorted pair; ustart[U] = n
+__global__ void k_named_groups(int64_t n, const uint32_t* __restrict__ sg, const int32_t* __restrict__ head,
+                               const int32_t* __restrict__ rank, int32_t* __restrict__ ug,
+                               int64_t* __restrict__ ustart) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    if (head[i]) {
+      ug[rank[i] - 1] = (int32_t)sg[i];
+      ustart[rank[i] - 1] = i;
+    }
+    if (i == n - 1) ustart[rank[i]] = n;
+  }
+}
+
+// size[u] = sum over the members m of group ug[u] of nnz(F[m]); size[U] = 0 (one warp per group)
+__global__ void __launch_bounds__(kBlock) k_named_sizes(int64_t U, const int32_t* __restrict__ ug,
+                                                        const int64_t* __restrict__ gptr,
+                                                        const int32_t* __restrict__ gidx,
+                                                        const int64_t* __restrict__ fptr, int64_t* __restrict__ size) {
+  const int lane = threadIdx.x & 31;
+  const int64_t nw = (int64_t)gridDim.x * (kBlock / 32);
+  for (int64_t u = blockIdx.x * (int64_t)(kBlock / 32) + (threadIdx.x >> 5); u <= U; u += nw) {
+    int64_t s = 0;
+    if (u < U) {
+      const int32_t g = ug[u];
+      for (int64_t t = gptr[g] + lane; t < gptr[g + 1]; t += 32) {
+        const int32_t m = gidx[t];
+        s += fptr[m + 1] - fptr[m];
+      }
+    }
+    for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(kFull, s, o);
+    if (lane == 0) size[u] = s;
+  }
+}
+
+// expansion of the named groups [u0, u1): one warp per group, its members in order, 32 at a time
+// (a warp scan of their row lengths places them); key = (u - u0) << 32 | column
+__global__ void __launch_bounds__(kBlock) k_expand_named(
+    int64_t u0, int64_t u1, int64_t base, const int32_t* __restrict__ ug, const int64_t* __restrict__ uoff,
+    const int64_t* __restrict__ gptr, const int32_t* __restrict__ gidx, const int64_t* __restrict__ fptr,
+    const int32_t* __restrict__ fidx, const float* __restrict__ fval, uint64_t* __restrict__ keys,
+    float* __restrict__ vals) {
+  const int lane = threadIdx.x & 31;
+  const int64_t nw = (int64_t)gridDim.x * (kBlock / 32);
+  for (int64_t u = u0 + blockIdx.x * (int64_t)(kBlock / 32) + (threadIdx.x >> 5); u < u1; u += nw) {
+    const int32_t g = ug[u];
+    const uint64_t hi = (uint64_t)(u - u0) << 32;
+    const int64_t t1 = gptr[g + 1];
+    int64_t dst = uoff[u] - base;
+    for (int64_t tb = gptr[g]; tb < t1; tb += 32) {
+      int64_t src = 0, len = 0;
+      if (tb + lane < t1) {
+        const int32_t m = gidx[tb + lane];
+        src = fptr[m];
+        len = fptr[m + 1] - src;
+      }
+      int64_t incl = len;
+      for (int o = 1; o < 32; o <<= 1) {
+        const int64_t v = __shfl_up_sync(kFull, incl, o);
+        if (lane >= o) incl += v;
+      }
+      const int64_t excl = incl - len;
+      const int members = t1 - tb < 32 ? (int)(t1 - tb) : 32;
+      for (int j = 0; j < members; ++j) {
+        const int64_t s = __shfl_sync(kFull, src, j), l = __shfl_sync(kFull, len, j);
+        const int64_t d = dst + __shfl_sync(kFull, excl, j);
+        for (int64_t k = lane; k < l; k += 32) {
+          keys[d + k] = hi | (uint32_t)fidx[s + k];
+          vals[d + k] = fval[s + k];
+        }
+      }
+      dst += __shfl_sync(kFull, incl, 31);
+    }
+  }
+}
+
+// out[order[i]] = J(X[px[order[i]]], centroid row u - u0) for the sorted pairs [i0, i1) of the named
+// groups [u0, u1) (u = rank[i] - 1); consecutive threads mostly share a centroid row
+__global__ void __launch_bounds__(kBlock) k_merge_named(
+    int64_t i0, int64_t i1, int64_t u0, const int32_t* __restrict__ order, const int32_t* __restrict__ rank,
+    const int32_t* __restrict__ ug, const int64_t* __restrict__ gptr, const int32_t* __restrict__ px,
+    const int64_t* __restrict__ xptr, const int32_t* __restrict__ xidx, const float* __restrict__ xval,
+    const int64_t* __restrict__ cptr, const int32_t* __restrict__ cidx, const float* __restrict__ cval,
+    float* __restrict__ out) {
+  for (int64_t i = i0 + blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < i1;
+       i += (int64_t)gridDim.x * blockDim.x) {
+    const int32_t p = order[i];
+    const int64_t u = rank[i] - 1;
+    const int32_t g = ug[u];
+    out[p] = gptr[g + 1] == gptr[g] ? 0.f   // a group without members has no centroid
+                                    : jaccard_pair(xptr, xidx, xval, px[p], cptr, cidx, cval, u - u0);
+  }
 }
 
 }  // namespace
@@ -403,6 +548,133 @@ int hge_jaccard_centroid(hge_ctx* ctx, const int64_t* xptr, const int32_t* xidx,
     return HGE_ERR_CUDA;
   }
   return s_out.finish();
+}
+
+int hge_jaccard_centroid_grouped(hge_ctx* ctx, hge_incidence* inc, int group_side, const int64_t* xptr,
+                                 const int32_t* xidx, const float* xval, int64_t xrows, int64_t xnnz,
+                                 const int64_t* fptr, const int32_t* fidx, const float* fval, int64_t frows,
+                                 int64_t fnnz, const int32_t* px, const int32_t* pg, int64_t num_pairs,
+                                 int64_t workspace_mb, float* out) {
+  HGE_REQUIRE(ctx && inc, "hge_jaccard_centroid_grouped: NULL argument");
+  HGE_REQUIRE(!inc->sharded, "hge_jaccard_centroid_grouped: needs a whole (not sharded) incidence");
+  HGE_REQUIRE(group_side == 0 || group_side == 1, "hge_jaccard_centroid_grouped: group_side must be 0 or 1");
+  HGE_REQUIRE(xptr && fptr && xrows >= 0 && frows >= 0 && xnnz >= 0 && fnnz >= 0 && (xidx || xnnz == 0) &&
+                  (xval || xnnz == 0) && (fidx || fnnz == 0) && (fval || fnnz == 0),
+              "hge_jaccard_centroid_grouped: bad matrix");
+  // groups are edges with node members (F = node features), or nodes with edge members
+  const int64_t groups = group_side == 1 ? inc->E : inc->N, members = group_side == 1 ? inc->N : inc->E;
+  HGE_REQUIRE(frows == members, "hge_jaccard_centroid_grouped: F has %lld rows, the members number %lld",
+              (long long)frows, (long long)members);
+  HGE_REQUIRE(num_pairs >= 0 && num_pairs < (1ll << 31) && (num_pairs == 0 || (px && pg && out)),
+              "hge_jaccard_centroid_grouped: bad pairs");
+  HGE_REQUIRE(workspace_mb >= 0, "hge_jaccard_centroid_grouped: negative workspace");
+  HGE_CUDA(cudaSetDevice(ctx->device));
+  if (num_pairs == 0) return HGE_OK;
+  const int64_t* gptr = group_side == 1 ? inc->e2n_ptr : inc->n2e_ptr;
+  const int32_t* gidx = group_side == 1 ? inc->e2n_idx : inc->n2e_idx;
+  const int64_t n = num_pairs;
+
+  // 1. pairs stably sorted by group
+  DevBuf<uint32_t> key(ctx), key2(ctx);
+  DevBuf<int32_t> idx(ctx), idx2(ctx), head(ctx), rank(ctx);
+  DevBuf<int> status(ctx);
+  DevBuf<char> temp(ctx);
+  HGE_TRY(key.alloc((size_t)n));
+  HGE_TRY(key2.alloc((size_t)n));
+  HGE_TRY(idx.alloc((size_t)n));
+  HGE_TRY(idx2.alloc((size_t)n));
+  HGE_TRY(status.alloc(1));
+  HGE_CUDA(cudaMemsetAsync(status.p, 0, sizeof(int), ctx->stream));
+  k_pair_keys<<<grid_for(ctx, n), kBlock, 0, ctx->stream>>>(n, px, xrows, pg, groups, key.p, idx.p, status.p);
+  HGE_CHECK_LAUNCH(ctx);
+  int bad = 0;
+  HGE_TRY(read_back(ctx, status.p, &bad, 1));
+  HGE_REQUIRE(!(bad & kBadX), "hge_jaccard_centroid_grouped: a pair names a row outside X's %lld",
+              (long long)xrows);
+  HGE_REQUIRE(!(bad & kBadGroup), "hge_jaccard_centroid_grouped: a pair names a group outside [0, %lld)",
+              (long long)groups);
+  int group_bits = 1;
+  while ((1ll << group_bits) < groups) ++group_bits;
+  cub::DoubleBuffer<uint32_t> dk(key.p, key2.p);
+  cub::DoubleBuffer<int32_t> dv(idx.p, idx2.p);
+  size_t bytes = 0;
+  HGE_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, bytes, dk, dv, n, 0, group_bits, ctx->stream));
+  HGE_TRY(temp.alloc(bytes));
+  HGE_CUDA(cub::DeviceRadixSort::SortPairs(temp.p, bytes, dk, dv, n, 0, group_bits, ctx->stream));
+  ctx->launches++;
+  const uint32_t* sg = dk.Current();
+  const int32_t* order = dv.Current();
+
+  // 2. the named groups, their pair ranges and expansion sizes
+  HGE_TRY(head.alloc((size_t)n));
+  HGE_TRY(rank.alloc((size_t)n));
+  k_pair_heads<<<grid_for(ctx, n), kBlock, 0, ctx->stream>>>(n, sg, head.p);
+  HGE_CHECK_LAUNCH(ctx);
+  HGE_CUDA(cub::DeviceScan::InclusiveSum(nullptr, bytes, head.p, rank.p, n, ctx->stream));
+  HGE_TRY(temp.alloc(bytes));
+  HGE_CUDA(cub::DeviceScan::InclusiveSum(temp.p, bytes, head.p, rank.p, n, ctx->stream));
+  ctx->launches++;
+  int32_t U32 = 0;
+  HGE_TRY(read_back(ctx, rank.p + n - 1, &U32, 1));
+  const int64_t U = U32;
+  DevBuf<int32_t> ug(ctx);
+  DevBuf<int64_t> ustart(ctx), usize(ctx), uoff(ctx);
+  HGE_TRY(ug.alloc((size_t)U));
+  HGE_TRY(ustart.alloc((size_t)U + 1));
+  HGE_TRY(usize.alloc((size_t)U + 1));
+  HGE_TRY(uoff.alloc((size_t)U + 1));
+  k_named_groups<<<grid_for(ctx, n), kBlock, 0, ctx->stream>>>(n, sg, head.p, rank.p, ug.p, ustart.p);
+  HGE_CHECK_LAUNCH(ctx);
+  hge_dev_free(ctx, head.p);
+  k_named_sizes<<<grid_for(ctx, U + 1, kBlock / 32), kBlock, 0, ctx->stream>>>(U, ug.p, gptr, gidx, fptr, usize.p);
+  HGE_CHECK_LAUNCH(ctx);
+  HGE_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, bytes, usize.p, uoff.p, U + 1, ctx->stream));
+  HGE_TRY(temp.alloc(bytes));
+  HGE_CUDA(cub::DeviceScan::ExclusiveSum(temp.p, bytes, usize.p, uoff.p, U + 1, ctx->stream));
+  ctx->launches++;
+  hge_dev_free(ctx, temp.p);
+  hge_dev_free(ctx, usize.p);
+  std::vector<int64_t> h_uoff((size_t)U + 1), h_ustart((size_t)U + 1);
+  HGE_TRY(read_back(ctx, uoff.p, h_uoff.data(), (size_t)U + 1));
+  HGE_TRY(read_back(ctx, ustart.p, h_ustart.data(), (size_t)U + 1));
+
+  // 3. batches of consecutive named groups whose expansion fits the budget (a single larger group
+  //    is its own batch): centroid rows, then the merge of the batch's pairs
+  const int64_t mb = workspace_mb ? workspace_mb : kDefaultWorkspaceMb;
+  const int64_t budget = std::max<int64_t>(1, (mb << 20) / kBytesPerEntry);
+  for (int64_t u0 = 0; u0 < U;) {
+    int64_t u1 = u0 + 1;
+    while (u1 < U && h_uoff[(size_t)u1 + 1] - h_uoff[(size_t)u0] <= budget) ++u1;
+    const int64_t L = u1 - u0, m = h_uoff[(size_t)u1] - h_uoff[(size_t)u0];
+    DevBuf<int64_t> cptr(ctx);
+    DevBuf<int32_t> cidx(ctx);
+    DevBuf<float> cval(ctx);
+    HGE_TRY(cptr.alloc((size_t)L + 1));
+    if (m == 0) {   // no member of these groups has a feature: every centroid row is empty
+      HGE_CUDA(cudaMemsetAsync(cptr.p, 0, ((size_t)L + 1) * sizeof(int64_t), ctx->stream));
+    } else {
+      DevBuf<uint64_t> keys(ctx);
+      DevBuf<float> vals(ctx);
+      int rc = keys.alloc((size_t)m);
+      if (rc == HGE_OK) rc = vals.alloc((size_t)m);
+      if (rc == HGE_ERR_NOMEM)
+        hge_set_error("hge_jaccard_centroid_grouped: %lld groups expand to %lld entries, more than the device holds",
+                      (long long)L, (long long)m);
+      HGE_TRY(rc);
+      k_expand_named<<<grid_for(ctx, L, kBlock / 32), kBlock, 0, ctx->stream>>>(
+          u0, u1, h_uoff[(size_t)u0], ug.p, uoff.p, gptr, gidx, fptr, fidx, fval, keys.p, vals.p);
+      HGE_CHECK_LAUNCH(ctx);
+      int64_t runs = 0;
+      HGE_TRY(centroid_batch(ctx, m, L, 0, ug.p + u0, gptr, keys, vals, cptr.p, 0, 0, true, &cidx.p, &cval.p,
+                             &runs));
+    }
+    const int64_t i0 = h_ustart[(size_t)u0], i1 = h_ustart[(size_t)u1];
+    k_merge_named<<<grid_for(ctx, i1 - i0), kBlock, 0, ctx->stream>>>(i0, i1, u0, order, rank.p, ug.p, gptr, px,
+                                                                    xptr, xidx, xval, cptr.p, cidx.p, cval.p, out);
+    HGE_CHECK_LAUNCH(ctx);
+    u0 = u1;
+  }
+  return HGE_OK;
 }
 
 }  // extern "C"

@@ -17,7 +17,7 @@ from .hg2v_model import (BooleanModel, EarlyStopping, Hg2vModel, KerasModelToEmb
                          UnweightedFloatModel)
 from .hg2v_sample import (AlgebraicDistanceSamples, AlgebraicDistanceSamplesDevice, BooleanSamples,
                           BooleanSamplesDevice, PlotDistributions, SamplesToModelInput,
-                          WeightedJaccardSamples, _Graph)
+                          WeightedJaccardSamples, WeightedJaccardSamplesDevice, _Graph)
 from .hg2v_weighting import UniformWeight, WeightByNeighborhood
 from .hypergraph_util import CompressRange, ToCsrMatrix, ToEdgeCsrMatrix
 
@@ -179,6 +179,48 @@ def EmbedHg2vAlgDistDevice(hypergraph, dimension, num_neighbors=5, num_samples=2
   embedding = _hypergraph2vec_device(hypergraph, dimension, num_neighbors, sampler_fn, "relu",
                                      "mean_squared_error", batch_size, epochs, seed)
   embedding.method_name = "HG2V_ALG_DIST"
+  return embedding
+
+
+def _jaccard_device(hypergraph, dimension, features_fn, num_neighbors, num_samples, batch_size, epochs,
+                    seed, chunk_rows):
+  """The Jaccard methods as a seeded pipeline whose samples never leave the GPU: features_fn(the
+  compressed hypergraph) on the host, WeightedJaccardSamplesDevice (per-row counts from the node /
+  edge weights, as WeightedJaccardSamples), an UnweightedFloatModel with seeded tables, per-epoch
+  orders from hge_shuffle_order."""
+
+  def sampler_fn(g, hg):
+    node2features, edge2features = features_fn(hg)
+    nw = [hg.node[i].weight for i in range(g.num_nodes)]
+    ew = [hg.edge[i].weight for i in range(g.num_edges)]
+    return WeightedJaccardSamplesDevice(g, node2features, edge2features, num_neighbors, num_samples,
+                                        node_weights=nw, edge_weights=ew, seed=seed, chunk_rows=chunk_rows,
+                                        keep_on_device=True)
+
+  return _hypergraph2vec_device(hypergraph, dimension, num_neighbors, sampler_fn, "relu",
+                                "mean_squared_error", batch_size, epochs, seed)
+
+
+def EmbedHg2vAdjJaccardDevice(hypergraph, dimension, num_neighbors=5, num_samples=200, batch_size=256,
+                              epochs=10, seed=0, chunk_rows=0):
+  """EmbedHg2vAdjJaccard (uniform features) as a seeded pipeline whose samples never leave the GPU
+  (see _jaccard_device).  The result depends on `seed`, not on numpy's global RNG, which is
+  neither read nor advanced."""
+  embedding = _jaccard_device(hypergraph, dimension, UniformWeight, num_neighbors, num_samples, batch_size,
+                              epochs, seed, chunk_rows)
+  embedding.method_name = "HG2V_ADJ_JAC"
+  return embedding
+
+
+def EmbedHg2vNeighborhoodWeightedJaccardDevice(hypergraph, dimension, alpha=0, num_neighbors=5,
+                                               num_samples=200, batch_size=256, epochs=10, seed=0,
+                                               chunk_rows=0):
+  """EmbedHg2vNeighborhoodWeightedJaccard (WeightByNeighborhood(alpha) features) as a seeded
+  pipeline whose samples never leave the GPU (see _jaccard_device).  numpy's global RNG is neither
+  read nor advanced."""
+  embedding = _jaccard_device(hypergraph, dimension, lambda hg: WeightByNeighborhood(hg, alpha),
+                              num_neighbors, num_samples, batch_size, epochs, seed, chunk_rows)
+  embedding.method_name = "HG2V_NEIGH_JAC"
   return embedding
 
 

@@ -450,17 +450,20 @@ def _per_row(weights, count, base):
 
 class _DeviceBlock(object):
   """One block of device sampler output: int32 CUDA tensors of the index columns it has ([m, k]
-  for the neighbour arrays), and the one probability column it fills, `prob_field`, as an fp32
-  CUDA tensor `prob` or the constant `prob_value`."""
+  for the neighbour arrays), the one probability column it fills, `prob_field`, as an fp32
+  CUDA tensor `prob` or the constant `prob_value`, and optionally the fp32 CUDA tensors
+  `left_weight` / `right_weight` (the Jaccard factors of node-edge records)."""
 
   INDEX = ("left_node", "left_edge", "right_node", "right_edge", "neigh_node", "neigh_edge")
   PROB_SLOT = {"nn_prob": 0, "ee_prob": 1, "ne_prob": 2}
 
-  def __init__(self, count, prob_field=None, prob=None, prob_value=1.0, **cols):
+  def __init__(self, count, prob_field=None, prob=None, prob_value=1.0, left_weight=None,
+               right_weight=None, **cols):
     assert set(cols) <= set(self.INDEX)
     self.count = int(count)
     self.cols = {name: cols.get(name) for name in self.INDEX}
     self.prob_field, self.prob, self.prob_value = prob_field, prob, float(prob_value)
+    self.left_weight, self.right_weight = left_weight, right_weight
 
   @property
   def prob_slot(self):
@@ -474,6 +477,7 @@ class _DeviceBlock(object):
       return t if t is None or t.untyped_storage().nbytes() == t.nbytes else t.clone()
     self.cols = {name: own(t) for name, t in self.cols.items()}
     self.prob = own(self.prob)
+    self.left_weight, self.right_weight = own(self.left_weight), own(self.right_weight)
     return self
 
   def to_host(self, k):
@@ -481,11 +485,15 @@ class _DeviceBlock(object):
     if self.prob_field is not None:
       cols[self.prob_field] = (_host(self.prob) if self.prob is not None else
                                np.broadcast_to(np.float32(self.prob_value), (self.count,)))
+    for name in ("left_weight", "right_weight"):
+      if getattr(self, name) is not None:
+        cols[name] = _host(getattr(self, name))
     return SampleColumns.build(k, self.count, **cols)
 
 
 class DeviceSampleColumns(object):
-  """Output of BooleanSamplesDevice / AlgebraicDistanceSamplesDevice with ``keep_on_device=True``:
+  """Output of BooleanSamplesDevice / AlgebraicDistanceSamplesDevice /
+  WeightedJaccardSamplesDevice with ``keep_on_device=True``:
   the sampler's blocks in record order, each a set of CUDA tensors (``blocks[i].cols``,
   ``.prob``) with its record count.  ``to_host()`` is the SampleColumns the default call returns;
   ``Hg2vModel.fit_device`` packs the blocks into the model's sample buffer on the device."""
@@ -706,6 +714,76 @@ def WeightedJaccardSamples(hypergraph, node2features, edge2features, num_neighbo
                                    left_weight=prob_by_node, right_weight=prob_by_edge,
                                    ne_prob=prob_by_node * prob_by_edge))
   return SampleColumns.concatenate(parts)
+
+
+def WeightedJaccardSamplesDevice(incidence, node2features, edge2features, num_neighbors, num_samples,
+                                 node_weights=None, edge_weights=None, seed=0, chunk_rows=0, stream=False,
+                                 timings=None, keep_on_device=False, workspace_mb=0):
+  """WeightedJaccardSamples on an N x E incidence CSR (or a _Graph) with the pairs and neighbour
+  arrays drawn on the GPU from seeded Philox streams, as AlgebraicDistanceSamplesDevice draws them
+  (numpy's global MT19937 is neither read nor advanced), and every probability computed on the
+  device from the drawn pairs.  Row r emits int(weight_r * num_samples) samples (weights default
+  to 1).  Same blocks and columns as the reference's Jaccard sampler: node-node (nn_prob),
+  edge-edge (ee_prob), then node-edge rows and edge-node rows with left_weight = J(node features,
+  centroid of the edge's nodes' features), right_weight = J(edge features, centroid of the node's
+  edges' features) and ne_prob their fp32 product; not the reference's stream.  The feature
+  matrices (any scipy sparse matrices) are uploaded once per call.  The result depends on the
+  graph, the features, the counts and `seed`, not on `chunk_rows` or `workspace_mb` (megabytes of
+  one expansion batch of the candidate and centroid rows, 0 = 2048).  With ``stream=True`` returns
+  an iterator of SampleColumns chunks of about `chunk_rows` rows, with ``keep_on_device=True`` a
+  DeviceSampleColumns (see BooleanSamplesDevice).  `timings` (a dict) receives the seconds spent
+  drawing pairs ("pairs") and neighbour arrays ("neighbours") and uploading the features and
+  computing the probabilities ("probabilities"); it is filled when the result is complete."""
+  import time
+  import torch
+  assert num_neighbors >= 0
+  assert num_samples >= 0
+  g = incidence if isinstance(incidence, _Graph) else _Graph.from_csr(incidence)
+  assert g.num_nodes == node2features.shape[0]     # hg2v_sample.py:430
+  assert g.num_edges == edge2features.shape[0]     # hg2v_sample.py:458
+  nf, ef = _native.FeatureCsr(node2features), _native.FeatureCsr(edge2features)
+  node_s = _per_row(node_weights, g.num_nodes, num_samples)
+  edge_s = _per_row(edge_weights, g.num_edges, num_samples)
+  assert node_s.min(initial=0) >= 0 and edge_s.min(initial=0) >= 0
+  k = num_neighbors
+
+  def blocks():
+    ctx = _native.default_context()
+    spent = {"probabilities": 0.0}
+
+    def prob(fn, *args, **kw):
+      t = time.perf_counter()
+      out = fn(*args, **kw)
+      ctx.sync()
+      spent["probabilities"] += time.perf_counter() - t
+      return out
+
+    dev = torch.device("cuda", ctx.device)
+    nfd, efd = prob(nf.to_device, dev), prob(ef.to_device, dev)
+    inc = g.incidence(ctx)
+    s = _DeviceSampler(g, ctx, inc, k, seed, chunk_rows, workspace_mb)
+    try:
+      for side, samples, phase, left, right, field, feat in (
+          (0, node_s, _native.PHASE_NN, "left_node", "right_node", "nn_prob", nfd),
+          (1, edge_s, _native.PHASE_EE, "left_edge", "right_edge", "ee_prob", efd)):
+        for r, c in s.pairs(side, 2, samples, phase):
+          p = prob(_native.jaccard_rows, ctx, feat, r, c)
+          yield _DeviceBlock(p.shape[0], field, p, **{left: r, right: c})
+      phases = (_native.PHASE_NE, _native.PHASE_EN, _native.PHASE_NEIGHBORS)
+      for nodes, edges, nbr_n, nbr_e in s.node_edge(node_s, edge_s, 3, phases):
+        # centroid of an edge = mean of its member nodes' feature rows, and vice versa
+        by_node = prob(_native.jaccard_centroid_grouped, ctx, inc, 1, nfd, nfd, nodes, edges, workspace_mb)
+        by_edge = prob(_native.jaccard_centroid_grouped, ctx, inc, 0, efd, efd, edges, nodes, workspace_mb)
+        yield _DeviceBlock(nodes.shape[0], "ne_prob", by_node * by_edge, left_weight=by_node,
+                           right_weight=by_edge, left_node=nodes, right_edge=edges, neigh_node=nbr_n,
+                           neigh_edge=nbr_e)
+    finally:
+      inc.close()
+    if timings is not None:
+      timings.update(s.spent)
+      timings.update(spent)
+
+  return _device_result(blocks(), k, stream, keep_on_device)
 
 
 ################################################################################

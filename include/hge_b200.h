@@ -274,6 +274,22 @@ int hge_jaccard_centroid(hge_ctx* ctx, const int64_t* xptr, const int32_t* xidx,
                          const float* fval, int64_t frows, int64_t fnnz, const int32_t* px,
                          const int32_t* pg, int64_t num_pairs, float* out, int mem);
 
+/* The same factor with the groups taken from the incidence's own CSR, for pairs held on the
+ * device: group_side 1 = groups are edges with their member nodes (edge -> node CSR, F = node
+ * features, frows = nodes), group_side 0 = groups are nodes with their edges (node -> edge CSR,
+ * F = edge features, frows = edges).  All pointers are device pointers.  The pairs are stably
+ * sorted by group; the centroid rows of the named groups are built once per call, in batches of
+ * consecutive named groups whose expansion fits workspace_mb megabytes (0 = 2048, 48 bytes per
+ * expanded entry), each batch freed after the merge of its pairs.  A single group larger than the
+ * budget is its own batch; one the device cannot hold is HGE_ERR_NOMEM.  Besides the budget the
+ * call holds at most 52 bytes per pair.  Bit-equal to hge_jaccard_centroid on the same inputs for
+ * every workspace_mb.  A pair index outside X or outside the groups is HGE_ERR_INVALID. */
+int hge_jaccard_centroid_grouped(hge_ctx* ctx, hge_incidence* inc, int group_side, const int64_t* xptr,
+                                 const int32_t* xidx, const float* xval, int64_t xrows, int64_t xnnz,
+                                 const int64_t* fptr, const int32_t* fidx, const float* fval, int64_t frows,
+                                 int64_t fnnz, const int32_t* px, const int32_t* pg, int64_t num_pairs,
+                                 int64_t workspace_mb, float* out);
+
 /* ---- candidate rows and bit-exact sampling (host code; all pointers are host pointers) ---
  * The reference draws every sample from numpy's process-global legacy MT19937, sequentially
  * and with data-dependent rejection, so this part of the path runs on the host; the drawn

@@ -135,6 +135,10 @@ SIGNATURES = {
     "hge_hg2v_get_samples": (ctypes.c_int, [c_vp, c_vp, c_vp, ctypes.c_int]),
     "hge_shuffle_order": (ctypes.c_int, [c_vp, ctypes.c_uint64, ctypes.c_uint32, ctypes.c_int64, c_vp,
                                          ctypes.c_int]),
+    "hge_lp_svm_predict": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int, c_vp, ctypes.c_int, c_vp, c_vp, ctypes.c_int64,
+                                          ctypes.c_uint64, ctypes.c_double, ctypes.c_double, ctypes.c_double,
+                                          ctypes.c_int64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
+                                          ctypes.c_int64, c_vp]),
     "hge_mt19937_random_raw": (ctypes.c_int, [c_vp, ctypes.c_int64, c_vp]),
     "hge_mt19937_interval": (ctypes.c_int, [c_vp, ctypes.c_uint32, ctypes.c_int64, c_vp]),
     "hge_spgemm_rows": (ctypes.c_int, [ctypes.c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
@@ -768,6 +772,7 @@ PHASE_NN, PHASE_EE, PHASE_NE, PHASE_EN, PHASE_NEIGHBORS = 1, 2, 3, 4, 5
 PHASE_NEG_NN, PHASE_NEG_EE, PHASE_NEG_EE_AGAIN, PHASE_NEG_NE, PHASE_NEG_EN = 6, 7, 8, 9, 10
 PHASE_NEG_NEIGHBORS = 11
 PHASE_SHUFFLE, PHASE_INIT_NODES, PHASE_INIT_EDGES = 12, 13, 14
+PHASE_LP_EDGE_OWNERS, PHASE_LP_NODE_OWNERS = 15, 16
 
 
 def sample_pairs_device(ctx, inc, side, factors, row0, samples, seed, phase, negative=False,
@@ -814,6 +819,55 @@ def shuffle_order(ctx, seed, epoch, n, out=None):
   assert out.dtype == torch.int32 and out.is_cuda and int(out.shape[0]) == int(n)
   check(ctx.lib.hge_shuffle_order(ctx.handle, int(seed) & 0xFFFFFFFFFFFFFFFF, int(epoch), int(n), ptr(out),
                                   MEM_DEVICE), "hge_shuffle_order")
+  return out
+
+
+class LpSvmModel(object):
+  """The classifiers of one hge_lp_svm_predict call, on the host: named owners in ascending id with
+  their rho, SMO iterations and first training point (offset, U + 1 entries), and per training point
+  its item id and alpha_i y_i.  capped = owners that hit the iteration cap."""
+
+  def __init__(self, owner_ids, rho, iterations, offset, point_ids, coef, capped):
+    self.owner_ids, self.rho, self.iterations, self.offset = owner_ids, rho, iterations, offset
+    self.point_ids, self.coef, self.capped = point_ids, coef, capped
+
+
+def lp_svm_predict(ctx, inc, owner_side, vectors, items, owners, seed, C=1.0, gamma=0.1, tol=1e-3,
+                   workspace_mb=0, return_model=False, timings=None):
+  """hge_lp_svm_predict on CUDA tensors: vectors fp32 [num items, d], items / owners int32 [L].
+  Returns (keep bool [L], decision fp64 [L], owners at the iteration cap) as CUDA tensors and an
+  int, plus an LpSvmModel when `return_model`.  `timings` (a dict) receives the seconds of the
+  grouping, negatives, solve and predict phases, each ended by a synchronise."""
+  import torch
+  dev = vectors.device
+  L = int(items.shape[0])
+  assert int(owners.shape[0]) == L and vectors.dim() == 2 and vectors.dtype == torch.float32
+  assert items.dtype == torch.int32 and owners.dtype == torch.int32
+  keep = torch.empty(max(L, 1), dtype=torch.uint8, device=dev)[:L]
+  decision = torch.empty(max(L, 1), dtype=torch.float64, device=dev)[:L]
+  counts = np.zeros(3, dtype=np.int64)
+  phase = np.zeros(4, dtype=np.float64) if timings is not None else None
+  model = [None] * 6
+  cap = 0
+  if return_model:
+    cap = 3 * max(inc.nnz_of(0), inc.nnz_of(1))   # an owner trains on at most 3 x its members
+    model = [torch.empty(max(L, 1), dtype=torch.int32, device=dev), torch.empty(max(L, 1), dtype=torch.float64, device=dev),
+             torch.empty(max(L, 1), dtype=torch.int64, device=dev), torch.empty(L + 1, dtype=torch.int64, device=dev),
+             torch.empty(max(cap, 1), dtype=torch.int32, device=dev), torch.empty(max(cap, 1), dtype=torch.float64, device=dev)]
+  vectors = vectors.contiguous()
+  check(ctx.lib.hge_lp_svm_predict(ctx.handle, inc.handle, int(owner_side), ptr(vectors), int(vectors.shape[1]),
+                                   ptr(items.contiguous()), ptr(owners.contiguous()), L,
+                                   int(seed) & 0xFFFFFFFFFFFFFFFF, float(C), float(gamma), float(tol),
+                                   int(workspace_mb), ptr(keep), ptr(decision), ptr(counts),
+                                   *[ptr(m) for m in model], cap, ptr(phase)), "hge_lp_svm_predict")
+  if timings is not None:
+    timings.update(zip(("grouping", "negatives", "solve", "predict"), (phase / 1e3).tolist()))
+  U, T, capped = (int(v) for v in counts)
+  out = (keep.bool(), decision, capped)
+  if return_model:
+    host = [m.cpu().numpy() for m in model]
+    out += (LpSvmModel(host[0][:U], host[1][:U], host[2][:U], host[3][:U + 1], host[4][:T], host[5][:T],
+                       capped),)
   return out
 
 

@@ -365,43 +365,6 @@ constexpr int64_t kDefaultWorkspaceMb = 2048;
 // (8), run heads and their scan (16), the centroid entry (8)
 constexpr int64_t kBytesPerEntry = 48;
 
-enum : int { kBadX = 1, kBadGroup = 2 };
-
-// sort input of the pairs: key = group, value = pair index; out-of-range ids are flagged
-__global__ void k_pair_keys(int64_t num_pairs, const int32_t* __restrict__ px, int64_t xrows,
-                            const int32_t* __restrict__ pg, int64_t groups, uint32_t* __restrict__ key,
-                            int32_t* __restrict__ idx, int* __restrict__ status) {
-  for (int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; p < num_pairs;
-       p += (int64_t)gridDim.x * blockDim.x) {
-    const int32_t x = px[p], g = pg[p];
-    if (x < 0 || x >= xrows) atomicOr(status, kBadX);
-    const bool bad_g = g < 0 || g >= groups;
-    if (bad_g) atomicOr(status, kBadGroup);
-    key[p] = bad_g ? 0u : (uint32_t)g;
-    idx[p] = (int32_t)p;
-  }
-}
-
-// head[i] = 1 where the run of pairs of one group starts (sorted group ids)
-__global__ void k_pair_heads(int64_t n, const uint32_t* __restrict__ sg, int32_t* __restrict__ head) {
-  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-    head[i] = (i == 0 || sg[i] != sg[i - 1]) ? 1 : 0;
-}
-
-// named group u = run u of the sorted pairs (u = rank[i] - 1, rank = inclusive scan of the heads):
-// ug[u] its group id, ustart[u] its first sorted pair; ustart[U] = n
-__global__ void k_named_groups(int64_t n, const uint32_t* __restrict__ sg, const int32_t* __restrict__ head,
-                               const int32_t* __restrict__ rank, int32_t* __restrict__ ug,
-                               int64_t* __restrict__ ustart) {
-  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-    if (head[i]) {
-      ug[rank[i] - 1] = (int32_t)sg[i];
-      ustart[rank[i] - 1] = i;
-    }
-    if (i == n - 1) ustart[rank[i]] = n;
-  }
-}
-
 // size[u] = sum over the members m of group ug[u] of nnz(F[m]); size[U] = 0 (one warp per group)
 __global__ void __launch_bounds__(kBlock) k_named_sizes(int64_t U, const int32_t* __restrict__ ug,
                                                         const int64_t* __restrict__ gptr,
@@ -575,57 +538,25 @@ int hge_jaccard_centroid_grouped(hge_ctx* ctx, hge_incidence* inc, int group_sid
   const int64_t n = num_pairs;
 
   // 1. pairs stably sorted by group
-  DevBuf<uint32_t> key(ctx), key2(ctx);
-  DevBuf<int32_t> idx(ctx), idx2(ctx), head(ctx), rank(ctx);
-  DevBuf<int> status(ctx);
-  DevBuf<char> temp(ctx);
-  HGE_TRY(key.alloc((size_t)n));
-  HGE_TRY(key2.alloc((size_t)n));
-  HGE_TRY(idx.alloc((size_t)n));
-  HGE_TRY(idx2.alloc((size_t)n));
-  HGE_TRY(status.alloc(1));
-  HGE_CUDA(cudaMemsetAsync(status.p, 0, sizeof(int), ctx->stream));
-  k_pair_keys<<<grid_for(ctx, n), kBlock, 0, ctx->stream>>>(n, px, xrows, pg, groups, key.p, idx.p, status.p);
-  HGE_CHECK_LAUNCH(ctx);
+  PairGroups pg_sorted(ctx);
   int bad = 0;
-  HGE_TRY(read_back(ctx, status.p, &bad, 1));
+  HGE_TRY(pg_sorted.build(ctx, n, px, xrows, pg, groups, &bad));
   HGE_REQUIRE(!(bad & kBadX), "hge_jaccard_centroid_grouped: a pair names a row outside X's %lld",
               (long long)xrows);
   HGE_REQUIRE(!(bad & kBadGroup), "hge_jaccard_centroid_grouped: a pair names a group outside [0, %lld)",
               (long long)groups);
-  int group_bits = 1;
-  while ((1ll << group_bits) < groups) ++group_bits;
-  cub::DoubleBuffer<uint32_t> dk(key.p, key2.p);
-  cub::DoubleBuffer<int32_t> dv(idx.p, idx2.p);
-  size_t bytes = 0;
-  HGE_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, bytes, dk, dv, n, 0, group_bits, ctx->stream));
-  HGE_TRY(temp.alloc(bytes));
-  HGE_CUDA(cub::DeviceRadixSort::SortPairs(temp.p, bytes, dk, dv, n, 0, group_bits, ctx->stream));
-  ctx->launches++;
-  const uint32_t* sg = dk.Current();
-  const int32_t* order = dv.Current();
+  const int32_t* order = pg_sorted.order;
+  const int64_t U = pg_sorted.U;
+  DevBuf<int32_t>& ug = pg_sorted.ug;
+  DevBuf<int32_t>& rank = pg_sorted.rank;
+  DevBuf<int64_t>& ustart = pg_sorted.ustart;
 
-  // 2. the named groups, their pair ranges and expansion sizes
-  HGE_TRY(head.alloc((size_t)n));
-  HGE_TRY(rank.alloc((size_t)n));
-  k_pair_heads<<<grid_for(ctx, n), kBlock, 0, ctx->stream>>>(n, sg, head.p);
-  HGE_CHECK_LAUNCH(ctx);
-  HGE_CUDA(cub::DeviceScan::InclusiveSum(nullptr, bytes, head.p, rank.p, n, ctx->stream));
-  HGE_TRY(temp.alloc(bytes));
-  HGE_CUDA(cub::DeviceScan::InclusiveSum(temp.p, bytes, head.p, rank.p, n, ctx->stream));
-  ctx->launches++;
-  int32_t U32 = 0;
-  HGE_TRY(read_back(ctx, rank.p + n - 1, &U32, 1));
-  const int64_t U = U32;
-  DevBuf<int32_t> ug(ctx);
-  DevBuf<int64_t> ustart(ctx), usize(ctx), uoff(ctx);
-  HGE_TRY(ug.alloc((size_t)U));
-  HGE_TRY(ustart.alloc((size_t)U + 1));
+  // 2. the named groups' expansion sizes
+  DevBuf<int64_t> usize(ctx), uoff(ctx);
+  DevBuf<char> temp(ctx);
+  size_t bytes = 0;
   HGE_TRY(usize.alloc((size_t)U + 1));
   HGE_TRY(uoff.alloc((size_t)U + 1));
-  k_named_groups<<<grid_for(ctx, n), kBlock, 0, ctx->stream>>>(n, sg, head.p, rank.p, ug.p, ustart.p);
-  HGE_CHECK_LAUNCH(ctx);
-  hge_dev_free(ctx, head.p);
   k_named_sizes<<<grid_for(ctx, U + 1, kBlock / 32), kBlock, 0, ctx->stream>>>(U, ug.p, gptr, gidx, fptr, usize.p);
   HGE_CHECK_LAUNCH(ctx);
   HGE_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, bytes, usize.p, uoff.p, U + 1, ctx->stream));

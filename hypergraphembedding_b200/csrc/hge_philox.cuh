@@ -1,7 +1,8 @@
 // Philox4x32-10 (Salmon et al., "Parallel random numbers: as easy as 1, 2, 3", SC'11) and the
 // word-stream layout of the device sampler (csrc/hge_device_sampler.cu).  oracle/
 // device_sampler_ref.py restates everything in this file in numpy; oracle/seeded_training_ref.py
-// restates the training phases (epoch order, initial tables).
+// restates the training phases (epoch order, initial tables), oracle/lp_svm_ref.py the negatives of
+// the link-prediction classifiers.
 //
 // Layout.  Every item owns one stream of 32-bit words:
 //   key     = { (uint32)seed, (uint32)(seed >> 32) }
@@ -40,6 +41,10 @@ enum HgePhase : uint32_t {
   // initial embedding tables: item = row, word c is column c
   HGE_PHASE_INIT_NODES = 13,
   HGE_PHASE_INIT_EDGES = 14,
+  // negatives of the personalized link-prediction classifiers (csrc/hge_lp_svm.cu): item = owner
+  // row, Floyd's selection over the owner's non-members
+  HGE_PHASE_LP_EDGE_OWNERS = 15,
+  HGE_PHASE_LP_NODE_OWNERS = 16,
 };
 
 #ifdef __CUDACC__

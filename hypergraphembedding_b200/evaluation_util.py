@@ -17,6 +17,8 @@ embeddings and out of scope (SURVEY.md section 2 row 11); ``EXPERIMENT_OPTIONS``
 caller fills with ``RegisterExperiment`` -- ``RunLinkPredictionExperiment`` looks the predictor up
 in it exactly as the reference does.  The per-edge / per-node SVC predictors are provided on top
 of scikit-learn (imported on first use) because they need nothing else; the Keras one raises.
+Their GPU forms (``Personalized*ClassifierPredictionDevice``, csrc/hge_lp_svm.cu) train the same
+classifiers with seeded negatives and are not registered.
 """
 import logging
 import random
@@ -24,6 +26,7 @@ from collections import namedtuple
 
 import numpy as np
 
+from . import _native
 from .hypergraph_pb2 import EvaluationMetrics, ExperimentalResult, Hypergraph
 
 log = logging.getLogger()
@@ -199,6 +202,95 @@ def PersonalizedEdgeClassifierPrediction(hypergraph, embedding, links, run_in_pa
 
 def PersonalizedNodeClassifierPrediction(hypergraph, embedding, links, run_in_parallel=False):
   return _personalized_classifier_prediction(hypergraph, embedding, links, per_edge=False)
+
+
+def PersonalizedClassifierPredictionDevice(incidence, item_vectors, links, per_edge, seed=0, C=1.0, gamma=0.1,
+                                          tol=1e-3, workspace_mb=0, return_model=False):
+  """The personalized classifiers on the GPU (csrc/hge_lp_svm.cu) over dense row ids.  `incidence`
+  is an N x E incidence CSR (or an hg2v_sample._Graph), `item_vectors` fp32 [N, d] node vectors
+  (`per_edge`: one classifier per edge over its nodes) or [E, d] edge vectors (one per node over its
+  edges), `links` an [L, 2] array of (node, edge) rows.  Each owner named by a link trains an RBF
+  SVC (C, gamma, tol as libsvm) on its members against min(non-members, 2 x members) non-members
+  drawn from the owner's own Philox stream of `seed`; the draw and the result depend only on
+  (seed, side, owner, graph), never on the links' order or `workspace_mb` (megabytes of solver
+  workspace per batch of large owners, 0 = 2048).  Returns the boolean keep mask of the links (a
+  numpy array), and with ``return_model`` also the _native.LpSvmModel.  Python's ``random`` and
+  numpy's global RNG are neither read nor advanced; owners that hit libsvm's iteration cap are
+  logged as a warning, as libsvm warns."""
+  import torch
+  from .hg2v_sample import _Graph
+  g = incidence if isinstance(incidence, _Graph) else _Graph.from_csr(incidence)
+  links = np.asarray(links, dtype=np.int64).reshape(-1, 2)
+  items, owners = (links[:, 0], links[:, 1]) if per_edge else (links[:, 1], links[:, 0])
+  ctx = _native.default_context()
+  dev = torch.device("cuda", ctx.device)
+  if torch.is_tensor(item_vectors):
+    vectors = item_vectors.to(dev, torch.float32).contiguous()
+  else:
+    vectors = torch.as_tensor(np.ascontiguousarray(item_vectors, dtype=np.float32)).to(dev)
+  assert vectors.dim() == 2 and vectors.shape[0] == (g.num_nodes if per_edge else g.num_edges)
+  as_i32 = lambda a: torch.as_tensor(np.asarray(a).astype(np.int32)).to(dev)
+  inc = g.incidence(ctx)
+  try:
+    out = _native.lp_svm_predict(ctx, inc, 1 if per_edge else 0, vectors, as_i32(items), as_i32(owners), seed,
+                                 C, gamma, tol, workspace_mb, return_model)
+  finally:
+    inc.close()
+  if out[2]:
+    log.warning("%d personalized classifiers reached the maximum number of iterations", out[2])
+  keep = out[0].cpu().numpy()
+  return (keep, out[3]) if return_model else keep
+
+
+def _personalized_classifier_prediction_device(hypergraph, embedding, links, per_edge, seed, **kw):
+  """The host form's semantics on PersonalizedClassifierPredictionDevice: the asked links are those
+  whose node and edge both have vectors, item rows are the embedding's sorted ids, an owner absent
+  from the hypergraph has no members, a member without a vector is a KeyError; the kept links come
+  back in the asked order."""
+  from .hypergraph_util import embedding_from_wire
+  ids_n, ptr_n, val_n, ids_e, ptr_e, val_e, _ = embedding_from_wire(embedding)
+  table = []
+  for ids, ptr, val in ((ids_n, ptr_n, val_n), (ids_e, ptr_e, val_e)):
+    order = np.argsort(ids, kind="stable")
+    width = int(ptr[1] - ptr[0]) if len(ids) else 0
+    assert width > 0 and np.all(np.diff(ptr) == width), "embedding rows must all have the same length"
+    table.append((ids[order].astype(np.int64), val.reshape(-1, width)[order]))
+  (node_ids, xn), (edge_ids, xe) = table
+  pairs = np.asarray(_pairs(links), dtype=np.int64).reshape(-1, 2)
+  asked = pairs[np.isin(pairs[:, 0], node_ids) & np.isin(pairs[:, 1], edge_ids)]
+  rows = np.stack([np.searchsorted(node_ids, asked[:, 0]), np.searchsorted(edge_ids, asked[:, 1])], axis=1)
+  owner_ids, member_ids, owner_map = (edge_ids, node_ids, hypergraph.edge) if per_edge else (
+      node_ids, edge_ids, hypergraph.node)
+  member_rows = {int(i): r for r, i in enumerate(member_ids.tolist())}
+  inc = []   # (node row, edge row) of every named owner's members
+  for r in np.unique(rows[:, 1 if per_edge else 0]).tolist():
+    owner = int(owner_ids[r])
+    if owner not in owner_map:
+      continue
+    members = set(owner_map[owner].nodes if per_edge else owner_map[owner].edges)
+    for m in members:
+      inc.append((member_rows[m], r) if per_edge else (r, member_rows[m]))   # KeyError: no vector
+  import scipy.sparse as sps
+  inc = np.asarray(inc, dtype=np.int64).reshape(-1, 2)
+  A = sps.csr_matrix((np.ones(len(inc), dtype=np.int8), (inc[:, 0], inc[:, 1])),
+                     shape=(len(node_ids), len(edge_ids)))
+  A.sum_duplicates()
+  A.sort_indices()
+  keep = PersonalizedClassifierPredictionDevice(A, xn if per_edge else xe, rows, per_edge, seed=seed, **kw)
+  return [(int(n), int(e)) for n, e in asked[keep]]
+
+
+def PersonalizedEdgeClassifierPredictionDevice(hypergraph, embedding, links, seed=0, **kw):
+  """LP_EDGE_CLASSIFIERS with the classifiers trained on the GPU from `seed` (not registered in
+  EXPERIMENT_OPTIONS: add it with RegisterExperiment(name, functools.partial(fn, seed=s))).  `kw`:
+  C, gamma, tol, workspace_mb of PersonalizedClassifierPredictionDevice."""
+  return _personalized_classifier_prediction_device(hypergraph, embedding, links, True, seed, **kw)
+
+
+def PersonalizedNodeClassifierPredictionDevice(hypergraph, embedding, links, seed=0, **kw):
+  """LP_NODE_CLASSIFIERS with the classifiers trained on the GPU from `seed` (see
+  PersonalizedEdgeClassifierPredictionDevice)."""
+  return _personalized_classifier_prediction_device(hypergraph, embedding, links, False, seed, **kw)
 
 
 def NodeEdgeEmbeddingPrediction(hypergraph, embedding, potential_links, classifier=None,

@@ -431,6 +431,39 @@ int hge_hg2v_get_samples(hge_hg2v_model* m, int32_t* features, float* targets, i
  * index.  The result is hge_hg2v_fit_epoch's order. */
 int hge_shuffle_order(hge_ctx* ctx, uint64_t seed, uint32_t epoch, int64_t n, int32_t* order, int mem);
 
+/* Personalized link-prediction classifiers (csrc/hge_lp_svm.cu): one RBF C-SVC per owner named by
+ * a link (item, owner), as LP_EDGE_CLASSIFIERS / LP_NODE_CLASSIFIERS train them.  owner_side 1:
+ * owners are edges, their members their nodes (edge -> node CSR), items the nodes; owner_side 0:
+ * owners are nodes, members their edges, items the edges.  item_vectors: fp32 [items, d], d >= 1.
+ * An owner with M members among N items trains on M (label +1, ascending) and k = min(N - M, 2M)
+ * distinct non-members (label -1, ascending) chosen uniformly by Floyd's algorithm over the
+ * positions of its ascending non-member list, from the Philox stream (csrc/hge_philox.cuh) of item =
+ * owner row, phase HGE_PHASE_LP_EDGE_OWNERS (15) / HGE_PHASE_LP_NODE_OWNERS (16); k = N - M takes
+ * them all and draws nothing.  The dual is libsvm's (Solver, WSS3, no shrinking) with K(x, z) =
+ * exp(-gamma ||x - z||^2) in fp32, gradient and alpha in fp64, stop at tol, at most
+ * max(10^7, 100 n) iterations.  out_keep[l] = 1 iff sum_i alpha_i y_i K(x_i, x_item) - rho > 0
+ * (out_decision, optional, receives that value).  An owner without members rejects its links
+ * (rho = +inf), one whose members are every item keeps them (rho = -inf); neither has points.
+ * Owners of more than 32 points are solved in batches whose workspace fits workspace_mb megabytes
+ * (0 = 2048; 24 + 4 d bytes a point); a single larger owner is its own batch, one the device cannot
+ * hold is HGE_ERR_NOMEM.  Besides that the call holds 16 bytes a training point and 24 a
+ * link.  Everything is bit-identical for every workspace_mb and from run to run.
+ * All array pointers are device pointers except out_counts and phase_ms (host, optional):
+ *   out_counts[3] = { named owners U, training points T, owners that hit the iteration cap };
+ *   phase_ms[4]   = milliseconds of grouping, negatives, solve and predict, each ended by a
+ *                   stream synchronise (only when phase_ms is given).
+ * Optional model outputs, named owners in ascending owner id: owner_ids [U], owner_rho [U],
+ * owner_iters [U], owner_offset [U + 1] (first training point of each owner); point_ids [T] and
+ * point_coef [T] (alpha_i y_i) in training order, T <= point_capacity (U <= num_links).  A link
+ * naming an item or owner out of range, or a bad owner_side, is HGE_ERR_INVALID and nothing is
+ * written. */
+int hge_lp_svm_predict(hge_ctx* ctx, hge_incidence* inc, int owner_side, const float* item_vectors, int d,
+                       const int32_t* link_items, const int32_t* link_owners, int64_t num_links, uint64_t seed,
+                       double C, double gamma, double tol, int64_t workspace_mb, uint8_t* out_keep,
+                       double* out_decision, int64_t* out_counts, int32_t* owner_ids, double* owner_rho,
+                       int64_t* owner_iters, int64_t* owner_offset, int32_t* point_ids, double* point_coef,
+                       int64_t point_capacity, double* phase_ms);
+
 /* ---- hypergraph.proto wire format (host code; all pointers are host pointers) --------------
  * The data formats either side of the path: a serialized Hypergraph (hypergraph.proto:6-23) is
  * read straight into arrays, replacing the per-incidence Python loops of ToCsrMatrix /

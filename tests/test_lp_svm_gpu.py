@@ -1,9 +1,12 @@
 """hge_lp_svm_predict and the device personalized classifiers: negatives bit-equal to their numpy
-restatement (oracle/lp_svm_ref.py) on both sides, decision values against scikit-learn fitted on
-the exported training sets, the KKT gap of the exported model, every owner size class and the
-degenerate owners in one call, bit-identical output for every workspace budget and run, the
-refusals, the untouched global RNGs, the proto-level wrappers against the host predictors, and a
-100 000-node run."""
+restatement (oracle/lp_svm_ref.py) on both sides; the exported model (coef, rho) against
+scikit-learn fitted on the exported training sets, through its KKT gap and through decision values
+recomputed from it on the host (ref.decision), with the keep mask's sign checked where
+scikit-learn's value is clear of zero; every owner size class and the degenerate owners in one
+call, bit-identical output for every workspace budget and run, the refusals, the untouched global
+RNGs, the proto-level wrappers against the host predictors, and a 100 000-node run.  The device's
+own coef, rho, iterations and decision values are pinned bit for bit to the restatement in
+tests/test_lp_svm_exact_gpu.py."""
 import functools
 import random
 

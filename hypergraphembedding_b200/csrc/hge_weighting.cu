@@ -357,6 +357,52 @@ __global__ void __launch_bounds__(kBlock) k_diff_type_prob(
   }
 }
 
+// ---- pair index range checks ------------------------------------------------------------------
+// The kernels above trust their pair indices: k_same_type_prob and k_diff_type_prob read row
+// pointers at them, k_pair_l2 skips a negative one and leaves its output unwritten.  The entry
+// points therefore check every index before any of those kernels runs.
+__global__ void k_check_pairs(int64_t n, const int32_t* __restrict__ a, int64_t rows_a,
+                              const int32_t* __restrict__ b, int64_t rows_b, int* __restrict__ bad) {
+  for (int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; p < n;
+       p += (int64_t)gridDim.x * blockDim.x) {
+    const int32_t x = __ldcs(a + p), y = __ldcs(b + p);
+    if (x < 0 || x >= rows_a || y < 0 || y >= rows_b) *bad = 1;
+  }
+}
+
+// *ok = every a[p] in [0, rows_a) and every b[p] in [0, rows_b).  Host arrays are scanned on the
+// host; device arrays by k_check_pairs, then one flag read-back.
+int pairs_in_range(hge_ctx* ctx, int64_t n, const int32_t* a, int64_t rows_a, const int32_t* b,
+                   int64_t rows_b, int mem, bool* ok) {
+  if (mem != HGE_MEM_DEVICE) {
+    bool all = true;
+    for (int64_t p = 0; p < n; ++p)
+      all &= a[p] >= 0 && a[p] < rows_a && b[p] >= 0 && b[p] < rows_b;
+    *ok = all;
+    return HGE_OK;
+  }
+  int* d_bad = nullptr;
+  HGE_TRY(hge_dev_alloc(ctx, &d_bad, 1));
+  int h_bad = 0;
+  cudaError_t e = cudaMemsetAsync(d_bad, 0, sizeof(int), ctx->stream);
+  if (e == cudaSuccess) {
+    k_check_pairs<<<grid_for(ctx, n, kBlock * 8), kBlock, 0, ctx->stream>>>(n, a, rows_a, b, rows_b,
+                                                                          d_bad);
+    ctx->launches++;
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess)
+    e = cudaMemcpyAsync(&h_bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);   // h_bad is on this stack frame
+  hge_dev_free(ctx, d_bad);
+  if (e != cudaSuccess) {
+    hge_set_error("pair index check: %s", cudaGetErrorString(e));
+    return HGE_ERR_CUDA;
+  }
+  *ok = h_bad == 0;
+  return HGE_OK;
+}
+
 // rows -> segments of at most kSegment incidences, on the device: per row ceil(deg / kSegment)
 // segments, an exclusive prefix sum for their positions (cub; set-up), one thread per row writes
 // them.  (A host loop over the row pointers did this before: two passes over 1.5 M rows, a 24 MB
@@ -475,6 +521,10 @@ int hge_pair_l2(hge_ctx* ctx, const float* xa, int64_t rows_a, const float* xb, 
   HGE_REQUIRE(R >= 1 && R <= 1024, "hge_pair_l2: dimension %d not in [1, 1024]", R);
   if (num_pairs == 0) return HGE_OK;
   HGE_CUDA(cudaSetDevice(ctx->device));
+  bool ok = false;
+  HGE_TRY(pairs_in_range(ctx, num_pairs, ia, rows_a, ib, rows_b, mem, &ok));
+  HGE_REQUIRE(ok, "hge_pair_l2: a pair names a row outside [0, %lld) x [0, %lld)", (long long)rows_a,
+              (long long)rows_b);
   Staged<float> s_xa, s_xb, s_out;
   Staged<int32_t> s_ia, s_ib;
   HGE_TRY(s_xa.init(ctx, xa, (size_t)rows_a * R, mem, true, false));
@@ -639,6 +689,9 @@ int hge_same_type_prob(hge_ctx* ctx, hge_incidence* inc, int side, const float* 
   if (num_pairs == 0) return HGE_OK;
   HGE_CUDA(cudaSetDevice(ctx->device));
   const HgeHalfSchedule& half = side == 0 ? inc->node_half : inc->edge_half;
+  bool ok = false;
+  HGE_TRY(pairs_in_range(ctx, num_pairs, pi, half.rows, pj, half.rows, mem, &ok));
+  HGE_REQUIRE(ok, "hge_same_type_prob: a pair names a row outside [0, %d)", half.rows);
   Staged<float> s_w, s_out;
   Staged<int32_t> s_i, s_j;
   HGE_TRY(s_w.init(ctx, w, (size_t)half.nnz, mem, true, false));
@@ -665,6 +718,10 @@ int hge_diff_type_prob(hge_ctx* ctx, hge_incidence* inc, const float* w_e2n, con
   HGE_REQUIRE(num_pairs >= 0 && (num_pairs == 0 || (pn && pe)), "hge_diff_type_prob: bad pairs");
   if (num_pairs == 0) return HGE_OK;
   HGE_CUDA(cudaSetDevice(ctx->device));
+  bool ok = false;
+  HGE_TRY(pairs_in_range(ctx, num_pairs, pn, inc->N, pe, inc->E, mem, &ok));
+  HGE_REQUIRE(ok, "hge_diff_type_prob: a pair names a node outside [0, %d) or an edge outside [0, %d)",
+              inc->N, inc->E);
   Staged<float> s_w, s_out;
   Staged<int32_t> s_n, s_e;
   HGE_TRY(s_w.init(ctx, w_e2n, (size_t)inc->edge_half.nnz, mem, true, false));

@@ -210,7 +210,8 @@ int hge_incidence_l2(hge_ctx* ctx, hge_incidence* inc, const float* xn, const fl
 
 /* dist[p] = || xa[ia[p]] - xb[ib[p]] ||_2 for arbitrary (node,node), (node,edge) or
  * (edge,edge) sample pairs: the distance part of WeightBySameTypeDistance
- * (hg2v_weighting.py:37-45) and of the 100M-pair weighting of BASELINE.json configs[2]. */
+ * (hg2v_weighting.py:37-45) and of the 100M-pair weighting of BASELINE.json configs[2].
+ * An index outside [0, rows_a) / [0, rows_b) is HGE_ERR_INVALID; nothing is computed then. */
 int hge_pair_l2(hge_ctx* ctx, const float* xa, int64_t rows_a, const float* xb, int64_t rows_b,
                 int R, const int32_t* ia, const int32_t* ib, int64_t num_pairs, float* dist,
                 int mem);
@@ -240,14 +241,16 @@ int hge_row_span(hge_ctx* ctx, hge_incidence* inc, const float* xn, const float*
 /* HOBE same-type probability (hg2v_sample.py:527-543) for num_pairs pairs (i, j) of rows of
  * the node->edge CSR (side == 0) or of the edge->node CSR (side == 1):
  *     prob = max over shared columns k of min(w(i,k), w(j,k)),  0 without a shared column,
- * with w the incidence weights in that CSR's storage order (hge_incidence_l2, as_weight). */
+ * with w the incidence weights in that CSR's storage order (hge_incidence_l2, as_weight).  An index
+ * outside the side's rows is HGE_ERR_INVALID; nothing is computed then. */
 int hge_same_type_prob(hge_ctx* ctx, hge_incidence* inc, int side, const float* w,
                        const int32_t* pi, const int32_t* pj, int64_t num_pairs, float* prob,
                        int mem);
 
 /* HOBE node-edge probability (hg2v_sample.py:606-629) for pairs (node n, edge e):
  *     prob = max(0, max over the node's edges e' of same_type_prob_edges(e, e')),
- * w_e2n = incidence weights in edge->node storage order. */
+ * w_e2n = incidence weights in edge->node storage order.  A node outside [0, N) or an edge outside
+ * [0, E) is HGE_ERR_INVALID; nothing is computed then. */
 int hge_diff_type_prob(hge_ctx* ctx, hge_incidence* inc, const float* w_e2n, const int32_t* pn,
                        const int32_t* pe, int64_t num_pairs, float* prob, int mem);
 

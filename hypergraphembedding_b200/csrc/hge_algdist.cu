@@ -308,62 +308,54 @@ __global__ void k_edge_finalize(int64_t row0, int64_t rows, int R, int ld,
 // host side: schedule construction
 // ----------------------------------------------------------------------------------------
 
-int grid_1d(const hge_ctx* ctx, int64_t work, int block) {
-  int64_t want = (work + block - 1) / block;
-  int64_t cap = (int64_t)ctx->num_sms * 32;
-  if (want < 1) want = 1;
-  return (int)std::min(want, cap);
-}
+constexpr int kBlocksPerSm = 32;   // grid cap of the kernels of this file, per multiprocessor
 
 // wsum[r] = sum over the row's neighbours b of 1 / other_deg[b] (f64, device).
 // Transposes a CSR whose column ids are sorted inside every row: a stable sort of the
 // (column, row) pairs by column keeps the rows of a column in ascending order.
 int transpose_csr(hge_ctx* ctx, int32_t rows, int32_t cols, int64_t nnz, const int64_t* d_ptr,
                   const int32_t* d_idx, int64_t* t_ptr, int32_t* t_idx) {
-  int32_t *row_of = nullptr, *cols_sorted = nullptr;
-  HGE_TRY(hge_dev_alloc(ctx, &row_of, (size_t)nnz));
-  HGE_TRY(hge_dev_alloc(ctx, &cols_sorted, (size_t)nnz));
-  k_expand_rows<<<grid_1d(ctx, (int64_t)rows * 8, kBlock), kBlock, 0, ctx->stream>>>(rows, d_ptr, row_of);
+  DevBuf<int32_t> row_of(ctx), cols_sorted(ctx);
+  DevBuf<char> temp(ctx);
+  HGE_TRY(row_of.alloc((size_t)nnz));
+  HGE_TRY(cols_sorted.alloc((size_t)nnz));
+  k_expand_rows<<<grid_for(ctx, (int64_t)rows * 8, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(rows, d_ptr,
+                                                                                                 row_of.p);
   HGE_CHECK_LAUNCH(ctx);
   int bits = 1;
   while (bits < 31 && ((int64_t)1 << bits) < cols) ++bits;
   size_t temp_bytes = 0;
-  HGE_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, d_idx, cols_sorted, row_of, t_idx, nnz, 0, bits,
-                                           ctx->stream));
-  char* temp = nullptr;
-  HGE_TRY(hge_dev_alloc(ctx, &temp, temp_bytes));
-  HGE_CUDA(cub::DeviceRadixSort::SortPairs(temp, temp_bytes, d_idx, cols_sorted, row_of, t_idx, nnz, 0, bits,
-                                           ctx->stream));
+  HGE_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, d_idx, cols_sorted.p, row_of.p, t_idx, nnz, 0,
+                                           bits, ctx->stream));
+  HGE_TRY(temp.alloc(temp_bytes));
+  HGE_CUDA(cub::DeviceRadixSort::SortPairs(temp.p, temp_bytes, d_idx, cols_sorted.p, row_of.p, t_idx, nnz, 0,
+                                           bits, ctx->stream));
   ctx->launches += 3;
-  k_transpose_ptr<<<grid_1d(ctx, (int64_t)cols + 1, kBlock), kBlock, 0, ctx->stream>>>(cols, nnz, cols_sorted,
-                                                                                      t_ptr);
+  k_transpose_ptr<<<grid_for(ctx, (int64_t)cols + 1, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(
+      cols, nnz, cols_sorted.p, t_ptr);
   HGE_CHECK_LAUNCH(ctx);
-  hge_dev_free(ctx, temp);
-  hge_dev_free(ctx, row_of);
-  hge_dev_free(ctx, cols_sorted);
   return HGE_OK;
 }
 
 int compute_wsum(hge_ctx* ctx, int32_t rows, const int64_t* d_ptr, const int32_t* d_idx,
-                 const int32_t* d_other_deg, double** wsum) {
-  HGE_TRY(hge_dev_alloc(ctx, wsum, (size_t)rows));
-  int32_t* long_rows = nullptr;   // [0] = count, [1..] = row ids
-  HGE_TRY(hge_dev_alloc(ctx, &long_rows, (size_t)rows + 1));
-  HGE_CUDA(cudaMemsetAsync(long_rows, 0, sizeof(int32_t), ctx->stream));
-  k_row_wsum<<<grid_1d(ctx, (int64_t)rows * 8, kBlock), kBlock, 0, ctx->stream>>>(
-      rows, d_ptr, d_idx, d_other_deg, *wsum, long_rows + 1, long_rows);
+                 const int32_t* d_other_deg, DevBuf<double>& wsum) {
+  HGE_TRY(wsum.alloc((size_t)rows));
+  DevBuf<int32_t> long_rows(ctx);   // [0] = count, [1..] = row ids
+  HGE_TRY(long_rows.alloc((size_t)rows + 1));
+  HGE_CUDA(cudaMemsetAsync(long_rows.p, 0, sizeof(int32_t), ctx->stream));
+  k_row_wsum<<<grid_for(ctx, (int64_t)rows * 8, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(
+      rows, d_ptr, d_idx, d_other_deg, wsum.p, long_rows.p + 1, long_rows.p);
   HGE_CHECK_LAUNCH(ctx);
-  k_row_wsum_long<<<ctx->num_sms * 4, kBlock, 0, ctx->stream>>>(long_rows + 1, long_rows, d_ptr, d_idx,
-                                                               d_other_deg, *wsum);
+  k_row_wsum_long<<<ctx->num_sms * 4, kBlock, 0, ctx->stream>>>(long_rows.p + 1, long_rows.p, d_ptr, d_idx,
+                                                               d_other_deg, wsum.p);
   HGE_CHECK_LAUNCH(ctx);
-  hge_dev_free(ctx, long_rows);
   return HGE_OK;
 }
 
 // invs = 1 / wsum as fp32 (device).
 int invert_wsum(hge_ctx* ctx, int32_t rows, const double* wsum, float** invs) {
   HGE_TRY(hge_dev_alloc(ctx, invs, (size_t)rows));
-  k_invert<<<grid_1d(ctx, rows, kBlock), kBlock, 0, ctx->stream>>>(rows, wsum, *invs);
+  k_invert<<<grid_for(ctx, rows, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(rows, wsum, *invs);
   HGE_CHECK_LAUNCH(ctx);
   return HGE_OK;
 }
@@ -535,9 +527,7 @@ static int incidence_create_impl(hge_ctx* ctx, int32_t num_nodes, int32_t num_ed
     inc->n2e_idx = const_cast<int32_t*>(n2e_idx);
     if (build_e2n) {
       // only the last row pointer is needed on the host: the number of incidences
-      e = cudaMemcpyAsync(&nnz_a, n2e_ptr + num_nodes, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-      if (e != cudaSuccess) return cuda_fail(e, "reading the incidence count");
+      if ((rc = read_back(ctx, n2e_ptr + num_nodes, &nnz_a, 1)) != HGE_OK) return fail(rc);
       inc->owns_e2n = true;
       if ((rc = hge_dev_alloc(ctx, &inc->e2n_ptr, (size_t)num_edges + 1)) != HGE_OK) return fail(rc);
       if ((rc = hge_dev_alloc(ctx, &inc->e2n_idx, (size_t)nnz_a)) != HGE_OK) return fail(rc);
@@ -563,11 +553,11 @@ static int incidence_create_impl(hge_ctx* ctx, int32_t num_nodes, int32_t num_ed
   inc->num_slices = num_slices;
   if ((rc = hge_dev_alloc(ctx, &nh.deg, (size_t)num_nodes)) != HGE_OK) return fail(rc);
   if ((rc = hge_dev_alloc(ctx, &eh.deg, (size_t)num_edges)) != HGE_OK) return fail(rc);
-  k_row_degree<<<grid_1d(ctx, num_nodes, kBlock), kBlock, 0, ctx->stream>>>(num_nodes, inc->n2e_ptr,
-                                                                          nh.deg);
+  k_row_degree<<<grid_for(ctx, num_nodes, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(
+      num_nodes, inc->n2e_ptr, nh.deg);
   ctx->launches++;
-  k_row_degree<<<grid_1d(ctx, num_edges, kBlock), kBlock, 0, ctx->stream>>>(num_edges, inc->e2n_ptr,
-                                                                          eh.deg);
+  k_row_degree<<<grid_for(ctx, num_edges, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(
+      num_edges, inc->e2n_ptr, eh.deg);
   ctx->launches++;
   if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "degree kernel launch");
 
@@ -596,8 +586,10 @@ static int incidence_create_impl(hge_ctx* ctx, int32_t num_nodes, int32_t num_ed
     if (e != cudaSuccess) return cuda_fail(e, "column-id upload");
   }
   // edge weight sums: sum over (local) members n of 1 / deg(n); node degrees are complete
-  rc = compute_wsum(ctx, num_edges, inc->e2n_ptr, inc->e2n_idx, nh.deg, &inc->edge_wsum);
+  DevBuf<double> edge_wsum(ctx);
+  rc = compute_wsum(ctx, num_edges, inc->e2n_ptr, inc->e2n_idx, nh.deg, edge_wsum);
   if (rc != HGE_OK) return fail(rc);
+  inc->edge_wsum = edge_wsum.release();
   if (!sharded && !defer_finish) {
     rc = incidence_finish(inc);
     if (rc != HGE_OK) return fail(rc);
@@ -612,11 +604,10 @@ static int incidence_finish(hge_incidence* inc) {
   hge_ctx* ctx = inc->ctx;
   HgeHalfSchedule& nh = inc->node_half;
   HgeHalfSchedule& eh = inc->edge_half;
-  double* node_wsum = nullptr;
-  HGE_TRY(compute_wsum(ctx, inc->N, inc->n2e_ptr, inc->n2e_idx, eh.deg, &node_wsum));
-  int rc = invert_wsum(ctx, inc->N, node_wsum, &nh.invs);
-  hge_dev_free(ctx, node_wsum);
-  if (rc != HGE_OK) return rc;
+  DevBuf<double> node_wsum(ctx);
+  HGE_TRY(compute_wsum(ctx, inc->N, inc->n2e_ptr, inc->n2e_idx, eh.deg, node_wsum));
+  HGE_TRY(invert_wsum(ctx, inc->N, node_wsum.p, &nh.invs));
+  node_wsum.reset();
   HGE_TRY(invert_wsum(ctx, inc->E, inc->edge_wsum, &eh.invs));
   HGE_TRY(hge_sched_finish(ctx, "node", &nh));
   HGE_TRY(hge_sched_finish(ctx, "edge", &eh));
@@ -711,7 +702,7 @@ static int ensure_edge_tiles(hge_ctx* ctx, hge_incidence* inc, int32_t tile_rows
   if (tiles <= 1) return HGE_OK;
   const HgeHalfSchedule& eh = inc->edge_half;
   HGE_TRY(hge_dev_alloc(ctx, &inc->tile_pos, (size_t)(tiles + 1) * inc->E));
-  k_tile_offsets<<<grid_1d(ctx, (int64_t)inc->E * (tiles + 1), kBlock), kBlock, 0, ctx->stream>>>(
+  k_tile_offsets<<<grid_for(ctx, (int64_t)inc->E * (tiles + 1), kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(
       inc->E, inc->e2n_ptr, inc->e2n_idx, tiles, tile_rows, inc->tile_pos);
   HGE_CHECK_LAUNCH(ctx);
   // Tiling adds work per non-empty (edge, tile) pair (a work item, a read-modify-write of the
@@ -720,18 +711,18 @@ static int ensure_edge_tiles(hge_ctx* ctx, hge_incidence* inc, int32_t tile_rows
   // 0.24 -> 0.45 ms).  Below kMinPerPair incidences per pair the half-sweep stays untiled.
   {
     constexpr double kMinPerPair = 16.0;
-    unsigned long long* d_pairs = nullptr;
-    HGE_TRY(hge_dev_alloc(ctx, &d_pairs, 1));
-    HGE_CUDA(cudaMemsetAsync(d_pairs, 0, sizeof(unsigned long long), ctx->stream));
-    k_count_tile_pairs<<<grid_1d(ctx, (int64_t)inc->E * tiles, kBlock), kBlock, 0, ctx->stream>>>(
-        (int64_t)inc->E * tiles, inc->E, inc->tile_pos, d_pairs);
+    DevBuf<unsigned long long> d_pairs(ctx);
+    HGE_TRY(d_pairs.alloc(1));
+    HGE_CUDA(cudaMemsetAsync(d_pairs.p, 0, sizeof(unsigned long long), ctx->stream));
+    k_count_tile_pairs<<<grid_for(ctx, (int64_t)inc->E * tiles, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(
+        (int64_t)inc->E * tiles, inc->E, inc->tile_pos, d_pairs.p);
     HGE_CHECK_LAUNCH(ctx);
     unsigned long long* h_pairs = static_cast<unsigned long long*>(hge_ctx_pinned_slot(ctx));
     if (!h_pairs) return HGE_ERR_NOMEM;
-    HGE_CUDA(cudaMemcpyAsync(h_pairs, d_pairs, sizeof(unsigned long long), cudaMemcpyDeviceToHost,
+    HGE_CUDA(cudaMemcpyAsync(h_pairs, d_pairs.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost,
                              ctx->stream));
     HGE_CUDA(cudaStreamSynchronize(ctx->stream));
-    hge_dev_free(ctx, d_pairs);
+    d_pairs.reset();
     const double per_pair = *h_pairs ? (double)eh.nnz / (double)*h_pairs : 0.0;
     if (per_pair < kMinPerPair && !ctx->tile_force) {
       hge_dev_free(ctx, inc->tile_pos);
@@ -883,13 +874,13 @@ static int algdist_load_impl(hge_algdist* st, const float* xn, const float* xe, 
     dn = ctx->stage;
     de = ctx->stage + (size_t)inc->N * st->R;
   }
-  k_fill_minmax<<<grid_1d(ctx, (int64_t)std::max(1, st->max_iters) * 2 * st->ld, kBlock), kBlock, 0,
+  k_fill_minmax<<<grid_for(ctx, (int64_t)std::max(1, st->max_iters) * 2 * st->ld, kBlock, kBlocksPerSm), kBlock, 0,
                   ctx->stream>>>(st->mm, std::max(1, st->max_iters), st->ld);
   HGE_CHECK_LAUNCH(ctx);
-  k_load_rows<<<grid_1d(ctx, (int64_t)inc->N * st->ld, kBlock), kBlock, 0, ctx->stream>>>(
+  k_load_rows<<<grid_for(ctx, (int64_t)inc->N * st->ld, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(
       inc->N, st->R, st->ld, dn, inc->node_half.deg, st->yn);
   HGE_CHECK_LAUNCH(ctx);
-  k_load_rows<<<grid_1d(ctx, (int64_t)inc->E * st->ld, kBlock), kBlock, 0, ctx->stream>>>(
+  k_load_rows<<<grid_for(ctx, (int64_t)inc->E * st->ld, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(
       inc->E, st->R, st->ld, de, inc->edge_half.deg, st->ye);
   HGE_CHECK_LAUNCH(ctx);
   if (mem == HGE_MEM_HOST) HGE_CUDA(cudaEventRecord(ctx->stage_idle, ctx->stream));
@@ -920,7 +911,7 @@ int hge_algdist_edge_half(hge_algdist* st, int sweep) {
   HGE_REQUIRE(st->ld <= 1024, "hge_algdist_edge_half: dimension too large for the tiled edge half");
   const int32_t* mm_prev = sweep > 0 ? st->mm + (size_t)(sweep - 1) * 2 * st->ld : nullptr;
   int32_t* mm_cur = st->mm + (size_t)sweep * 2 * st->ld;
-  k_edge_finalize<<<grid_1d(ctx, (int64_t)inc->E * st->ld, kBlock), kBlock, 0, ctx->stream>>>(
+  k_edge_finalize<<<grid_for(ctx, (int64_t)inc->E * st->ld, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(
       0, inc->E, st->R, st->ld, st->tile_raw, inc->edge_half.deg, inc->edge_half.invs, mm_prev, mm_cur,
       st->ye);
   HGE_CHECK_LAUNCH(ctx);
@@ -949,7 +940,7 @@ int hge_algdist_edge_finalize(hge_algdist* st, int sweep, int slice, const float
   int32_t* mm_cur = st->mm + (size_t)sweep * 2 * st->ld;
   const int64_t row0 = inc->slice_bounds[(size_t)slice];
   const int64_t rows = inc->slice_bounds[(size_t)slice + 1] - row0;
-  k_edge_finalize<<<grid_1d(ctx, rows * st->ld, kBlock), kBlock, 0, ctx->stream>>>(
+  k_edge_finalize<<<grid_for(ctx, rows * st->ld, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(
       row0, rows, st->R, st->ld, partial, inc->edge_half.deg, inc->edge_half.invs, mm_prev, mm_cur,
       st->ye);
   HGE_CHECK_LAUNCH(ctx);
@@ -975,7 +966,7 @@ int hge_internal_edge_push(hge_algdist* st, int sweep, int slice) {
   HgeOwnerMap map;
   map.slice_rows = p->slice_rows;
   map.sub_rows = p->sub_rows;
-  k_push_rows<<<grid_1d(ctx, (int64_t)inc->E * st->ld4, kBlock), kBlock, 0, ctx->stream>>>(
+  k_push_rows<<<grid_for(ctx, (int64_t)inc->E * st->ld4, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(
       0, inc->E, st->ld4, reinterpret_cast<const float4*>(st->tile_raw), p->d_peer_stage, p->own_rows,
       p->rank, map);
   HGE_CHECK_LAUNCH(ctx);
@@ -1098,10 +1089,10 @@ int hge_algdist_store(hge_algdist* st, int sweeps_done, float* xn, float* xe, in
     dn = stage;
     de = stage + (size_t)inc->N * st->R;
   }
-  k_store_rows<<<grid_1d(ctx, (int64_t)inc->N * st->R, kBlock), kBlock, 0, ctx->stream>>>(
+  k_store_rows<<<grid_for(ctx, (int64_t)inc->N * st->R, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(
       inc->N, st->R, st->ld, st->yn, inc->node_half.deg, mm, dn);
   HGE_CHECK_LAUNCH(ctx);
-  k_store_rows<<<grid_1d(ctx, (int64_t)inc->E * st->R, kBlock), kBlock, 0, ctx->stream>>>(
+  k_store_rows<<<grid_for(ctx, (int64_t)inc->E * st->R, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(
       inc->E, st->R, st->ld, st->ye, inc->edge_half.deg, mm, de);
   HGE_CHECK_LAUNCH(ctx);
   if (mem == HGE_MEM_HOST) {
@@ -1130,19 +1121,19 @@ int hge_column_rescale(hge_ctx* ctx, float* xn, int64_t num_nodes, float* xe, in
     HGE_CUDA(cudaMemcpyAsync(dn, xn, nn * 4, cudaMemcpyHostToDevice, ctx->stream));
     HGE_CUDA(cudaMemcpyAsync(de, xe, ne * 4, cudaMemcpyHostToDevice, ctx->stream));
   }
-  int32_t* mm = nullptr;
-  HGE_TRY(hge_dev_alloc(ctx, &mm, (size_t)2 * R));
-  k_fill_minmax<<<grid_1d(ctx, 2 * R, kBlock), kBlock, 0, ctx->stream>>>(mm, 1, R);
+  DevBuf<int32_t> mm(ctx);
+  HGE_TRY(mm.alloc((size_t)2 * R));
+  k_fill_minmax<<<grid_for(ctx, 2 * R, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(mm.p, 1, R);
   HGE_CHECK_LAUNCH(ctx);
-  k_dense_minmax<<<grid_1d(ctx, (int64_t)nn, kBlock), kBlock, 0, ctx->stream>>>(num_nodes, R, dn, mm);
+  k_dense_minmax<<<grid_for(ctx, (int64_t)nn, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(num_nodes, R, dn, mm.p);
   HGE_CHECK_LAUNCH(ctx);
-  k_dense_minmax<<<grid_1d(ctx, (int64_t)ne, kBlock), kBlock, 0, ctx->stream>>>(num_edges, R, de, mm);
+  k_dense_minmax<<<grid_for(ctx, (int64_t)ne, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(num_edges, R, de, mm.p);
   HGE_CHECK_LAUNCH(ctx);
-  k_dense_rescale<<<grid_1d(ctx, (int64_t)nn, kBlock), kBlock, 0, ctx->stream>>>(num_nodes, R, dn, mm);
+  k_dense_rescale<<<grid_for(ctx, (int64_t)nn, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(num_nodes, R, dn, mm.p);
   HGE_CHECK_LAUNCH(ctx);
-  k_dense_rescale<<<grid_1d(ctx, (int64_t)ne, kBlock), kBlock, 0, ctx->stream>>>(num_edges, R, de, mm);
+  k_dense_rescale<<<grid_for(ctx, (int64_t)ne, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(num_edges, R, de, mm.p);
   HGE_CHECK_LAUNCH(ctx);
-  hge_dev_free(ctx, mm);
+  mm.reset();
   if (mem == HGE_MEM_HOST) {
     HGE_CUDA(cudaMemcpyAsync(xn, dn, nn * 4, cudaMemcpyDeviceToHost, ctx->stream));
     HGE_CUDA(cudaMemcpyAsync(xe, de, ne * 4, cudaMemcpyDeviceToHost, ctx->stream));

@@ -7,6 +7,8 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <algorithm>
+
 #include "../../include/hge_b200.h"
 
 void hge_set_error(const char* fmt, ...);
@@ -67,6 +69,10 @@ struct hge_ctx {
   cudaStream_t copy_stream;
   cudaEvent_t copy_done;    // recorded on copy_stream after an upload into `stage`
   cudaEvent_t stage_idle;   // recorded on `stream` after the last reader / writer of `stage`
+  // HGE_FAIL_ALLOC_AT = n > 0: the n-th device allocation after the last tuning reset fails with
+  // HGE_ERR_NOMEM, so that the error paths of every entry point can be exercised (0: off)
+  int64_t fail_alloc_at;
+  mutable int64_t allocs;
 };
 
 // Staging block of at least `floats` floats (contents undefined).  Growing it drains the stream.
@@ -81,9 +87,13 @@ void* hge_ctx_pinned_slot(hge_ctx* ctx);
 // reused instead of being returned to the driver).  Everything is released explicitly by the
 // owning object; all work of a context is queued on one stream, so stream order is enough.
 template <typename T>
-static inline int hge_dev_alloc(const hge_ctx* ctx, T** p, size_t count) {
+[[nodiscard]] static inline int hge_dev_alloc(const hge_ctx* ctx, T** p, size_t count) {
   *p = nullptr;
   if (count == 0) count = 1;
+  if (ctx->fail_alloc_at > 0 && ++ctx->allocs == ctx->fail_alloc_at) {
+    hge_set_error("device allocation %lld failed (HGE_FAIL_ALLOC_AT)", (long long)ctx->allocs);
+    return HGE_ERR_NOMEM;
+  }
   cudaError_t e = cudaMallocAsync(reinterpret_cast<void**>(p), count * sizeof(T), ctx->stream);
   if (e != cudaSuccess) {
     hge_set_error("cudaMallocAsync of %zu bytes failed: %s", count * sizeof(T),
@@ -98,6 +108,76 @@ template <typename T>
 static inline void hge_dev_free(const hge_ctx* ctx, T*& p) {
   if (p) cudaFreeAsync(p, ctx->stream);
   p = nullptr;
+}
+
+// Owner of a device buffer that lives for one call: freed (stream-ordered) when the owner goes
+// out of scope or at reset(), or handed with release() to an object that frees it itself.
+template <typename T>
+struct DevBuf {
+  const hge_ctx* ctx;
+  T* p = nullptr;
+  explicit DevBuf(const hge_ctx* c) : ctx(c) {}
+  DevBuf(DevBuf&& o) noexcept : ctx(o.ctx), p(o.release()) {}
+  DevBuf& operator=(DevBuf&& o) {
+    reset();
+    p = o.release();
+    return *this;
+  }
+  ~DevBuf() { reset(); }
+  [[nodiscard]] int alloc(size_t n) {
+    reset();
+    return hge_dev_alloc(ctx, &p, n);
+  }
+  void reset() { hge_dev_free(ctx, p); }
+  [[nodiscard]] T* release() {
+    T* q = p;
+    p = nullptr;
+    return q;
+  }
+};
+
+// n elements device -> host, waited for
+template <typename T>
+int read_back(const hge_ctx* ctx, const T* dev, T* host, size_t n) {
+  HGE_CUDA(cudaMemcpyAsync(host, dev, n * sizeof(T), cudaMemcpyDeviceToHost, ctx->stream));
+  HGE_CUDA(cudaStreamSynchronize(ctx->stream));
+  return HGE_OK;
+}
+
+// Host <-> device staging for the HGE_MEM_HOST flavour of the entry points: `dev` is the
+// caller's array for HGE_MEM_DEVICE, otherwise a device copy, uploaded by init() when `in` and
+// copied back by finish() when `out`.
+template <typename T>
+struct Staged {
+  DevBuf<T> copy;
+  T* dev = nullptr;
+  T* host = nullptr;
+  size_t count = 0;
+  bool copy_out = false;
+  explicit Staged(const hge_ctx* c) : copy(c) {}
+
+  int init(const T* p, size_t n, int mem, bool in, bool out) {
+    count = n;
+    copy_out = out && mem == HGE_MEM_HOST;
+    host = const_cast<T*>(p);
+    if (mem == HGE_MEM_DEVICE || p == nullptr) {
+      dev = const_cast<T*>(p);
+      return HGE_OK;
+    }
+    HGE_TRY(copy.alloc(n));
+    dev = copy.p;
+    if (in && n)
+      HGE_CUDA(cudaMemcpyAsync(dev, p, n * sizeof(T), cudaMemcpyHostToDevice, copy.ctx->stream));
+    return HGE_OK;
+  }
+  int finish() { return copy_out && count ? read_back(copy.ctx, dev, host, count) : HGE_OK; }
+};
+
+// Blocks of a grid-stride launch over `work` items, `per_block` a block: at least one, at most
+// `per_sm` a multiprocessor.
+static inline int grid_for(const hge_ctx* ctx, int64_t work, int per_block = 256, int per_sm = 16) {
+  const int64_t want = std::max<int64_t>(1, (work + per_block - 1) / per_block);
+  return (int)std::min<int64_t>(want, (int64_t)ctx->num_sms * per_sm);
 }
 
 #ifdef __CUDACC__

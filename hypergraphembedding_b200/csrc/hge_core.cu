@@ -86,6 +86,9 @@ static void set_default_tuning(hge_ctx* ctx) {
   if (const char* env = getenv("HGE_TILE_MB")) ctx->tile_mb = atoi(env);
   if (const char* env = getenv("HGE_TILE_MIN_MB")) ctx->tile_min_mb = atoi(env);
   ctx->tile_force = ctx->tile_min_mb == 0;
+  ctx->fail_alloc_at = 0;
+  if (const char* env = getenv("HGE_FAIL_ALLOC_AT")) ctx->fail_alloc_at = std::max(0ll, atoll(env));
+  ctx->allocs = 0;
 }
 
 extern "C" {

@@ -27,7 +27,6 @@
 #include "hge_expand.cuh"
 #include "hge_incidence.cuh"
 #include "hge_philox.cuh"
-#include "hge_staged.cuh"
 
 namespace {
 
@@ -255,8 +254,8 @@ struct PairSampler {
     HGE_TRY(temp.alloc(bytes));
     HGE_CUDA(cub::DeviceRadixSort::SortKeys(temp.p, bytes, keys.p, keys2.p, n, 0, 32 + row_bits, ctx->stream));
     ctx->launches++;
-    hge_dev_free(ctx, temp.p);
-    hge_dev_free(ctx, keys.p);
+    temp.reset();
+    keys.reset();
     HGE_TRY(head.alloc((size_t)n + 1));
     HGE_TRY(pos.alloc((size_t)n + 1));
     k_run_heads<<<grid_for(ctx, n), kBlock, 0, ctx->stream>>>(n, keys2.p, head.p);
@@ -395,10 +394,10 @@ int hge_sample_pairs_device(hge_ctx* ctx, hge_incidence* inc, int side, int fact
   const DevCsr m1 = side == 0 ? n2e : e2n, m2 = side == 0 ? e2n : n2e;
   // columns of M1 (M1 * M2 (* M3)): E / N alternate with the number of factors
   const uint32_t out_cols = (uint32_t)(((side == 0) == (factors != 2)) ? inc->E : inc->N);
-  Staged<int32_t> s_k, s_row, s_col;
-  HGE_TRY(s_k.init(ctx, samples_per_row, (size_t)L, mem, true, false));
-  HGE_TRY(s_row.init(ctx, out_row, (size_t)capacity, mem, false, true));
-  HGE_TRY(s_col.init(ctx, out_col, (size_t)capacity, mem, false, true));
+  Staged<int32_t> s_k(ctx), s_row(ctx), s_col(ctx);
+  HGE_TRY(s_k.init(samples_per_row, (size_t)L, mem, true, false));
+  HGE_TRY(s_row.init(out_row, (size_t)capacity, mem, false, true));
+  HGE_TRY(s_col.init(out_col, (size_t)capacity, mem, false, true));
   DevBuf<int> status(ctx);
   HGE_TRY(status.alloc(1));
   HGE_CUDA(cudaMemsetAsync(status.p, 0, sizeof(int), ctx->stream));
@@ -426,11 +425,11 @@ int hge_sample_neighbors_device(hge_ctx* ctx, hge_incidence* inc, const int32_t*
   HGE_REQUIRE(mem == HGE_MEM_HOST || mem == HGE_MEM_DEVICE, "hge_sample_neighbors_device: bad mem %d", mem);
   HGE_CUDA(cudaSetDevice(ctx->device));
   if (count == 0 || k == 0) return HGE_OK;
-  Staged<int32_t> s_n, s_e, s_oe, s_on;
-  HGE_TRY(s_n.init(ctx, nodes, (size_t)count, mem, true, false));
-  HGE_TRY(s_e.init(ctx, edges, (size_t)count, mem, true, false));
-  HGE_TRY(s_oe.init(ctx, out_nbr_edges, (size_t)count * k, mem, false, true));
-  HGE_TRY(s_on.init(ctx, out_nbr_nodes, (size_t)count * k, mem, false, true));
+  Staged<int32_t> s_n(ctx), s_e(ctx), s_oe(ctx), s_on(ctx);
+  HGE_TRY(s_n.init(nodes, (size_t)count, mem, true, false));
+  HGE_TRY(s_e.init(edges, (size_t)count, mem, true, false));
+  HGE_TRY(s_oe.init(out_nbr_edges, (size_t)count * k, mem, false, true));
+  HGE_TRY(s_on.init(out_nbr_nodes, (size_t)count * k, mem, false, true));
   DevBuf<int> status(ctx);
   HGE_TRY(status.alloc(1));
   HGE_CUDA(cudaMemsetAsync(status.p, 0, sizeof(int), ctx->stream));

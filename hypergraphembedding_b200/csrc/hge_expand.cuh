@@ -8,38 +8,11 @@
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
-#include <algorithm>
-
 #include "hge_common.cuh"
 
 namespace {
 
 constexpr int kExpandBlock = 256;
-
-int grid_for(const hge_ctx* ctx, int64_t work, int per_block = kExpandBlock) {
-  const int64_t want = std::max<int64_t>(1, (work + per_block - 1) / per_block);
-  return (int)std::min<int64_t>(want, (int64_t)ctx->num_sms * 16);
-}
-
-// device buffer released when it goes out of scope (stream-ordered)
-template <typename T>
-struct DevBuf {
-  const hge_ctx* ctx;
-  T* p = nullptr;
-  explicit DevBuf(const hge_ctx* c) : ctx(c) {}
-  ~DevBuf() { hge_dev_free(ctx, p); }
-  int alloc(size_t n) {
-    hge_dev_free(ctx, p);
-    return hge_dev_alloc(ctx, &p, n);
-  }
-};
-
-template <typename T>
-int read_back(hge_ctx* ctx, const T* dev, T* host, size_t n) {
-  HGE_CUDA(cudaMemcpyAsync(host, dev, n * sizeof(T), cudaMemcpyDeviceToHost, ctx->stream));
-  HGE_CUDA(cudaStreamSynchronize(ctx->stream));
-  return HGE_OK;
-}
 
 // head[i] = 1 where a run of equal keys starts
 __global__ void k_run_heads(int64_t n, const uint64_t* __restrict__ keys, int64_t* __restrict__ head) {

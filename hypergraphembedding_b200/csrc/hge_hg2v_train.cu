@@ -40,7 +40,6 @@
 #include "hge_common.cuh"
 #include "hge_expand.cuh"
 #include "hge_philox.cuh"
-#include "hge_staged.cuh"
 
 namespace cg = cooperative_groups;
 
@@ -597,16 +596,9 @@ int hge_hg2v_set_samples(hge_hg2v_model* m, const int32_t* features, const float
   HGE_REQUIRE(mem == HGE_MEM_HOST || mem == HGE_MEM_DEVICE, "hge_hg2v_set_samples: bad mem %d", mem);
   hge_ctx* ctx = m->ctx;
   HGE_CUDA(cudaSetDevice(ctx->device));
-  hge_dev_free(ctx, m->feat);
-  hge_dev_free(ctx, m->target);
-  hge_dev_free(ctx, m->order);
-  m->reserved = false;
-  m->M = num_samples;
   const size_t cols = 4 + 2 * (size_t)m->k;
-  HGE_TRY(upload(ctx, &m->feat, features, cols * (size_t)num_samples, mem));
-  HGE_TRY(upload(ctx, &m->target, targets, 3 * (size_t)num_samples, mem));
-  HGE_TRY(hge_dev_alloc(ctx, &m->order, (size_t)num_samples));
-  // every index must address a table row: check once here instead of in the hot loop
+  // every index must address a table row: check once here instead of in the hot loop, and before
+  // the model changes, so that a refused call leaves the samples it had
   if (mem == HGE_MEM_HOST) {
     for (size_t c = 0; c < cols; ++c) {
       const bool node = c == 0 || c == 2 || (c >= 4 && c < 4 + (size_t)m->k);
@@ -618,6 +610,15 @@ int hge_hg2v_set_samples(hge_hg2v_model* m, const int32_t* features, const float
                     "table of %d rows", c, (long long)i, col[i], limit);
     }
   }
+  hge_dev_free(ctx, m->feat);
+  hge_dev_free(ctx, m->target);
+  hge_dev_free(ctx, m->order);
+  m->reserved = false;
+  m->M = 0;
+  HGE_TRY(upload(ctx, &m->feat, features, cols * (size_t)num_samples, mem));
+  HGE_TRY(upload(ctx, &m->target, targets, 3 * (size_t)num_samples, mem));
+  HGE_TRY(hge_dev_alloc(ctx, &m->order, (size_t)num_samples));
+  m->M = num_samples;
   return HGE_OK;
 }
 
@@ -699,8 +700,7 @@ int hge_hg2v_fit_epoch(hge_hg2v_model* m, const int32_t* order, int batch_size, 
   m->last_clusters = clusters;
   ctx->launches++;
   double total = 0.0;
-  HGE_CUDA(cudaMemcpyAsync(&total, m->d_loss, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-  HGE_CUDA(cudaStreamSynchronize(ctx->stream));
+  HGE_TRY(read_back(ctx, m->d_loss, &total, 1));
   *epoch_loss = total / (double)m->M;
   return HGE_OK;
 }
@@ -799,44 +799,26 @@ int hge_shuffle_order(hge_ctx* ctx, uint64_t seed, uint32_t epoch, int64_t n, in
   HGE_REQUIRE(mem == HGE_MEM_HOST || mem == HGE_MEM_DEVICE, "hge_shuffle_order: bad mem %d", mem);
   if (n == 0) return HGE_OK;
   HGE_CUDA(cudaSetDevice(ctx->device));
-  Staged<int32_t> out;
-  HGE_TRY(out.init(ctx, order, (size_t)n, mem, false, true));
-  uint64_t *k0 = nullptr, *k1 = nullptr;
-  int32_t* v1 = nullptr;
-  char* temp = nullptr;
-  int rc = hge_dev_alloc(ctx, &k0, (size_t)n);
-  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &k1, (size_t)n);
-  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &v1, (size_t)n);
-  cub::DoubleBuffer<uint64_t> keys(k0, k1);
-  cub::DoubleBuffer<int32_t> vals(out.dev, v1);
+  Staged<int32_t> out(ctx);
+  HGE_TRY(out.init(order, (size_t)n, mem, false, true));
+  DevBuf<uint64_t> k0(ctx), k1(ctx);
+  DevBuf<int32_t> v1(ctx);
+  DevBuf<char> temp(ctx);
+  HGE_TRY(k0.alloc((size_t)n));
+  HGE_TRY(k1.alloc((size_t)n));
+  HGE_TRY(v1.alloc((size_t)n));
+  cub::DoubleBuffer<uint64_t> keys(k0.p, k1.p);
+  cub::DoubleBuffer<int32_t> vals(out.dev, v1.p);
+  k_shuffle_keys<<<grid_for(ctx, n), kExpandBlock, 0, ctx->stream>>>(n, seed, epoch, k0.p, out.dev);
+  HGE_CHECK_LAUNCH(ctx);
+  // LSD radix sort: stable, so equal keys keep ascending item order
   size_t bytes = 0;
-  if (rc == HGE_OK) {
-    k_shuffle_keys<<<grid_for(ctx, n), kExpandBlock, 0, ctx->stream>>>(n, seed, epoch, k0, out.dev);
-    ctx->launches++;
-    cudaError_t e = cudaGetLastError();
-    // LSD radix sort: stable, so equal keys keep ascending item order
-    if (e == cudaSuccess) e = cub::DeviceRadixSort::SortPairs(nullptr, bytes, keys, vals, n, 0, 64, ctx->stream);
-    if (e != cudaSuccess) {
-      hge_set_error("hge_shuffle_order: %s", cudaGetErrorString(e));
-      rc = HGE_ERR_CUDA;
-    }
-  }
-  if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &temp, bytes);
-  if (rc == HGE_OK) {
-    cudaError_t e = cub::DeviceRadixSort::SortPairs(temp, bytes, keys, vals, n, 0, 64, ctx->stream);
-    ctx->launches++;
-    if (e == cudaSuccess && vals.Current() != out.dev)
-      e = cudaMemcpyAsync(out.dev, vals.Current(), (size_t)n * 4, cudaMemcpyDeviceToDevice, ctx->stream);
-    if (e != cudaSuccess) {
-      hge_set_error("hge_shuffle_order: %s", cudaGetErrorString(e));
-      rc = HGE_ERR_CUDA;
-    }
-  }
-  hge_dev_free(ctx, temp);
-  hge_dev_free(ctx, k0);
-  hge_dev_free(ctx, k1);
-  hge_dev_free(ctx, v1);
-  HGE_TRY(rc);
+  HGE_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, bytes, keys, vals, n, 0, 64, ctx->stream));
+  HGE_TRY(temp.alloc(bytes));
+  HGE_CUDA(cub::DeviceRadixSort::SortPairs(temp.p, bytes, keys, vals, n, 0, 64, ctx->stream));
+  ctx->launches++;
+  if (vals.Current() != out.dev)
+    HGE_CUDA(cudaMemcpyAsync(out.dev, vals.Current(), (size_t)n * 4, cudaMemcpyDeviceToDevice, ctx->stream));
   return out.finish();
 }
 

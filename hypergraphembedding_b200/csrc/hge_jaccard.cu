@@ -35,7 +35,6 @@
 #include "hge_common.cuh"
 #include "hge_expand.cuh"
 #include "hge_incidence.cuh"
-#include "hge_staged.cuh"
 
 namespace {
 
@@ -184,20 +183,22 @@ struct FeatureMatrix {
   Staged<int64_t> ptr;
   Staged<int32_t> idx;
   Staged<float> val;
-  int init(hge_ctx* c, const int64_t* p, const int32_t* i, const float* v, int64_t rows, int64_t nnz, int mem) {
-    HGE_TRY(ptr.init(c, p, (size_t)rows + 1, mem, true, false));
-    HGE_TRY(idx.init(c, i, (size_t)nnz, mem, true, false));
-    HGE_TRY(val.init(c, v, (size_t)nnz, mem, true, false));
+  explicit FeatureMatrix(const hge_ctx* c) : ptr(c), idx(c), val(c) {}
+  int init(const int64_t* p, const int32_t* i, const float* v, int64_t rows, int64_t nnz, int mem) {
+    HGE_TRY(ptr.init(p, (size_t)rows + 1, mem, true, false));
+    HGE_TRY(idx.init(i, (size_t)nnz, mem, true, false));
+    HGE_TRY(val.init(v, (size_t)nnz, mem, true, false));
     return HGE_OK;
   }
 };
 
 // Centroid rows of the groups named by pg[0 .. num_pairs): CSR over ALL groups (rows of the
-// groups no pair names are empty).  Everything on ctx->stream; the arrays are the caller's to free.
+// groups no pair names are empty).  Everything on ctx->stream.
 struct CentroidRows {
-  int64_t* ptr = nullptr;
-  int32_t* idx = nullptr;
-  float* val = nullptr;
+  DevBuf<int64_t> ptr;
+  DevBuf<int32_t> idx;
+  DevBuf<float> val;
+  explicit CentroidRows(const hge_ctx* c) : ptr(c), idx(c), val(c) {}
 };
 
 // Centroid rows of one batch of L groups from its expansion: keys ((local group << 32) | column)
@@ -205,10 +206,10 @@ struct CentroidRows {
 // the members stay in ascending order), run heads, then one sequential fp32 sum per run.  Local
 // group l is group gid[l] of the group CSR (g0 + l when gid is NULL).  The rows' start offsets go to
 // start[s0 + l] = rows_before + first run of l (and start[s0 + L] when last); the n_runs column ids
-// and values to *cidx / *cval, which the caller frees.  keys / vals are used as sort buffers.
+// and values to cidx / cval.  keys / vals are used as sort buffers.
 int centroid_batch(hge_ctx* ctx, int64_t n, int64_t L, int64_t g0, const int32_t* gid, const int64_t* gptr,
                    DevBuf<uint64_t>& keys, DevBuf<float>& vals, int64_t* start, int64_t s0, int64_t rows_before,
-                   bool last, int32_t** cidx, float** cval, int64_t* n_runs) {
+                   bool last, DevBuf<int32_t>& cidx, DevBuf<float>& cval, int64_t* n_runs) {
   DevBuf<uint64_t> keys2(ctx);
   DevBuf<float> vals2(ctx);
   DevBuf<int64_t> head(ctx), pos(ctx);
@@ -236,9 +237,9 @@ int centroid_batch(hge_ctx* ctx, int64_t n, int64_t L, int64_t g0, const int32_t
   HGE_CUDA(cub::DeviceScan::ExclusiveSum(temp.p, bytes, head.p, pos.p, n + 1, ctx->stream));
   ctx->launches++;
   HGE_TRY(read_back(ctx, pos.p + n, n_runs, 1));
-  HGE_TRY(hge_dev_alloc(ctx, cidx, (size_t)std::max<int64_t>(1, *n_runs)));
-  HGE_TRY(hge_dev_alloc(ctx, cval, (size_t)std::max<int64_t>(1, *n_runs)));
-  k_run_sums<<<grid_for(ctx, n), kBlock, 0, ctx->stream>>>(n, g0, gid, sk, sv, pos.p, gptr, *cidx, *cval);
+  HGE_TRY(cidx.alloc((size_t)std::max<int64_t>(1, *n_runs)));
+  HGE_TRY(cval.alloc((size_t)std::max<int64_t>(1, *n_runs)));
+  k_run_sums<<<grid_for(ctx, n), kBlock, 0, ctx->stream>>>(n, g0, gid, sk, sv, pos.p, gptr, cidx.p, cval.p);
   HGE_CHECK_LAUNCH(ctx);
   k_run_starts<<<grid_for(ctx, L + 1), kBlock, 0, ctx->stream>>>(s0, s0 + L, n, *n_runs, rows_before, sk, pos.p,
                                                                start, last);
@@ -248,46 +249,46 @@ int centroid_batch(hge_ctx* ctx, int64_t n, int64_t L, int64_t g0, const int32_t
 
 int build_centroids(hge_ctx* ctx, const int64_t* gptr, const int32_t* gidx, int64_t groups, int64_t gnnz,
                     const FeatureMatrix& f, const int32_t* pg, int64_t num_pairs, CentroidRows* out) {
-  int32_t* flag = nullptr;
-  int64_t *w = nullptr, *off = nullptr, *goff = nullptr;
-  HGE_TRY(hge_dev_alloc(ctx, &flag, (size_t)groups));
-  HGE_TRY(hge_dev_alloc(ctx, &w, (size_t)gnnz + 1));
-  HGE_TRY(hge_dev_alloc(ctx, &off, (size_t)gnnz + 1));
-  HGE_TRY(hge_dev_alloc(ctx, &goff, (size_t)groups + 1));
-  HGE_TRY(hge_dev_alloc(ctx, &out->ptr, (size_t)groups + 1));
-  HGE_CUDA(cudaMemsetAsync(flag, 0, (size_t)groups * sizeof(int32_t), ctx->stream));
-  HGE_CUDA(cudaMemsetAsync(w, 0, ((size_t)gnnz + 1) * sizeof(int64_t), ctx->stream));
-  k_flag_groups<<<grid_for(ctx, num_pairs), kBlock, 0, ctx->stream>>>(num_pairs, pg, flag);
+  DevBuf<int32_t> flag(ctx);
+  DevBuf<int64_t> w(ctx), off(ctx), goff(ctx);
+  DevBuf<char> scan_temp(ctx);
+  HGE_TRY(flag.alloc((size_t)groups));
+  HGE_TRY(w.alloc((size_t)gnnz + 1));
+  HGE_TRY(off.alloc((size_t)gnnz + 1));
+  HGE_TRY(goff.alloc((size_t)groups + 1));
+  HGE_TRY(out->ptr.alloc((size_t)groups + 1));
+  HGE_CUDA(cudaMemsetAsync(flag.p, 0, (size_t)groups * sizeof(int32_t), ctx->stream));
+  HGE_CUDA(cudaMemsetAsync(w.p, 0, ((size_t)gnnz + 1) * sizeof(int64_t), ctx->stream));
+  k_flag_groups<<<grid_for(ctx, num_pairs), kBlock, 0, ctx->stream>>>(num_pairs, pg, flag.p);
   HGE_CHECK_LAUNCH(ctx);
-  k_member_weights<<<grid_for(ctx, groups, kBlock / 32), kBlock, 0, ctx->stream>>>(groups, gptr, gidx, flag,
-                                                                                 f.ptr.dev, w);
+  k_member_weights<<<grid_for(ctx, groups, kBlock / 32), kBlock, 0, ctx->stream>>>(groups, gptr, gidx, flag.p,
+                                                                                 f.ptr.dev, w.p);
   HGE_CHECK_LAUNCH(ctx);
   size_t scan_bytes = 0;
-  HGE_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, w, off, gnnz + 1, ctx->stream));
-  char* scan_temp = nullptr;
-  HGE_TRY(hge_dev_alloc(ctx, &scan_temp, scan_bytes));
-  HGE_CUDA(cub::DeviceScan::ExclusiveSum(scan_temp, scan_bytes, w, off, gnnz + 1, ctx->stream));
+  HGE_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, w.p, off.p, gnnz + 1, ctx->stream));
+  HGE_TRY(scan_temp.alloc(scan_bytes));
+  HGE_CUDA(cub::DeviceScan::ExclusiveSum(scan_temp.p, scan_bytes, w.p, off.p, gnnz + 1, ctx->stream));
   ctx->launches++;
-  hge_dev_free(ctx, scan_temp);
+  scan_temp.reset();
   int64_t total = 0;
-  HGE_TRY(read_back(ctx, off + gnnz, &total, 1));
-  k_group_offsets<<<grid_for(ctx, groups + 1), kBlock, 0, ctx->stream>>>(groups, gnnz, total, gptr, off, goff);
+  HGE_TRY(read_back(ctx, off.p + gnnz, &total, 1));
+  k_group_offsets<<<grid_for(ctx, groups + 1), kBlock, 0, ctx->stream>>>(groups, gnnz, total, gptr, off.p,
+                                                                         goff.p);
   HGE_CHECK_LAUNCH(ctx);
   std::vector<int64_t> h_goff((size_t)groups + 1), h_gptr((size_t)groups + 1);
-  HGE_TRY(read_back(ctx, goff, h_goff.data(), (size_t)groups + 1));
+  HGE_TRY(read_back(ctx, goff.p, h_goff.data(), (size_t)groups + 1));
   HGE_TRY(read_back(ctx, gptr, h_gptr.data(), (size_t)groups + 1));
 
   // batches of consecutive groups whose expansion fits the budget (a single group larger than
   // the budget is its own batch)
   struct Part {
-    int32_t* idx;
-    float* val;
+    DevBuf<int32_t> idx;
+    DevBuf<float> val;
     int64_t n;
   };
   std::vector<Part> parts;
   int64_t rows_before = 0;
-  int rc = HGE_OK;
-  for (int64_t g0 = 0; g0 < groups && rc == HGE_OK;) {
+  for (int64_t g0 = 0; g0 < groups;) {
     int64_t g1 = g0 + 1;
     while (g1 < groups && h_goff[(size_t)g1 + 1] - h_goff[(size_t)g0] <= kBatchEntries && g1 - g0 < (1ll << 31) - 1)
       ++g1;
@@ -296,66 +297,48 @@ int build_centroids(hge_ctx* ctx, const int64_t* gptr, const int32_t* gidx, int6
     if (n == 0) {
       // no pair names any of these groups: empty rows
       k_run_starts<<<grid_for(ctx, g1 - g0 + 1), kBlock, 0, ctx->stream>>>(g0, g1, 0, 0, rows_before, nullptr,
-                                                                         nullptr, out->ptr, last);
+                                                                         nullptr, out->ptr.p, last);
       HGE_CHECK_LAUNCH(ctx);
       g0 = g1;
       continue;
     }
     DevBuf<uint64_t> keys(ctx);
     DevBuf<float> vals(ctx);
-    Part part = {nullptr, nullptr, 0};
-    auto batch = [&]() -> int {
-      HGE_TRY(keys.alloc((size_t)n));
-      HGE_TRY(vals.alloc((size_t)n));
-      k_expand<<<grid_for(ctx, h_gptr[(size_t)g1] - h_gptr[(size_t)g0], kBlock / 32), kBlock, 0, ctx->stream>>>(
-          h_gptr[(size_t)g0], h_gptr[(size_t)g1], g0, g1, h_goff[(size_t)g0], gptr, gidx, off, w, f.ptr.dev,
-          f.idx.dev, f.val.dev, keys.p, vals.p);
-      HGE_CHECK_LAUNCH(ctx);
-      return centroid_batch(ctx, n, g1 - g0, g0, nullptr, gptr, keys, vals, out->ptr, g0, rows_before, last,
-                            &part.idx, &part.val, &part.n);
-    };
-    rc = batch();
-    if (rc == HGE_OK) {
-      parts.push_back(part);
-      rows_before += part.n;
-    } else {
-      hge_dev_free(ctx, part.idx);
-      hge_dev_free(ctx, part.val);
-    }
+    Part part = {DevBuf<int32_t>(ctx), DevBuf<float>(ctx), 0};
+    HGE_TRY(keys.alloc((size_t)n));
+    HGE_TRY(vals.alloc((size_t)n));
+    k_expand<<<grid_for(ctx, h_gptr[(size_t)g1] - h_gptr[(size_t)g0], kBlock / 32), kBlock, 0, ctx->stream>>>(
+        h_gptr[(size_t)g0], h_gptr[(size_t)g1], g0, g1, h_goff[(size_t)g0], gptr, gidx, off.p, w.p, f.ptr.dev,
+        f.idx.dev, f.val.dev, keys.p, vals.p);
+    HGE_CHECK_LAUNCH(ctx);
+    HGE_TRY(centroid_batch(ctx, n, g1 - g0, g0, nullptr, gptr, keys, vals, out->ptr.p, g0, rows_before, last,
+                           part.idx, part.val, &part.n));
+    rows_before += part.n;
+    parts.push_back(std::move(part));
     g0 = g1;
   }
-  hge_dev_free(ctx, flag);
-  hge_dev_free(ctx, w);
-  hge_dev_free(ctx, off);
-  hge_dev_free(ctx, goff);
-  if (rc == HGE_OK) {
-    if (parts.size() == 1) {
-      out->idx = parts[0].idx;
-      out->val = parts[0].val;
-      parts.clear();
-    } else {
-      rc = hge_dev_alloc(ctx, &out->idx, (size_t)std::max<int64_t>(1, rows_before));
-      if (rc == HGE_OK) rc = hge_dev_alloc(ctx, &out->val, (size_t)std::max<int64_t>(1, rows_before));
-      int64_t at = 0;
-      for (const Part& p : parts) {
-        if (rc == HGE_OK && p.n) {
-          cudaMemcpyAsync(out->idx + at, p.idx, (size_t)p.n * sizeof(int32_t), cudaMemcpyDeviceToDevice, ctx->stream);
-          cudaMemcpyAsync(out->val + at, p.val, (size_t)p.n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream);
-        }
-        at += p.n;
-      }
+  flag.reset();
+  w.reset();
+  off.reset();
+  goff.reset();
+  if (parts.size() == 1) {
+    out->idx = std::move(parts[0].idx);
+    out->val = std::move(parts[0].val);
+    return HGE_OK;
+  }
+  HGE_TRY(out->idx.alloc((size_t)std::max<int64_t>(1, rows_before)));
+  HGE_TRY(out->val.alloc((size_t)std::max<int64_t>(1, rows_before)));
+  int64_t at = 0;
+  for (const Part& p : parts) {
+    if (p.n) {
+      HGE_CUDA(cudaMemcpyAsync(out->idx.p + at, p.idx.p, (size_t)p.n * sizeof(int32_t), cudaMemcpyDeviceToDevice,
+                               ctx->stream));
+      HGE_CUDA(cudaMemcpyAsync(out->val.p + at, p.val.p, (size_t)p.n * sizeof(float), cudaMemcpyDeviceToDevice,
+                               ctx->stream));
     }
+    at += p.n;
   }
-  for (Part& p : parts) {
-    hge_dev_free(ctx, p.idx);
-    hge_dev_free(ctx, p.val);
-  }
-  if (rc != HGE_OK) {
-    hge_dev_free(ctx, out->ptr);
-    hge_dev_free(ctx, out->idx);
-    hge_dev_free(ctx, out->val);
-  }
-  return rc;
+  return HGE_OK;
 }
 
 // ---- centroid rows of the named groups, batch by batch (hge_jaccard_centroid_grouped) ----------
@@ -458,13 +441,13 @@ int hge_jaccard_rows(hge_ctx* ctx, const int64_t* ptr, const int32_t* idx, const
   HGE_REQUIRE(mem == HGE_MEM_HOST || mem == HGE_MEM_DEVICE, "hge_jaccard_rows: bad mem %d", mem);
   HGE_CUDA(cudaSetDevice(ctx->device));
   if (num_pairs == 0) return HGE_OK;
-  FeatureMatrix f;
-  Staged<int32_t> s_i, s_j;
-  Staged<float> s_out;
-  HGE_TRY(f.init(ctx, ptr, idx, val, rows, nnz, mem));
-  HGE_TRY(s_i.init(ctx, pi, (size_t)num_pairs, mem, true, false));
-  HGE_TRY(s_j.init(ctx, pj, (size_t)num_pairs, mem, true, false));
-  HGE_TRY(s_out.init(ctx, out, (size_t)num_pairs, mem, false, true));
+  FeatureMatrix f(ctx);
+  Staged<int32_t> s_i(ctx), s_j(ctx);
+  Staged<float> s_out(ctx);
+  HGE_TRY(f.init(ptr, idx, val, rows, nnz, mem));
+  HGE_TRY(s_i.init(pi, (size_t)num_pairs, mem, true, false));
+  HGE_TRY(s_j.init(pj, (size_t)num_pairs, mem, true, false));
+  HGE_TRY(s_out.init(out, (size_t)num_pairs, mem, false, true));
   k_jaccard_merge<<<grid_for(ctx, num_pairs), kBlock, 0, ctx->stream>>>(
       num_pairs, f.ptr.dev, f.idx.dev, f.val.dev, f.ptr.dev, f.idx.dev, f.val.dev, s_i.dev, s_j.dev, nullptr,
       s_out.dev);
@@ -483,33 +466,25 @@ int hge_jaccard_centroid(hge_ctx* ctx, const int64_t* xptr, const int32_t* xidx,
   HGE_REQUIRE(mem == HGE_MEM_HOST || mem == HGE_MEM_DEVICE, "hge_jaccard_centroid: bad mem %d", mem);
   HGE_CUDA(cudaSetDevice(ctx->device));
   if (num_pairs == 0) return HGE_OK;
-  FeatureMatrix x, f;
+  FeatureMatrix x(ctx), f(ctx);
   const bool same = xptr == fptr && xidx == fidx && xval == fval;   // usual case: X is F
-  Staged<int64_t> s_gptr;
-  Staged<int32_t> s_gidx, s_px, s_pg;
-  Staged<float> s_out;
-  HGE_TRY(f.init(ctx, fptr, fidx, fval, frows, fnnz, mem));
-  if (!same) HGE_TRY(x.init(ctx, xptr, xidx, xval, xrows, xnnz, mem));
-  HGE_TRY(s_gptr.init(ctx, gptr, (size_t)grows + 1, mem, true, false));
-  HGE_TRY(s_gidx.init(ctx, gidx, (size_t)gnnz, mem, true, false));
-  HGE_TRY(s_px.init(ctx, px, (size_t)num_pairs, mem, true, false));
-  HGE_TRY(s_pg.init(ctx, pg, (size_t)num_pairs, mem, true, false));
-  HGE_TRY(s_out.init(ctx, out, (size_t)num_pairs, mem, false, true));
-  CentroidRows c;
+  Staged<int64_t> s_gptr(ctx);
+  Staged<int32_t> s_gidx(ctx), s_px(ctx), s_pg(ctx);
+  Staged<float> s_out(ctx);
+  HGE_TRY(f.init(fptr, fidx, fval, frows, fnnz, mem));
+  if (!same) HGE_TRY(x.init(xptr, xidx, xval, xrows, xnnz, mem));
+  HGE_TRY(s_gptr.init(gptr, (size_t)grows + 1, mem, true, false));
+  HGE_TRY(s_gidx.init(gidx, (size_t)gnnz, mem, true, false));
+  HGE_TRY(s_px.init(px, (size_t)num_pairs, mem, true, false));
+  HGE_TRY(s_pg.init(pg, (size_t)num_pairs, mem, true, false));
+  HGE_TRY(s_out.init(out, (size_t)num_pairs, mem, false, true));
+  CentroidRows c(ctx);
   HGE_TRY(build_centroids(ctx, s_gptr.dev, s_gidx.dev, grows, gnnz, f, s_pg.dev, num_pairs, &c));
   const FeatureMatrix& xr = same ? f : x;
   k_jaccard_merge<<<grid_for(ctx, num_pairs), kBlock, 0, ctx->stream>>>(
-      num_pairs, xr.ptr.dev, xr.idx.dev, xr.val.dev, c.ptr, c.idx, c.val, s_px.dev, s_pg.dev, s_gptr.dev,
+      num_pairs, xr.ptr.dev, xr.idx.dev, xr.val.dev, c.ptr.p, c.idx.p, c.val.p, s_px.dev, s_pg.dev, s_gptr.dev,
       s_out.dev);
-  ctx->launches++;
-  const bool launched = cudaGetLastError() == cudaSuccess;
-  hge_dev_free(ctx, c.ptr);
-  hge_dev_free(ctx, c.idx);
-  hge_dev_free(ctx, c.val);
-  if (!launched) {
-    hge_set_error("hge_jaccard_centroid: kernel launch failed");
-    return HGE_ERR_CUDA;
-  }
+  HGE_CHECK_LAUNCH(ctx);
   return s_out.finish();
 }
 
@@ -563,8 +538,8 @@ int hge_jaccard_centroid_grouped(hge_ctx* ctx, hge_incidence* inc, int group_sid
   HGE_TRY(temp.alloc(bytes));
   HGE_CUDA(cub::DeviceScan::ExclusiveSum(temp.p, bytes, usize.p, uoff.p, U + 1, ctx->stream));
   ctx->launches++;
-  hge_dev_free(ctx, temp.p);
-  hge_dev_free(ctx, usize.p);
+  temp.reset();
+  usize.reset();
   std::vector<int64_t> h_uoff((size_t)U + 1), h_ustart((size_t)U + 1);
   HGE_TRY(read_back(ctx, uoff.p, h_uoff.data(), (size_t)U + 1));
   HGE_TRY(read_back(ctx, ustart.p, h_ustart.data(), (size_t)U + 1));
@@ -596,8 +571,7 @@ int hge_jaccard_centroid_grouped(hge_ctx* ctx, hge_incidence* inc, int group_sid
           u0, u1, h_uoff[(size_t)u0], ug.p, uoff.p, gptr, gidx, fptr, fidx, fval, keys.p, vals.p);
       HGE_CHECK_LAUNCH(ctx);
       int64_t runs = 0;
-      HGE_TRY(centroid_batch(ctx, m, L, 0, ug.p + u0, gptr, keys, vals, cptr.p, 0, 0, true, &cidx.p, &cval.p,
-                             &runs));
+      HGE_TRY(centroid_batch(ctx, m, L, 0, ug.p + u0, gptr, keys, vals, cptr.p, 0, 0, true, cidx, cval, &runs));
     }
     const int64_t i0 = h_ustart[(size_t)u0], i1 = h_ustart[(size_t)u1];
     k_merge_named<<<grid_for(ctx, i1 - i0), kBlock, 0, ctx->stream>>>(i0, i1, u0, order, rank.p, ug.p, gptr, px,

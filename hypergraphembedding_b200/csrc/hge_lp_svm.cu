@@ -548,7 +548,7 @@ int hge_lp_svm_predict(hge_ctx* ctx, hge_incidence* inc, int owner_side, const f
   k_training_sets<<<grid_for(ctx, U, kBlock / 32), kBlock, 0, ctx->stream>>>(U, grp.ug.p, mptr, midx, items, poff.p,
                                                                            seed, phase, pid.p, scratch.p);
   HGE_CHECK_LAUNCH(ctx);
-  hge_dev_free(ctx, scratch.p);
+  scratch.reset();
   HGE_TRY(mark(1, last));
 
   // 3. solve: small owners a warp each in one launch, larger ones a CTA each in batches whose

@@ -325,17 +325,17 @@ int hge_p2p_open_peers(hge_p2p* p, const void* handles) {
     tables[2][r] = p->peer_base[r] + p->off_mmx;
     tables[3][r] = p->peer_base[r] + p->off_flags;
   }
-  void** dev[4];
+  DevBuf<void*> dev[4] = {DevBuf<void*>(ctx), DevBuf<void*>(ctx), DevBuf<void*>(ctx), DevBuf<void*>(ctx)};
   for (int k = 0; k < 4; ++k) {
-    HGE_TRY(hge_dev_alloc(ctx, &dev[k], (size_t)p->world));
-    HGE_CUDA(cudaMemcpyAsync(dev[k], tables[k], sizeof(void*) * p->world, cudaMemcpyHostToDevice,
+    HGE_TRY(dev[k].alloc((size_t)p->world));
+    HGE_CUDA(cudaMemcpyAsync(dev[k].p, tables[k], sizeof(void*) * p->world, cudaMemcpyHostToDevice,
                              ctx->stream));
   }
   HGE_CUDA(cudaStreamSynchronize(ctx->stream));
-  p->d_peer_stage = reinterpret_cast<float4**>(dev[0]);
-  p->d_peer_ye = reinterpret_cast<float4**>(dev[1]);
-  p->d_peer_mmx = reinterpret_cast<int32_t**>(dev[2]);
-  p->d_peer_flags = reinterpret_cast<uint32_t**>(dev[3]);
+  p->d_peer_stage = reinterpret_cast<float4**>(dev[0].release());
+  p->d_peer_ye = reinterpret_cast<float4**>(dev[1].release());
+  p->d_peer_mmx = reinterpret_cast<int32_t**>(dev[2].release());
+  p->d_peer_flags = reinterpret_cast<uint32_t**>(dev[3].release());
   p->peers_open = true;
   return HGE_OK;
 }

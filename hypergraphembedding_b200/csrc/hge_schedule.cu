@@ -268,11 +268,6 @@ __global__ void k_piece_bounds(int pieces, int32_t n_units, int unit_cost,
   }
 }
 
-int grid_for(const hge_ctx* ctx, int64_t work, int per_block) {
-  const int64_t want = std::max<int64_t>(1, (work + per_block - 1) / per_block);
-  return (int)std::min<int64_t>(want, (int64_t)ctx->num_sms * 16);
-}
-
 }  // namespace
 
 int hge_sched_begin(hge_ctx* ctx, int32_t row0, int32_t row1, const int64_t* d_ptr,
@@ -293,12 +288,12 @@ int hge_sched_begin_ranges(hge_ctx* ctx, int32_t row0, int32_t row1, const int64
   int bits = 1;
   while (bits < 31 && ((int64_t)1 << bits) <= max_degree_possible) ++bits;
   const uint32_t key_max = (uint32_t)(((int64_t)1 << bits) - 1);
-  uint32_t* keys_in = nullptr;
-  uint32_t* keys_out = nullptr;
-  int32_t* vals_in = nullptr;
-  HGE_TRY(hge_dev_alloc(ctx, &keys_in, (size_t)rows));
-  HGE_TRY(hge_dev_alloc(ctx, &keys_out, (size_t)rows));
-  HGE_TRY(hge_dev_alloc(ctx, &vals_in, (size_t)rows));
+  DevBuf<uint32_t> keys_in(ctx), keys_out(ctx);
+  DevBuf<int32_t> vals_in(ctx);
+  DevBuf<char> temp(ctx);
+  HGE_TRY(keys_in.alloc((size_t)rows));
+  HGE_TRY(keys_out.alloc((size_t)rows));
+  HGE_TRY(vals_in.alloc((size_t)rows));
   HGE_TRY(hge_dev_alloc(ctx, &s->sorted_rows, (size_t)rows));
   HGE_TRY(hge_dev_alloc(ctx, &s->d_stats, (size_t)kStatWords));
   s->h_stats = static_cast<long long*>(hge_ctx_pinned_slot(ctx));
@@ -306,21 +301,16 @@ int hge_sched_begin_ranges(hge_ctx* ctx, int32_t row0, int32_t row1, const int64
   k_sched_init<<<1, 32, 0, ctx->stream>>>(s->d_stats);
   HGE_CHECK_LAUNCH(ctx);
   k_sched_keys<<<grid_for(ctx, rows, kBlock), kBlock, 0, ctx->stream>>>(
-      row0, rows, row_begin, row_end, ctx->light_max_deg, ctx->chunk, key_max, keys_in, vals_in,
+      row0, rows, row_begin, row_end, ctx->light_max_deg, ctx->chunk, key_max, keys_in.p, vals_in.p,
       s->d_stats);
   HGE_CHECK_LAUNCH(ctx);
   size_t temp_bytes = 0;
-  HGE_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, keys_in, keys_out, vals_in,
+  HGE_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, keys_in.p, keys_out.p, vals_in.p,
                                            s->sorted_rows, (int64_t)rows, 0, bits, ctx->stream));
-  char* temp = nullptr;
-  HGE_TRY(hge_dev_alloc(ctx, &temp, temp_bytes));
-  HGE_CUDA(cub::DeviceRadixSort::SortPairs(temp, temp_bytes, keys_in, keys_out, vals_in,
+  HGE_TRY(temp.alloc(temp_bytes));
+  HGE_CUDA(cub::DeviceRadixSort::SortPairs(temp.p, temp_bytes, keys_in.p, keys_out.p, vals_in.p,
                                            s->sorted_rows, (int64_t)rows, 0, bits, ctx->stream));
   ctx->launches += 3;   // histogram + onesweep passes (library kernels, counted approximately)
-  hge_dev_free(ctx, temp);
-  hge_dev_free(ctx, keys_in);
-  hge_dev_free(ctx, keys_out);
-  hge_dev_free(ctx, vals_in);
   HGE_CUDA(cudaMemcpyAsync(s->h_stats, s->d_stats, kStatWords * sizeof(long long),
                            cudaMemcpyDeviceToHost, ctx->stream));
   if (!s->stats_ready) HGE_CUDA(cudaEventCreateWithFlags(&s->stats_ready, cudaEventDisableTiming));
@@ -364,29 +354,24 @@ int hge_sched_finish(hge_ctx* ctx, const char* what, HgeHalfSchedule* s) {
   }
   if (s->n_hrows) {
     const int32_t nh = s->n_hrows;
-    int32_t *nch = nullptr, *npart = nullptr, *coff = nullptr, *poff = nullptr;
-    HGE_TRY(hge_dev_alloc(ctx, &nch, (size_t)nh));
-    HGE_TRY(hge_dev_alloc(ctx, &npart, (size_t)nh));
-    HGE_TRY(hge_dev_alloc(ctx, &coff, (size_t)nh));
-    HGE_TRY(hge_dev_alloc(ctx, &poff, (size_t)nh));
+    DevBuf<int32_t> nch(ctx), npart(ctx), coff(ctx), poff(ctx);
+    DevBuf<char> temp(ctx);
+    HGE_TRY(nch.alloc((size_t)nh));
+    HGE_TRY(npart.alloc((size_t)nh));
+    HGE_TRY(coff.alloc((size_t)nh));
+    HGE_TRY(poff.alloc((size_t)nh));
     k_sched_heavy_counts<<<grid_for(ctx, nh, kBlock), kBlock, 0, ctx->stream>>>(
-        nh, s->sorted_rows, s->ptr, s->row_end, s->chunk_sz, nch, npart);
+        nh, s->sorted_rows, s->ptr, s->row_end, s->chunk_sz, nch.p, npart.p);
     HGE_CHECK_LAUNCH(ctx);
     size_t temp_bytes = 0;
-    HGE_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, nch, coff, nh, ctx->stream));
-    char* temp = nullptr;
-    HGE_TRY(hge_dev_alloc(ctx, &temp, temp_bytes));
-    HGE_CUDA(cub::DeviceScan::ExclusiveSum(temp, temp_bytes, nch, coff, nh, ctx->stream));
-    HGE_CUDA(cub::DeviceScan::ExclusiveSum(temp, temp_bytes, npart, poff, nh, ctx->stream));
+    HGE_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, nch.p, coff.p, nh, ctx->stream));
+    HGE_TRY(temp.alloc(temp_bytes));
+    HGE_CUDA(cub::DeviceScan::ExclusiveSum(temp.p, temp_bytes, nch.p, coff.p, nh, ctx->stream));
+    HGE_CUDA(cub::DeviceScan::ExclusiveSum(temp.p, temp_bytes, npart.p, poff.p, nh, ctx->stream));
     ctx->launches += 2;
     k_sched_heavy_write<<<grid_for(ctx, nh, kBlock / 32), kBlock, 0, ctx->stream>>>(
-        nh, s->sorted_rows, s->ptr, s->row_end, s->invs, s->chunk_sz, coff, poff, s->hrows, s->chunks);
+        nh, s->sorted_rows, s->ptr, s->row_end, s->invs, s->chunk_sz, coff.p, poff.p, s->hrows, s->chunks);
     HGE_CHECK_LAUNCH(ctx);
-    hge_dev_free(ctx, temp);
-    hge_dev_free(ctx, nch);
-    hge_dev_free(ctx, npart);
-    hge_dev_free(ctx, coff);
-    hge_dev_free(ctx, poff);
   }
   hge_dev_free(ctx, s->sorted_rows);
   hge_dev_free(ctx, s->d_stats);
@@ -425,20 +410,20 @@ int hge_sched_stream(hge_ctx* ctx, HgeHalfSchedule* s, int G, int with_own, uint
   t.unit_cost = unit_cost;
   t.n_units = (int32_t)n_units;
   t.n_quads = (int32_t)n_quads;
-  uint32_t* steps = nullptr;
-  HGE_TRY(hge_dev_alloc(ctx, &steps, (size_t)n_units + 1));
+  DevBuf<uint32_t> steps(ctx);
+  DevBuf<char> temp(ctx);
+  HGE_TRY(steps.alloc((size_t)n_units + 1));
   HGE_TRY(hge_dev_alloc(ctx, &t.uoff, (size_t)n_units + 1));
   k_unit_steps<<<grid_for(ctx, n_units + 1, kBlock), kBlock, 0, ctx->stream>>>(
-      t.n_units, s->n_chunks, s->n_light, G, with_own, s->chunk_sz, s->chunks, s->hrows, s->light, steps);
+      t.n_units, s->n_chunks, s->n_light, G, with_own, s->chunk_sz, s->chunks, s->hrows, s->light, steps.p);
   HGE_CHECK_LAUNCH(ctx);
   size_t temp_bytes = 0;
-  HGE_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, steps, t.uoff, n_units + 1, ctx->stream));
-  char* temp = nullptr;
-  HGE_TRY(hge_dev_alloc(ctx, &temp, temp_bytes));
-  HGE_CUDA(cub::DeviceScan::ExclusiveSum(temp, temp_bytes, steps, t.uoff, n_units + 1, ctx->stream));
+  HGE_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, steps.p, t.uoff, n_units + 1, ctx->stream));
+  HGE_TRY(temp.alloc(temp_bytes));
+  HGE_CUDA(cub::DeviceScan::ExclusiveSum(temp.p, temp_bytes, steps.p, t.uoff, n_units + 1, ctx->stream));
   ctx->launches += 1;
-  hge_dev_free(ctx, temp);
-  hge_dev_free(ctx, steps);
+  temp.reset();
+  steps.reset();
   // the one host wait: the stream's length (a 32-bit sum that wrapped shows as a mismatch with
   // the 64-bit bound below)
   uint32_t* h_total = static_cast<uint32_t*>(hge_ctx_pinned_slot(ctx));

@@ -12,18 +12,11 @@
 #include <new>
 
 #include "hge_incidence.cuh"
-#include "hge_staged.cuh"
 
 namespace {
 
 constexpr int kBlock = 256;
 constexpr unsigned kFull = 0xffffffffu;
-
-int grid_for(const hge_ctx* ctx, int64_t work_items, int items_per_block) {
-  int64_t want = (work_items + items_per_block - 1) / items_per_block;
-  if (want < 1) want = 1;
-  return (int)std::min<int64_t>(want, (int64_t)ctx->num_sms * 16);
-}
 
 int lanes_per_row(int ld4) {
   int lpr = 1;
@@ -44,24 +37,20 @@ __global__ void k_pad_rows(int64_t rows, int R, int ld, const float* __restrict_
 
 // Dense [rows, R] rows as float4-addressable [rows, ld]: the input itself when R % 4 == 0.
 struct PaddedRows {
-  const hge_ctx* ctx = nullptr;
+  DevBuf<float> padded;
   const float4* rows4 = nullptr;
-  float* owned = nullptr;
-  int init(hge_ctx* c, const float* x, int64_t rows, int R) {
-    ctx = c;
+  explicit PaddedRows(const hge_ctx* c) : padded(c) {}
+  int init(hge_ctx* ctx, const float* x, int64_t rows, int R) {
     if (R % 4 == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0) {
       rows4 = reinterpret_cast<const float4*>(x);
       return HGE_OK;
     }
     const int ld = (R + 3) & ~3;
-    HGE_TRY(hge_dev_alloc(ctx, &owned, (size_t)rows * ld));
-    k_pad_rows<<<grid_for(c, rows * ld, kBlock), kBlock, 0, c->stream>>>(rows, R, ld, x, owned);
-    HGE_CHECK_LAUNCH(c);
-    rows4 = reinterpret_cast<const float4*>(owned);
+    HGE_TRY(padded.alloc((size_t)rows * ld));
+    k_pad_rows<<<grid_for(ctx, rows * ld, kBlock), kBlock, 0, ctx->stream>>>(rows, R, ld, x, padded.p);
+    HGE_CHECK_LAUNCH(ctx);
+    rows4 = reinterpret_cast<const float4*>(padded.p);
     return HGE_OK;
-  }
-  ~PaddedRows() {
-    if (owned) hge_dev_free(ctx, owned);
   }
 };
 
@@ -381,24 +370,13 @@ int pairs_in_range(hge_ctx* ctx, int64_t n, const int32_t* a, int64_t rows_a, co
     *ok = all;
     return HGE_OK;
   }
-  int* d_bad = nullptr;
-  HGE_TRY(hge_dev_alloc(ctx, &d_bad, 1));
+  DevBuf<int> d_bad(ctx);
+  HGE_TRY(d_bad.alloc(1));
+  HGE_CUDA(cudaMemsetAsync(d_bad.p, 0, sizeof(int), ctx->stream));
+  k_check_pairs<<<grid_for(ctx, n, kBlock * 8), kBlock, 0, ctx->stream>>>(n, a, rows_a, b, rows_b, d_bad.p);
+  HGE_CHECK_LAUNCH(ctx);
   int h_bad = 0;
-  cudaError_t e = cudaMemsetAsync(d_bad, 0, sizeof(int), ctx->stream);
-  if (e == cudaSuccess) {
-    k_check_pairs<<<grid_for(ctx, n, kBlock * 8), kBlock, 0, ctx->stream>>>(n, a, rows_a, b, rows_b,
-                                                                          d_bad);
-    ctx->launches++;
-    e = cudaGetLastError();
-  }
-  if (e == cudaSuccess)
-    e = cudaMemcpyAsync(&h_bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);   // h_bad is on this stack frame
-  hge_dev_free(ctx, d_bad);
-  if (e != cudaSuccess) {
-    hge_set_error("pair index check: %s", cudaGetErrorString(e));
-    return HGE_ERR_CUDA;
-  }
+  HGE_TRY(read_back(ctx, d_bad.p, &h_bad, 1));
   *ok = h_bad == 0;
   return HGE_OK;
 }
@@ -431,37 +409,29 @@ __global__ void k_segment_write(int32_t rows, const int64_t* __restrict__ ptr,
   }
 }
 
-int build_segments(hge_ctx* ctx, int32_t rows, const int64_t* d_ptr, int64_t nnz, Segment** d_segs,
+int build_segments(hge_ctx* ctx, int32_t rows, const int64_t* d_ptr, int64_t nnz, DevBuf<Segment>& segs,
                    int64_t* count) {
-  *d_segs = nullptr;
   *count = 0;
   if (rows <= 0) return HGE_OK;
-  int64_t *counts = nullptr, *offset = nullptr;
-  HGE_TRY(hge_dev_alloc(ctx, &counts, (size_t)rows + 1));
-  HGE_TRY(hge_dev_alloc(ctx, &offset, (size_t)rows + 1));
-  HGE_CUDA(cudaMemsetAsync(counts + rows, 0, sizeof(int64_t), ctx->stream));
+  DevBuf<int64_t> counts(ctx), offset(ctx);
+  DevBuf<char> temp(ctx);
+  HGE_TRY(counts.alloc((size_t)rows + 1));
+  HGE_TRY(offset.alloc((size_t)rows + 1));
+  HGE_CUDA(cudaMemsetAsync(counts.p + rows, 0, sizeof(int64_t), ctx->stream));
   const int grid = grid_for(ctx, rows, kBlock);
-  k_segment_counts<<<grid, kBlock, 0, ctx->stream>>>(rows, d_ptr, counts);
+  k_segment_counts<<<grid, kBlock, 0, ctx->stream>>>(rows, d_ptr, counts.p);
   HGE_CHECK_LAUNCH(ctx);
   size_t temp_bytes = 0;
-  HGE_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, counts, offset, rows + 1, ctx->stream));
-  char* temp = nullptr;
-  HGE_TRY(hge_dev_alloc(ctx, &temp, temp_bytes));
-  HGE_CUDA(cub::DeviceScan::ExclusiveSum(temp, temp_bytes, counts, offset, rows + 1, ctx->stream));
+  HGE_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, temp_bytes, counts.p, offset.p, rows + 1, ctx->stream));
+  HGE_TRY(temp.alloc(temp_bytes));
+  HGE_CUDA(cub::DeviceScan::ExclusiveSum(temp.p, temp_bytes, counts.p, offset.p, rows + 1, ctx->stream));
   ctx->launches += 1;
   // the segment count is bounded without a read-back: every row adds at most one partial segment
   const int64_t bound = nnz / kSegment + rows;
-  HGE_TRY(hge_dev_alloc(ctx, d_segs, (size_t)bound));
-  k_segment_write<<<grid, kBlock, 0, ctx->stream>>>(rows, d_ptr, offset, *d_segs);
+  HGE_TRY(segs.alloc((size_t)bound));
+  k_segment_write<<<grid, kBlock, 0, ctx->stream>>>(rows, d_ptr, offset.p, segs.p);
   HGE_CHECK_LAUNCH(ctx);
-  int64_t total = 0;
-  HGE_CUDA(cudaMemcpyAsync(&total, offset + rows, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
-  HGE_CUDA(cudaStreamSynchronize(ctx->stream));
-  hge_dev_free(ctx, temp);
-  hge_dev_free(ctx, counts);
-  hge_dev_free(ctx, offset);
-  *count = total;
-  return HGE_OK;
+  return read_back(ctx, offset.p + rows, count, 1);
 }
 
 #define HGE_DISPATCH_LPR(lpr, CALL) \
@@ -485,16 +455,16 @@ int hge_incidence_l2(hge_ctx* ctx, hge_incidence* inc, const float* xn, const fl
   HGE_REQUIRE(order == 0 || order == 1, "hge_incidence_l2: order must be 0 or 1");
   HGE_CUDA(cudaSetDevice(ctx->device));
   const HgeHalfSchedule& half = order == 0 ? inc->node_half : inc->edge_half;
-  Staged<float> s_xn, s_xe, s_out;
-  HGE_TRY(s_xn.init(ctx, xn, (size_t)inc->N * R, mem, true, false));
-  HGE_TRY(s_xe.init(ctx, xe, (size_t)inc->E * R, mem, true, false));
-  HGE_TRY(s_out.init(ctx, dist, (size_t)half.nnz, mem, false, true));
-  PaddedRows pn, pe;
+  Staged<float> s_xn(ctx), s_xe(ctx), s_out(ctx);
+  HGE_TRY(s_xn.init(xn, (size_t)inc->N * R, mem, true, false));
+  HGE_TRY(s_xe.init(xe, (size_t)inc->E * R, mem, true, false));
+  HGE_TRY(s_out.init(dist, (size_t)half.nnz, mem, false, true));
+  PaddedRows pn(ctx), pe(ctx);
   HGE_TRY(pn.init(ctx, s_xn.dev, inc->N, R));
   HGE_TRY(pe.init(ctx, s_xe.dev, inc->E, R));
-  Segment* segs = nullptr;
+  DevBuf<Segment> segs(ctx);
   int64_t nseg = 0;
-  HGE_TRY(build_segments(ctx, half.rows, half.ptr, half.nnz, &segs, &nseg));
+  HGE_TRY(build_segments(ctx, half.rows, half.ptr, half.nnz, segs, &nseg));
   const int ld4 = ((R + 3) & ~3) / 4;
   const float max_dist = (float)sqrt((double)R);
   const float4* self = order == 0 ? pn.rows4 : pe.rows4;
@@ -502,14 +472,8 @@ int hge_incidence_l2(hge_ctx* ctx, hge_incidence* inc, const float* xn, const fl
   const int grid = grid_for(ctx, nseg, kBlock / 32);
   HGE_DISPATCH_LPR(lanes_per_row(ld4),
                    (k_incidence_l2<L><<<grid, kBlock, 0, ctx->stream>>>(
-                       nseg, segs, half.idx, self, other, ld4, max_dist, as_weight, s_out.dev)));
-  ctx->launches++;
-  cudaError_t e = cudaGetLastError();
-  hge_dev_free(ctx, segs);
-  if (e != cudaSuccess) {
-    hge_set_error("hge_incidence_l2: launch failed: %s", cudaGetErrorString(e));
-    return HGE_ERR_CUDA;
-  }
+                       nseg, segs.p, half.idx, self, other, ld4, max_dist, as_weight, s_out.dev)));
+  HGE_CHECK_LAUNCH(ctx);
   return s_out.finish();
 }
 
@@ -525,31 +489,24 @@ int hge_pair_l2(hge_ctx* ctx, const float* xa, int64_t rows_a, const float* xb, 
   HGE_TRY(pairs_in_range(ctx, num_pairs, ia, rows_a, ib, rows_b, mem, &ok));
   HGE_REQUIRE(ok, "hge_pair_l2: a pair names a row outside [0, %lld) x [0, %lld)", (long long)rows_a,
               (long long)rows_b);
-  Staged<float> s_xa, s_xb, s_out;
-  Staged<int32_t> s_ia, s_ib;
-  HGE_TRY(s_xa.init(ctx, xa, (size_t)rows_a * R, mem, true, false));
-  if (xb == xa) {
-    s_xb.ctx = ctx;
-    s_xb.dev = s_xa.dev;
-  } else {
-    HGE_TRY(s_xb.init(ctx, xb, (size_t)rows_b * R, mem, true, false));
-  }
-  HGE_TRY(s_ia.init(ctx, ia, (size_t)num_pairs, mem, true, false));
-  HGE_TRY(s_ib.init(ctx, ib, (size_t)num_pairs, mem, true, false));
-  HGE_TRY(s_out.init(ctx, dist, (size_t)num_pairs, mem, false, true));
-  PaddedRows pa, pb;
+  // xb == xa (distances inside one table) is staged and padded once
+  const bool same = xb == xa;
+  Staged<float> s_xa(ctx), s_xb(ctx), s_out(ctx);
+  Staged<int32_t> s_ia(ctx), s_ib(ctx);
+  HGE_TRY(s_xa.init(xa, (size_t)rows_a * R, mem, true, false));
+  if (!same) HGE_TRY(s_xb.init(xb, (size_t)rows_b * R, mem, true, false));
+  HGE_TRY(s_ia.init(ia, (size_t)num_pairs, mem, true, false));
+  HGE_TRY(s_ib.init(ib, (size_t)num_pairs, mem, true, false));
+  HGE_TRY(s_out.init(dist, (size_t)num_pairs, mem, false, true));
+  PaddedRows pa(ctx), pb(ctx);
   HGE_TRY(pa.init(ctx, s_xa.dev, rows_a, R));
-  if (s_xb.dev == s_xa.dev) {
-    pb.ctx = ctx;
-    pb.rows4 = pa.rows4;
-  } else {
-    HGE_TRY(pb.init(ctx, s_xb.dev, rows_b, R));
-  }
+  if (!same) HGE_TRY(pb.init(ctx, s_xb.dev, rows_b, R));
+  const float4* rows_b4 = same ? pa.rows4 : pb.rows4;
   const int ld4 = ((R + 3) & ~3) / 4;
   const int grid = grid_for(ctx, (num_pairs + 31) / 32, kBlock / 32);
   HGE_DISPATCH_LPR(lanes_per_row(ld4),
                    (k_pair_l2<L><<<grid, kBlock, 0, ctx->stream>>>(
-                       num_pairs, s_ia.dev, s_ib.dev, pa.rows4, pb.rows4, ld4, s_out.dev)));
+                       num_pairs, s_ia.dev, s_ib.dev, pa.rows4, rows_b4, ld4, s_out.dev)));
   HGE_CHECK_LAUNCH(ctx);
   return s_out.finish();
 }
@@ -562,38 +519,24 @@ int hge_scale_transform(hge_ctx* ctx, float* values, int64_t n, double alpha, fl
   HGE_REQUIRE(n >= 0, "hge_scale_transform: negative count");
   if (n == 0) return HGE_OK;   // ZeroOneScaleValues({}) == {}
   HGE_CUDA(cudaSetDevice(ctx->device));
-  Staged<float> s_v;
-  HGE_TRY(s_v.init(ctx, values, (size_t)n, mem, true, true));
-  int32_t* mm = nullptr;
-  HGE_TRY(hge_dev_alloc(ctx, &mm, 2));
-  k_minmax_init<<<1, 1, 0, ctx->stream>>>(mm);
+  Staged<float> s_v(ctx);
+  HGE_TRY(s_v.init(values, (size_t)n, mem, true, true));
+  DevBuf<int32_t> mm(ctx);
+  HGE_TRY(mm.alloc(2));
+  k_minmax_init<<<1, 1, 0, ctx->stream>>>(mm.p);
   ctx->launches++;
   const int grid = grid_for(ctx, n, kBlock * 8);
-  k_minmax<<<grid, kBlock, 0, ctx->stream>>>(n, s_v.dev, mm);
+  k_minmax<<<grid, kBlock, 0, ctx->stream>>>(n, s_v.dev, mm.p);
   ctx->launches++;
-  k_scale_transform<<<grid, kBlock, 0, ctx->stream>>>(n, s_v.dev, mm, (float)alpha,
+  k_scale_transform<<<grid, kBlock, 0, ctx->stream>>>(n, s_v.dev, mm.p, (float)alpha,
                                                       (float)(1.0 - alpha));
-  ctx->launches++;
-  cudaError_t e = cudaGetLastError();
-  int rc = HGE_OK;
-  if (e != cudaSuccess) {
-    hge_set_error("hge_scale_transform: launch failed: %s", cudaGetErrorString(e));
-    rc = HGE_ERR_CUDA;
-  }
-  if (rc == HGE_OK && minmax) {
+  HGE_CHECK_LAUNCH(ctx);
+  if (minmax) {
     int32_t h[2];
-    e = cudaMemcpyAsync(h, mm, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) {
-      hge_set_error("hge_scale_transform: reading min/max failed: %s", cudaGetErrorString(e));
-      rc = HGE_ERR_CUDA;
-    } else {
-      minmax[0] = hge_dec(h[0]);
-      minmax[1] = hge_dec(h[1]);
-    }
+    HGE_TRY(read_back(ctx, mm.p, h, 2));
+    minmax[0] = hge_dec(h[0]);
+    minmax[1] = hge_dec(h[1]);
   }
-  hge_dev_free(ctx, mm);
-  if (rc != HGE_OK) return rc;
   return s_v.finish();
 }
 
@@ -605,22 +548,16 @@ int hge_scale_minmax(hge_ctx* ctx, const float* values, int64_t n, float* minmax
   minmax[0] = INFINITY;
   minmax[1] = -INFINITY;
   if (n == 0) return HGE_OK;
-  Staged<float> s_v;
-  HGE_TRY(s_v.init(ctx, values, (size_t)n, mem, true, false));
-  int32_t* mm = nullptr;
-  HGE_TRY(hge_dev_alloc(ctx, &mm, 2));
-  k_minmax_init<<<1, 1, 0, ctx->stream>>>(mm);
+  Staged<float> s_v(ctx);
+  HGE_TRY(s_v.init(values, (size_t)n, mem, true, false));
+  DevBuf<int32_t> mm(ctx);
+  HGE_TRY(mm.alloc(2));
+  k_minmax_init<<<1, 1, 0, ctx->stream>>>(mm.p);
   ctx->launches++;
-  k_minmax<<<grid_for(ctx, n, kBlock * 8), kBlock, 0, ctx->stream>>>(n, s_v.dev, mm);
-  ctx->launches++;
+  k_minmax<<<grid_for(ctx, n, kBlock * 8), kBlock, 0, ctx->stream>>>(n, s_v.dev, mm.p);
+  HGE_CHECK_LAUNCH(ctx);
   int32_t h[2];
-  cudaError_t e = cudaMemcpyAsync(h, mm, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-  hge_dev_free(ctx, mm);
-  if (e != cudaSuccess) {
-    hge_set_error("hge_scale_minmax: %s", cudaGetErrorString(e));
-    return HGE_ERR_CUDA;
-  }
+  HGE_TRY(read_back(ctx, mm.p, h, 2));
   minmax[0] = hge_dec(h[0]);
   minmax[1] = hge_dec(h[1]);
   return HGE_OK;
@@ -634,24 +571,16 @@ int hge_scale_apply(hge_ctx* ctx, float* values, int64_t n, double alpha, float 
   HGE_REQUIRE(lo <= hi, "hge_scale_apply: min %g > max %g", lo, hi);
   if (n == 0) return HGE_OK;
   HGE_CUDA(cudaSetDevice(ctx->device));
-  Staged<float> s_v;
-  HGE_TRY(s_v.init(ctx, values, (size_t)n, mem, true, true));
-  int32_t* mm = nullptr;
-  HGE_TRY(hge_dev_alloc(ctx, &mm, 2));
+  Staged<float> s_v(ctx);
+  HGE_TRY(s_v.init(values, (size_t)n, mem, true, true));
+  DevBuf<int32_t> mm(ctx);
+  HGE_TRY(mm.alloc(2));
   const int32_t h[2] = {hge_enc(lo), hge_enc(hi)};
-  cudaError_t e = cudaMemcpyAsync(mm, h, sizeof(h), cudaMemcpyHostToDevice, ctx->stream);
-  if (e == cudaSuccess) {
-    k_scale_transform<<<grid_for(ctx, n, kBlock * 8), kBlock, 0, ctx->stream>>>(
-        n, s_v.dev, mm, (float)alpha, (float)(1.0 - alpha));
-    ctx->launches++;
-    e = cudaGetLastError();
-  }
-  if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);   // h is on this stack frame
-  hge_dev_free(ctx, mm);
-  if (e != cudaSuccess) {
-    hge_set_error("hge_scale_apply: %s", cudaGetErrorString(e));
-    return HGE_ERR_CUDA;
-  }
+  HGE_CUDA(cudaMemcpyAsync(mm.p, h, sizeof(h), cudaMemcpyHostToDevice, ctx->stream));
+  k_scale_transform<<<grid_for(ctx, n, kBlock * 8), kBlock, 0, ctx->stream>>>(
+      n, s_v.dev, mm.p, (float)alpha, (float)(1.0 - alpha));
+  HGE_CHECK_LAUNCH(ctx);
+  HGE_CUDA(cudaStreamSynchronize(ctx->stream));   // h is on this stack frame
   return s_v.finish();
 }
 
@@ -662,11 +591,11 @@ int hge_row_span(hge_ctx* ctx, hge_incidence* inc, const float* xn, const float*
   HGE_REQUIRE(side == 0 || side == 1, "hge_row_span: side must be 0 or 1");
   HGE_CUDA(cudaSetDevice(ctx->device));
   const HgeHalfSchedule& half = side == 0 ? inc->node_half : inc->edge_half;
-  Staged<float> s_xn, s_xe, s_out;
-  HGE_TRY(s_xn.init(ctx, xn, (size_t)inc->N * R, mem, true, false));
-  HGE_TRY(s_xe.init(ctx, xe, (size_t)inc->E * R, mem, true, false));
-  HGE_TRY(s_out.init(ctx, span, (size_t)half.rows, mem, false, true));
-  PaddedRows pn, pe;
+  Staged<float> s_xn(ctx), s_xe(ctx), s_out(ctx);
+  HGE_TRY(s_xn.init(xn, (size_t)inc->N * R, mem, true, false));
+  HGE_TRY(s_xe.init(xe, (size_t)inc->E * R, mem, true, false));
+  HGE_TRY(s_out.init(span, (size_t)half.rows, mem, false, true));
+  PaddedRows pn(ctx), pe(ctx);
   HGE_TRY(pn.init(ctx, s_xn.dev, inc->N, R));
   HGE_TRY(pe.init(ctx, s_xe.dev, inc->E, R));
   const int ld4 = ((R + 3) & ~3) / 4;
@@ -692,12 +621,12 @@ int hge_same_type_prob(hge_ctx* ctx, hge_incidence* inc, int side, const float* 
   bool ok = false;
   HGE_TRY(pairs_in_range(ctx, num_pairs, pi, half.rows, pj, half.rows, mem, &ok));
   HGE_REQUIRE(ok, "hge_same_type_prob: a pair names a row outside [0, %d)", half.rows);
-  Staged<float> s_w, s_out;
-  Staged<int32_t> s_i, s_j;
-  HGE_TRY(s_w.init(ctx, w, (size_t)half.nnz, mem, true, false));
-  HGE_TRY(s_i.init(ctx, pi, (size_t)num_pairs, mem, true, false));
-  HGE_TRY(s_j.init(ctx, pj, (size_t)num_pairs, mem, true, false));
-  HGE_TRY(s_out.init(ctx, prob, (size_t)num_pairs, mem, false, true));
+  Staged<float> s_w(ctx), s_out(ctx);
+  Staged<int32_t> s_i(ctx), s_j(ctx);
+  HGE_TRY(s_w.init(w, (size_t)half.nnz, mem, true, false));
+  HGE_TRY(s_i.init(pi, (size_t)num_pairs, mem, true, false));
+  HGE_TRY(s_j.init(pj, (size_t)num_pairs, mem, true, false));
+  HGE_TRY(s_out.init(prob, (size_t)num_pairs, mem, false, true));
   const double mean_deg = (double)half.nnz / std::max(1, half.rows);
   if (mean_deg <= 24.0) {
     const int grid = grid_for(ctx, num_pairs, kBlock / 8);
@@ -722,12 +651,12 @@ int hge_diff_type_prob(hge_ctx* ctx, hge_incidence* inc, const float* w_e2n, con
   HGE_TRY(pairs_in_range(ctx, num_pairs, pn, inc->N, pe, inc->E, mem, &ok));
   HGE_REQUIRE(ok, "hge_diff_type_prob: a pair names a node outside [0, %d) or an edge outside [0, %d)",
               inc->N, inc->E);
-  Staged<float> s_w, s_out;
-  Staged<int32_t> s_n, s_e;
-  HGE_TRY(s_w.init(ctx, w_e2n, (size_t)inc->edge_half.nnz, mem, true, false));
-  HGE_TRY(s_n.init(ctx, pn, (size_t)num_pairs, mem, true, false));
-  HGE_TRY(s_e.init(ctx, pe, (size_t)num_pairs, mem, true, false));
-  HGE_TRY(s_out.init(ctx, prob, (size_t)num_pairs, mem, false, true));
+  Staged<float> s_w(ctx), s_out(ctx);
+  Staged<int32_t> s_n(ctx), s_e(ctx);
+  HGE_TRY(s_w.init(w_e2n, (size_t)inc->edge_half.nnz, mem, true, false));
+  HGE_TRY(s_n.init(pn, (size_t)num_pairs, mem, true, false));
+  HGE_TRY(s_e.init(pe, (size_t)num_pairs, mem, true, false));
+  HGE_TRY(s_out.init(prob, (size_t)num_pairs, mem, false, true));
   const int grid = grid_for(ctx, num_pairs, kBlock / 32);
   k_diff_type_prob<<<grid, kBlock, 0, ctx->stream>>>(num_pairs, inc->n2e_ptr, inc->n2e_idx,
                                                      inc->e2n_ptr, inc->e2n_idx, s_w.dev, s_n.dev,

@@ -148,10 +148,10 @@ class Hg2vModel(object):
     feats = np.ascontiguousarray(np.stack([np.asarray(c).reshape(-1) for c in x]), dtype=np.int32)
     targets = np.ascontiguousarray(np.stack([np.asarray(c).reshape(-1) for c in y]), dtype=np.float32)
     assert feats.shape[1] == targets.shape[1]
-    self.num_samples = feats.shape[1]
     _native.check(self.ctx.lib.hge_hg2v_set_samples(self.handle, _native.ptr(feats), _native.ptr(targets),
-                                                    self.num_samples, _native.MEM_HOST),
+                                                    feats.shape[1], _native.MEM_HOST),
                   "hge_hg2v_set_samples")
+    self.num_samples = feats.shape[1]
 
   def fit_epoch(self, order, batch_size):
     order = np.ascontiguousarray(order, dtype=np.int32)

@@ -144,14 +144,37 @@ def test_fit_shuffles_with_the_global_rng_and_stops_early():
 
 
 def test_bad_indices_are_refused():
+  import ctypes
   from hypergraphembedding_b200.hg2v_model import UnweightedFloatModel
   feats, targets = _random_problem(0, k=1, m=50)
   model = UnweightedFloatModel(_Graph(300, 120), 4, 1)
   feats[0][7] = 302                                  # rows are 0 .. 300
+  good, good_targets = _random_problem(1, k=1, m=40)
+  model.set_samples(good, good_targets)
   with pytest.raises(AssertionError):
     model.set_samples(feats, targets)
   with pytest.raises(AssertionError):
     model.set_samples(feats[:-1], targets)
+  # a refused call leaves the samples of the last accepted one
+  assert model.num_samples == 40
+  got, got_targets = model.samples()
+  assert all(np.array_equal(a, b) for a, b in zip(got + got_targets, good + good_targets))
+  model.close()
+  # and on a fresh model, none: there is nothing to read back and nothing to train on
+  from hypergraphembedding_b200 import _native
+  fresh = UnweightedFloatModel(_Graph(300, 120), 4, 1)
+  try:
+    with pytest.raises(AssertionError):
+      fresh.set_samples(feats, targets)
+    lib = fresh.ctx.lib
+    _native.check(lib.hge_hg2v_get_samples(fresh.handle, None, None, _native.MEM_HOST), "hge_hg2v_get_samples")
+    order = np.arange(50, dtype=np.int32)
+    loss = ctypes.c_double()
+    with pytest.raises(AssertionError, match="no samples"):
+      _native.check(lib.hge_hg2v_fit_epoch(fresh.handle, _native.ptr(order), 8, _native.MEM_HOST,
+                                           ctypes.byref(loss)))
+  finally:
+    fresh.close()
 
 
 @pytest.mark.parametrize("method", ["HG2V_ALG_DIST", "HG2V_BOOLEAN", "HG2V_NEIGH_JAC"])

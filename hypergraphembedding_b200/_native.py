@@ -83,7 +83,7 @@ SIGNATURES = {
     "hge_algdist_ld": (ctypes.c_int, [c_vp]),
     "hge_algdist_store": (ctypes.c_int, [c_vp, ctypes.c_int, c_vp, c_vp, ctypes.c_int]),
     "hge_p2p_create": (ctypes.c_int, [c_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int32, ctypes.c_int32,
-                                      ctypes.c_int, ctypes.c_int, ctypes.POINTER(c_vp)]),
+                                      ctypes.c_int, ctypes.POINTER(c_vp)]),
     "hge_p2p_export": (ctypes.c_int, [c_vp, c_vp]),
     "hge_p2p_open_peers": (ctypes.c_int, [c_vp, c_vp]),
     "hge_p2p_check": (ctypes.c_int, [c_vp]),
@@ -874,11 +874,10 @@ def lp_svm_predict(ctx, inc, owner_side, vectors, items, owners, seed, C=1.0, ga
 class PeerArena(object):
   """hge_p2p: the IPC-shared exchange arena of one shard."""
 
-  def __init__(self, ctx, rank, world, num_local_nodes, num_edges, ld, slices=0):
-    """slices: pipelining depth of the exchange (0 = the library's default, 1 = not pipelined)."""
+  def __init__(self, ctx, rank, world, num_local_nodes, num_edges, ld):
     self.ctx = ctx
     handle = c_vp()
-    check(ctx.lib.hge_p2p_create(ctx.handle, rank, world, num_local_nodes, num_edges, ld, int(slices),
+    check(ctx.lib.hge_p2p_create(ctx.handle, rank, world, num_local_nodes, num_edges, ld,
                                  ctypes.byref(handle)), "hge_p2p_create")
     self.handle = handle
     self.world = world

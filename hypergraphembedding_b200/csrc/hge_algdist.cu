@@ -187,8 +187,7 @@ __global__ void k_count_tile_pairs(int64_t total, int32_t rows, const int64_t* _
 // Reduce-scatter of locally accumulated partial rows [row0, row0 + rows): a row goes to the
 // staging block of its owner, slot `rank` (the push the gather kernel does itself when untiled).
 __global__ void k_push_rows(int32_t row0, int32_t rows, int ld4, const float4* __restrict__ raw,
-                            float4* const* __restrict__ peer_stage, int32_t own_rows, int rank,
-                            HgeOwnerMap map) {
+                            float4* const* __restrict__ peer_stage, int rank, HgeOwnerMap map) {
   const int64_t total = (int64_t)rows * ld4;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total;
        i += (int64_t)gridDim.x * blockDim.x) {
@@ -197,7 +196,7 @@ __global__ void k_push_rows(int32_t row0, int32_t rows, int ld4, const float4* _
     int owner;
     int32_t idx;
     map.locate(r, owner, idx);
-    peer_stage[owner][((size_t)rank * own_rows + idx) * ld4 + c4] = __ldcs(raw + (size_t)r * ld4 + c4);
+    peer_stage[owner][((size_t)rank * map.sub_rows + idx) * ld4 + c4] = __ldcs(raw + (size_t)r * ld4 + c4);
   }
 }
 
@@ -388,40 +387,6 @@ int sweep_blocks(const hge_algdist* st, const HgeHalfSchedule& s, int G) {
   return (int)std::min<int64_t>((int64_t)per_sm * ctx->num_sms, want);
 }
 
-HgeSweepSrc sweep_src(const hge_algdist* st, const HgeHalfSchedule& s, float4* partials, int32_t* counters) {
-  const HgeStream& t = s.stream;
-  HgeSweepSrc src;
-  src.stream = t.ids;
-  src.items = t.items;
-  src.uoff = t.uoff;
-  src.piece = t.piece;
-  src.hrows = s.hrows;
-  src.chunks = s.chunks;
-  src.n_chunks = s.n_chunks;
-  src.n_hrows = s.n_hrows;
-  src.partials = partials;
-  src.counters = counters;
-  (void)st;
-  return src;
-}
-
-// everything of the launch arguments that does not depend on the schedule
-void fill_sweep_args(const hge_algdist* st, bool node_half, int sweep, float* raw, const hge_p2p* push,
-                     HgeSweepArgs* a) {
-  a->base = reinterpret_cast<const float4*>(st->ye);
-  a->own = reinterpret_cast<float4*>(node_half ? st->yn : st->ye);
-  a->mm_prev = sweep > 0 ? st->mm + (size_t)(sweep - 1) * 2 * st->ld : nullptr;
-  a->mm_cur = st->mm + (size_t)sweep * 2 * st->ld;
-  a->raw = reinterpret_cast<float4*>(raw);
-  a->push_stage = push ? push->d_peer_stage : nullptr;
-  a->push_rows = push ? push->own_rows : 1;
-  a->push_rank = push ? push->rank : 0;
-  a->push_map.slice_rows = push ? push->slice_rows : 1;
-  a->push_map.sub_rows = push ? push->sub_rows : 1;
-  a->R = st->R;
-  a->ld4 = st->ld4;
-}
-
 int run_half_stream(hge_algdist* st, HgeHalfSchedule& s, bool node_half, int sweep, float* raw,
                     const hge_p2p* push, bool accumulate) {
   hge_ctx* ctx = st->ctx;
@@ -438,8 +403,26 @@ int run_half_stream(hge_algdist* st, HgeHalfSchedule& s, bool node_half, int swe
   const int blocks = sweep_blocks(st, s, G);
   HGE_TRY(hge_sched_stream(ctx, &s, G, with_own, gather0, own0, st->zero_row, blocks * kWarps));
   HgeSweepArgs a = {};
-  a.src = sweep_src(st, s, st->partials, st->counters);
-  fill_sweep_args(st, node_half, sweep, raw, push, &a);
+  a.src.stream = s.stream.ids;
+  a.src.items = s.stream.items;
+  a.src.uoff = s.stream.uoff;
+  a.src.piece = s.stream.piece;
+  a.src.hrows = s.hrows;
+  a.src.chunks = s.chunks;
+  a.src.n_chunks = s.n_chunks;
+  a.src.n_hrows = s.n_hrows;
+  a.src.partials = st->partials;
+  a.src.counters = st->counters;
+  a.base = reinterpret_cast<const float4*>(st->ye);
+  a.own = reinterpret_cast<float4*>(node_half ? st->yn : st->ye);
+  a.mm_prev = sweep > 0 ? st->mm + (size_t)(sweep - 1) * 2 * st->ld : nullptr;
+  a.mm_cur = st->mm + (size_t)sweep * 2 * st->ld;
+  a.raw = reinterpret_cast<float4*>(raw);
+  a.push_stage = push ? push->d_peer_stage : nullptr;
+  a.push_rank = push ? push->rank : 0;
+  a.push_map.sub_rows = push ? push->sub_rows : 1;
+  a.R = st->R;
+  a.ld4 = st->ld4;
   return hge_sweep_launch(ctx, a, st->lpr, mode, blocks, st->slabs);
 }
 
@@ -947,123 +930,21 @@ int hge_algdist_edge_finalize(hge_algdist* st, int sweep, int slice, const float
   return HGE_OK;
 }
 
-// The sharded edge gather with the partial rows pushed to their owners: slice >= 0 gathers only
-// that slice of the edge rows (the pipelined peer-memory sweep), slice < 0 all of them.
-int hge_internal_edge_push(hge_algdist* st, int sweep, int slice) {
+// The sharded edge gather with the partial rows pushed to their owners.
+int hge_internal_edge_push(hge_algdist* st, int sweep) {
   hge_p2p* p = st->p2p;
-  if (!st->tile_raw) {
-    HgeHalfSchedule* sched = slice >= 0 ? &p->slice_sched[(size_t)slice] : nullptr;
-    return run_half(st, false, sweep, nullptr, -1, p, sched);
-  }
-  // tiled: the local partial sums are accumulated tile by tile, then pushed to their owners (in
-  // one piece: the tiles already walk all edges, there is nothing to pipeline the exchange with)
+  if (!st->tile_raw) return run_half(st, false, sweep, nullptr, -1, p);
+  // tiled: the local partial sums are accumulated tile by tile, then pushed to their owners
   hge_ctx* ctx = st->ctx;
   hge_incidence* inc = st->inc;
-  HGE_REQUIRE(slice < 0, "hge_internal_edge_push: the tiled edge half is not sliced");
   HGE_CUDA(cudaMemsetAsync(st->tile_raw, 0, (size_t)inc->E * st->ld * sizeof(float), ctx->stream));
   for (size_t t = 0; t < inc->edge_tiles.size(); ++t)
     HGE_TRY(run_half(st, false, sweep, st->tile_raw, -1, nullptr, &inc->edge_tiles[t], true));
   HgeOwnerMap map;
-  map.slice_rows = p->slice_rows;
   map.sub_rows = p->sub_rows;
   k_push_rows<<<grid_for(ctx, (int64_t)inc->E * st->ld4, kBlock, kBlocksPerSm), kBlock, 0, ctx->stream>>>(
-      0, inc->E, st->ld4, reinterpret_cast<const float4*>(st->tile_raw), p->d_peer_stage, p->own_rows,
-      p->rank, map);
+      0, inc->E, st->ld4, reinterpret_cast<const float4*>(st->tile_raw), p->d_peer_stage, p->rank, map);
   HGE_CHECK_LAUNCH(ctx);
-  return HGE_OK;
-}
-
-// The pipelined peer-memory sweep: ONE launch gathers all slices of the edge rows, slice-major
-// (HgeSweepDyn, hge_sweep.cuh), and announces every finished slice to all ranks.  The grid leaves
-// p->reserve_blocks block slots free so that the owner-side kernels of the finished slices run
-// next to it.
-int hge_internal_edge_push_dynamic(hge_algdist* st, int sweep) {
-  hge_p2p* p = st->p2p;
-  hge_ctx* ctx = st->ctx;
-  HGE_REQUIRE(!p->slice_sched.empty() && !st->tile_raw, "hge_internal_edge_push_dynamic: no slice schedules");
-  const int G = 32 / st->lpr;
-  const int S = (int)p->slice_sched.size();
-  const int64_t yn_row = (st->yn - st->ye) / st->ld;
-  const int resident = ctx->num_sms * st->sweep_resident;
-  const int blocks = std::max(ctx->num_sms, resident - p->reserve_blocks);
-  // pieces per slice: a few per warp, so that the claims even out what the cost model of the
-  // pieces gets wrong (the static launches use a second wave of blocks for that)
-  int per_warp = 2;
-  if (const char* env = getenv("HGE_DYN_PIECES_PER_WARP")) per_warp = std::max(1, std::min(16, atoi(env)));
-  const int pieces = blocks * kWarps * per_warp;
-  std::vector<HgeSweepSrc> srcs((size_t)S);
-  size_t part_off = 0, cnt_off = 0;
-  for (int k = 0; k < S; ++k) {
-    HgeHalfSchedule& sl = p->slice_sched[(size_t)k];
-    HGE_TRY(hge_sched_stream(ctx, &sl, G, 0, (uint32_t)yn_row, 0u, st->zero_row, pieces));
-    srcs[(size_t)k] = sweep_src(st, sl, st->partials + part_off * st->ld4, st->counters + cnt_off * st->slabs);
-    part_off += (size_t)sl.n_partials;
-    cnt_off += (size_t)sl.n_hrows;
-  }
-  const size_t bytes = srcs.size() * sizeof(HgeSweepSrc);
-  if (!p->d_dyn_src) {
-    HGE_CUDA(cudaMalloc(&p->d_dyn_src, 16 * sizeof(HgeSweepSrc)));
-    HGE_CUDA(cudaMalloc(reinterpret_cast<void**>(&p->d_dyn_ctr), 17 * sizeof(int32_t)));
-    HGE_CUDA(cudaMemsetAsync(p->d_dyn_ctr, 0, 17 * sizeof(int32_t), ctx->stream));
-  }
-  if (p->h_dyn_src.size() != bytes || memcmp(p->h_dyn_src.data(), srcs.data(), bytes) != 0) {
-    p->h_dyn_src.assign(reinterpret_cast<const char*>(srcs.data()), reinterpret_cast<const char*>(srcs.data()) + bytes);
-    // pageable source: the copy has left the host buffer when the call returns
-    HGE_CUDA(cudaMemcpyAsync(p->d_dyn_src, p->h_dyn_src.data(), bytes, cudaMemcpyHostToDevice, ctx->stream));
-  }
-  p->dyn_pieces = pieces;
-  HGE_CUDA(cudaMemsetAsync(p->d_dyn_ctr, 0, sizeof(int32_t), ctx->stream));   // the work-item counter
-  HgeSweepArgs a = {};
-  a.src = srcs[0];
-  fill_sweep_args(st, false, sweep, nullptr, p, &a);
-  a.dyn.src = static_cast<const HgeSweepSrc*>(p->d_dyn_src);
-  a.dyn.slices = S;
-  a.dyn.pieces = pieces;
-  a.dyn.next = p->d_dyn_ctr;
-  a.dyn.done = p->d_dyn_ctr + 1;
-  a.dyn.peer_flags = p->d_peer_flags;
-  a.dyn.seq = p->sweep_seq;
-  a.dyn.flag0 = p->world;          // the first `world` flags are the plain barrier's
-  a.dyn.rank = p->rank;
-  a.dyn.world = p->world;
-  a.dyn.flag_stride = 32;
-  return hge_sweep_launch(ctx, a, st->lpr, kSweepPush, blocks, st->slabs);
-}
-
-// Builds the per-slice schedules of a shard's edge half (hge_algdist_attach_p2p).
-int hge_internal_slice_schedules(hge_algdist* st) {
-  hge_p2p* p = st->p2p;
-  hge_incidence* inc = st->inc;
-  hge_ctx* ctx = st->ctx;
-  for (HgeHalfSchedule& sl : p->slice_sched) hge_sched_release(ctx, &sl);
-  p->slice_sched.clear();
-  if (p->slices <= 1 || st->tile_raw) return HGE_OK;
-  p->slice_sched.resize((size_t)p->slices);
-  for (int k = 0; k < p->slices; ++k) {
-    const int32_t r0 = (int32_t)std::min<int64_t>((int64_t)k * p->slice_rows, inc->E);
-    const int32_t r1 = (int32_t)std::min<int64_t>((int64_t)(k + 1) * p->slice_rows, inc->E);
-    HGE_TRY(hge_sched_begin(ctx, r0, r1, inc->e2n_ptr, inc->N, &p->slice_sched[(size_t)k]));
-  }
-  size_t n_part = 0, n_cnt = 0;
-  for (HgeHalfSchedule& sl : p->slice_sched) {
-    sl.idx = inc->edge_half.idx;
-    sl.deg = inc->edge_half.deg;
-    sl.invs = inc->edge_half.invs;
-    HGE_TRY(hge_sched_finish(ctx, "edge", &sl));
-    n_part = std::max(n_part, (size_t)sl.n_partials);
-    n_cnt = std::max(n_cnt, (size_t)sl.n_hrows);
-  }
-  // the parked chunk sums / arrival counters were sized for the whole-half schedules; the slices
-  // partition the edge rows, so together they need no more (every slice gets its own region:
-  // one launch walks them all)
-  size_t sum_part = 0, sum_cnt = 0;
-  for (const HgeHalfSchedule& sl : p->slice_sched) {
-    sum_part += (size_t)sl.n_partials;
-    sum_cnt += (size_t)sl.n_hrows;
-  }
-  HGE_REQUIRE(sum_part <= (size_t)std::max(inc->node_half.n_partials, inc->edge_half.n_partials) &&
-                  sum_cnt <= (size_t)std::max(inc->node_half.n_hrows, inc->edge_half.n_hrows),
-              "hge_internal_slice_schedules: slice schedules larger than the whole");
   return HGE_OK;
 }
 

@@ -70,12 +70,6 @@ static void set_default_tuning(hge_ctx* ctx) {
   // cut the stream into pieces of equal cost
   ctx->unit_cost = 1;
   if (const char* env = getenv("HGE_UNIT_COST")) ctx->unit_cost = atoi(env);
-  // peer-memory exchange of the sharded edge half: pipelined in this many slices of edge rows.
-  // Measured at 2 GPUs on config 2 (profiles/r2_multi_gpu.md): every extra slice costs ~23 us per
-  // sweep in launches (gather, barrier, reduce) and buys back less than that, so the default is
-  // one slice; the pipeline is there for shapes whose exchange tail is longer.
-  ctx->p2p_slices = 1;
-  if (const char* env = getenv("HGE_P2P_SLICES")) ctx->p2p_slices = std::max(1, std::min(16, atoi(env)));
   ctx->trainer_max_clusters = 0;
   if (const char* env = getenv("HGE_TRAIN_MAX_CLUSTERS")) ctx->trainer_max_clusters = std::max(0, atoi(env));
   // random 128-byte gathers over 8 GB of rows run at a third of the rate they reach inside 1 GB;

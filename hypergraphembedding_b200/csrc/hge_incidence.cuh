@@ -140,10 +140,9 @@ struct hge_p2p {
   hge_ctx* ctx = nullptr;
   int rank = 0, world = 1;
   int32_t E = 0, N = 0, ld = 0;                // N = local node rows
-  // Ownership of the edge rows: the rows are cut into `slices` slices of slice_rows consecutive
-  // rows (the unit the exchange is pipelined in), every slice into `world` runs of sub_rows rows,
-  // run o of every slice belongs to rank o.  own_rows = slices * sub_rows rows per rank.
-  int32_t slices = 1, slice_rows = 0, sub_rows = 0, own_rows = 0;
+  // Ownership of the edge rows: rank o owns the sub_rows consecutive rows from o * sub_rows on
+  // (HgeOwnerMap), clipped at E (the last runs may be short or empty)
+  int32_t sub_rows = 0;
   char* base = nullptr;                      // local arena
   size_t off_ye = 0, off_stage = 0, off_mmx = 0, off_flags = 0, off_err = 0, off_yn = 0, bytes = 0;
   char* peer_base[16] = {nullptr};           // peer arenas (own slot = base)
@@ -154,20 +153,6 @@ struct hge_p2p {
   uint32_t** d_peer_flags = nullptr;
   uint32_t seq = 0;                          // barrier sequence number (same on every rank)
   bool peers_open = false;
-  // pipelined exchange: the owner-side work of the finished slices runs on `side` while the
-  // gather launch goes on with the next slices on the context's stream
-  cudaStream_t side = nullptr;
-  cudaEvent_t reduced = nullptr;
-  std::vector<HgeHalfSchedule> slice_sched;  // the shard's edge half, one schedule per slice
-  // pipelined sweep (slices > 1): one dynamic gather launch over all slice schedules
-  // (hge_internal_edge_push_dynamic); the owner-side work follows slice by slice on `side`
-  void* d_dyn_src = nullptr;                 // device HgeSweepSrc[slices]
-  std::vector<char> h_dyn_src;               // what was uploaded last
-  int32_t* d_dyn_ctr = nullptr;              // [1 + slices]: next work item, finished pieces per slice
-  int dyn_pieces = 0;
-  int reserve_blocks = 0;                    // block slots the gather leaves to the owner-side kernels
-  uint32_t sweep_seq = 0;                    // sequence number of the per-slice arrival flags
-  cudaEvent_t node_done = nullptr;
   // HGE_P2P_TIMING=1: events around the phases of every sweep (node half, gather + push,
   // barrier A, owner reduce + all-gather, barrier B), read by hge_p2p_phase_ms
   bool timing = false;
@@ -177,12 +162,10 @@ struct hge_p2p {
 // (owner rank, row inside the owner's block) of an edge row -- shared by the kernels that push
 // partial rows to their owners and by the owner-side reduce
 struct HgeOwnerMap {
-  int32_t slice_rows, sub_rows;
+  int32_t sub_rows;   // rows owned per rank (= rows per source rank in a staging block)
   __host__ __device__ void locate(int32_t row, int& owner, int32_t& idx) const {
-    const int32_t k = row / slice_rows;
-    const int32_t w = row - k * slice_rows;
-    owner = w / sub_rows;
-    idx = k * sub_rows + (w - owner * sub_rows);
+    owner = row / sub_rows;
+    idx = row - owner * sub_rows;
   }
 };
 
@@ -206,8 +189,5 @@ struct hge_algdist {
   hge_p2p* p2p = nullptr;
 };
 
-// internal: the sharded edge gather with the partial rows pushed to their owners (slice < 0: all
-// edge rows), and the per-slice schedules it runs over
-extern "C" int hge_internal_edge_push(hge_algdist* st, int sweep, int slice);
-extern "C" int hge_internal_edge_push_dynamic(hge_algdist* st, int sweep);
-extern "C" int hge_internal_slice_schedules(hge_algdist* st);
+// internal: the sharded edge gather with the partial rows pushed to their owners
+extern "C" int hge_internal_edge_push(hge_algdist* st, int sweep);

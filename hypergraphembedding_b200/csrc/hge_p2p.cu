@@ -12,21 +12,9 @@
 //                                      peers, signals, waits, and reduces them locally
 //                                                                   -> all-reduce(min / max)
 //
-// Pipelining.  The edge rows are cut into `slices` slices; inside a slice the ownership is split
-// over the ranks (HgeOwnerMap).  ONE gather launch walks all slices, slice-major, with warps
-// claiming (slice, piece) work items from a counter (HgeSweepDyn, hge_sweep.cuh); the warp that
-// finishes a slice's last piece raises that slice's arrival flag on every rank.  On a second,
-// higher-priority stream a one-block kernel waits for a slice's flags from all ranks and the
-// owner-side reduce of that slice follows -- in the block slots the gather launch leaves free
-// (reserve_blocks), while the gather goes on with the next slices, so that the serial tail of a
-// sweep (owner pass + `world` peer stores per row + two barriers: 0.115 of 0.42 ms per sweep at 4
-// and 8 GPUs) shrinks to the last slice's.  MEASURED (profiles/r2_multi_gpu.md): it does hide the
-// tail, but the gather launch pays more than the tail was worth -- 0.16 -> 0.25 ms at 8 GPUs
-// (fewer resident warps, the claim per piece, and the owner-side traffic now competes with the
-// gather for the same memory system) -- so `slices` defaults to 1 (no pipeline) and this path is
-// opt-in (HGE_P2P_SLICES, hge_p2p_create).  Round 2's first attempt, one gather launch per
-// slice, lost more: a launch fills every slot the previous one frees, so the owner-side kernels
-// only ran between the waves of the next gather.
+// Rank o owns the edge rows [o sub_rows, (o + 1) sub_rows) (HgeOwnerMap).  Each phase is one
+// launch on the context's stream.  Overlapping the owner-side reduce with the gather was tried
+// and was slower (profiles/r2_multi_gpu.md, section 4).
 //
 // Each rank owns one cudaMalloc arena [edge rows | row of zeros | staging | bounds | flags |
 // error | local node rows] that the other ranks of the node map through CUDA IPC (the node rows
@@ -107,27 +95,12 @@ __global__ void k_exchange(int rank, int world, uint32_t seq, uint32_t* const* p
   }
 }
 
-// Waits until every rank has announced slice `slice` of the sweep numbered `seq` (the flags the
-// dynamic gather launch raises).  One block.
-__global__ void k_wait_slice(int world, uint32_t seq, const uint32_t* my_flags, int err_after_ns_hi, int* err) {
-  const int tid = threadIdx.x;
-  if (tid < world) {
-    const unsigned long long t0 = global_ns();
-    while ((int32_t)(ld_acquire_sys(my_flags + (size_t)tid * kFlagStride) - seq) < 0) {
-      if (global_ns() - t0 > kTimeoutNs) {
-        *err = 1;
-        break;
-      }
-    }
-  }
-  (void)err_after_ns_hi;
-}
-
 // Owner-side reduce of the staged partial rows + row update + push of the new row to all ranks.
-// row0 = first edge row of the run, stage0 = its row inside the owner's staging block.
+// row0 = first edge row of this rank's run; every source rank's block of the staging area holds
+// sub_rows rows.
 template <int LPR>
 __global__ void __launch_bounds__(kBlock) k_edge_reduce_push(
-    int rank, int world, int32_t row0, int32_t stage0, int32_t rows, int32_t own_rows, int R, int ld4,
+    int rank, int world, int32_t row0, int32_t rows, int32_t sub_rows, int R, int ld4,
     const float4* __restrict__ stage, const float4* __restrict__ ye_local,
     float4* const* __restrict__ peer_ye, const int32_t* __restrict__ deg,
     const float* __restrict__ invs, const int32_t* __restrict__ mm_prev, int32_t* mm_cur) {
@@ -156,7 +129,7 @@ __global__ void __launch_bounds__(kBlock) k_edge_reduce_push(
     const int32_t row = row0 + (int32_t)i;
     float4 acc = hge_f4_zero();
     for (int p = 0; p < world; ++p)     // rank order: the sum is the same on every run
-      hge_f4_add(acc, __ldcs(stage + ((size_t)p * own_rows + stage0 + i) * ld4 + c4));
+      hge_f4_add(acc, __ldcs(stage + ((size_t)p * sub_rows + i) * ld4 + c4));
     const float4 y = __ldcs(ye_local + (size_t)row * ld4 + c4);
     const float degf = (float)deg[row];
     const float hd = 0.5f * degf, hs = 0.5f * invs[row];
@@ -206,13 +179,13 @@ __global__ void __launch_bounds__(kBlock) k_edge_reduce_push(
   }
 }
 
-int launch_exchange(hge_algdist* st, int sweep_for_mm, cudaStream_t stream) {
+int launch_exchange(hge_algdist* st, int sweep_for_mm) {
   hge_p2p* p = st->p2p;
   hge_ctx* ctx = st->ctx;
   p->seq += 1;
   const bool with_mm = sweep_for_mm >= 0;
   int32_t* mm_cur = with_mm ? st->mm + (size_t)sweep_for_mm * 2 * st->ld : nullptr;
-  k_exchange<<<1, 128, 0, stream>>>(
+  k_exchange<<<1, 128, 0, ctx->stream>>>(
       p->rank, p->world, p->seq, p->d_peer_flags, reinterpret_cast<uint32_t*>(p->base + p->off_flags),
       p->d_peer_mmx, reinterpret_cast<int32_t*>(p->base + p->off_mmx), with_mm ? (sweep_for_mm & 1) : 0,
       st->ld, mm_cur, reinterpret_cast<int*>(p->base + p->off_err));
@@ -225,17 +198,13 @@ int launch_exchange(hge_algdist* st, int sweep_for_mm, cudaStream_t stream) {
 extern "C" {
 
 int hge_p2p_create(hge_ctx* ctx, int rank, int world, int32_t num_local_nodes, int32_t num_edges,
-                   int ld, int slices, hge_p2p** out) {
+                   int ld, hge_p2p** out) {
   HGE_REQUIRE(ctx && out, "hge_p2p_create: NULL argument");
   *out = nullptr;
   HGE_REQUIRE(num_local_nodes >= 0, "hge_p2p_create: negative node count");
   HGE_REQUIRE(world >= 1 && world <= 16 && rank >= 0 && rank < world,
               "hge_p2p_create: rank %d / world %d not supported (world <= 16)", rank, world);
   HGE_REQUIRE(num_edges > 0 && ld > 0 && ld % 4 == 0, "hge_p2p_create: bad shape");
-  HGE_REQUIRE(slices >= 0 && slices <= 16, "hge_p2p_create: slices %d not in [0, 16] (0 = default)", slices);
-  if (slices == 0) slices = ctx->p2p_slices;
-  if (world == 1 && !getenv("HGE_P2P_SLICES_ONE_RANK")) slices = 1;   // one rank: nothing to overlap (the override is for profiling the gather launch)
-  slices = std::max(1, std::min(slices, num_edges / std::max(1, 64 * world)));   // no sliver slices
   HGE_CUDA(cudaSetDevice(ctx->device));
   hge_p2p* p = new (std::nothrow) hge_p2p();
   if (!p) return HGE_ERR_NOMEM;
@@ -245,19 +214,16 @@ int hge_p2p_create(hge_ctx* ctx, int rank, int world, int32_t num_local_nodes, i
   p->E = num_edges;
   p->N = num_local_nodes;
   p->ld = ld;
-  p->slices = slices;
-  p->slice_rows = (num_edges + slices - 1) / slices;
-  p->sub_rows = (p->slice_rows + world - 1) / world;
-  p->own_rows = slices * p->sub_rows;
+  p->sub_rows = (num_edges + world - 1) / world;
   size_t off = 0;
   p->off_ye = off;
   off = align_up(off + ((size_t)num_edges + 1) * ld * 4, 256);   // + the row of zeros
   p->off_stage = off;
-  off = align_up(off + (size_t)world * p->own_rows * ld * 4, 256);
+  off = align_up(off + (size_t)world * p->sub_rows * ld * 4, 256);
   p->off_mmx = off;
   off = align_up(off + (size_t)2 * world * 2 * ld * 4, 256);
   p->off_flags = off;
-  off = align_up(off + (size_t)(1 + 16) * world * kFlagStride * 4, 256);   // barrier + per-slice arrival flags
+  off = align_up(off + (size_t)world * kFlagStride * 4, 256);
   p->off_err = off;
   off = align_up(off + 256, 256);
   // offsets above are the same on every rank (peers address them); the node rows differ in size
@@ -282,9 +248,6 @@ int hge_p2p_create(hge_ctx* ctx, int rank, int world, int32_t num_local_nodes, i
   }
   p->peer_base[rank] = p->base;
   if (const char* env = getenv("HGE_P2P_TIMING")) p->timing = atoi(env) != 0;
-  // block slots (of 256 threads) the pipelined gather leaves to the owner-side kernels
-  p->reserve_blocks = 32;
-  if (const char* env = getenv("HGE_P2P_RESERVE")) p->reserve_blocks = std::max(8, atoi(env));
   *out = p;
   return HGE_OK;
 }
@@ -358,17 +321,7 @@ int hge_p2p_destroy(hge_p2p* p) {
   if (!p) return HGE_OK;
   hge_ctx* ctx = p->ctx;
   hge_p2p_close_peers(p);
-  for (HgeHalfSchedule& sl : p->slice_sched) hge_sched_release(ctx, &sl);
-  p->slice_sched.clear();
-  if (p->side) {
-    cudaStreamSynchronize(p->side);
-    cudaStreamDestroy(p->side);
-    if (p->reduced) cudaEventDestroy(p->reduced);
-  }
   for (cudaEvent_t e : p->marks) cudaEventDestroy(e);
-  if (p->node_done) cudaEventDestroy(p->node_done);
-  if (p->d_dyn_src) cudaFree(p->d_dyn_src);
-  if (p->d_dyn_ctr) cudaFree(p->d_dyn_ctr);
   hge_dev_free(ctx, p->d_peer_stage);
   hge_dev_free(ctx, p->d_peer_ye);
   hge_dev_free(ctx, p->d_peer_mmx);
@@ -389,19 +342,11 @@ int hge_algdist_attach_p2p(hge_algdist* st, hge_p2p* p) {
   st->yn = reinterpret_cast<float*>(p->base + p->off_yn);
   st->zero_row = (uint32_t)p->E;
   st->p2p = p;
-  if (p->slices > 1 && !p->side) {
-    int lo = 0, hi = 0;
-    HGE_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-    HGE_CUDA(cudaStreamCreateWithPriority(&p->side, cudaStreamNonBlocking, hi));
-    HGE_CUDA(cudaEventCreateWithFlags(&p->reduced, cudaEventDisableTiming));
-    HGE_CUDA(cudaEventCreateWithFlags(&p->node_done, cudaEventDisableTiming));
-  }
-  // a pooled arena may come back from a relaxation over another incidence of the same shape
-  return hge_internal_slice_schedules(st);
+  return HGE_OK;
 }
 
-// Owner-side reduce of one run of this rank's rows (slice k, or all slices when k < 0).
-static int launch_reduce_push(hge_algdist* st, int sweep, int k, cudaStream_t stream) {
+// Owner-side reduce of this rank's run of edge rows.
+static int launch_reduce_push(hge_algdist* st, int sweep) {
   hge_p2p* p = st->p2p;
   hge_ctx* ctx = st->ctx;
   hge_incidence* inc = st->inc;
@@ -409,34 +354,28 @@ static int launch_reduce_push(hge_algdist* st, int sweep, int k, cudaStream_t st
   int32_t* mm_cur = st->mm + (size_t)sweep * 2 * st->ld;
   const float4* stage = reinterpret_cast<const float4*>(p->base + p->off_stage);
   const float4* ye = reinterpret_cast<const float4*>(st->ye);
-  const int k0 = k < 0 ? 0 : k, k1 = k < 0 ? p->slices : k + 1;
-  for (int kk = k0; kk < k1; ++kk) {
-    // this rank's run of slice kk: rows [kk slice_rows + rank sub_rows, + sub_rows), clipped
-    const int64_t s0 = (int64_t)kk * p->slice_rows;
-    const int64_t s1 = std::min<int64_t>(s0 + p->slice_rows, p->E);
-    const int64_t r0 = std::min<int64_t>(s0 + (int64_t)p->rank * p->sub_rows, s1);
-    const int64_t r1 = std::min<int64_t>(r0 + p->sub_rows, s1);
-    const int32_t rows = (int32_t)(r1 - r0);
-    if (rows <= 0) continue;
-    const int G = 32 / st->lpr;
-    int blocks = (int)std::min<int64_t>(((int64_t)rows + (kBlock / 32) * G - 1) / ((kBlock / 32) * G),
-                                        (int64_t)ctx->num_sms * 8);
-    dim3 grid(std::max(1, blocks), st->slabs);
+  // rows [rank sub_rows, + sub_rows), clipped at E
+  const int64_t r0 = std::min<int64_t>((int64_t)p->rank * p->sub_rows, p->E);
+  const int32_t rows = (int32_t)(std::min<int64_t>(r0 + p->sub_rows, p->E) - r0);
+  if (rows <= 0) return HGE_OK;
+  const int G = 32 / st->lpr;
+  int blocks = (int)std::min<int64_t>(((int64_t)rows + (kBlock / 32) * G - 1) / ((kBlock / 32) * G),
+                                      (int64_t)ctx->num_sms * 8);
+  dim3 grid(std::max(1, blocks), st->slabs);
 #define HGE_LAUNCH_RP(L)                                                                              \
-  k_edge_reduce_push<L><<<grid, kBlock, 0, stream>>>(p->rank, p->world, (int32_t)r0, kk * p->sub_rows, rows, \
-                                                     p->own_rows, st->R, st->ld4, stage, ye, p->d_peer_ye,    \
-                                                     inc->edge_half.deg, inc->edge_half.invs, mm_prev, mm_cur)
-    switch (st->lpr) {
-      case 1: HGE_LAUNCH_RP(1); break;
-      case 2: HGE_LAUNCH_RP(2); break;
-      case 4: HGE_LAUNCH_RP(4); break;
-      case 8: HGE_LAUNCH_RP(8); break;
-      case 16: HGE_LAUNCH_RP(16); break;
-      default: HGE_LAUNCH_RP(32); break;
-    }
-#undef HGE_LAUNCH_RP
-    HGE_CHECK_LAUNCH(ctx);
+  k_edge_reduce_push<L><<<grid, kBlock, 0, ctx->stream>>>(p->rank, p->world, (int32_t)r0, rows, p->sub_rows, \
+                                                          st->R, st->ld4, stage, ye, p->d_peer_ye,            \
+                                                          inc->edge_half.deg, inc->edge_half.invs, mm_prev, mm_cur)
+  switch (st->lpr) {
+    case 1: HGE_LAUNCH_RP(1); break;
+    case 2: HGE_LAUNCH_RP(2); break;
+    case 4: HGE_LAUNCH_RP(4); break;
+    case 8: HGE_LAUNCH_RP(8); break;
+    case 16: HGE_LAUNCH_RP(16); break;
+    default: HGE_LAUNCH_RP(32); break;
   }
+#undef HGE_LAUNCH_RP
+  HGE_CHECK_LAUNCH(ctx);
   return HGE_OK;
 }
 
@@ -461,35 +400,13 @@ int hge_algdist_sweep_p2p(hge_algdist* st, int sweep) {
   mark();
   HGE_TRY(hge_algdist_node_half(st, sweep));
   mark();
-  if (p->slice_sched.empty()) {
-    HGE_TRY(hge_internal_edge_push(st, sweep, -1));       // gather + reduce-scatter (peer stores)
-    mark();
-    HGE_TRY(launch_exchange(st, -1, ctx->stream));        // barrier A
-    mark();
-    HGE_TRY(launch_reduce_push(st, sweep, -1, ctx->stream));
-    mark();
-  } else {
-    // one dynamic gather launch on the main stream; on the side stream, per slice: wait for the
-    // slice's arrival flags of all ranks, then the owner-side reduce + all-gather of the slice
-    p->sweep_seq += 1;
-    HGE_CUDA(cudaEventRecord(p->node_done, ctx->stream));
-    HGE_CUDA(cudaStreamWaitEvent(p->side, p->node_done, 0));
-    HGE_TRY(hge_internal_edge_push_dynamic(st, sweep));
-    uint32_t* my_flags = reinterpret_cast<uint32_t*>(p->base + p->off_flags);
-    for (int k = 0; k < p->slices; ++k) {
-      k_wait_slice<<<1, 32, 0, p->side>>>(p->world, p->sweep_seq,
-                                          my_flags + (size_t)(p->world + k * p->world) * kFlagStride, 0,
-                                          reinterpret_cast<int*>(p->base + p->off_err));
-      HGE_CHECK_LAUNCH(ctx);
-      HGE_TRY(launch_reduce_push(st, sweep, k, p->side));
-    }
-    mark();   // pipelined: the gather launch alone ...
-    HGE_CUDA(cudaEventRecord(p->reduced, p->side));
-    HGE_CUDA(cudaStreamWaitEvent(ctx->stream, p->reduced, 0));
-    mark();   // ... what is left of the owner-side work of the slices after it ...
-    mark();   // ... (nothing: slot kept so that the five phases line up with the unpipelined sweep)
-  }
-  HGE_TRY(launch_exchange(st, sweep, ctx->stream));       // barrier B + all-reduce(min / max)
+  HGE_TRY(hge_internal_edge_push(st, sweep));             // gather + reduce-scatter (peer stores)
+  mark();
+  HGE_TRY(launch_exchange(st, -1));                       // barrier A
+  mark();
+  HGE_TRY(launch_reduce_push(st, sweep));                 // owner reduce + all-gather
+  mark();
+  HGE_TRY(launch_exchange(st, sweep));                    // barrier B + all-reduce(min / max)
   mark();
   if (timed && p->marks.size() != mark0 + 6) {            // an event could not be created: drop the sweep
     while (p->marks.size() > mark0) {

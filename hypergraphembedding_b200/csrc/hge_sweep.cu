@@ -125,7 +125,7 @@ __device__ __forceinline__ void kahan_add4(float4& s, float4& c, const float4& v
   y = v.w - c.w; t = s.w + y; c.w = (t - s.w) - y; s.w = t;
 }
 
-template <int LPR, int MODE, bool DYN>
+template <int LPR, int MODE>
 __global__ void __launch_bounds__(kBlock, HGE_SWEEP_MIN_BLOCKS) k_sweep(const HgeSweepArgs a) {
   constexpr int G = 32 / LPR;                      // lane groups (rows in flight) per warp
   constexpr int K = LPR >= 4 ? 1 : 4 / LPR;        // id registers per lane and step
@@ -220,7 +220,7 @@ __global__ void __launch_bounds__(kBlock, HGE_SWEEP_MIN_BLOCKS) k_sweep(const Hg
       int owner;
       int32_t idx;
       a.push_map.locate(row, owner, idx);
-      float4* dst = a.push_stage[owner] + ((size_t)a.push_rank * a.push_rows + idx) * ld4 + c4;
+      float4* dst = a.push_stage[owner] + ((size_t)a.push_rank * a.push_map.sub_rows + idx) * ld4 + c4;
       *dst = acc;
     } else if (MODE == kSweepRawAdd) {
       float4 prev = a.raw[off];
@@ -284,8 +284,9 @@ __global__ void __launch_bounds__(kBlock, HGE_SWEEP_MIN_BLOCKS) k_sweep(const Hg
   };
 
   // ---- one piece of one schedule ----------------------------------------------------------------
+  // (kept as a lambda: unwrapped, the same code gets a different register and stack-slot
+  // allocation in every instantiation)
   auto run_piece = [&](const HgeSweepSrc& src, const int pi) {
-  // the schedule the piece belongs to: the launch's own, or (dynamic mode) a slice's
   const int32_t* const stream0 = src.stream;
   const int32_t* const sp = stream0 + g * 4 + (K == 1 ? (gl & 3) : gl);   // this lane's column of the id stream
   auto load_ids = [&](uint32_t step, int (&r)[K]) {
@@ -466,41 +467,7 @@ __global__ void __launch_bounds__(kBlock, HGE_SWEEP_MIN_BLOCKS) k_sweep(const Hg
   }
   };   // run_piece
 
-  if (!DYN) {
-    run_piece(a.src, blockIdx.x * kWarps + warp);
-  } else {
-    const int32_t total_items = a.dyn.slices * a.dyn.pieces;
-    for (;;) {
-      int32_t w = 0;
-      if (lane == 0) w = atomicAdd(a.dyn.next, 1);
-      w = __shfl_sync(kFull, w, 0);
-      if (w >= total_items) break;
-      const int32_t slice = w / a.dyn.pieces;
-      const HgeSweepSrc& src = a.dyn.src[slice];
-      run_piece(src, w - slice * a.dyn.pieces);
-      // This warp's partial rows are on their way to their owners.  The count is a release at
-      // GPU scope (orders the lanes' stores, made visible to the counting lane by the warp
-      // barrier, before the increment); the warp that takes the last count acquires it, fences at
-      // system scope once and raises the flag on every rank.  One system-scope fence per piece
-      // instead (MEMBAR.SYS, ~7 us each) was 15 % of the launch.
-      __syncwarp();
-      if (lane == 0) {
-        int32_t before;
-        asm volatile("atom.add.acq_rel.gpu.global.s32 %0, [%1], 1;" : "=r"(before) : "l"(a.dyn.done + slice) : "memory");
-        if (before == a.dyn.pieces - 1) {
-          // last piece of the slice on this rank: every rank may reduce its rows of the slice
-          // as soon as it has seen this from all ranks
-          a.dyn.done[slice] = 0;
-          __threadfence_system();
-          for (int p = 0; p < a.dyn.world; ++p) {
-            uint32_t* flag = a.dyn.peer_flags[p] +
-                             (size_t)(a.dyn.flag0 + slice * a.dyn.world + a.dyn.rank) * a.dyn.flag_stride;
-            asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(flag), "r"(a.dyn.seq) : "memory");
-          }
-        }
-      }
-    }
-  }
+  run_piece(a.src, blockIdx.x * kWarps + warp);
 
   // ---- per-column min / max of the rows this block produced -------------------------------------
   if (kOwn) {
@@ -548,14 +515,11 @@ __global__ void __launch_bounds__(kBlock, HGE_SWEEP_MIN_BLOCKS) k_sweep(const Hg
 template <int LPR>
 int launch_mode(const HgeSweepArgs& a, int mode, dim3 grid, cudaStream_t stream) {
   switch (mode) {
-    case kSweepNode: k_sweep<LPR, kSweepNode, false><<<grid, kBlock, 0, stream>>>(a); break;
-    case kSweepEdge: k_sweep<LPR, kSweepEdge, false><<<grid, kBlock, 0, stream>>>(a); break;
-    case kSweepRaw: k_sweep<LPR, kSweepRaw, false><<<grid, kBlock, 0, stream>>>(a); break;
-    case kSweepRawAdd: k_sweep<LPR, kSweepRawAdd, false><<<grid, kBlock, 0, stream>>>(a); break;
-    default:
-      if (a.dyn.src) k_sweep<LPR, kSweepPush, true><<<grid, kBlock, 0, stream>>>(a);
-      else k_sweep<LPR, kSweepPush, false><<<grid, kBlock, 0, stream>>>(a);
-      break;
+    case kSweepNode: k_sweep<LPR, kSweepNode><<<grid, kBlock, 0, stream>>>(a); break;
+    case kSweepEdge: k_sweep<LPR, kSweepEdge><<<grid, kBlock, 0, stream>>>(a); break;
+    case kSweepRaw: k_sweep<LPR, kSweepRaw><<<grid, kBlock, 0, stream>>>(a); break;
+    case kSweepRawAdd: k_sweep<LPR, kSweepRawAdd><<<grid, kBlock, 0, stream>>>(a); break;
+    default: k_sweep<LPR, kSweepPush><<<grid, kBlock, 0, stream>>>(a); break;
   }
   return HGE_OK;
 }
@@ -563,7 +527,7 @@ int launch_mode(const HgeSweepArgs& a, int mode, dim3 grid, cudaStream_t stream)
 template <int LPR>
 int resident_blocks(int* out) {
   int per_sm = 0;
-  HGE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sweep<LPR, kSweepNode, false>, kBlock, 0));
+  HGE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sweep<LPR, kSweepNode>, kBlock, 0));
   *out = per_sm < 1 ? 1 : per_sm;
   return HGE_OK;
 }

@@ -26,33 +26,14 @@ struct HgeSweepSrc {
   int32_t* counters;           // [slabs, n_hrows]
 };
 
-// Dynamic mode of the push kernel (the pipelined peer-memory sweep): one launch walks the gather
-// streams of all `slices` slices of the edge rows.  Warps claim (slice, piece) work items from a
-// counter in slice-major order, so slice k is complete on this rank about k / slices into the
-// launch; the warp that finishes a slice's last piece tells every rank so (release store of `seq`
-// into flag (flag0 + slice * world + rank) of every peer), and the owners start reducing that
-// slice while the launch goes on with the next.
-struct HgeSweepDyn {
-  const HgeSweepSrc* src;      // device array [slices]
-  int32_t slices;
-  int32_t pieces;              // pieces per slice
-  int32_t* next;               // work-item counter, zero at launch
-  int32_t* done;               // [slices] finished pieces, zero at launch, left zero
-  uint32_t* const* peer_flags; // flag arrays of all ranks
-  uint32_t seq;
-  int32_t flag0, rank, world, flag_stride;
-};
-
 struct HgeSweepArgs {
-  HgeSweepSrc src;             // static mode: piece blockIdx.x * warps + warp of this schedule
-  HgeSweepDyn dyn;             // dyn.src != nullptr: dynamic mode (kSweepPush only)
+  HgeSweepSrc src;             // a warp runs piece blockIdx.x * warps + warp of this schedule
   const float4* base;          // row 0 of the allocation the stream's row indices refer to
   float4* own;                 // owned rows [rows, ld4]
   const int32_t* mm_prev;      // affine map of the previous sweep, or nullptr (identity)
   int32_t* mm_cur;             // min / max slots of this sweep
   float4* raw;
   float4* const* push_stage;   // kSweepPush: staging blocks of all ranks
-  int32_t push_rows;           //   rows owned per rank (= rows per source rank in a staging block)
   int32_t push_rank;
   HgeOwnerMap push_map;        //   edge row -> (owner, row inside the owner's block)
   int32_t R;

@@ -176,11 +176,9 @@ int hge_algdist_store(hge_algdist* st, int sweeps_done, float* xn, float* xe, in
  * met within 20 s raises an error flag (hge_p2p_check) instead of hanging. */
 typedef struct hge_p2p hge_p2p;
 /* num_local_nodes: this rank's node rows (they live in the arena next to the edge rows, though no
- * peer touches them).  slices: the exchange is pipelined in this many slices of edge rows -- slice
- * k's barrier and owner-side reduce overlap the gather of slice k + 1 (0 = default: 1 = off,
- * HGE_P2P_SLICES overrides). */
+ * peer touches them). */
 int hge_p2p_create(hge_ctx* ctx, int rank, int world, int32_t num_local_nodes, int32_t num_edges,
-                   int ld, int slices, hge_p2p** out);
+                   int ld, hge_p2p** out);
 int hge_p2p_export(hge_p2p* p, void* handle64);
 int hge_p2p_open_peers(hge_p2p* p, const void* handles /* world x 64 bytes */);
 int hge_p2p_check(hge_p2p* p);

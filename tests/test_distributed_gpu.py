@@ -72,29 +72,6 @@ def test_two_ranks(tmp_path, comm, R):
 
 
 @pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
-@pytest.mark.parametrize("slices,R", [(2, 32), (4, 32), (3, 10)])
-def test_two_ranks_pipelined_exchange(tmp_path, monkeypatch, slices, R):
-  """The pipelined peer-memory sweep (HGE_P2P_SLICES > 1): one dynamic gather launch over the
-  slices of the edge rows, owner-side reduce of every finished slice next to it.  Same result as
-  the oracle, and bit for bit the result of the unpipelined sweep (the owner adds the staged rows
-  in rank order either way)."""
-  graph_args = (10, 30000, 900, 250000)
-  outs = []
-  for s in (slices, 1):
-    monkeypatch.setenv("HGE_P2P_SLICES", str(s))
-    d = tmp_path / ("slices%d" % s)
-    d.mkdir()
-    mp.spawn(dist_helpers.worker,
-             args=(2, _free_port(), "nccl", graph_args, R, 8, 1, str(d), True, "p2p"),
-             nprocs=2, join=True)
-    _check(d, 2, graph_args, R, 8)
-    outs.append([np.load(d / ("rank%d.npz" % r)) for r in range(2)])
-  for r in range(2):
-    assert np.array_equal(outs[0][r]["xn"], outs[1][r]["xn"])
-    assert np.array_equal(outs[0][r]["xe"], outs[1][r]["xe"])
-
-
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 def test_two_ranks_p2p_is_reproducible(tmp_path):
   graph_args = (11, 20000, 500, 200000)
   outs = []

@@ -1,7 +1,7 @@
 """The peer-memory sweep on ONE rank (world size 1: every push goes to the rank's own staging
-block), for timing / profiling the gather launch of the pipelined sweep without a second GPU:
+block), for the phase split of a p2p sweep without a second GPU:
 
-    HGE_P2P_SLICES=4 HGE_P2P_SLICES_ONE_RANK=1 python tools/p2p_one_rank.py
+    python tools/p2p_one_rank.py
 """
 import json
 import os
@@ -38,8 +38,8 @@ def main():
       relax.sweep(t)
     ms5, n = relax.ops.arena.phase_ms()
     relax.ops.arena.set_timing(False)
-  print(json.dumps({"slices": os.environ.get("HGE_P2P_SLICES", "1"), "sweeps": n,
-                    "phases_ms": dict(zip(("node_half", "gather", "barrier_a_or_tail", "reduce", "barrier_b"),
+  print(json.dumps({"sweeps": n,
+                    "phases_ms": dict(zip(("node_half", "gather", "barrier_a", "reduce", "barrier_b"),
                                           [round(v, 4) for v in ms5]))}), flush=True)
   relax.close()
   hd.release_peer_arenas(dist)

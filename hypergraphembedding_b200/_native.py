@@ -11,8 +11,7 @@ import threading
 import numpy as np
 
 _PKG_DIR = os.path.dirname(os.path.abspath(__file__))
-# HGE_LIB_PATH selects an experimental build of the same library (tools/sweep_variants.py)
-LIB_PATH = os.environ.get("HGE_LIB_PATH") or os.path.join(_PKG_DIR, "libhge_b200.so")
+LIB_PATH = os.path.join(_PKG_DIR, "libhge_b200.so")
 
 HGE_OK = 0
 HGE_ERR_INVALID = -1
@@ -899,7 +898,7 @@ class PeerArena(object):
 
   def phase_ms(self):
     """(mean ms per sweep of [node half, gather + push, barrier A, reduce + all-gather, barrier B],
-    sweeps averaged over) since the last call; needs HGE_P2P_TIMING=1 when the arena was created."""
+    sweeps averaged over) since the last call; records only while set_timing(True) is on."""
     out = np.zeros(5, dtype=np.float64)
     n = ctypes.c_int(0)
     check(self.ctx.lib.hge_p2p_phase_ms(self.handle, ptr(out), ctypes.byref(n)), "hge_p2p_phase_ms")

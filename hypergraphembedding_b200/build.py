@@ -45,15 +45,13 @@ def needs_build():
   return any(os.path.getmtime(d) > built for d in deps)
 
 
-def build(force=False, verbose=False, defines=(), out=None, tag=""):
-  """Compiles every CUDA / C++ source under csrc/ into one shared library.  `defines`, `out`
-  and `tag` build an experimental variant (tools/sweep_variants.py) next to the default."""
-  out = out or LIB_PATH
-  if not defines and not force and not needs_build():
-    return out
+def build(force=False, verbose=False):
+  """Compiles every CUDA / C++ source under csrc/ into one shared library."""
+  if not force and not needs_build():
+    return LIB_PATH
   nvcc = find_nvcc()
   objs = []
-  obj_dir = os.path.join(PKG_DIR, "csrc", "_obj" + tag)
+  obj_dir = os.path.join(CSRC, "_obj")
   os.makedirs(obj_dir, exist_ok=True)
   procs = []
   for src in sources():
@@ -61,10 +59,9 @@ def build(force=False, verbose=False, defines=(), out=None, tag=""):
     objs.append(obj)
     if src.endswith(".cpp"):
       cuda_inc = os.path.join(os.path.dirname(os.path.dirname(nvcc)), "include")
-      cmd = [os.environ.get("CXX", "g++")] + CXX_FLAGS + ["-I", cuda_inc] + ["-D" + d for d in defines] + [
-          "-c", src, "-o", obj]
+      cmd = [os.environ.get("CXX", "g++")] + CXX_FLAGS + ["-I", cuda_inc, "-c", src, "-o", obj]
     else:
-      cmd = [nvcc] + NVCC_FLAGS + ["-D" + d for d in defines] + ["-x", "cu", "-c", src, "-o", obj]
+      cmd = [nvcc] + NVCC_FLAGS + ["-x", "cu", "-c", src, "-o", obj]
     procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT,
                                         text=True)))
   log = []
@@ -79,12 +76,12 @@ def build(force=False, verbose=False, defines=(), out=None, tag=""):
     sys.stderr.write("\n".join(log) + "\n")
   if failed:
     raise RuntimeError("nvcc failed; see the log above")
-  tmp = out + ".tmp"
+  tmp = LIB_PATH + ".tmp"
   subprocess.check_call([nvcc, "-shared", "-o", tmp] + objs + ["-gencode",
                                                                "arch=compute_100a,code=sm_100a",
                                                                "-Xlinker", "-lpthread"])
-  os.replace(tmp, out)
-  return out
+  os.replace(tmp, LIB_PATH)
+  return LIB_PATH
 
 
 if __name__ == "__main__":

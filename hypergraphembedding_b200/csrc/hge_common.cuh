@@ -52,7 +52,6 @@ struct hge_ctx {
   int light_max_deg;
   int chunk;
   int blocks_per_sm;
-  int unit_cost;         // per-unit cost in steps when the stream is cut into pieces
   int trainer_max_clusters;  // cap on the clusters of one hg2v training launch (0: what fits)
   int tile_mb;           // node-range tile of the single-GPU edge half in MB of rows (0 = off)
   int tile_min_mb;       // ... used when the node rows exceed this many MB

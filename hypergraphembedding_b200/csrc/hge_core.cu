@@ -58,28 +58,22 @@ int hge_ctx_stage(hge_ctx* ctx, size_t floats, float** out) {
   return HGE_OK;
 }
 
-// Schedule / kernel defaults (hge_ctx_create, hge_ctx_reset_tuning); the environment variables
-// are read on every reset so a variant sweep can steer a whole process.
+// Schedule / kernel defaults (hge_ctx_create, hge_ctx_reset_tuning).  The API setters change
+// them; the only environment variable read is the allocation-failure countdown of the tests,
+// re-read on every reset.
 static void set_default_tuning(hge_ctx* ctx) {
   // schedule defaults from the sweep in profiles/r1_half_sweep_experiments.md (config 2, 4-block
-  // kernel): sub-warp rows up to degree 128, chunks of 1024, a grid of 4 x the resident blocks
+  // kernel): sub-warp rows up to degree 128, chunks of 1024
   ctx->light_max_deg = 128;
   ctx->chunk = 1024;
-  ctx->blocks_per_sm = 0;  // 0: 4 x what the occupancy calculator says is resident
-  // cost of a unit (a chunk of a long row, a group of short rows) in steps of 4 gathers, used to
-  // cut the stream into pieces of equal cost
-  ctx->unit_cost = 1;
-  if (const char* env = getenv("HGE_UNIT_COST")) ctx->unit_cost = atoi(env);
+  ctx->blocks_per_sm = 0;  // 0: 2 x what the occupancy calculator says is resident
   ctx->trainer_max_clusters = 0;
-  if (const char* env = getenv("HGE_TRAIN_MAX_CLUSTERS")) ctx->trainer_max_clusters = std::max(0, atoi(env));
   // random 128-byte gathers over 8 GB of rows run at a third of the rate they reach inside 1 GB;
   // the edge half over more than 512 MB of node rows is tiled by node range into L2-sized tiles
   // when the edges are large enough for that to pay (profiles/r1_tiled_edge_half.md)
   ctx->tile_mb = 64;
   ctx->tile_min_mb = 512;
-  if (const char* env = getenv("HGE_TILE_MB")) ctx->tile_mb = atoi(env);
-  if (const char* env = getenv("HGE_TILE_MIN_MB")) ctx->tile_min_mb = atoi(env);
-  ctx->tile_force = ctx->tile_min_mb == 0;
+  ctx->tile_force = 0;
   ctx->fail_alloc_at = 0;
   if (const char* env = getenv("HGE_FAIL_ALLOC_AT")) ctx->fail_alloc_at = std::max(0ll, atoll(env));
   ctx->allocs = 0;

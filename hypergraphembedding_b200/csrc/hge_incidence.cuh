@@ -43,13 +43,12 @@ struct HgeHeavyRow {    // 32 B
 // padding), so a slot costs one multiply-add and one load, with no predicate.  With with_own
 // the last slot of a short row's last step is the row itself: its old value arrives through
 // the same pipeline as the neighbours'.  `piece` cuts the unit list into `pieces` contiguous
-// runs of equal cost (steps + unit_cost per unit), one per warp of the grid.
+// runs of equal cost (steps + 1 per unit), one per warp of the grid.
 struct HgeStream {
   int G = 0;
   int with_own = 0;
   uint32_t gather0 = 0, own0 = 0, zero = 0;
   int pieces = 0;
-  int unit_cost = 0;
   int32_t* ids = nullptr;        // [(total_steps + kStreamSlackSteps) * 4 G]
   int4* items = nullptr;         // [n_quads * G + kStreamSlackItems]: {row (-1: none), degree, steps of the unit, 1 / weight sum}
   uint32_t* uoff = nullptr;      // [n_units + 1] first step of every unit
@@ -153,7 +152,7 @@ struct hge_p2p {
   uint32_t** d_peer_flags = nullptr;
   uint32_t seq = 0;                          // barrier sequence number (same on every rank)
   bool peers_open = false;
-  // HGE_P2P_TIMING=1: events around the phases of every sweep (node half, gather + push,
+  // hge_p2p_set_timing: events around the phases of every sweep (node half, gather + push,
   // barrier A, owner reduce + all-gather, barrier B), read by hge_p2p_phase_ms
   bool timing = false;
   std::vector<cudaEvent_t> marks;            // 6 per recorded sweep

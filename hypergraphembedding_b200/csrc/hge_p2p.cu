@@ -247,7 +247,6 @@ int hge_p2p_create(hge_ctx* ctx, int rank, int world, int32_t num_local_nodes, i
     return HGE_ERR_CUDA;
   }
   p->peer_base[rank] = p->base;
-  if (const char* env = getenv("HGE_P2P_TIMING")) p->timing = atoi(env) != 0;
   *out = p;
   return HGE_OK;
 }
@@ -386,7 +385,7 @@ int hge_algdist_sweep_p2p(hge_algdist* st, int sweep) {
   hge_p2p* p = st->p2p;
   hge_ctx* ctx = st->ctx;
   HGE_CUDA(cudaSetDevice(ctx->device));
-  // phase marks (HGE_P2P_TIMING): 6 events per sweep, up to 256 sweeps between two read-outs
+  // phase marks (hge_p2p_set_timing): 6 events per sweep, up to 256 sweeps between two read-outs
   const bool timed = p->timing && p->marks.size() < 6 * 256;
   size_t mark0 = p->marks.size();
   auto mark = [&]() {
@@ -423,7 +422,7 @@ int hge_p2p_set_timing(hge_p2p* p, int on) {
   return HGE_OK;
 }
 
-// Mean milliseconds per sweep of the five phases recorded since the last call (HGE_P2P_TIMING=1):
+// Mean milliseconds per sweep of the five phases recorded since the last call (hge_p2p_set_timing):
 // node half, edge gather with the partial rows pushed to their owners, barrier A, owner-side
 // reduce + all-gather, barrier B with the min / max exchange.  *sweeps = sweeps averaged over.
 int hge_p2p_phase_ms(hge_p2p* p, double* out5, int* sweeps) {

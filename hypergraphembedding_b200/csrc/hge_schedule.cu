@@ -247,11 +247,11 @@ __global__ void k_stream_slack(int n, uint32_t zero, int32_t* __restrict__ dst, 
     items[i] = make_int4(-1, 0, 0x7fffffff, 0);
 }
 
-// piece[p] = first unit whose cost prefix (steps before it + unit_cost per unit before it)
-// reaches p / pieces of the total
-__global__ void k_piece_bounds(int pieces, int32_t n_units, int unit_cost,
-                               const uint32_t* __restrict__ uoff, int32_t* __restrict__ piece) {
-  const unsigned long long total = (unsigned long long)uoff[n_units] + (unsigned long long)unit_cost * n_units;
+// piece[p] = first unit whose cost prefix (steps before it + 1 per unit before it) reaches
+// p / pieces of the total
+__global__ void k_piece_bounds(int pieces, int32_t n_units, const uint32_t* __restrict__ uoff,
+                               int32_t* __restrict__ piece) {
+  const unsigned long long total = (unsigned long long)uoff[n_units] + (unsigned long long)n_units;
   for (int p = blockIdx.x * blockDim.x + threadIdx.x; p <= pieces; p += gridDim.x * blockDim.x) {
     if (p == pieces) {
       piece[p] = n_units;
@@ -261,7 +261,7 @@ __global__ void k_piece_bounds(int pieces, int32_t n_units, int unit_cost,
     int32_t lo = 0, hi = n_units;
     while (lo < hi) {
       const int32_t mid = lo + ((hi - lo) >> 1);
-      const unsigned long long c = (unsigned long long)uoff[mid] + (unsigned long long)unit_cost * mid;
+      const unsigned long long c = (unsigned long long)uoff[mid] + (unsigned long long)mid;
       if (c < want) lo = mid + 1; else hi = mid;
     }
     piece[p] = lo;
@@ -389,9 +389,8 @@ static void stream_release(const hge_ctx* ctx, HgeStream* t) {
 int hge_sched_stream(hge_ctx* ctx, HgeHalfSchedule* s, int G, int with_own, uint32_t gather0,
                      uint32_t own0, uint32_t zero, int pieces) {
   HgeStream& t = s->stream;
-  const int unit_cost = ctx->unit_cost;
   if (t.ids && t.G == G && t.with_own == with_own && t.gather0 == gather0 && t.own0 == own0 &&
-      t.zero == zero && t.pieces == pieces && t.unit_cost == unit_cost)
+      t.zero == zero && t.pieces == pieces)
     return HGE_OK;
   stream_release(ctx, &t);
   HGE_REQUIRE(G >= 1 && G <= 32 && pieces >= 1, "hge_sched_stream: bad group count / piece count");
@@ -407,7 +406,6 @@ int hge_sched_stream(hge_ctx* ctx, HgeHalfSchedule* s, int G, int with_own, uint
   t.own0 = own0;
   t.zero = zero;
   t.pieces = pieces;
-  t.unit_cost = unit_cost;
   t.n_units = (int32_t)n_units;
   t.n_quads = (int32_t)n_quads;
   DevBuf<uint32_t> steps(ctx);
@@ -455,8 +453,8 @@ int hge_sched_stream(hge_ctx* ctx, HgeHalfSchedule* s, int G, int with_own, uint
                                                 t.ids + (size_t)t.total_steps * 4 * G,
                                                 t.items + (size_t)n_quads * G);
   HGE_CHECK_LAUNCH(ctx);
-  k_piece_bounds<<<grid_for(ctx, pieces + 1, kBlock), kBlock, 0, ctx->stream>>>(pieces, t.n_units, unit_cost,
-                                                                              t.uoff, t.piece);
+  k_piece_bounds<<<grid_for(ctx, pieces + 1, kBlock), kBlock, 0, ctx->stream>>>(pieces, t.n_units, t.uoff,
+                                                                              t.piece);
   HGE_CHECK_LAUNCH(ctx);
   return HGE_OK;
 }

@@ -17,7 +17,7 @@
 //     pipeline instead of a dependent load per row;
 //   * a warp issues two steps (8 rows per lane) back to back and only then adds them up; a group
 //     of rows may end after either step, and the loads never sit inside a branch;
-//   * every warp owns one contiguous, cost-balanced piece of the unit list, one wave of blocks.
+//   * every warp owns one contiguous, cost-balanced piece of the unit list, two waves of blocks.
 #include <algorithm>
 
 #include "hge_incidence.cuh"
@@ -28,43 +28,8 @@ namespace {
 constexpr int kBlock = 256;
 constexpr int kWarps = kBlock / 32;
 constexpr unsigned kFull = 0xffffffffu;
-
-#ifndef HGE_SWEEP_MIN_BLOCKS
-#define HGE_SWEEP_MIN_BLOCKS 4
-#endif
-// 1: the running per-column min / max of the rows a thread produced live in registers (8) instead
-// of shared memory (a 128-bit shared-memory access of a warp is 4 wavefronts of the L1 data pipe,
-// the busiest unit of the node half: 67 % in profiles/r2_half_sweep.md)
-#ifndef HGE_SWEEP_MINMAX_REGS
-#define HGE_SWEEP_MINMAX_REGS 0     // measured: 64 registers do not hold them without spills
-#endif
-// 1: the constants of the lazily applied affine map live in registers (8) as well
-#ifndef HGE_SWEEP_AFFINE_REGS
-#define HGE_SWEEP_AFFINE_REGS 0
-#endif
-// bit 0: the node half stores its rows with the streaming (evict-first) hint, bit 1: the edge half
-// does.  The rows a half writes compete for L2 with the table it gathers from; measured on
-// config 2 (profiles/r2_half_sweep.md): 0.3069 -> 0.3042 ms per sweep with both.
-#ifndef HGE_SWEEP_STORE_CS
-#define HGE_SWEEP_STORE_CS 3
-#endif
-// measurement-only builds (wrong results): 1 = finished rows are dropped, 2 = ids are not
-// broadcast inside the lane group, 4 = descriptors are not read
-#ifndef HGE_SWEEP_DEBUG
-#define HGE_SWEEP_DEBUG 0
-#endif
-// distance, in groups of rows, at which the rows a warp will update are requested into L2 (0: off)
-#ifndef HGE_SWEEP_PREFETCH_OWN
-#define HGE_SWEEP_PREFETCH_OWN 1
-#endif
-// 1: while a round's rows are in flight, L2 is asked for the rows of the NEXT round (their ids are
-// in registers a round ahead): the loads of a round then mostly wait for L2, not for DRAM
-#ifndef HGE_SWEEP_PREFETCH_ROWS
-#define HGE_SWEEP_PREFETCH_ROWS 0
-#endif
-#ifndef HGE_SWEEP_PREFETCH_STEPS
-#define HGE_SWEEP_PREFETCH_STEPS 24
-#endif
+constexpr int kMinBlocks = 4;          // resident blocks per SM the register budget is cut for
+constexpr int kPrefetchSteps = 24;     // distance, in steps, of the L2 prefetch of the id stream
 
 // A gathered float4 is one 128-bit virtual register from the load to the add.  ptxas gives such
 // a register an aligned quad, so the software-pipelined (loop-carried) slots are loaded in place;
@@ -126,15 +91,16 @@ __device__ __forceinline__ void kahan_add4(float4& s, float4& c, const float4& v
 }
 
 template <int LPR, int MODE>
-__global__ void __launch_bounds__(kBlock, HGE_SWEEP_MIN_BLOCKS) k_sweep(const HgeSweepArgs a) {
+__global__ void __launch_bounds__(kBlock, kMinBlocks) k_sweep(const HgeSweepArgs a) {
   constexpr int G = 32 / LPR;                      // lane groups (rows in flight) per warp
   constexpr int K = LPR >= 4 ? 1 : 4 / LPR;        // id registers per lane and step
   constexpr int D = kStreamStepAlign;              // id look-ahead ring = unroll, in steps
   constexpr bool kOwn = MODE == kSweepNode || MODE == kSweepEdge;
 
   // per-thread constants of the lazily applied affine map and the running min / max of the rows
-  // this thread produced: shared memory instead of 16 registers (touched once per finished row)
-  __shared__ float4 s_state[kOwn ? ((HGE_SWEEP_MINMAX_REGS ? 0 : 2) + (HGE_SWEEP_AFFINE_REGS ? 0 : 2)) * kBlock + 1 : 1];
+  // this thread produced: shared memory instead of 16 registers (touched once per finished row;
+  // 64 registers do not hold them without spills)
+  __shared__ float4 s_state[kOwn ? 4 * kBlock + 1 : 1];
   __shared__ float4 s_min[kOwn ? kWarps : 1][LPR];
   __shared__ float4 s_max[kOwn ? kWarps : 1][LPR];
   // row descriptors of the short rows, two halves of 32 per warp, filled by asynchronous copies
@@ -154,7 +120,6 @@ __global__ void __launch_bounds__(kBlock, HGE_SWEEP_MIN_BLOCKS) k_sweep(const Hg
   const char* const basel = reinterpret_cast<const char*>(a.base + c4c);
   const uint32_t row_bytes = (uint32_t)ld4 * 16u;
 
-  float4 rinv = make_float4(1.f, 1.f, 1.f, 1.f), rc3 = make_float4(0.f, 0.f, 0.f, 0.f);
   if (kOwn) {
     float lo[4] = {0.f, 0.f, 0.f, 0.f}, inv[4] = {1.f, 1.f, 1.f, 1.f};
     if (a.mm_prev && active) {
@@ -170,50 +135,25 @@ __global__ void __launch_bounds__(kBlock, HGE_SWEEP_MIN_BLOCKS) k_sweep(const Hg
     // x' = c1 y + (c2 acc - c3):  c1 = inv deg / 2;  node half (the gathered rows carry the map
     // too): c2 = inv invs / 2, c3 = inv lo;  edge half: c2 = invs / 2, c3 = inv lo / 2
     const float h = MODE == kSweepNode ? 1.0f : 0.5f;
-    rinv = make_float4(inv[0], inv[1], inv[2], inv[3]);
-    rc3 = make_float4(h * (lo[0] * inv[0]), h * (lo[1] * inv[1]), h * (lo[2] * inv[2]), h * (lo[3] * inv[3]));
-#if !HGE_SWEEP_AFFINE_REGS
-    sst[0] = rinv;
-    sst[kBlock] = rc3;
-#endif
-#if !HGE_SWEEP_MINMAX_REGS
+    sst[0] = make_float4(inv[0], inv[1], inv[2], inv[3]);
+    sst[kBlock] = make_float4(h * (lo[0] * inv[0]), h * (lo[1] * inv[1]), h * (lo[2] * inv[2]), h * (lo[3] * inv[3]));
     const float inf = __int_as_float(0x7f800000);
     sst[2 * kBlock] = make_float4(inf, inf, inf, inf);
     sst[3 * kBlock] = make_float4(-inf, -inf, -inf, -inf);
-#endif
   }
-  const float kInf = __int_as_float(0x7f800000);
-  float4 rmin = make_float4(kInf, kInf, kInf, kInf), rmax = make_float4(-kInf, -kInf, -kInf, -kInf);
 
   // ---- feeding ----------------------------------------------------------------------------
   auto issue_one = [&](quad& v, const int (&r)[K], const int j) {
-#if HGE_SWEEP_DEBUG & 2
-    const int c = (r[0] + j) & 0xffff;
-#else
     const int c = __shfl_sync(kFull, r[K == 1 ? 0 : j / LPR], K == 1 ? j : j % LPR, LPR);
-#endif
     v = ldg_quad(basel + (size_t)(uint32_t)c * row_bytes);
   };
   auto issue = [&](quad (&v)[4], const int (&r)[K]) {
 #pragma unroll
     for (int j = 0; j < 4; ++j) issue_one(v[j], r, j);
   };
-  auto prefetch_rows = [&](const int (&r)[K]) {
-#if HGE_SWEEP_PREFETCH_ROWS
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int c = __shfl_sync(kFull, r[K == 1 ? 0 : j / LPR], K == 1 ? j : j % LPR, LPR);
-      asm volatile("prefetch.global.L2 [%0];" ::"l"(basel + (size_t)(uint32_t)c * row_bytes));
-    }
-#endif
-  };
   // ---- finishing ----------------------------------------------------------------------------
   // called by the lanes that own (row, c4); acc is the full gathered sum of the row
   auto finish_row = [&](int row, float degf, float invs, const float4& yown, const float4& acc) {
-#if HGE_SWEEP_DEBUG & 1
-    if (acc.x == 123.456f && yown.x == 654.321f) a.own[0] = acc;
-    return;
-#endif
     const size_t off = (size_t)row * ld4 + c4;
     if (MODE == kSweepPush) {
       // fused reduce-scatter: the partial row goes straight into the owning GPU's staging block
@@ -229,11 +169,7 @@ __global__ void __launch_bounds__(kBlock, HGE_SWEEP_MIN_BLOCKS) k_sweep(const Hg
     } else if (MODE == kSweepRaw) {
       a.raw[off] = acc;
     } else {
-#if HGE_SWEEP_AFFINE_REGS
-      const float4 inv = rinv, c3 = rc3;
-#else
       const float4 inv = sst[0], c3 = sst[kBlock];
-#endif
       const float hd = 0.5f * degf, hs = 0.5f * invs;
       float4 x;
       if (MODE == kSweepNode) {
@@ -249,17 +185,10 @@ __global__ void __launch_bounds__(kBlock, HGE_SWEEP_MIN_BLOCKS) k_sweep(const Hg
       }
       const float w = __frcp_rn(degf);
       const float4 y = make_float4(x.x * w, x.y * w, x.z * w, x.w * w);
-      if ((MODE == kSweepNode && (HGE_SWEEP_STORE_CS & 1)) || (MODE == kSweepEdge && (HGE_SWEEP_STORE_CS & 2)))
-        __stcs(a.own + off, y);
-      else
-        a.own[off] = y;
+      // streaming (evict-first) store: the rows a half writes compete for L2 with the table it
+      // gathers from (config 2, profiles/r2_half_sweep.md: 0.3069 -> 0.3042 ms per sweep)
+      __stcs(a.own + off, y);
       // padding columns (>= R) stay 0 and are not published, so no per-column mask here
-#if HGE_SWEEP_MINMAX_REGS
-      rmin.x = fminf(rmin.x, x.x); rmax.x = fmaxf(rmax.x, x.x);
-      rmin.y = fminf(rmin.y, x.y); rmax.y = fmaxf(rmax.y, x.y);
-      rmin.z = fminf(rmin.z, x.z); rmax.z = fmaxf(rmax.z, x.z);
-      rmin.w = fminf(rmin.w, x.w); rmax.w = fmaxf(rmax.w, x.w);
-#else
       float4 lo4 = sst[2 * kBlock], hi4 = sst[3 * kBlock];
       lo4.x = fminf(lo4.x, x.x); hi4.x = fmaxf(hi4.x, x.x);
       lo4.y = fminf(lo4.y, x.y); hi4.y = fmaxf(hi4.y, x.y);
@@ -267,7 +196,6 @@ __global__ void __launch_bounds__(kBlock, HGE_SWEEP_MIN_BLOCKS) k_sweep(const Hg
       lo4.w = fminf(lo4.w, x.w); hi4.w = fmaxf(hi4.w, x.w);
       sst[2 * kBlock] = lo4;
       sst[3 * kBlock] = hi4;
-#endif
     }
   };
   auto reduce_groups = [&](float4& v) {
@@ -296,8 +224,8 @@ __global__ void __launch_bounds__(kBlock, HGE_SWEEP_MIN_BLOCKS) k_sweep(const Hg
   // the id stream is read once, front to back: one lane per warp asks L2 for the line a few
   // steps ahead, so the register ring above only has to cover an L2 hit
   auto prefetch_ids = [&](uint32_t step) {
-    if (HGE_SWEEP_PREFETCH_STEPS > 0 && lane == 0)
-      asm volatile("prefetch.global.L2 [%0];" ::"l"(stream0 + (size_t)(step + HGE_SWEEP_PREFETCH_STEPS) * (4 * G)));
+    if (lane == 0)
+      asm volatile("prefetch.global.L2 [%0];" ::"l"(stream0 + (size_t)(step + kPrefetchSteps) * (4 * G)));
   };
   const int32_t u0 = src.piece[pi], u1 = src.piece[pi + 1];
 
@@ -321,8 +249,6 @@ __global__ void __launch_bounds__(kBlock, HGE_SWEEP_MIN_BLOCKS) k_sweep(const Hg
         quad va[4], vb[4];
         issue(va, r[d]);
         issue(vb, r[d + 1]);
-        prefetch_rows(r[(d + 2) % D]);
-        prefetch_rows(r[(d + 3) % D]);
         load_ids(pos + i + d + D, r[d]);
         load_ids(pos + i + d + 1 + D, r[d + 1]);
         if (d == 0) prefetch_ids(pos + i);
@@ -391,7 +317,7 @@ __global__ void __launch_bounds__(kBlock, HGE_SWEEP_MIN_BLOCKS) k_sweep(const Hg
     // in the ring ahead of their use, so each lane asks L2 for the row of one descriptor half a
     // ring (16 / G .. 48 / G groups of rows) before it is gathered.
     auto prefetch_own = [&](int half) {
-      if (kOwn && HGE_SWEEP_PREFETCH_OWN) {
+      if (kOwn) {
         const int row = ring[half][lane].x;
         if (row >= 0)
           asm volatile("prefetch.global.L2 [%0];" ::"l"(a.own + (size_t)row * ld4 + slab * LPR));
@@ -418,7 +344,7 @@ __global__ void __launch_bounds__(kBlock, HGE_SWEEP_MIN_BLOCKS) k_sweep(const Hg
         ++blk_next;
         slot &= 63;
       }
-      if (kOwn && HGE_SWEEP_PREFETCH_OWN && G <= 16 && (slot & 31) == 16 + g) {
+      if (kOwn && G <= 16 && (slot & 31) == 16 + g) {
         // half way through this half of the ring: the other half (requested when this one was
         // entered) has landed by now -- ask L2 for the rows it describes
         cp_async_wait<0>();
@@ -437,8 +363,6 @@ __global__ void __launch_bounds__(kBlock, HGE_SWEEP_MIN_BLOCKS) k_sweep(const Hg
         quad va[4], vb[4];
         issue(va, r[d]);
         issue(vb, r[d + 1]);
-        prefetch_rows(r[(d + 2) % D]);
-        prefetch_rows(r[(d + 3) % D]);
         load_ids(pos + i + d + D, r[d]);
         load_ids(pos + i + d + 1 + D, r[d + 1]);
         if (d == 0) prefetch_ids(pos + i);
@@ -471,11 +395,7 @@ __global__ void __launch_bounds__(kBlock, HGE_SWEEP_MIN_BLOCKS) k_sweep(const Hg
 
   // ---- per-column min / max of the rows this block produced -------------------------------------
   if (kOwn) {
-#if HGE_SWEEP_MINMAX_REGS
-    float4 lo4 = rmin, hi4 = rmax;
-#else
     float4 lo4 = sst[2 * kBlock], hi4 = sst[3 * kBlock];
-#endif
 #pragma unroll
     for (int off = LPR; off < 32; off <<= 1) {
       lo4.x = fminf(lo4.x, __shfl_xor_sync(kFull, lo4.x, off));

@@ -182,8 +182,8 @@ int hge_p2p_create(hge_ctx* ctx, int rank, int world, int32_t num_local_nodes, i
 int hge_p2p_export(hge_p2p* p, void* handle64);
 int hge_p2p_open_peers(hge_p2p* p, const void* handles /* world x 64 bytes */);
 int hge_p2p_check(hge_p2p* p);
-/* Phase timing of the peer-memory sweep (off by default; hge_p2p_set_timing or HGE_P2P_TIMING=1
- * in the environment at hge_p2p_create): CUDA events around the five phases of every sweep.
+/* Phase timing of the peer-memory sweep (off by default, switched by hge_p2p_set_timing): CUDA
+ * events around the five phases of every sweep.
  * hge_p2p_phase_ms returns the mean ms per sweep of each since the last call -- node half, edge
  * gather + push, barrier A, owner reduce + all-gather, barrier B + min/max -- and the number of
  * sweeps averaged over (0: nothing recorded). */

@@ -113,8 +113,9 @@ def make_graph(seed, n, e, nnz):
 
 
 def worker(rank, world, port, backend, graph_args, R, iters, slices, out_dir, use_native,
-           comm="nccl"):
-  """Runs the sharded relaxation on one rank and writes its node block to out_dir."""
+           comm="nccl", tile_mb=0):
+  """Runs the sharded relaxation on one rank and writes its node block to out_dir.  tile_mb > 0
+  forces node-range tiles of that many MB on the rank's context, whatever the edge sizes."""
   os.environ["MASTER_ADDR"] = "127.0.0.1"
   os.environ["MASTER_PORT"] = str(port)
   import torch
@@ -129,6 +130,9 @@ def worker(rank, world, port, backend, graph_args, R, iters, slices, out_dir, us
     xn0 = rng.random((A.shape[0], R)).astype(np.float32)
     xe0 = rng.random((A.shape[1], R)).astype(np.float32)
     A_loc, r0, r1 = hd.local_shard(A, rank, world)
+    if tile_mb:
+      from hypergraphembedding_b200 import _native
+      _native.default_context().set_tile_mb(tile_mb, 0)
     relax = hd.ShardedRelaxation(A_loc, R, iters, num_slices=slices, comm=comm,
                                  ops_factory=None if use_native else NumpyOps)
     assert relax.use_p2p == (comm == "p2p")

@@ -45,16 +45,14 @@ def test_one_rank(tmp_path, slices, comm):
 
 
 @pytest.mark.parametrize("world", [1, 2])
-def test_peer_memory_sweep_with_node_range_tiles(tmp_path, world, monkeypatch):
-  """The shard's edge gather in node-range tiles (1 MB tiles forced through the environment the
-  workers inherit): partial sums accumulated per tile, then pushed to their owners."""
+def test_peer_memory_sweep_with_node_range_tiles(tmp_path, world):
+  """The shard's edge gather in node-range tiles (1 MB tiles forced on every worker's context):
+  partial sums accumulated per tile, then pushed to their owners."""
   if torch.cuda.device_count() < world:
     pytest.skip("needs %d GPUs" % world)
-  monkeypatch.setenv("HGE_TILE_MB", "1")
-  monkeypatch.setenv("HGE_TILE_MIN_MB", "0")
   graph_args = (12, 60000, 800, 400000)
   mp.spawn(dist_helpers.worker,
-           args=(world, _free_port(), "nccl", graph_args, 32, 6, 1, str(tmp_path), True, "p2p"),
+           args=(world, _free_port(), "nccl", graph_args, 32, 6, 1, str(tmp_path), True, "p2p", 1),
            nprocs=world, join=True)
   _check(tmp_path, world, graph_args, 32, 6)
 

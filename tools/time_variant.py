@@ -1,5 +1,8 @@
-"""Times the half-sweep kernel of the library selected by HGE_LIB_PATH on config 2 and reports
-its error on the youtube golden.  Prints one JSON line.  Used by tools/sweep_variants.py."""
+"""Times the node and edge half-sweeps of the built library on one bench workload (config 2 by
+default) and reports its error on the youtube golden.  Prints one JSON line.
+
+    python tools/time_variant.py [WORKLOAD [LIGHT_MAX_DEG CHUNK BLOCKS_PER_SM]]
+"""
 import json
 import os
 import sys
@@ -39,7 +42,7 @@ def main():
   ctx = _native.default_context(0)
   if tuning:
     ctx.set_tuning(*tuning)
-  out = dict(lib=os.path.basename(_native.LIB_PATH), tuning=tuning)
+  out = dict(tuning=tuning)
   out.update(golden_error(ctx))
   A, B = build_workload(spec)
   N, E = A.shape

@@ -267,8 +267,7 @@ struct PairSampler {
     HGE_TRY(uptr.alloc((size_t)L + 1));
     k_run_cols<<<grid_for(ctx, n), kBlock, 0, ctx->stream>>>(n, keys2.p, pos.p, ucol.p);
     HGE_CHECK_LAUNCH(ctx);
-    k_run_starts<<<grid_for(ctx, L + 1), kBlock, 0, ctx->stream>>>(0, L, n, *n_runs, 0, keys2.p, pos.p, uptr.p,
-                                                                  true);
+    k_run_starts<<<grid_for(ctx, L + 1), kBlock, 0, ctx->stream>>>(L, n, *n_runs, keys2.p, pos.p, uptr.p);
     HGE_CHECK_LAUNCH(ctx);
     return HGE_OK;
   }

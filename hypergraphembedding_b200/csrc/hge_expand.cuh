@@ -2,7 +2,8 @@
 // by the centroid rows of csrc/hge_jaccard.cu and the candidate rows of
 // csrc/hge_device_sampler.cu.  Keys are (local row << 32) | column, sorted ascending, so the runs
 // of one row are its distinct columns in ascending order.  Also the grouping of (x, group) pairs
-// by group shared by hge_jaccard_centroid_grouped and hge_lp_svm_predict (csrc/hge_lp_svm.cu).
+// by group shared by the centroid factors of csrc/hge_jaccard.cu and hge_lp_svm_predict
+// (csrc/hge_lp_svm.cu).
 #pragma once
 
 #include <cub/device/device_radix_sort.cuh>
@@ -21,14 +22,11 @@ __global__ void k_run_heads(int64_t n, const uint64_t* __restrict__ keys, int64_
     head[i] = (i == 0 || keys[i] != keys[i - 1]) ? 1 : 0;
 }
 
-// start[g0 + k] for k in [0, g1 - g0) (and k = g1 - g0 when last_batch): rows_before + position,
-// among the runs of the sorted keys, of the first run of local row k (pos = exclusive scan of
-// the run heads, n_runs = number of runs)
-__global__ void k_run_starts(int64_t g0, int64_t g1, int64_t n, int64_t n_runs, int64_t rows_before,
-                             const uint64_t* __restrict__ keys, const int64_t* __restrict__ pos,
-                             int64_t* __restrict__ start, bool last_batch) {
-  const int64_t count = g1 - g0 + (last_batch ? 1 : 0);
-  for (int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; k < count;
+// start[k] for k in [0, L]: position, among the runs of the sorted keys, of the first run of
+// local row k (pos = exclusive scan of the run heads, n_runs = number of runs = start[L])
+__global__ void k_run_starts(int64_t L, int64_t n, int64_t n_runs, const uint64_t* __restrict__ keys,
+                             const int64_t* __restrict__ pos, int64_t* __restrict__ start) {
+  for (int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; k <= L;
        k += (int64_t)gridDim.x * blockDim.x) {
     const uint64_t want = (uint64_t)k << 32;
     int64_t lo = 0, hi = n;
@@ -36,7 +34,7 @@ __global__ void k_run_starts(int64_t g0, int64_t g1, int64_t n, int64_t n_runs, 
       const int64_t mid = (lo + hi) >> 1;
       if (keys[mid] < want) lo = mid + 1; else hi = mid;
     }
-    start[g0 + k] = rows_before + (lo < n ? pos[lo] : n_runs);
+    start[k] = lo < n ? pos[lo] : n_runs;
   }
 }
 

@@ -19,13 +19,13 @@
 //               y = (sum_{t in group} F[t]) / |group|  (CentroidFromRows, :284-299,
 //               DiffTypeJaccardSample, :343-392).  The reference materialises the centroid rows
 //               with scipy (column sums of F[rows]: the members are added in ascending order,
-//               fp32, then one division); so does this file, for the groups the pairs name:
-//               expand (group, column, value) triples in member order, stable radix sort by
-//               (group, column), one sequential sum per run -- the classic expand / sort /
-//               compress product, batched so that the expansion stays inside a memory budget.
-//               hge_jaccard_centroid keeps every named centroid row resident until its merge;
-//               hge_jaccard_centroid_grouped sorts the pairs by group and builds, merges and
-//               frees the rows batch by batch, so its peak is the budget plus O(pairs).
+//               fp32, then one division); so does this file, for the groups the pairs name.
+//               centroid_factor, which both centroid entry points call, sorts the pairs by
+//               group, then cuts the named groups into batches whose expansion fits a memory
+//               budget.  Per batch it expands (group, column, value) triples in member order,
+//               stable radix sorts them by (group, column) and sums each run in order -- the
+//               classic expand / sort / compress product -- then merges the batch's pairs and
+//               frees its rows, so the peak is the budget plus O(pairs).
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
@@ -35,13 +35,12 @@
 #include "hge_common.cuh"
 #include "hge_expand.cuh"
 #include "hge_incidence.cuh"
+#include "hge_pairs.cuh"
 
 namespace {
 
 constexpr int kBlock = 256;
 constexpr unsigned kFull = 0xffffffffu;
-// entries of one expansion batch (12 bytes each, twice for the sort's double buffer)
-constexpr int64_t kBatchEntries = 192ll << 20;
 
 // one step of SparseWeightedJaccard's loop (hg2v_sample.py:264-271)
 __device__ __forceinline__ void jaccard_step(float x, float y, float& num, float& den) {
@@ -81,98 +80,31 @@ __device__ __forceinline__ float jaccard_pair(const int64_t* __restrict__ aptr, 
   return den == 0.f ? 0.f : __fdiv_rn(num, den);
 }
 
-// out[p] = J(A[pa[p]], B[pb[p]]), one thread per pair.
-// b_members (optional): a pair whose group rb has no members gives 0.
+// out[p] = J(F[pi[p]], F[pj[p]]), one thread per pair
 __global__ void __launch_bounds__(kBlock) k_jaccard_merge(
-    int64_t num_pairs, const int64_t* __restrict__ aptr, const int32_t* __restrict__ aidx,
-    const float* __restrict__ aval, const int64_t* __restrict__ bptr, const int32_t* __restrict__ bidx,
-    const float* __restrict__ bval, const int32_t* __restrict__ pa, const int32_t* __restrict__ pb,
-    const int64_t* __restrict__ b_members, float* __restrict__ out) {
-  for (int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; p < num_pairs;
-       p += (int64_t)gridDim.x * blockDim.x) {
-    const int32_t ra = pa[p], rb = pb[p];
-    if (b_members && b_members[rb + 1] == b_members[rb]) {   // a group without members has no centroid
-      out[p] = 0.f;
-      continue;
-    }
-    out[p] = jaccard_pair(aptr, aidx, aval, ra, bptr, bidx, bval, rb);
-  }
-}
-
-// ---- centroid rows -----------------------------------------------------------------------------
-
-__global__ void k_flag_groups(int64_t num_pairs, const int32_t* __restrict__ pg, int32_t* __restrict__ flag) {
+    int64_t num_pairs, const int64_t* __restrict__ ptr, const int32_t* __restrict__ idx,
+    const float* __restrict__ val, const int32_t* __restrict__ pi, const int32_t* __restrict__ pj,
+    float* __restrict__ out) {
   for (int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; p < num_pairs;
        p += (int64_t)gridDim.x * blockDim.x)
-    flag[pg[p]] = 1;
+    out[p] = jaccard_pair(ptr, idx, val, pi[p], ptr, idx, val, pj[p]);
 }
 
-// w[t] = non-zeros of F[gidx[t]] when t's group is named by a pair, else 0 (one warp per group)
-__global__ void __launch_bounds__(kBlock) k_member_weights(
-    int64_t groups, const int64_t* __restrict__ gptr, const int32_t* __restrict__ gidx,
-    const int32_t* __restrict__ flag, const int64_t* __restrict__ fptr, int64_t* __restrict__ w) {
-  const int lane = threadIdx.x & 31;
-  const int64_t nw = (int64_t)gridDim.x * (kBlock / 32);
-  for (int64_t g = blockIdx.x * (int64_t)(kBlock / 32) + (threadIdx.x >> 5); g < groups; g += nw) {
-    const bool on = flag[g] != 0;
-    for (int64_t t = gptr[g] + lane; t < gptr[g + 1]; t += 32) {
-      const int32_t m = gidx[t];
-      w[t] = on ? fptr[m + 1] - fptr[m] : 0;
-    }
-  }
-}
-
-// goff[g] = off[gptr[g]]: first expanded entry of group g (goff[groups] = total)
-__global__ void k_group_offsets(int64_t groups, int64_t gnnz, int64_t total, const int64_t* __restrict__ gptr,
-                                const int64_t* __restrict__ off, int64_t* __restrict__ goff) {
-  for (int64_t g = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; g <= groups;
-       g += (int64_t)gridDim.x * blockDim.x) {
-    const int64_t t = gptr[g];
-    goff[g] = t < gnnz ? off[t] : total;
-  }
-}
-
-// expansion of the member positions [t0, t1) (groups [g0, g1)): one warp per member position,
-// entries in member order; key = (group - g0) << 32 | column
-__global__ void __launch_bounds__(kBlock) k_expand(
-    int64_t t0, int64_t t1, int64_t g0, int64_t g1, int64_t base, const int64_t* __restrict__ gptr,
-    const int32_t* __restrict__ gidx, const int64_t* __restrict__ off, const int64_t* __restrict__ w,
-    const int64_t* __restrict__ fptr, const int32_t* __restrict__ fidx, const float* __restrict__ fval,
-    uint64_t* __restrict__ keys, float* __restrict__ vals) {
-  const int lane = threadIdx.x & 31;
-  const int64_t nw = (int64_t)gridDim.x * (kBlock / 32);
-  for (int64_t t = t0 + blockIdx.x * (int64_t)(kBlock / 32) + (threadIdx.x >> 5); t < t1; t += nw) {
-    const int64_t n = w[t];
-    if (n == 0) continue;
-    // group of t: last g in [g0, g1) with gptr[g] <= t
-    int64_t lo = g0, hi = g1;
-    while (hi - lo > 1) {
-      const int64_t mid = (lo + hi) >> 1;
-      if (gptr[mid] <= t) lo = mid; else hi = mid;
-    }
-    const uint64_t gkey = (uint64_t)(lo - g0) << 32;
-    const int64_t src = fptr[gidx[t]], dst = off[t] - base;
-    for (int64_t k = lane; k < n; k += 32) {
-      keys[dst + k] = gkey | (uint32_t)fidx[src + k];
-      vals[dst + k] = fval[src + k];
-    }
-  }
-}
+// ---- centroid rows of the named groups, batch by batch ----------------------------------------
 
 // head of a run: the members' values added in member order, then one division by the group size
 // (targets2features[rows].sum(axis=0) / len(rows), hg2v_sample.py:293).  Local group l is group
-// gid[l] of the group CSR, or g0 + l when gid is NULL.
-__global__ void k_run_sums(int64_t n, int64_t g0, const int32_t* __restrict__ gid,
-                           const uint64_t* __restrict__ keys, const float* __restrict__ vals,
-                           const int64_t* __restrict__ pos, const int64_t* __restrict__ gptr,
-                           int32_t* __restrict__ cidx, float* __restrict__ cval) {
+// gid[l] of the group CSR.
+__global__ void k_run_sums(int64_t n, const int32_t* __restrict__ gid, const uint64_t* __restrict__ keys,
+                           const float* __restrict__ vals, const int64_t* __restrict__ pos,
+                           const int64_t* __restrict__ gptr, int32_t* __restrict__ cidx, float* __restrict__ cval) {
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n;
        i += (int64_t)gridDim.x * blockDim.x) {
     const uint64_t key = keys[i];
     if (i > 0 && keys[i - 1] == key) continue;
     float s = 0.f;
     for (int64_t k = i; k < n && keys[k] == key; ++k) s = __fadd_rn(s, vals[k]);
-    const int64_t l = (int64_t)(key >> 32), g = gid ? (int64_t)gid[l] : g0 + l;
+    const int64_t g = gid[key >> 32];
     const int64_t o = pos[i];
     cidx[o] = (int32_t)(uint32_t)key;
     cval[o] = __fdiv_rn(s, (float)(gptr[g + 1] - gptr[g]));
@@ -192,24 +124,14 @@ struct FeatureMatrix {
   }
 };
 
-// Centroid rows of the groups named by pg[0 .. num_pairs): CSR over ALL groups (rows of the
-// groups no pair names are empty).  Everything on ctx->stream.
-struct CentroidRows {
-  DevBuf<int64_t> ptr;
-  DevBuf<int32_t> idx;
-  DevBuf<float> val;
-  explicit CentroidRows(const hge_ctx* c) : ptr(c), idx(c), val(c) {}
-};
-
 // Centroid rows of one batch of L groups from its expansion: keys ((local group << 32) | column)
 // and vals, n > 0 entries in member order.  Stable radix sort by key (inside a (group, column) run
 // the members stay in ascending order), run heads, then one sequential fp32 sum per run.  Local
-// group l is group gid[l] of the group CSR (g0 + l when gid is NULL).  The rows' start offsets go to
-// start[s0 + l] = rows_before + first run of l (and start[s0 + L] when last); the n_runs column ids
-// and values to cidx / cval.  keys / vals are used as sort buffers.
-int centroid_batch(hge_ctx* ctx, int64_t n, int64_t L, int64_t g0, const int32_t* gid, const int64_t* gptr,
-                   DevBuf<uint64_t>& keys, DevBuf<float>& vals, int64_t* start, int64_t s0, int64_t rows_before,
-                   bool last, DevBuf<int32_t>& cidx, DevBuf<float>& cval, int64_t* n_runs) {
+// group l is group gid[l] of the group CSR.  The rows go to the CSR (cptr [L + 1], cidx, cval);
+// keys / vals are used as sort buffers.
+int centroid_batch(hge_ctx* ctx, int64_t n, int64_t L, const int32_t* gid, const int64_t* gptr,
+                   DevBuf<uint64_t>& keys, DevBuf<float>& vals, int64_t* cptr, DevBuf<int32_t>& cidx,
+                   DevBuf<float>& cval) {
   DevBuf<uint64_t> keys2(ctx);
   DevBuf<float> vals2(ctx);
   DevBuf<int64_t> head(ctx), pos(ctx);
@@ -236,112 +158,16 @@ int centroid_batch(hge_ctx* ctx, int64_t n, int64_t L, int64_t g0, const int32_t
   HGE_TRY(temp.alloc(bytes));
   HGE_CUDA(cub::DeviceScan::ExclusiveSum(temp.p, bytes, head.p, pos.p, n + 1, ctx->stream));
   ctx->launches++;
-  HGE_TRY(read_back(ctx, pos.p + n, n_runs, 1));
-  HGE_TRY(cidx.alloc((size_t)std::max<int64_t>(1, *n_runs)));
-  HGE_TRY(cval.alloc((size_t)std::max<int64_t>(1, *n_runs)));
-  k_run_sums<<<grid_for(ctx, n), kBlock, 0, ctx->stream>>>(n, g0, gid, sk, sv, pos.p, gptr, cidx.p, cval.p);
+  int64_t n_runs = 0;
+  HGE_TRY(read_back(ctx, pos.p + n, &n_runs, 1));
+  HGE_TRY(cidx.alloc((size_t)std::max<int64_t>(1, n_runs)));
+  HGE_TRY(cval.alloc((size_t)std::max<int64_t>(1, n_runs)));
+  k_run_sums<<<grid_for(ctx, n), kBlock, 0, ctx->stream>>>(n, gid, sk, sv, pos.p, gptr, cidx.p, cval.p);
   HGE_CHECK_LAUNCH(ctx);
-  k_run_starts<<<grid_for(ctx, L + 1), kBlock, 0, ctx->stream>>>(s0, s0 + L, n, *n_runs, rows_before, sk, pos.p,
-                                                               start, last);
+  k_run_starts<<<grid_for(ctx, L + 1), kBlock, 0, ctx->stream>>>(L, n, n_runs, sk, pos.p, cptr);
   HGE_CHECK_LAUNCH(ctx);
   return HGE_OK;
 }
-
-int build_centroids(hge_ctx* ctx, const int64_t* gptr, const int32_t* gidx, int64_t groups, int64_t gnnz,
-                    const FeatureMatrix& f, const int32_t* pg, int64_t num_pairs, CentroidRows* out) {
-  DevBuf<int32_t> flag(ctx);
-  DevBuf<int64_t> w(ctx), off(ctx), goff(ctx);
-  DevBuf<char> scan_temp(ctx);
-  HGE_TRY(flag.alloc((size_t)groups));
-  HGE_TRY(w.alloc((size_t)gnnz + 1));
-  HGE_TRY(off.alloc((size_t)gnnz + 1));
-  HGE_TRY(goff.alloc((size_t)groups + 1));
-  HGE_TRY(out->ptr.alloc((size_t)groups + 1));
-  HGE_CUDA(cudaMemsetAsync(flag.p, 0, (size_t)groups * sizeof(int32_t), ctx->stream));
-  HGE_CUDA(cudaMemsetAsync(w.p, 0, ((size_t)gnnz + 1) * sizeof(int64_t), ctx->stream));
-  k_flag_groups<<<grid_for(ctx, num_pairs), kBlock, 0, ctx->stream>>>(num_pairs, pg, flag.p);
-  HGE_CHECK_LAUNCH(ctx);
-  k_member_weights<<<grid_for(ctx, groups, kBlock / 32), kBlock, 0, ctx->stream>>>(groups, gptr, gidx, flag.p,
-                                                                                 f.ptr.dev, w.p);
-  HGE_CHECK_LAUNCH(ctx);
-  size_t scan_bytes = 0;
-  HGE_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, w.p, off.p, gnnz + 1, ctx->stream));
-  HGE_TRY(scan_temp.alloc(scan_bytes));
-  HGE_CUDA(cub::DeviceScan::ExclusiveSum(scan_temp.p, scan_bytes, w.p, off.p, gnnz + 1, ctx->stream));
-  ctx->launches++;
-  scan_temp.reset();
-  int64_t total = 0;
-  HGE_TRY(read_back(ctx, off.p + gnnz, &total, 1));
-  k_group_offsets<<<grid_for(ctx, groups + 1), kBlock, 0, ctx->stream>>>(groups, gnnz, total, gptr, off.p,
-                                                                         goff.p);
-  HGE_CHECK_LAUNCH(ctx);
-  std::vector<int64_t> h_goff((size_t)groups + 1), h_gptr((size_t)groups + 1);
-  HGE_TRY(read_back(ctx, goff.p, h_goff.data(), (size_t)groups + 1));
-  HGE_TRY(read_back(ctx, gptr, h_gptr.data(), (size_t)groups + 1));
-
-  // batches of consecutive groups whose expansion fits the budget (a single group larger than
-  // the budget is its own batch)
-  struct Part {
-    DevBuf<int32_t> idx;
-    DevBuf<float> val;
-    int64_t n;
-  };
-  std::vector<Part> parts;
-  int64_t rows_before = 0;
-  for (int64_t g0 = 0; g0 < groups;) {
-    int64_t g1 = g0 + 1;
-    while (g1 < groups && h_goff[(size_t)g1 + 1] - h_goff[(size_t)g0] <= kBatchEntries && g1 - g0 < (1ll << 31) - 1)
-      ++g1;
-    const int64_t n = h_goff[(size_t)g1] - h_goff[(size_t)g0];
-    const bool last = g1 == groups;
-    if (n == 0) {
-      // no pair names any of these groups: empty rows
-      k_run_starts<<<grid_for(ctx, g1 - g0 + 1), kBlock, 0, ctx->stream>>>(g0, g1, 0, 0, rows_before, nullptr,
-                                                                         nullptr, out->ptr.p, last);
-      HGE_CHECK_LAUNCH(ctx);
-      g0 = g1;
-      continue;
-    }
-    DevBuf<uint64_t> keys(ctx);
-    DevBuf<float> vals(ctx);
-    Part part = {DevBuf<int32_t>(ctx), DevBuf<float>(ctx), 0};
-    HGE_TRY(keys.alloc((size_t)n));
-    HGE_TRY(vals.alloc((size_t)n));
-    k_expand<<<grid_for(ctx, h_gptr[(size_t)g1] - h_gptr[(size_t)g0], kBlock / 32), kBlock, 0, ctx->stream>>>(
-        h_gptr[(size_t)g0], h_gptr[(size_t)g1], g0, g1, h_goff[(size_t)g0], gptr, gidx, off.p, w.p, f.ptr.dev,
-        f.idx.dev, f.val.dev, keys.p, vals.p);
-    HGE_CHECK_LAUNCH(ctx);
-    HGE_TRY(centroid_batch(ctx, n, g1 - g0, g0, nullptr, gptr, keys, vals, out->ptr.p, g0, rows_before, last,
-                           part.idx, part.val, &part.n));
-    rows_before += part.n;
-    parts.push_back(std::move(part));
-    g0 = g1;
-  }
-  flag.reset();
-  w.reset();
-  off.reset();
-  goff.reset();
-  if (parts.size() == 1) {
-    out->idx = std::move(parts[0].idx);
-    out->val = std::move(parts[0].val);
-    return HGE_OK;
-  }
-  HGE_TRY(out->idx.alloc((size_t)std::max<int64_t>(1, rows_before)));
-  HGE_TRY(out->val.alloc((size_t)std::max<int64_t>(1, rows_before)));
-  int64_t at = 0;
-  for (const Part& p : parts) {
-    if (p.n) {
-      HGE_CUDA(cudaMemcpyAsync(out->idx.p + at, p.idx.p, (size_t)p.n * sizeof(int32_t), cudaMemcpyDeviceToDevice,
-                               ctx->stream));
-      HGE_CUDA(cudaMemcpyAsync(out->val.p + at, p.val.p, (size_t)p.n * sizeof(float), cudaMemcpyDeviceToDevice,
-                               ctx->stream));
-    }
-    at += p.n;
-  }
-  return HGE_OK;
-}
-
-// ---- centroid rows of the named groups, batch by batch (hge_jaccard_centroid_grouped) ----------
 
 constexpr int64_t kDefaultWorkspaceMb = 2048;
 // workspace bytes per expanded entry of a batch: keys and their sort buffer (16), values and theirs
@@ -428,98 +254,21 @@ __global__ void __launch_bounds__(kBlock) k_merge_named(
   }
 }
 
-}  // namespace
-
-extern "C" {
-
-int hge_jaccard_rows(hge_ctx* ctx, const int64_t* ptr, const int32_t* idx, const float* val,
-                     int64_t rows, int64_t nnz, const int32_t* pi, const int32_t* pj,
-                     int64_t num_pairs, float* out, int mem) {
-  HGE_REQUIRE(ctx && ptr && (idx || nnz == 0) && (val || nnz == 0) && rows >= 0 && nnz >= 0,
-              "hge_jaccard_rows: bad feature matrix");
-  HGE_REQUIRE(num_pairs >= 0 && (num_pairs == 0 || (pi && pj && out)), "hge_jaccard_rows: bad pairs");
-  HGE_REQUIRE(mem == HGE_MEM_HOST || mem == HGE_MEM_DEVICE, "hge_jaccard_rows: bad mem %d", mem);
-  HGE_CUDA(cudaSetDevice(ctx->device));
-  if (num_pairs == 0) return HGE_OK;
-  FeatureMatrix f(ctx);
-  Staged<int32_t> s_i(ctx), s_j(ctx);
-  Staged<float> s_out(ctx);
-  HGE_TRY(f.init(ptr, idx, val, rows, nnz, mem));
-  HGE_TRY(s_i.init(pi, (size_t)num_pairs, mem, true, false));
-  HGE_TRY(s_j.init(pj, (size_t)num_pairs, mem, true, false));
-  HGE_TRY(s_out.init(out, (size_t)num_pairs, mem, false, true));
-  k_jaccard_merge<<<grid_for(ctx, num_pairs), kBlock, 0, ctx->stream>>>(
-      num_pairs, f.ptr.dev, f.idx.dev, f.val.dev, f.ptr.dev, f.idx.dev, f.val.dev, s_i.dev, s_j.dev, nullptr,
-      s_out.dev);
-  HGE_CHECK_LAUNCH(ctx);
-  return s_out.finish();
-}
-
-int hge_jaccard_centroid(hge_ctx* ctx, const int64_t* xptr, const int32_t* xidx, const float* xval,
-                         int64_t xrows, int64_t xnnz, const int64_t* gptr, const int32_t* gidx,
-                         int64_t grows, int64_t gnnz, const int64_t* fptr, const int32_t* fidx,
-                         const float* fval, int64_t frows, int64_t fnnz, const int32_t* px,
-                         const int32_t* pg, int64_t num_pairs, float* out, int mem) {
-  HGE_REQUIRE(ctx && xptr && gptr && fptr && xrows >= 0 && grows >= 0 && frows >= 0 && xnnz >= 0 &&
-                  gnnz >= 0 && fnnz >= 0, "hge_jaccard_centroid: bad matrix");
-  HGE_REQUIRE(num_pairs >= 0 && (num_pairs == 0 || (px && pg && out)), "hge_jaccard_centroid: bad pairs");
-  HGE_REQUIRE(mem == HGE_MEM_HOST || mem == HGE_MEM_DEVICE, "hge_jaccard_centroid: bad mem %d", mem);
-  HGE_CUDA(cudaSetDevice(ctx->device));
-  if (num_pairs == 0) return HGE_OK;
-  FeatureMatrix x(ctx), f(ctx);
-  const bool same = xptr == fptr && xidx == fidx && xval == fval;   // usual case: X is F
-  Staged<int64_t> s_gptr(ctx);
-  Staged<int32_t> s_gidx(ctx), s_px(ctx), s_pg(ctx);
-  Staged<float> s_out(ctx);
-  HGE_TRY(f.init(fptr, fidx, fval, frows, fnnz, mem));
-  if (!same) HGE_TRY(x.init(xptr, xidx, xval, xrows, xnnz, mem));
-  HGE_TRY(s_gptr.init(gptr, (size_t)grows + 1, mem, true, false));
-  HGE_TRY(s_gidx.init(gidx, (size_t)gnnz, mem, true, false));
-  HGE_TRY(s_px.init(px, (size_t)num_pairs, mem, true, false));
-  HGE_TRY(s_pg.init(pg, (size_t)num_pairs, mem, true, false));
-  HGE_TRY(s_out.init(out, (size_t)num_pairs, mem, false, true));
-  CentroidRows c(ctx);
-  HGE_TRY(build_centroids(ctx, s_gptr.dev, s_gidx.dev, grows, gnnz, f, s_pg.dev, num_pairs, &c));
-  const FeatureMatrix& xr = same ? f : x;
-  k_jaccard_merge<<<grid_for(ctx, num_pairs), kBlock, 0, ctx->stream>>>(
-      num_pairs, xr.ptr.dev, xr.idx.dev, xr.val.dev, c.ptr.p, c.idx.p, c.val.p, s_px.dev, s_pg.dev, s_gptr.dev,
-      s_out.dev);
-  HGE_CHECK_LAUNCH(ctx);
-  return s_out.finish();
-}
-
-int hge_jaccard_centroid_grouped(hge_ctx* ctx, hge_incidence* inc, int group_side, const int64_t* xptr,
-                                 const int32_t* xidx, const float* xval, int64_t xrows, int64_t xnnz,
-                                 const int64_t* fptr, const int32_t* fidx, const float* fval, int64_t frows,
-                                 int64_t fnnz, const int32_t* px, const int32_t* pg, int64_t num_pairs,
-                                 int64_t workspace_mb, float* out) {
-  HGE_REQUIRE(ctx && inc, "hge_jaccard_centroid_grouped: NULL argument");
-  HGE_REQUIRE(!inc->sharded, "hge_jaccard_centroid_grouped: needs a whole (not sharded) incidence");
-  HGE_REQUIRE(group_side == 0 || group_side == 1, "hge_jaccard_centroid_grouped: group_side must be 0 or 1");
-  HGE_REQUIRE(xptr && fptr && xrows >= 0 && frows >= 0 && xnnz >= 0 && fnnz >= 0 && (xidx || xnnz == 0) &&
-                  (xval || xnnz == 0) && (fidx || fnnz == 0) && (fval || fnnz == 0),
-              "hge_jaccard_centroid_grouped: bad matrix");
-  // groups are edges with node members (F = node features), or nodes with edge members
-  const int64_t groups = group_side == 1 ? inc->E : inc->N, members = group_side == 1 ? inc->N : inc->E;
-  HGE_REQUIRE(frows == members, "hge_jaccard_centroid_grouped: F has %lld rows, the members number %lld",
-              (long long)frows, (long long)members);
-  HGE_REQUIRE(num_pairs >= 0 && num_pairs < (1ll << 31) && (num_pairs == 0 || (px && pg && out)),
-              "hge_jaccard_centroid_grouped: bad pairs");
-  HGE_REQUIRE(workspace_mb >= 0, "hge_jaccard_centroid_grouped: negative workspace");
-  HGE_CUDA(cudaSetDevice(ctx->device));
-  if (num_pairs == 0) return HGE_OK;
-  const int64_t* gptr = group_side == 1 ? inc->e2n_ptr : inc->n2e_ptr;
-  const int32_t* gidx = group_side == 1 ? inc->e2n_idx : inc->n2e_idx;
-  const int64_t n = num_pairs;
-
+// out[p] = J(X[px[p]], centroid of the members of group pg[p]) for p in [0, n), n in [1, 2^31): the
+// groups are the CSR (gptr, gidx) over the rows of F, groups of them (at most 2^31).  Every pointer
+// is a device pointer; the centroid rows are built in batches of at most workspace_mb MB.  A pair
+// naming a row outside [0, xrows) or a group outside [0, groups) is HGE_ERR_INVALID, reported under
+// the entry point's name `who`; nothing is computed then.
+int centroid_factor(hge_ctx* ctx, const char* who, const int64_t* gptr, const int32_t* gidx, int64_t groups,
+                    const int64_t* xptr, const int32_t* xidx, const float* xval, int64_t xrows,
+                    const int64_t* fptr, const int32_t* fidx, const float* fval, const int32_t* px,
+                    const int32_t* pg, int64_t n, int64_t workspace_mb, float* out) {
   // 1. pairs stably sorted by group
   PairGroups pg_sorted(ctx);
   int bad = 0;
   HGE_TRY(pg_sorted.build(ctx, n, px, xrows, pg, groups, &bad));
-  HGE_REQUIRE(!(bad & kBadX), "hge_jaccard_centroid_grouped: a pair names a row outside X's %lld",
-              (long long)xrows);
-  HGE_REQUIRE(!(bad & kBadGroup), "hge_jaccard_centroid_grouped: a pair names a group outside [0, %lld)",
-              (long long)groups);
+  HGE_REQUIRE(!(bad & kBadX), "%s: a pair names a row outside X's %lld", who, (long long)xrows);
+  HGE_REQUIRE(!(bad & kBadGroup), "%s: a pair names a group outside [0, %lld)", who, (long long)groups);
   const int32_t* order = pg_sorted.order;
   const int64_t U = pg_sorted.U;
   DevBuf<int32_t>& ug = pg_sorted.ug;
@@ -546,8 +295,7 @@ int hge_jaccard_centroid_grouped(hge_ctx* ctx, hge_incidence* inc, int group_sid
 
   // 3. batches of consecutive named groups whose expansion fits the budget (a single larger group
   //    is its own batch): centroid rows, then the merge of the batch's pairs
-  const int64_t mb = workspace_mb ? workspace_mb : kDefaultWorkspaceMb;
-  const int64_t budget = std::max<int64_t>(1, (mb << 20) / kBytesPerEntry);
+  const int64_t budget = std::max<int64_t>(1, (workspace_mb << 20) / kBytesPerEntry);
   for (int64_t u0 = 0; u0 < U;) {
     int64_t u1 = u0 + 1;
     while (u1 < U && h_uoff[(size_t)u1 + 1] - h_uoff[(size_t)u0] <= budget) ++u1;
@@ -564,14 +312,13 @@ int hge_jaccard_centroid_grouped(hge_ctx* ctx, hge_incidence* inc, int group_sid
       int rc = keys.alloc((size_t)m);
       if (rc == HGE_OK) rc = vals.alloc((size_t)m);
       if (rc == HGE_ERR_NOMEM)
-        hge_set_error("hge_jaccard_centroid_grouped: %lld groups expand to %lld entries, more than the device holds",
-                      (long long)L, (long long)m);
+        hge_set_error("%s: %lld groups expand to %lld entries, more than the device holds", who, (long long)L,
+                      (long long)m);
       HGE_TRY(rc);
       k_expand_named<<<grid_for(ctx, L, kBlock / 32), kBlock, 0, ctx->stream>>>(
           u0, u1, h_uoff[(size_t)u0], ug.p, uoff.p, gptr, gidx, fptr, fidx, fval, keys.p, vals.p);
       HGE_CHECK_LAUNCH(ctx);
-      int64_t runs = 0;
-      HGE_TRY(centroid_batch(ctx, m, L, 0, ug.p + u0, gptr, keys, vals, cptr.p, 0, 0, true, cidx, cval, &runs));
+      HGE_TRY(centroid_batch(ctx, m, L, ug.p + u0, gptr, keys, vals, cptr.p, cidx, cval));
     }
     const int64_t i0 = h_ustart[(size_t)u0], i1 = h_ustart[(size_t)u1];
     k_merge_named<<<grid_for(ctx, i1 - i0), kBlock, 0, ctx->stream>>>(i0, i1, u0, order, rank.p, ug.p, gptr, px,
@@ -580,6 +327,92 @@ int hge_jaccard_centroid_grouped(hge_ctx* ctx, hge_incidence* inc, int group_sid
     u0 = u1;
   }
   return HGE_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int hge_jaccard_rows(hge_ctx* ctx, const int64_t* ptr, const int32_t* idx, const float* val,
+                     int64_t rows, int64_t nnz, const int32_t* pi, const int32_t* pj,
+                     int64_t num_pairs, float* out, int mem) {
+  HGE_REQUIRE(ctx && ptr && (idx || nnz == 0) && (val || nnz == 0) && rows >= 0 && nnz >= 0,
+              "hge_jaccard_rows: bad feature matrix");
+  HGE_REQUIRE(num_pairs >= 0 && (num_pairs == 0 || (pi && pj && out)), "hge_jaccard_rows: bad pairs");
+  HGE_REQUIRE(mem == HGE_MEM_HOST || mem == HGE_MEM_DEVICE, "hge_jaccard_rows: bad mem %d", mem);
+  HGE_CUDA(cudaSetDevice(ctx->device));
+  if (num_pairs == 0) return HGE_OK;
+  bool ok = false;
+  HGE_TRY(pairs_in_range(ctx, num_pairs, pi, rows, pj, rows, mem, &ok));
+  HGE_REQUIRE(ok, "hge_jaccard_rows: a pair names a row outside [0, %lld)", (long long)rows);
+  FeatureMatrix f(ctx);
+  Staged<int32_t> s_i(ctx), s_j(ctx);
+  Staged<float> s_out(ctx);
+  HGE_TRY(f.init(ptr, idx, val, rows, nnz, mem));
+  HGE_TRY(s_i.init(pi, (size_t)num_pairs, mem, true, false));
+  HGE_TRY(s_j.init(pj, (size_t)num_pairs, mem, true, false));
+  HGE_TRY(s_out.init(out, (size_t)num_pairs, mem, false, true));
+  k_jaccard_merge<<<grid_for(ctx, num_pairs), kBlock, 0, ctx->stream>>>(num_pairs, f.ptr.dev, f.idx.dev, f.val.dev,
+                                                                       s_i.dev, s_j.dev, s_out.dev);
+  HGE_CHECK_LAUNCH(ctx);
+  return s_out.finish();
+}
+
+int hge_jaccard_centroid(hge_ctx* ctx, const int64_t* xptr, const int32_t* xidx, const float* xval,
+                         int64_t xrows, int64_t xnnz, const int64_t* gptr, const int32_t* gidx,
+                         int64_t grows, int64_t gnnz, const int64_t* fptr, const int32_t* fidx,
+                         const float* fval, int64_t frows, int64_t fnnz, const int32_t* px,
+                         const int32_t* pg, int64_t num_pairs, float* out, int mem) {
+  HGE_REQUIRE(ctx && xptr && gptr && fptr && xrows >= 0 && grows >= 0 && frows >= 0 && xnnz >= 0 &&
+                  gnnz >= 0 && fnnz >= 0, "hge_jaccard_centroid: bad matrix");
+  HGE_REQUIRE(num_pairs >= 0 && num_pairs < (1ll << 31) && (num_pairs == 0 || (px && pg && out)),
+              "hge_jaccard_centroid: bad pairs");
+  HGE_REQUIRE(mem == HGE_MEM_HOST || mem == HGE_MEM_DEVICE, "hge_jaccard_centroid: bad mem %d", mem);
+  HGE_CUDA(cudaSetDevice(ctx->device));
+  if (num_pairs == 0) return HGE_OK;
+  FeatureMatrix x(ctx), f(ctx);
+  const bool same = xptr == fptr && xidx == fidx && xval == fval;   // usual case: X is F
+  Staged<int64_t> s_gptr(ctx);
+  Staged<int32_t> s_gidx(ctx), s_px(ctx), s_pg(ctx);
+  Staged<float> s_out(ctx);
+  HGE_TRY(f.init(fptr, fidx, fval, frows, fnnz, mem));
+  if (!same) HGE_TRY(x.init(xptr, xidx, xval, xrows, xnnz, mem));
+  HGE_TRY(s_gptr.init(gptr, (size_t)grows + 1, mem, true, false));
+  HGE_TRY(s_gidx.init(gidx, (size_t)gnnz, mem, true, false));
+  HGE_TRY(s_px.init(px, (size_t)num_pairs, mem, true, false));
+  HGE_TRY(s_pg.init(pg, (size_t)num_pairs, mem, true, false));
+  HGE_TRY(s_out.init(out, (size_t)num_pairs, mem, false, true));
+  const FeatureMatrix& xr = same ? f : x;
+  // an int32 pg names no group at or past 2^31, so the clamp keeps the core's range check exact
+  HGE_TRY(centroid_factor(ctx, "hge_jaccard_centroid", s_gptr.dev, s_gidx.dev, std::min<int64_t>(grows, 1ll << 31),
+                          xr.ptr.dev, xr.idx.dev, xr.val.dev, xrows, f.ptr.dev, f.idx.dev, f.val.dev, s_px.dev,
+                          s_pg.dev, num_pairs, kDefaultWorkspaceMb, s_out.dev));
+  return s_out.finish();
+}
+
+int hge_jaccard_centroid_grouped(hge_ctx* ctx, hge_incidence* inc, int group_side, const int64_t* xptr,
+                                 const int32_t* xidx, const float* xval, int64_t xrows, int64_t xnnz,
+                                 const int64_t* fptr, const int32_t* fidx, const float* fval, int64_t frows,
+                                 int64_t fnnz, const int32_t* px, const int32_t* pg, int64_t num_pairs,
+                                 int64_t workspace_mb, float* out) {
+  HGE_REQUIRE(ctx && inc, "hge_jaccard_centroid_grouped: NULL argument");
+  HGE_REQUIRE(!inc->sharded, "hge_jaccard_centroid_grouped: needs a whole (not sharded) incidence");
+  HGE_REQUIRE(group_side == 0 || group_side == 1, "hge_jaccard_centroid_grouped: group_side must be 0 or 1");
+  HGE_REQUIRE(xptr && fptr && xrows >= 0 && frows >= 0 && xnnz >= 0 && fnnz >= 0 && (xidx || xnnz == 0) &&
+                  (xval || xnnz == 0) && (fidx || fnnz == 0) && (fval || fnnz == 0),
+              "hge_jaccard_centroid_grouped: bad matrix");
+  // groups are edges with node members (F = node features), or nodes with edge members
+  const int64_t groups = group_side == 1 ? inc->E : inc->N, members = group_side == 1 ? inc->N : inc->E;
+  HGE_REQUIRE(frows == members, "hge_jaccard_centroid_grouped: F has %lld rows, the members number %lld",
+              (long long)frows, (long long)members);
+  HGE_REQUIRE(num_pairs >= 0 && num_pairs < (1ll << 31) && (num_pairs == 0 || (px && pg && out)),
+              "hge_jaccard_centroid_grouped: bad pairs");
+  HGE_REQUIRE(workspace_mb >= 0, "hge_jaccard_centroid_grouped: negative workspace");
+  HGE_CUDA(cudaSetDevice(ctx->device));
+  if (num_pairs == 0) return HGE_OK;
+  return centroid_factor(ctx, "hge_jaccard_centroid_grouped", group_side == 1 ? inc->e2n_ptr : inc->n2e_ptr,
+                         group_side == 1 ? inc->e2n_idx : inc->n2e_idx, groups, xptr, xidx, xval, xrows, fptr, fidx,
+                         fval, px, pg, num_pairs, workspace_mb ? workspace_mb : kDefaultWorkspaceMb, out);
 }
 
 }  // extern "C"

@@ -12,6 +12,7 @@
 #include <new>
 
 #include "hge_incidence.cuh"
+#include "hge_pairs.cuh"
 
 namespace {
 
@@ -346,40 +347,9 @@ __global__ void __launch_bounds__(kBlock) k_diff_type_prob(
   }
 }
 
-// ---- pair index range checks ------------------------------------------------------------------
 // The kernels above trust their pair indices: k_same_type_prob and k_diff_type_prob read row
 // pointers at them, k_pair_l2 skips a negative one and leaves its output unwritten.  The entry
-// points therefore check every index before any of those kernels runs.
-__global__ void k_check_pairs(int64_t n, const int32_t* __restrict__ a, int64_t rows_a,
-                              const int32_t* __restrict__ b, int64_t rows_b, int* __restrict__ bad) {
-  for (int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; p < n;
-       p += (int64_t)gridDim.x * blockDim.x) {
-    const int32_t x = __ldcs(a + p), y = __ldcs(b + p);
-    if (x < 0 || x >= rows_a || y < 0 || y >= rows_b) *bad = 1;
-  }
-}
-
-// *ok = every a[p] in [0, rows_a) and every b[p] in [0, rows_b).  Host arrays are scanned on the
-// host; device arrays by k_check_pairs, then one flag read-back.
-int pairs_in_range(hge_ctx* ctx, int64_t n, const int32_t* a, int64_t rows_a, const int32_t* b,
-                   int64_t rows_b, int mem, bool* ok) {
-  if (mem != HGE_MEM_DEVICE) {
-    bool all = true;
-    for (int64_t p = 0; p < n; ++p)
-      all &= a[p] >= 0 && a[p] < rows_a && b[p] >= 0 && b[p] < rows_b;
-    *ok = all;
-    return HGE_OK;
-  }
-  DevBuf<int> d_bad(ctx);
-  HGE_TRY(d_bad.alloc(1));
-  HGE_CUDA(cudaMemsetAsync(d_bad.p, 0, sizeof(int), ctx->stream));
-  k_check_pairs<<<grid_for(ctx, n, kBlock * 8), kBlock, 0, ctx->stream>>>(n, a, rows_a, b, rows_b, d_bad.p);
-  HGE_CHECK_LAUNCH(ctx);
-  int h_bad = 0;
-  HGE_TRY(read_back(ctx, d_bad.p, &h_bad, 1));
-  *ok = h_bad == 0;
-  return HGE_OK;
-}
+// points therefore check every index with pairs_in_range (hge_pairs.cuh) first.
 
 // rows -> segments of at most kSegment incidences, on the device: per row ceil(deg / kSegment)
 // segments, an exclusive prefix sum for their positions (cub; set-up), one thread per row writes

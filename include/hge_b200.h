@@ -259,7 +259,8 @@ int hge_diff_type_prob(hge_ctx* ctx, hge_incidence* inc, const float* w_e2n, con
  * (ascending column, one value at a time), so the result equals the reference's bit for bit on
  * fp32 features. */
 
-/* out[p] = J(F[pi[p]], F[pj[p]]): SameTypeJaccardSample (:323-340). */
+/* out[p] = J(F[pi[p]], F[pj[p]]): SameTypeJaccardSample (:323-340).  An index outside [0, rows) is
+ * HGE_ERR_INVALID; nothing is computed then. */
 int hge_jaccard_rows(hge_ctx* ctx, const int64_t* ptr, const int32_t* idx, const float* val,
                      int64_t rows, int64_t nnz, const int32_t* pi, const int32_t* pj,
                      int64_t num_pairs, float* out, int mem);
@@ -268,7 +269,12 @@ int hge_jaccard_rows(hge_ctx* ctx, const int64_t* ptr, const int32_t* idx, const
  * (:343-392).  The centroid rows of the groups the pairs name are materialised on the device the
  * way CentroidFromRows (:284-299) computes them (members added in ascending order in fp32, one
  * division by the group size).  G is a boolean CSR (group -> member rows of F); X and F have the
- * same number of columns (X may be F itself).  An empty group gives 0. */
+ * same number of columns (X may be F itself).  An empty group gives 0.  The pairs are stably sorted
+ * by group and the centroid rows built in batches of consecutive named groups whose expansion fits
+ * 2048 MB (48 bytes per expanded entry), each batch freed after the merge of its pairs; besides that
+ * budget the call holds at most 52 bytes per pair and, for HGE_MEM_HOST, the device copies of its
+ * inputs.  A pair index outside [0, xrows) or outside [0, grows) is HGE_ERR_INVALID, and so is
+ * num_pairs >= 2^31 (refused before any array is read); nothing is computed then. */
 int hge_jaccard_centroid(hge_ctx* ctx, const int64_t* xptr, const int32_t* xidx, const float* xval,
                          int64_t xrows, int64_t xnnz, const int64_t* gptr, const int32_t* gidx,
                          int64_t grows, int64_t gnnz, const int64_t* fptr, const int32_t* fidx,
@@ -283,8 +289,10 @@ int hge_jaccard_centroid(hge_ctx* ctx, const int64_t* xptr, const int32_t* xidx,
  * consecutive named groups whose expansion fits workspace_mb megabytes (0 = 2048, 48 bytes per
  * expanded entry), each batch freed after the merge of its pairs.  A single group larger than the
  * budget is its own batch; one the device cannot hold is HGE_ERR_NOMEM.  Besides the budget the
- * call holds at most 52 bytes per pair.  Bit-equal to hge_jaccard_centroid on the same inputs for
- * every workspace_mb.  A pair index outside X or outside the groups is HGE_ERR_INVALID. */
+ * call holds at most 52 bytes per pair.  Both centroid entry points run the same code, so the
+ * result equals hge_jaccard_centroid's bit for bit on the same inputs, for every workspace_mb.  A
+ * pair index outside X or outside the groups is HGE_ERR_INVALID, and so is num_pairs >= 2^31;
+ * nothing is computed then. */
 int hge_jaccard_centroid_grouped(hge_ctx* ctx, hge_incidence* inc, int group_side, const int64_t* xptr,
                                  const int32_t* xidx, const float* xval, int64_t xrows, int64_t xnnz,
                                  const int64_t* fptr, const int32_t* fidx, const float* fval, int64_t frows,

@@ -1,5 +1,7 @@
-"""WeightedJaccardSamplesDevice and hge_jaccard_centroid_grouped: the grouped centroid kernel equal to
-hge_jaccard_centroid bit for bit whatever the budget; the sampler's index and neighbour columns equal
+"""WeightedJaccardSamplesDevice and the centroid factors: hge_jaccard_centroid (host arrays) and
+hge_jaccard_centroid_grouped (device arrays, every budget) equal to each other and to the fp32
+restatement of SparseWeightedJaccard / CentroidFromRows bit for bit on every pair; the range checks of
+hge_jaccard_centroid and hge_jaccard_rows; the sampler's index and neighbour columns equal
 to their numpy restatement (oracle/jaccard_device_ref.py), its probabilities and left / right weights
 equal to the fp32 restatement of SparseWeightedJaccard / CentroidFromRows bit for bit (and to the
 float64 one to the bars of tests/test_jaccard_samples_gpu.py); its result forms, the packing of its
@@ -45,9 +47,18 @@ def _dev(a):
       torch.device("cuda", _native.default_context().device))
 
 
-def _grouped_equals_the_reference(A, X, F, side, px, pg, budgets):
-  """hge_jaccard_centroid_grouped on the incidence A (groups: its edges for side 1, its nodes for
-  side 0) against hge_jaccard_centroid with the same group CSR given explicitly."""
+def _scipy(feat):
+  """The scipy CSR of a host FeatureCsr / CsrArrays: the rows exactly as the kernels read them."""
+  data = feat.val if hasattr(feat, "val") else np.ones(len(feat.idx), np.float32)
+  return sps.csr_matrix((data, feat.idx, feat.ptr), shape=feat.shape)
+
+
+def _centroid_factors_equal_the_restatement(A, X, F, side, px, pg, budgets):
+  """Both centroid entry points on the incidence A (groups: its edges for side 1, its nodes for
+  side 0): hge_jaccard_centroid on host arrays with the group CSR given explicitly, and
+  hge_jaccard_centroid_grouped on device arrays with the groups taken from the incidence, at every
+  budget.  The outputs are bit-equal to each other and, on every pair, to the fp32 restatement of
+  the reference (0 for a group without members)."""
   from hypergraphembedding_b200 import _native
   from hypergraphembedding_b200.hg2v_sample import _Graph
   ctx = _native.default_context()
@@ -65,20 +76,30 @@ def _grouped_equals_the_reference(A, X, F, side, px, pg, budgets):
       assert got.dtype == np.float32 and np.array_equal(got, want), (side, mb)
   finally:
     inc.close()
+  Xs, Fs, G = _scipy(x), _scipy(f), _scipy(groups)
+  centroids, expect = {}, {}
+  for i, key in enumerate(zip(np.asarray(px).tolist(), np.asarray(pg).tolist())):
+    if key not in expect:
+      a, grp = key
+      if grp not in centroids:
+        centroids[grp] = _centroid(G, grp, Fs) if G.indptr[grp + 1] > G.indptr[grp] else None
+      c = centroids[grp]
+      expect[key] = np.float32(0) if c is None else _reference_loop(*_row(Xs, a), *c)
+    assert want[i] == expect[key], (side, i)
   return want
 
 
 @pytest.mark.parametrize("name", GOLDEN)
-def test_grouped_kernel_equals_the_centroid_kernel_on_the_golden_graphs(name):
+def test_centroid_factors_equal_the_restatement_on_the_golden_graphs(name):
   A, NF, EF, _ = _golden_graph(name)
   N, E = A.shape
   rng = np.random.default_rng(11)
   nodes, edges = rng.integers(0, N, 3000), rng.integers(0, E, 3000)
-  _grouped_equals_the_reference(A, NF, NF, 1, nodes, edges, (0, 1))
-  _grouped_equals_the_reference(A, EF, EF, 0, edges, nodes, (0, 1))
+  _centroid_factors_equal_the_restatement(A, NF, NF, 1, nodes, edges, (0, 1))
+  _centroid_factors_equal_the_restatement(A, EF, EF, 0, edges, nodes, (0, 1))
 
 
-def test_grouped_kernel_on_signed_features_an_empty_group_and_a_group_above_the_budget():
+def test_centroid_factors_on_signed_features_an_empty_group_and_a_group_above_the_budget():
   g, F, G = _signed_golden()
   G = sps.vstack([G, sps.csr_matrix((1, G.shape[1]), dtype=G.dtype)]).tocsr()     # the last group is empty
   G.sort_indices()
@@ -88,14 +109,9 @@ def test_grouped_kernel_on_signed_features_an_empty_group_and_a_group_above_the_
   pg = np.concatenate([rng.integers(0, G.shape[0], 1999), [G.shape[0] - 1]])
   # groups on the edge side (the incidence's edge -> node CSR is G), then on the node side (its node
   # -> edge CSR is G)
-  want = _grouped_equals_the_reference(sps.csr_matrix(G.T), F, F, 1, px, pg, (0, 1))
+  want = _centroid_factors_equal_the_restatement(sps.csr_matrix(G.T), F, F, 1, px, pg, (0, 1))
   assert want[-1] == 0
-  assert np.array_equal(_grouped_equals_the_reference(G, F, F, 0, px, pg, (0, 1)), want)
-  # every value against the fp32 restatement of the reference
-  for i in range(0, len(px), 37):
-    members = G.indices[G.indptr[pg[i]]:G.indptr[pg[i] + 1]]
-    if len(members):
-      assert want[i] == _reference_loop(*_row(F, px[i]), *_centroid(G, pg[i], F)), i
+  assert np.array_equal(_centroid_factors_equal_the_restatement(G, F, F, 0, px, pg, (0, 1)), want)
   # one group expands to 2400 x 40 entries: about 4.6 MB of workspace, more than a 1 MB budget
   # (its own batch) and than 4 MB (a batch of its own next to batches of small groups)
   big = sps.random(3000, 500, density=0.08, random_state=5, format="csr", dtype=np.float32)
@@ -107,7 +123,7 @@ def test_grouped_kernel_on_signed_features_an_empty_group_and_a_group_above_the_
   inc.sort_indices()
   px = rng.integers(0, 3000, 5000)
   pg = np.concatenate([np.full(300, 7), rng.integers(0, 60, 4700)])
-  _grouped_equals_the_reference(inc, big, big, 1, px, pg, (0, 1, 4))
+  _centroid_factors_equal_the_restatement(inc, big, big, 1, px, pg, (0, 1, 4))
 
 
 @pytest.mark.parametrize("name", ["tiny_uniform", "rand25_uniform", "rand25_neighborhood"])
@@ -301,6 +317,62 @@ def test_refusals_leave_the_context_usable():
     assert np.array_equal(got, want)
   finally:
     inc.close()
+
+
+def test_centroid_and_rows_refuse_out_of_range_pairs_on_host_and_device_arrays():
+  """hge_jaccard_centroid and hge_jaccard_rows check every pair index before a kernel reads it: a
+  row or group outside the matrix is HGE_ERR_INVALID on host and on device arrays, as are 2^31
+  centroid pairs (refused before any array is read), and the context gives the restatement's
+  values afterwards."""
+  import torch
+  from hypergraphembedding_b200 import _native
+  A, NF, _ = _zipf()
+  N, E = A.shape
+  ctx = _native.default_context()
+  dev = torch.device("cuda", ctx.device)
+  feat = _native.FeatureCsr(NF)
+  groups = _native.CsrArrays(sps.csr_matrix(A.T))     # edges with their nodes
+  on = {False: (feat, groups.ptr, groups.idx),
+        True: (feat.to_device(dev), torch.from_numpy(groups.ptr).to(dev), torch.from_numpy(groups.idx).to(dev))}
+  P = _native.ptr
+
+  def centroid(px, pg, on_device, n=None):
+    f, gp, gi = on[on_device]
+    px, pg = (_dev(px), _dev(pg)) if on_device else (_native._as_i32(px), _native._as_i32(pg))
+    out = torch.empty(len(px), device=dev) if on_device else np.empty(len(px), np.float32)
+    return ctx.lib.hge_jaccard_centroid(
+        ctx.handle, P(f.ptr), P(f.idx), P(f.val), N, len(f.idx), P(gp), P(gi), E, len(gi), P(f.ptr), P(f.idx),
+        P(f.val), N, len(f.idx), P(px), P(pg), len(px) if n is None else n, P(out),
+        _native.MEM_DEVICE if on_device else _native.MEM_HOST)
+
+  ok = np.arange(10)
+  for on_device in (False, True):
+    for bad in (-1, N):
+      px = ok.copy()
+      px[3] = bad
+      assert centroid(px, ok, on_device) == _native.HGE_ERR_INVALID and "row" in _native.last_error()
+    for bad in (-1, E):
+      pg = ok.copy()
+      pg[7] = bad
+      assert centroid(ok, pg, on_device) == _native.HGE_ERR_INVALID and "group" in _native.last_error()
+  assert centroid(ok, ok, False, n=1 << 31) == _native.HGE_ERR_INVALID
+  for on_device in (False, True):
+    fr = on[on_device][0]
+    arr = _dev if on_device else np.asarray
+    for bad in (-1, N):
+      bad_i = ok.copy()
+      bad_i[5] = bad
+      with pytest.raises(AssertionError, match="outside"):
+        _native.jaccard_rows(ctx, fr, arr(bad_i), arr(ok))
+      with pytest.raises(AssertionError, match="outside"):
+        _native.jaccard_rows(ctx, fr, arr(ok), arr(bad_i))
+  # the context still works
+  Fs = _scipy(feat)
+  pi, pj = np.arange(10), np.arange(10)[::-1]
+  want = np.asarray([_reference_loop(*_row(Fs, a), *_row(Fs, b)) for a, b in zip(pi, pj)], np.float32)
+  assert np.array_equal(_native.jaccard_rows(ctx, feat, pi, pj), want)
+  assert np.array_equal(_native.jaccard_rows(ctx, on[True][0], _dev(pi), _dev(pj)).cpu().numpy(), want)
+  _centroid_factors_equal_the_restatement(A, NF, NF, 1, ok, ok, (0,))
 
 
 def test_sampler_at_100k_nodes_with_a_small_budget():

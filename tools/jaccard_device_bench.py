@@ -7,11 +7,7 @@ samples, dimension 32, 2 epochs at batch 256, uniform and neighbourhood (alpha 0
       probabilities split, packing into the model's buffer, 2 training epochs (fit_device); peak
       device memory in torch's allocator and in the device's default stream-ordered pool;
   (b) at 100 000 nodes only, the existing EmbedHg2vAdjJaccard / EmbedHg2vNeighborhoodWeightedJaccard
-      on the same graph built as a proto (proto construction timed separately);
-  (c) at both sizes, on the same device pairs (the node-edge block of the sampler, node rows and edge
-      rows), both centroid factors by hge_jaccard_centroid_grouped against hge_jaccard_centroid
-      called once per block on device pointers: time, peak pool memory, bit equality, or the
-      HGE_ERR_NOMEM the library returns.
+      on the same graph built as a proto (proto construction timed separately).
 
 Every timed step ends in a device synchronise.  The GPU's name and power limit are read in the
 same run.
@@ -128,64 +124,6 @@ def existing_path(hg, kind, pool):
   return {"features": kind, "total_s": dt, "method_name": emb.method_name, "peak_device": peaks(pool)}
 
 
-def kernels(A, kind, pool):
-  """Both centroid factors of the sampler's node-edge pairs: grouped kernel vs one
-  hge_jaccard_centroid call per block."""
-  import torch
-  from hypergraphembedding_b200 import _native
-  from hypergraphembedding_b200.hg2v_sample import _DeviceSampler, _Graph, _per_row
-  ctx = _native.default_context()
-  dev = torch.device("cuda", ctx.device)
-  NF, EF = features(A, kind)
-  g = _Graph.from_csr(A)
-  nf, ef = _native.FeatureCsr(NF).to_device(dev), _native.FeatureCsr(EF).to_device(dev)
-  inc = g.incidence(ctx)
-  out = {"features": kind, "blocks": []}
-  try:
-    s = _DeviceSampler(g, ctx, inc, K, SEED, 0)
-    phases = (_native.PHASE_NE, _native.PHASE_EN, _native.PHASE_NEIGHBORS)
-    blocks = [(n.clone(), e.clone()) for n, e, _, _ in
-              s.node_edge(_per_row(None, g.num_nodes, SAMPLES), _per_row(None, g.num_edges, SAMPLES), 3, phases)]
-    b_ptr = torch.from_numpy(g.b.ptr).to(dev)
-    b_idx = torch.from_numpy(g.b.idx).to(dev)
-    a_ptr = torch.from_numpy(g.a.ptr).to(dev)
-    a_idx = torch.from_numpy(g.a.idx).to(dev)
-    P = _native.ptr
-
-    def per_block(x, gp, gi, groups, px, pg):
-      res = torch.empty(int(px.shape[0]), dtype=torch.float32, device=dev)
-      _native.check(ctx.lib.hge_jaccard_centroid(
-          ctx.handle, P(x.ptr), P(x.idx), P(x.val), x.shape[0], int(x.idx.shape[0]), P(gp), P(gi), groups,
-          int(gi.shape[0]), P(x.ptr), P(x.idx), P(x.val), x.shape[0], int(x.idx.shape[0]), P(px), P(pg),
-          int(px.shape[0]), P(res), _native.MEM_DEVICE), "hge_jaccard_centroid")
-      return res
-
-    for nodes, edges in blocks:
-      rec = {"pairs": int(nodes.shape[0])}
-      for name, fn in (
-          ("grouped", lambda: (_native.jaccard_centroid_grouped(ctx, inc, 1, nf, nf, nodes, edges),
-                               _native.jaccard_centroid_grouped(ctx, inc, 0, ef, ef, edges, nodes))),
-          ("per_block", lambda: (per_block(nf, b_ptr, b_idx, g.num_edges, nodes, edges),
-                                 per_block(ef, a_ptr, a_idx, g.num_nodes, edges, nodes)))):
-        reset_peaks(pool)
-        try:
-          dt, res = sync_time(fn)
-          rec[name] = {"s": dt, "pool_peak_gb": peaks(pool)["pool_used_gb"]}
-          rec[name + "_result"] = res
-        except MemoryError as exc:
-          rec[name] = {"nomem": str(exc)}
-      if "grouped_result" in rec and "per_block_result" in rec:
-        rec["bit_equal"] = all(bool(torch.equal(a, b)) for a, b in zip(rec["grouped_result"],
-                                                                       rec["per_block_result"]))
-      rec.pop("grouped_result", None)
-      rec.pop("per_block_result", None)
-      out["blocks"].append(rec)
-      print(json.dumps(rec), flush=True)
-  finally:
-    inc.close()
-  return out
-
-
 def main():
   ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
   ap.add_argument("--out", required=True, help="directory for jaccard_device_bench.json")
@@ -201,17 +139,13 @@ def main():
   # warm-up: modules, memory pools, cub tuning of every kernel the paths launch
   small = synthetic.zipf_hypergraph(20000, 10000, seed=1)
   new_path(small, "uniform", pool)
-  kernels(small, "uniform", pool)
   existing_path(proto_from_csr(small), "uniform", pool)
   for n in (int(x) for x in args.sizes.split(",")):
     A = synthetic.zipf_hypergraph(n, n // 2, seed=2024)
-    run = {"graph": "zipf_hypergraph(%d, %d, seed=2024)" % (n, n // 2), "nnz": int(A.nnz), "new": [],
-           "kernels": []}
+    run = {"graph": "zipf_hypergraph(%d, %d, seed=2024)" % (n, n // 2), "nnz": int(A.nnz), "new": []}
     for kind in ("uniform", "neighborhood"):
       run["new"].append(new_path(A, kind, pool))
       print(json.dumps(run["new"][-1]), flush=True)
-    for kind in ("uniform", "neighborhood"):
-      run["kernels"].append(kernels(A, kind, pool))
     if n <= 100000:
       t = time.perf_counter()
       hg = proto_from_csr(A)

@@ -138,7 +138,14 @@ SIGNATURES = {
                                           ctypes.c_uint64, ctypes.c_double, ctypes.c_double, ctypes.c_double,
                                           ctypes.c_int64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
                                           ctypes.c_int64, c_vp]),
-    "hge_mt19937_random_raw": (ctypes.c_int, [c_vp, ctypes.c_int64, c_vp]),
+    "hge_lp_node_edge_train": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp, ctypes.c_int, ctypes.c_int, ctypes.c_uint64,
+                                              ctypes.c_int, ctypes.c_int, ctypes.c_float, ctypes.c_float, c_vp, c_vp,
+                                              c_vp, c_vp, c_vp, c_vp]),
+    "hge_lp_node_edge_samples": (ctypes.c_int, [c_vp, c_vp, ctypes.c_uint64, ctypes.c_int, c_vp, c_vp, c_vp]),
+    "hge_lp_node_edge_predict": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int64, c_vp, ctypes.c_int64, ctypes.c_int,
+                                                ctypes.c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, ctypes.c_int64, c_vp,
+                                                c_vp]),
+    "hge_mt19937_random_raw":(ctypes.c_int, [c_vp, ctypes.c_int64, c_vp]),
     "hge_mt19937_interval": (ctypes.c_int, [c_vp, ctypes.c_uint32, ctypes.c_int64, c_vp]),
     "hge_spgemm_rows": (ctypes.c_int, [ctypes.c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
                                        ctypes.c_int32, ctypes.c_int32, c_vp, ctypes.c_int64,
@@ -868,6 +875,65 @@ def lp_svm_predict(ctx, inc, owner_side, vectors, items, owners, seed, C=1.0, ga
     out += (LpSvmModel(host[0][:U], host[1][:U], host[2][:U], host[3][:U + 1], host[4][:T], host[5][:T],
                        capped),)
   return out
+
+
+def lp_node_edge_train(ctx, inc, xn, xe, seed, hidden=64, epochs=10, batch_size=256, lr=0.01, eps=1e-7,
+                       timings=None):
+  """hge_lp_node_edge_train on fp32 CUDA tensors xn [N, d], xe [E, d]: ((W1 [2d, hidden], b1 [hidden],
+  w2 [hidden], b2 [1]) as CUDA tensors, per-epoch losses as a numpy array).  `timings` (a dict)
+  receives the seconds of the set-up and of each epoch, each ended by a synchronise."""
+  import torch
+  assert xn.dim() == 2 and xe.dim() == 2 and xn.dtype == torch.float32 and xe.dtype == torch.float32
+  assert xn.shape[1] == xe.shape[1], "node and edge vectors must have the same length"
+  d, dev = int(xn.shape[1]), xn.device
+  W1 = torch.empty((max(2 * d, 1), max(int(hidden), 1)), dtype=torch.float32, device=dev)
+  b1 = torch.empty(max(int(hidden), 1), dtype=torch.float32, device=dev)
+  w2 = torch.empty(max(int(hidden), 1), dtype=torch.float32, device=dev)
+  b2 = torch.empty(1, dtype=torch.float32, device=dev)
+  losses = np.zeros(max(int(epochs), 1), dtype=np.float64)
+  phase = np.zeros(1 + max(int(epochs), 0), dtype=np.float64) if timings is not None else None
+  xn, xe = xn.contiguous(), xe.contiguous()
+  check(ctx.lib.hge_lp_node_edge_train(ctx.handle, inc.handle, ptr(xn), ptr(xe), d, int(hidden),
+                                       int(seed) & 0xFFFFFFFFFFFFFFFF, int(epochs), int(batch_size), float(lr),
+                                       float(eps), ptr(W1), ptr(b1), ptr(w2), ptr(b2), ptr(losses), ptr(phase)),
+        "hge_lp_node_edge_train")
+  if timings is not None:
+    timings["setup"] = float(phase[0]) / 1e3
+    timings["epochs"] = (phase[1:] / 1e3).tolist()
+  return (W1, b1, w2, b2), losses[:max(int(epochs), 0)]
+
+
+def lp_node_edge_samples(ctx, inc, seed, epochs):
+  """hge_lp_node_edge_samples: (sample nodes [2 nnz], sample edges [2 nnz], orders [epochs, 2 nnz]) as
+  int32 CUDA tensors."""
+  import torch
+  dev = torch.device("cuda", ctx.device)
+  M = 2 * inc.nnz
+  sn = torch.empty(max(M, 1), dtype=torch.int32, device=dev)
+  se = torch.empty(max(M, 1), dtype=torch.int32, device=dev)
+  orders = torch.empty((max(int(epochs), 1), max(M, 1)), dtype=torch.int32, device=dev)
+  check(ctx.lib.hge_lp_node_edge_samples(ctx.handle, inc.handle, int(seed) & 0xFFFFFFFFFFFFFFFF, int(epochs),
+                                         ptr(sn), ptr(se), ptr(orders)), "hge_lp_node_edge_samples")
+  return sn[:M], se[:M], orders[:int(epochs), :M]
+
+
+def lp_node_edge_predict(ctx, xn, xe, weights, nodes, edges):
+  """hge_lp_node_edge_predict on CUDA tensors: xn [N, d], xe [E, d] fp32, weights (W1, b1, w2, b2),
+  nodes / edges int32 [L].  Returns (probability fp32 [L], keep bool [L]) as CUDA tensors."""
+  import torch
+  W1, b1, w2, b2 = (w.contiguous() for w in weights)
+  assert xn.dim() == 2 and xe.dim() == 2 and xn.shape[1] == xe.shape[1]
+  assert xn.dtype == torch.float32 and xe.dtype == torch.float32
+  assert nodes.dtype == torch.int32 and edges.dtype == torch.int32 and nodes.shape == edges.shape
+  d, L, dev = int(xn.shape[1]), int(nodes.shape[0]), xn.device
+  prob = torch.empty(max(L, 1), dtype=torch.float32, device=dev)[:L]
+  keep = torch.empty(max(L, 1), dtype=torch.uint8, device=dev)[:L]
+  xn, xe = xn.contiguous(), xe.contiguous()
+  check(ctx.lib.hge_lp_node_edge_predict(ctx.handle, ptr(xn), int(xn.shape[0]), ptr(xe), int(xe.shape[0]), d,
+                                         int(W1.shape[1]), ptr(W1), ptr(b1), ptr(w2), ptr(b2),
+                                         ptr(nodes.contiguous()), ptr(edges.contiguous()), L, ptr(prob), ptr(keep)),
+        "hge_lp_node_edge_predict")
+  return prob, keep.bool()
 
 
 class PeerArena(object):

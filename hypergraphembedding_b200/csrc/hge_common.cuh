@@ -80,6 +80,11 @@ int hge_ctx_stage(hge_ctx* ctx, size_t floats, float** out);
 // stays untouched until 255 later requests on the same context.  nullptr on failure.
 void* hge_ctx_pinned_slot(hge_ctx* ctx);
 
+// hge_shuffle_order (csrc/hge_hg2v_train.cu) with the keys read from the streams of `phase`: the
+// epoch orders of every trainer that shuffles its samples.
+int hge_shuffle_order_phase(hge_ctx* ctx, uint64_t seed, uint32_t phase, uint32_t epoch, int64_t n,
+                            int32_t* order, int mem);
+
 // Device buffers come from the device's stream-ordered memory pool (cudaMallocAsync on the
 // context's stream; hge_ctx_create raises the pool's release threshold so freed blocks are
 // reused instead of being returned to the driver).  Everything is released explicitly by the

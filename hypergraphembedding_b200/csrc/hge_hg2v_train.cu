@@ -440,14 +440,14 @@ __global__ void k_hg2v_append(const AppendArgs a) {
 
 // ---- seeded epoch order and tables ------------------------------------------------------------
 
-// key of item i in epoch e: words 2e, 2e + 1 of its HGE_PHASE_SHUFFLE stream (high, low)
-__global__ void k_shuffle_keys(int64_t n, uint64_t seed, uint32_t epoch, uint64_t* __restrict__ keys,
-                               int32_t* __restrict__ idx) {
+// key of item i in epoch e: words 2e, 2e + 1 of its stream in `phase` (high, low)
+__global__ void k_shuffle_keys(int64_t n, uint64_t seed, uint32_t phase, uint32_t epoch,
+                               uint64_t* __restrict__ keys, int32_t* __restrict__ idx) {
   const int w = (int)(epoch & 1u) * 2;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n;
        i += (int64_t)gridDim.x * blockDim.x) {
     const HgeWords4 r = hge_philox4x32_10(epoch >> 1, (uint32_t)i, (uint32_t)((uint64_t)i >> 32),
-                                          HGE_PHASE_SHUFFLE, (uint32_t)seed, (uint32_t)(seed >> 32));
+                                          phase, (uint32_t)seed, (uint32_t)(seed >> 32));
     keys[i] = ((uint64_t)r.v[w] << 32) | r.v[w + 1];
     idx[i] = (int32_t)i;
   }
@@ -792,7 +792,10 @@ int hge_hg2v_get_samples(hge_hg2v_model* m, int32_t* features, float* targets, i
   return HGE_OK;
 }
 
-int hge_shuffle_order(hge_ctx* ctx, uint64_t seed, uint32_t epoch, int64_t n, int32_t* order, int mem) {
+}  // extern "C"
+
+int hge_shuffle_order_phase(hge_ctx* ctx, uint64_t seed, uint32_t phase, uint32_t epoch, int64_t n,
+                            int32_t* order, int mem) {
   HGE_REQUIRE(ctx, "hge_shuffle_order: NULL context");
   HGE_REQUIRE(n >= 0 && n < ((int64_t)1 << 31), "hge_shuffle_order: n = %lld not in [0, 2^31)", (long long)n);
   HGE_REQUIRE(n == 0 || order, "hge_shuffle_order: NULL order");
@@ -809,7 +812,7 @@ int hge_shuffle_order(hge_ctx* ctx, uint64_t seed, uint32_t epoch, int64_t n, in
   HGE_TRY(v1.alloc((size_t)n));
   cub::DoubleBuffer<uint64_t> keys(k0.p, k1.p);
   cub::DoubleBuffer<int32_t> vals(out.dev, v1.p);
-  k_shuffle_keys<<<grid_for(ctx, n), kExpandBlock, 0, ctx->stream>>>(n, seed, epoch, k0.p, out.dev);
+  k_shuffle_keys<<<grid_for(ctx, n), kExpandBlock, 0, ctx->stream>>>(n, seed, phase, epoch, k0.p, out.dev);
   HGE_CHECK_LAUNCH(ctx);
   // LSD radix sort: stable, so equal keys keep ascending item order
   size_t bytes = 0;
@@ -822,4 +825,7 @@ int hge_shuffle_order(hge_ctx* ctx, uint64_t seed, uint32_t epoch, int64_t n, in
   return out.finish();
 }
 
-}  // extern "C"
+extern "C" int hge_shuffle_order(hge_ctx* ctx, uint64_t seed, uint32_t epoch, int64_t n, int32_t* order,
+                                 int mem) {
+  return hge_shuffle_order_phase(ctx, seed, HGE_PHASE_SHUFFLE, epoch, n, order, mem);
+}

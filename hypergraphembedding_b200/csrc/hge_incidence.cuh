@@ -188,5 +188,15 @@ struct hge_algdist {
   hge_p2p* p2p = nullptr;
 };
 
+// id of position p of the ascending non-member list of the sorted member row mem[0 .. m)
+__device__ __forceinline__ int32_t hge_nonmember(const int32_t* __restrict__ mem, int64_t m, int64_t p) {
+  int64_t lo = 0, hi = m;   // first c with mem[c] - c > p
+  while (lo < hi) {
+    const int64_t c = (lo + hi) >> 1;
+    if (mem[c] - c > p) hi = c; else lo = c + 1;
+  }
+  return (int32_t)(p + lo);
+}
+
 // internal: the sharded edge gather with the partial rows pushed to their owners
 extern "C" int hge_internal_edge_push(hge_algdist* st, int sweep);

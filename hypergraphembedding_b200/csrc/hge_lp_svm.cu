@@ -232,16 +232,6 @@ __global__ void k_owner_sizes(int64_t U, const int32_t* __restrict__ ug, const i
   }
 }
 
-// id of position p of the ascending non-member list of the sorted member row mem[0 .. m)
-__device__ __forceinline__ int32_t nonmember(const int32_t* __restrict__ mem, int64_t m, int64_t p) {
-  int64_t lo = 0, hi = m;   // first c with mem[c] - c > p
-  while (lo < hi) {
-    const int64_t c = (lo + hi) >> 1;
-    if (mem[c] - c > p) hi = c; else lo = c + 1;
-  }
-  return (int32_t)(p + lo);
-}
-
 // training points of every named owner u at pid[poff[u] ..]: its members, then its negatives, both
 // ascending.  One warp per owner; every lane draws the same words of the owner's stream.
 __global__ void __launch_bounds__(kBlock) k_training_sets(
@@ -259,7 +249,7 @@ __global__ void __launch_bounds__(kBlock) k_training_sets(
     for (int64_t t = lane; t < m; t += 32) pid[base + t] = mem[t];
     int32_t* neg = pid + base + m;
     if (k == others) {   // every non-member, nothing drawn
-      for (int64_t p = lane; p < k; p += 32) neg[p] = nonmember(mem, m, p);
+      for (int64_t p = lane; p < k; p += 32) neg[p] = hge_nonmember(mem, m, p);
       continue;
     }
     int32_t* pos = scratch + base + m;
@@ -277,7 +267,7 @@ __global__ void __launch_bounds__(kBlock) k_training_sets(
       const int32_t v = pos[q];
       int64_t r = 0;
       for (int64_t x = 0; x < k; ++x) r += pos[x] < v;
-      neg[r] = nonmember(mem, m, v);
+      neg[r] = hge_nonmember(mem, m, v);
     }
     __syncwarp();
   }

@@ -2,7 +2,8 @@
 // word-stream layout of the device sampler (csrc/hge_device_sampler.cu).  oracle/
 // device_sampler_ref.py restates everything in this file in numpy; oracle/seeded_training_ref.py
 // restates the training phases (epoch order, initial tables), oracle/lp_svm_ref.py the negatives of
-// the link-prediction classifiers.
+// the link-prediction classifiers, oracle/lp_node_edge_ref.py the training set, epoch orders and
+// initial weights of the node-edge classifier.
 //
 // Layout.  Every item owns one stream of 32-bit words:
 //   key     = { (uint32)seed, (uint32)(seed >> 32) }
@@ -45,6 +46,13 @@ enum HgePhase : uint32_t {
   // row, Floyd's selection over the owner's non-members
   HGE_PHASE_LP_EDGE_OWNERS = 15,
   HGE_PHASE_LP_NODE_OWNERS = 16,
+  // node-edge link-prediction classifier (csrc/hge_lp_node_edge.cu): negative i of the training
+  // set (item = i, 64-bit masked rejection over the non-incidences), the epoch orders (item =
+  // sample index, as HGE_PHASE_SHUFFLE), the initial weights (item = row of W1, item 2d = w2;
+  // word j is column j)
+  HGE_PHASE_LP_NODE_EDGE_NEG = 17,
+  HGE_PHASE_LP_NODE_EDGE_SHUFFLE = 18,
+  HGE_PHASE_LP_NODE_EDGE_INIT = 19,
 };
 
 #ifdef __CUDACC__

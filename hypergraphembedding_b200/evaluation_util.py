@@ -18,7 +18,9 @@ caller fills with ``RegisterExperiment`` -- ``RunLinkPredictionExperiment`` look
 in it exactly as the reference does.  The per-edge / per-node SVC predictors are provided on top
 of scikit-learn (imported on first use) because they need nothing else; the Keras one raises.
 Their GPU forms (``Personalized*ClassifierPredictionDevice``, csrc/hge_lp_svm.cu) train the same
-classifiers with seeded negatives and are not registered.
+classifiers with seeded negatives and are not registered.  ``NodeEdgeEmbeddingPredictionDevice``
+(csrc/hge_lp_node_edge.cu) trains a seeded GPU classifier for the node-edge experiment, a documented
+model of the Keras kind rather than the reference's; it is not registered either.
 """
 import logging
 import random
@@ -242,11 +244,8 @@ def PersonalizedClassifierPredictionDevice(incidence, item_vectors, links, per_e
   return (keep, out[3]) if return_model else keep
 
 
-def _personalized_classifier_prediction_device(hypergraph, embedding, links, per_edge, seed, **kw):
-  """The host form's semantics on PersonalizedClassifierPredictionDevice: the asked links are those
-  whose node and edge both have vectors, item rows are the embedding's sorted ids, an owner absent
-  from the hypergraph has no members, a member without a vector is a KeyError; the kept links come
-  back in the asked order."""
+def _embedding_tables(embedding):
+  """((sorted node ids, fp32 rows in that order), (sorted edge ids, rows)) of an embedding proto."""
   from .hypergraph_util import embedding_from_wire
   ids_n, ptr_n, val_n, ids_e, ptr_e, val_e, _ = embedding_from_wire(embedding)
   table = []
@@ -255,7 +254,15 @@ def _personalized_classifier_prediction_device(hypergraph, embedding, links, per
     width = int(ptr[1] - ptr[0]) if len(ids) else 0
     assert width > 0 and np.all(np.diff(ptr) == width), "embedding rows must all have the same length"
     table.append((ids[order].astype(np.int64), val.reshape(-1, width)[order]))
-  (node_ids, xn), (edge_ids, xe) = table
+  return table
+
+
+def _personalized_classifier_prediction_device(hypergraph, embedding, links, per_edge, seed, **kw):
+  """The host form's semantics on PersonalizedClassifierPredictionDevice: the asked links are those
+  whose node and edge both have vectors, item rows are the embedding's sorted ids, an owner absent
+  from the hypergraph has no members, a member without a vector is a KeyError; the kept links come
+  back in the asked order."""
+  (node_ids, xn), (edge_ids, xe) = _embedding_tables(embedding)
   pairs = np.asarray(_pairs(links), dtype=np.int64).reshape(-1, 2)
   asked = pairs[np.isin(pairs[:, 0], node_ids) & np.isin(pairs[:, 1], edge_ids)]
   rows = np.stack([np.searchsorted(node_ids, asked[:, 0]), np.searchsorted(edge_ids, asked[:, 1])], axis=1)
@@ -308,6 +315,97 @@ def NodeEdgeEmbeddingPrediction(hypergraph, embedding, potential_links, classifi
     assert n in embedding.node and e in embedding.edge
   x = np.array([np.concatenate((embedding.node[n].values, embedding.edge[e].values)) for n, e in links])
   return [link for link, p in zip(links, classifier.predict(x)) if p > 0.5]
+
+
+def _device_f32(x, dev):
+  import torch
+  if torch.is_tensor(x):
+    return x.to(dev, torch.float32).contiguous()
+  return torch.as_tensor(np.ascontiguousarray(x, dtype=np.float32)).to(dev)
+
+
+class NodeEdgeClassifierDevice(object):
+  """The node-edge link classifier on the GPU (csrc/hge_lp_node_edge.cu): p = sigmoid(w2 . relu(W1^T
+  [xn[n], xe[e]] + b1) + b2), trained on the incidences (label 1) against as many non-incidences drawn
+  uniformly from `seed` (label 0), with Glorot-uniform kernels, zero biases, Adagrad and binary
+  cross-entropy.  This is a documented model of the usual Keras kind, not the reference's Keras
+  model, whose architecture is not recorded; oracle/lp_node_edge_ref.py restates it.  Weights and
+  losses are bit-identical from run to run; Python's ``random`` and numpy's global RNG are neither
+  read nor advanced.  Use ``fit``; the object satisfies the ``classifier=`` protocol of
+  NodeEdgeEmbeddingPrediction (``predict`` of [L, 2d] rows [node vector, edge vector])."""
+
+  def __init__(self, ctx, xn, xe, weights, losses):
+    self._ctx, self._xn, self._xe, self._weights, self.losses = ctx, xn, xe, weights, losses
+
+  @classmethod
+  def fit(cls, incidence, xn, xe, seed=0, hidden=64, epochs=10, batch_size=256, lr=0.01, timings=None):
+    """Trains on an N x E incidence CSR (or an hg2v_sample._Graph) with node vectors `xn` [N, d] and
+    edge vectors `xe` [E, d] (numpy or torch, fp32); 1 <= d, hidden <= 256.  ``losses``: the mean
+    sample loss of each epoch.  `timings` (a dict) receives the set-up and per-epoch seconds."""
+    import torch
+    from .hg2v_sample import _Graph
+    g = incidence if isinstance(incidence, _Graph) else _Graph.from_csr(incidence)
+    ctx = _native.default_context()
+    dev = torch.device("cuda", ctx.device)
+    xn, xe = _device_f32(xn, dev), _device_f32(xe, dev)
+    assert xn.dim() == 2 and xn.shape[0] == g.num_nodes and xe.dim() == 2 and xe.shape[0] == g.num_edges
+    inc = g.incidence(ctx)
+    try:
+      weights, losses = _native.lp_node_edge_train(ctx, inc, xn, xe, seed, hidden, epochs, batch_size, lr,
+                                                   timings=timings)
+    finally:
+      inc.close()
+    return cls(ctx, xn, xe, weights, losses)
+
+  def weights(self):
+    """(W1 [2d, hidden], b1 [hidden], w2 [hidden], b2 [1]) as numpy arrays."""
+    return tuple(w.cpu().numpy() for w in self._weights)
+
+  def _predict(self, xn, xe, nodes, edges):
+    import torch
+    dev = self._xn.device
+    as_i32 = lambda a: torch.as_tensor(np.asarray(a, dtype=np.int64).astype(np.int32)).to(dev)
+    prob, _ = _native.lp_node_edge_predict(self._ctx, xn, xe, self._weights, as_i32(nodes), as_i32(edges))
+    return prob.cpu().numpy()
+
+  def predict_links(self, nodes, edges):
+    """p of the links (nodes[l], edges[l]) over the training vectors (fp32 numpy array)."""
+    return self._predict(self._xn, self._xe, nodes, edges)
+
+  def predict(self, x):
+    """p of each row [node vector, edge vector] of the [L, 2d] matrix `x`, by the same kernel."""
+    x = _device_f32(x, self._xn.device)
+    d = int(self._xn.shape[1])
+    assert x.dim() == 2 and x.shape[1] == 2 * d, "rows must be [node vector, edge vector]"
+    rows = np.arange(int(x.shape[0]))
+    return self._predict(x[:, :d].contiguous(), x[:, d:].contiguous(), rows, rows)
+
+
+def NodeEdgeEmbeddingPredictionDevice(hypergraph, embedding, links, seed=0, **kw):
+  """LP_NODE_EDGE_CLASSIFIER with NodeEdgeClassifierDevice trained from `seed` (not registered in
+  EXPERIMENT_OPTIONS: add it with RegisterExperiment(name, functools.partial(fn, seed=s))).  Rows are
+  the embedding's sorted ids, the positives the hypergraph's connections (one without a vector is a
+  KeyError); the links are filtered as NodeEdgeEmbeddingPrediction filters them and the kept ones come
+  back in the asked order.  `kw`: hidden, epochs, batch_size, lr of NodeEdgeClassifierDevice.fit."""
+  import scipy.sparse as sps
+  (node_ids, xn), (edge_ids, xe) = _embedding_tables(embedding)
+  links = [(n, e) for n, e in _pairs(links) if n in hypergraph.node and e in hypergraph.edge]
+  if not links:
+    return []
+  for n, e in links:
+    assert n in embedding.node and e in embedding.edge
+  node_rows = {int(i): r for r, i in enumerate(node_ids.tolist())}
+  edge_rows = {int(i): r for r, i in enumerate(edge_ids.tolist())}
+  inc = [(node_rows[n], edge_rows[e]) for n, node in hypergraph.node.items() for e in node.edges]
+  inc = np.asarray(inc, dtype=np.int64).reshape(-1, 2)
+  A = sps.csr_matrix((np.ones(len(inc), dtype=np.int8), (inc[:, 0], inc[:, 1])),
+                     shape=(len(node_ids), len(edge_ids)))
+  A.sum_duplicates()
+  A.sort_indices()
+  model = NodeEdgeClassifierDevice.fit(A, xn, xe, seed=seed, **kw)
+  rows = np.asarray([(node_rows[n], edge_rows[e]) for n, e in links], dtype=np.int64)
+  p = model.predict_links(rows[:, 0], rows[:, 1])
+  return [link for link, q in zip(links, p) if q > 0.5]
 
 
 # Each entry is a function taking (hypergraph, embedding, links) -> predicted links

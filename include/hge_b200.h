@@ -473,6 +473,55 @@ int hge_lp_svm_predict(hge_ctx* ctx, hge_incidence* inc, int owner_side, const f
                        int64_t* owner_iters, int64_t* owner_offset, int32_t* point_ids, double* point_coef,
                        int64_t point_capacity, double* phase_ms);
 
+/* Node-edge link-prediction classifier (csrc/hge_lp_node_edge.cu), the GPU form of the classifier
+ * LP_NODE_EDGE_CLASSIFIER passes to NodeEdgeEmbeddingPrediction.  Not a port of the reference's
+ * Keras model (its architecture is not recorded): a model of the usual Keras kind,
+ *   x = [xn[n], xe[e]] (2d), h = relu(W1^T x + b1) (W1 [2d, hidden]), p = sigmoid(w2 . h + b2),
+ * 1 <= d <= 256, 1 <= hidden <= 256.
+ *
+ * hge_lp_node_edge_train: training set, initialisation and `epochs` epochs on the device.
+ *   Samples 0 .. nnz - 1 (label 1) are the incidences of `inc` in CSR order; sample nnz + i
+ *   (label 0) is a non-incidence drawn uniformly, with replacement, from the S = N E - nnz of them:
+ *   r = ((w0 << 32) | w1) & mask from the Philox stream (csrc/hge_philox.cuh) of item i, phase
+ *   HGE_PHASE_LP_NODE_EDGE_NEG (17), redrawn while r >= S (mask = smallest 2^k - 1 >= S - 1); node n
+ *   with C[n] <= r < C[n + 1] (C = exclusive prefix sum of E - deg(n)), edge = the (r - C[n])-th
+ *   edge id not in n's row.  nnz = 0, S = 0 or 2 nnz >= 2^31 is HGE_ERR_INVALID.
+ *   Weights: Keras glorot_uniform kernels, zero biases.  Row i of W1 is item i, w2 item 2d of
+ *   phase HGE_PHASE_LP_NODE_EDGE_INIT (19), word j for column j; value -L + (2L) u with
+ *   u = (w >> 8) 2^-24, each fp32 operation rounded on its own, L1 = fp32(sqrt(6 / (2d + hidden)))
+ *   for W1, L2 = fp32(sqrt(6 / (hidden + 1))) for w2.
+ *   Epoch e visits the samples in hge_shuffle_order's order with the keys of phase
+ *   HGE_PHASE_LP_NODE_EDGE_SHUFFLE (18), in batches of `batch` (the last one ragged); loss per
+ *   sample max(z, 0) - z y + log1p(exp(-|z|)) of the logit z, batch mean; Adagrad
+ *   (acc += g^2, w -= lr g / (sqrt(acc) + eps), accumulators from 0) on every parameter after each
+ *   batch.  epoch_loss[e] (host) = sum of the epoch's sample losses / 2 nnz.  Every sum has one
+ *   fixed order, so weights and losses are bit-identical from run to run.
+ *   W1 [2d, hidden] row-major, b1 [hidden], w2 [hidden], b2 [1]: caller-owned device arrays,
+ *   written with the trained weights (epochs = 0: the initial ones).  xn fp32 [N, d], xe fp32
+ *   [E, d] device.  phase_ms (host, optional) [1 + epochs]: milliseconds of the set-up (training
+ *   set, initialisation), then of each epoch, each phase ended by a stream synchronise.  Besides
+ *   the weights the call holds 8 bytes a sample for the training set, 4 for the epoch order (plus
+ *   the sort's 20), and the accumulators.
+ *
+ * hge_lp_node_edge_samples: what hge_lp_node_edge_train trains on, for inspection: the training
+ *   set (sample_nodes, sample_edges: device int32 [2 nnz]) and the orders of epochs 0 .. epochs - 1
+ *   (orders: device int32 [epochs][2 nnz], may be NULL when epochs = 0).
+ *
+ * hge_lp_node_edge_predict: p of each link (link_nodes[l], link_edges[l]) into out_prob (fp32,
+ *   optional) and out_keep[l] = p > 0.5 (optional); p depends on the model and the link's two rows
+ *   only, never on the other links.  All array pointers are device pointers.  A link naming a node
+ *   outside [0, num_nodes) or an edge outside [0, num_edges) is HGE_ERR_INVALID and nothing is
+ *   written. */
+int hge_lp_node_edge_train(hge_ctx* ctx, hge_incidence* inc, const float* xn, const float* xe, int d, int hidden,
+                           uint64_t seed, int epochs, int batch, float lr, float eps, float* W1, float* b1, float* w2,
+                           float* b2, double* epoch_loss, double* phase_ms);
+int hge_lp_node_edge_samples(hge_ctx* ctx, hge_incidence* inc, uint64_t seed, int epochs, int32_t* sample_nodes,
+                             int32_t* sample_edges, int32_t* orders);
+int hge_lp_node_edge_predict(hge_ctx* ctx, const float* xn, int64_t num_nodes, const float* xe, int64_t num_edges,
+                             int d, int hidden, const float* W1, const float* b1, const float* w2, const float* b2,
+                             const int32_t* link_nodes, const int32_t* link_edges, int64_t num_links, float* out_prob,
+                             uint8_t* out_keep);
+
 /* ---- hypergraph.proto wire format (host code; all pointers are host pointers) --------------
  * The data formats either side of the path: a serialized Hypergraph (hypergraph.proto:6-23) is
  * read straight into arrays, replacing the per-incidence Python loops of ToCsrMatrix /

@@ -145,6 +145,11 @@ SIGNATURES = {
     "hge_lp_node_edge_predict": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int64, c_vp, ctypes.c_int64, ctypes.c_int,
                                                 ctypes.c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, ctypes.c_int64, c_vp,
                                                 c_vp]),
+    "hge_nmf_init": (ctypes.c_int, [c_vp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int, ctypes.c_uint64,
+                                    ctypes.c_float, c_vp, c_vp, ctypes.c_int]),
+    "hge_nmf_fit": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int, c_vp, c_vp,
+                                   ctypes.c_int, ctypes.c_double, ctypes.c_int, ctypes.POINTER(ctypes.c_int), c_vp,
+                                   c_vp]),
     "hge_mt19937_random_raw":(ctypes.c_int, [c_vp, ctypes.c_int64, c_vp]),
     "hge_mt19937_interval": (ctypes.c_int, [c_vp, ctypes.c_uint32, ctypes.c_int64, c_vp]),
     "hge_spgemm_rows": (ctypes.c_int, [ctypes.c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
@@ -934,6 +939,42 @@ def lp_node_edge_predict(ctx, xn, xe, weights, nodes, edges):
                                          ptr(nodes.contiguous()), ptr(edges.contiguous()), L, ptr(prob), ptr(keep)),
         "hge_lp_node_edge_predict")
   return prob, keep.bool()
+
+
+def _factor_pair(W, Ht, k):
+  mem = _mem(W, Ht)
+  if mem == MEM_HOST:
+    assert isinstance(W, np.ndarray) and isinstance(Ht, np.ndarray)
+    assert W.dtype == np.float32 and Ht.dtype == np.float32
+  else:
+    import torch
+    assert W.dtype == torch.float32 and Ht.dtype == torch.float32
+  assert W.ndim == 2 and Ht.ndim == 2 and W.shape[1] == k and Ht.shape[1] == k, "factors must be [N, k], [E, k]"
+  return mem
+
+
+def nmf_init(ctx, num_nodes, num_edges, k, seed, scale, W, Ht):
+  """hge_nmf_init into fp32 W [num_nodes, k] and Ht [num_edges, k] (numpy, or CUDA tensors)."""
+  mem = _factor_pair(W, Ht, k)
+  assert tuple(W.shape) == (num_nodes, k) and tuple(Ht.shape) == (num_edges, k)
+  check(ctx.lib.hge_nmf_init(ctx.handle, int(num_nodes), int(num_edges), int(k), int(seed) & 0xFFFFFFFFFFFFFFFF,
+                             float(scale), ptr(W), ptr(Ht), mem), "hge_nmf_init")
+  return W, Ht
+
+
+def nmf_fit(ctx, inc, W, Ht, max_iter, tol, phase_ms=None):
+  """hge_nmf_fit in place on fp32 W [N, k] and Ht [E, k] (numpy, or CUDA tensors): (n_iter,
+  violations [n_iter] float64).  phase_ms: optional float64 [3] numpy array."""
+  k = int(W.shape[1]) if W.ndim == 2 else 0
+  mem = _factor_pair(W, Ht, k)
+  n_iter = ctypes.c_int(0)
+  viol = np.zeros(max(1, int(max_iter)), dtype=np.float64)
+  if phase_ms is not None:
+    assert phase_ms.dtype == np.float64 and phase_ms.shape == (3,)
+  check(ctx.lib.hge_nmf_fit(ctx.handle, inc.handle, int(W.shape[0]), int(Ht.shape[0]), k, ptr(W), ptr(Ht),
+                            int(max_iter), float(tol), mem, ctypes.byref(n_iter), ptr(viol), ptr(phase_ms)),
+        "hge_nmf_fit")
+  return n_iter.value, viol[:n_iter.value].copy()
 
 
 class PeerArena(object):

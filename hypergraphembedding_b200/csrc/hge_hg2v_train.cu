@@ -40,6 +40,7 @@
 #include "hge_common.cuh"
 #include "hge_expand.cuh"
 #include "hge_philox.cuh"
+#include "hge_seeded_table.cuh"
 
 namespace cg = cooperative_groups;
 
@@ -453,27 +454,6 @@ __global__ void k_shuffle_keys(int64_t n, uint64_t seed, uint32_t phase, uint32_
   }
 }
 
-// element (r, c) = -0.05 + 0.1 * ((word c of the stream of row r) >> 8) * 2^-24, each operation
-// rounded on its own (no contraction), so that the float32 numpy restatement gives the same bits
-__global__ void k_init_table(int64_t rows, int dim, uint64_t seed, uint32_t phase, float* __restrict__ t) {
-  const int blocks = (dim + 3) / 4;
-  for (int64_t g = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; g < rows * blocks;
-       g += (int64_t)gridDim.x * blockDim.x) {
-    const int64_t r = g / blocks;
-    const int b = (int)(g - r * blocks);
-    const HgeWords4 w = hge_philox4x32_10((uint32_t)b, (uint32_t)r, (uint32_t)((uint64_t)r >> 32), phase,
-                                          (uint32_t)seed, (uint32_t)(seed >> 32));
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int c = 4 * b + j;
-      if (c < dim) {
-        const float u = __fmul_rn(__uint2float_rn(w.v[j] >> 8), 0x1p-24f);
-        t[(size_t)r * dim + c] = __fadd_rn(-0.05f, __fmul_rn(0.1f, u));
-      }
-    }
-  }
-}
-
 // hge_hg2v_create and hge_hg2v_create_seeded: tables uploaded from node_init / edge_init, or
 // (seed != NULL) drawn on the device
 int create_model(hge_ctx* ctx, int32_t node_rows, int32_t edge_rows, int dim, int num_neighbors,
@@ -504,9 +484,9 @@ int create_model(hge_ctx* ctx, int32_t node_rows, int32_t edge_rows, int dim, in
     if (rc == HGE_OK) {
       const int blocks = (dim + 3) / 4;
       k_init_table<<<grid_for(ctx, (int64_t)node_rows * blocks), kExpandBlock, 0, ctx->stream>>>(
-          node_rows, dim, *seed, HGE_PHASE_INIT_NODES, m->N);
+          node_rows, dim, *seed, HGE_PHASE_INIT_NODES, -0.05f, 0.1f, m->N);
       k_init_table<<<grid_for(ctx, (int64_t)edge_rows * blocks), kExpandBlock, 0, ctx->stream>>>(
-          edge_rows, dim, *seed, HGE_PHASE_INIT_EDGES, m->E);
+          edge_rows, dim, *seed, HGE_PHASE_INIT_EDGES, -0.05f, 0.1f, m->E);
       ctx->launches += 2;
       const cudaError_t e = cudaGetLastError();
       if (e != cudaSuccess) {

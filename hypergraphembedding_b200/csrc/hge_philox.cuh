@@ -3,7 +3,7 @@
 // device_sampler_ref.py restates everything in this file in numpy; oracle/seeded_training_ref.py
 // restates the training phases (epoch order, initial tables), oracle/lp_svm_ref.py the negatives of
 // the link-prediction classifiers, oracle/lp_node_edge_ref.py the training set, epoch orders and
-// initial weights of the node-edge classifier.
+// initial weights of the node-edge classifier, oracle/nmf_ref.py the factorization's start.
 //
 // Layout.  Every item owns one stream of 32-bit words:
 //   key     = { (uint32)seed, (uint32)(seed >> 32) }
@@ -53,6 +53,10 @@ enum HgePhase : uint32_t {
   HGE_PHASE_LP_NODE_EDGE_NEG = 17,
   HGE_PHASE_LP_NODE_EDGE_SHUFFLE = 18,
   HGE_PHASE_LP_NODE_EDGE_INIT = 19,
+  // seeded start of the non-negative factorization (csrc/hge_nmf.cu): item = row of W (node) or
+  // of H^T (edge), word c is column c
+  HGE_PHASE_NMF_W = 20,
+  HGE_PHASE_NMF_H = 21,
 };
 
 #ifdef __CUDACC__
@@ -115,3 +119,4 @@ struct HgeStreamRng {
     return (uint32_t)(m >> 32);
   }
 };
+

@@ -19,7 +19,10 @@ from .hg2v_sample import (AlgebraicDistanceSamples, AlgebraicDistanceSamplesDevi
                           BooleanSamplesDevice, PlotDistributions, SamplesToModelInput,
                           WeightedJaccardSamples, WeightedJaccardSamplesDevice, _Graph)
 from .hg2v_weighting import UniformWeight, WeightByNeighborhood
-from .hypergraph_util import CompressRange, ToCsrMatrix, ToEdgeCsrMatrix
+from .hypergraph_pb2 import HypergraphEmbedding
+from .hypergraph_util import (CompressRange, ToCsrMatrix, ToEdgeCsrMatrix, compressed_incidence,
+                              embedding_to_wire)
+from .nmf import NonNegativeFactorizationDevice
 
 log = logging.getLogger()
 
@@ -221,6 +224,20 @@ def EmbedHg2vNeighborhoodWeightedJaccardDevice(hypergraph, dimension, alpha=0, n
   embedding = _jaccard_device(hypergraph, dimension, lambda hg: WeightByNeighborhood(hg, alpha),
                               num_neighbors, num_samples, batch_size, epochs, seed, chunk_rows)
   embedding.method_name = "HG2V_NEIGH_JAC"
+  return embedding
+
+
+def EmbedNMFDevice(hypergraph, dimension, max_iter=200, tol=1e-4, seed=0):
+  """The NMF baseline (embedding.py:110-261 of the reference) on the GPU: the compressed incidence
+  A ~ W H by NonNegativeFactorizationDevice with the seeded start of `seed`; node vectors are the
+  rows of W, edge vectors the columns of H, keyed by the original ids, method_name "NMF".  Not the
+  reference's NMF, whose start (init="nndsvda") draws numpy's global RNG: this one neither reads
+  nor advances it, so it is not in EMBEDDING_OPTIONS."""
+  node_ids, edge_ids, A = compressed_incidence(hypergraph)
+  W, H, _ = NonNegativeFactorizationDevice(A, dimension, seed=seed, max_iter=max_iter, tol=tol)
+  embedding = HypergraphEmbedding()
+  embedding.ParseFromString(embedding_to_wire(node_ids, W, edge_ids, np.ascontiguousarray(H.T), dimension,
+                                              "NMF"))
   return embedding
 
 

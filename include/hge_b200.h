@@ -522,6 +522,36 @@ int hge_lp_node_edge_predict(hge_ctx* ctx, const float* xn, int64_t num_nodes, c
                              const int32_t* link_nodes, const int32_t* link_edges, int64_t num_links, float* out_prob,
                              uint8_t* out_keep);
 
+/* ---- non-negative factorization of the incidence (csrc/hge_nmf.cu) -------------------------
+ * The NMF baseline embedder (embedding.py:110-261 of the reference runs scikit-learn's NMF):
+ * A [N, E] (the 0/1 incidence of `inc`) ~ W [N, k] H [k, E], 1 <= k <= 256, by scikit-learn's
+ * coordinate descent (solver "cd", Frobenius loss, no regularization, no shuffling).  W and
+ * Ht = H^T [E, k] are dense fp32 row-major; `mem` applies to both.
+ *
+ * hge_nmf_init: a seeded start in the style of scikit-learn's init="random": element (r, c) =
+ *   scale * ((w >> 8) * 2^-24) in fp32, each operation rounded on its own, w = word c of the Philox
+ *   stream (csrc/hge_philox.cuh) of item r, phase HGE_PHASE_NMF_W (20) for W and HGE_PHASE_NMF_H
+ *   (21) for Ht.  NonNegativeFactorizationDevice passes scale = 2 fp32(sqrt(nnz / (N E k))).
+ *
+ * hge_nmf_fit: W and Ht hold the start on entry and the factors on return.  Iteration it updates
+ *   every row of W from P = A Ht and G = Ht^T Ht, then every row of Ht from P = A^T W and
+ *   G = W^T W (with the new W), and sums the projected-gradient violations of both; it stops after
+ *   the first iteration when that sum is 0, when violation / violation of iteration 1 <= tol, or
+ *   after max_iter.  *n_iter receives the iterations done, violations (host, optional,
+ *   [max_iter]) each iteration's violation, phase_ms (host, optional, [3]) the milliseconds spent
+ *   in the products, the Gram matrices and the coordinate-descent passes, summed over the
+ *   iterations (CUDA events; each half then ends with an event wait).  Every sum has one fixed
+ *   order (DESIGN.md section 9.10), so the result is bit-identical from run to run.  k outside
+ *   [1, 256], max_iter < 1, tol negative or NaN, num_nodes / num_edges different from the
+ *   incidence's, a start with a negative or non-finite entry, or a W or Ht that is all zero is
+ *   HGE_ERR_INVALID; nothing is written then.  Besides the staged copies of host arguments the
+ *   call holds 4 ld (N + E + max(N, E)) bytes (ld = k rounded up to a multiple of 4), one k x k
+ *   partial per 4096 rows and 8 bytes per 64 rows. */
+int hge_nmf_init(hge_ctx* ctx, int32_t num_nodes, int32_t num_edges, int k, uint64_t seed, float scale, float* W,
+                 float* Ht, int mem);
+int hge_nmf_fit(hge_ctx* ctx, hge_incidence* inc, int32_t num_nodes, int32_t num_edges, int k, float* W, float* Ht,
+                int max_iter, double tol, int mem, int* n_iter, double* violations, double* phase_ms);
+
 /* ---- hypergraph.proto wire format (host code; all pointers are host pointers) --------------
  * The data formats either side of the path: a serialized Hypergraph (hypergraph.proto:6-23) is
  * read straight into arrays, replacing the per-incidence Python loops of ToCsrMatrix /

@@ -20,8 +20,9 @@ from .hg2v_model import BooleanModel, KerasModelToEmbedding, UnweightedFloatMode
 from .embedding import (EMBEDDING_OPTIONS, EmbedHg2vAdjJaccard, EmbedHg2vAdjJaccardDevice,
                         EmbedHg2vAlgDist, EmbedHg2vAlgDistDevice, EmbedHg2vBoolean,
                         EmbedHg2vBooleanDevice, EmbedHg2vNeighborhoodWeightedJaccard,
-                        EmbedHg2vNeighborhoodWeightedJaccardDevice, EmbedNMFDevice)
+                        EmbedHg2vNeighborhoodWeightedJaccardDevice, EmbedNMFDevice, EmbedSVDDevice)
 from .nmf import NonNegativeFactorizationDevice
+from .svd import TruncatedSVDDevice
 from .hg2v_weighting import (AlphaScaleValues, ComputeSpans, DictToSparseRow, OneMinusValues,
                              UniformWeight, WeightByAlgebraicSpan, WeightByDistance,
                              WeightByDistanceCluster, WeightByNeighborhood,
@@ -40,7 +41,7 @@ __all__ = [
     "EmbedHg2vBoolean", "EmbedHg2vAdjJaccard", "EmbedHg2vNeighborhoodWeightedJaccard",
     "EmbedHg2vAlgDist", "EmbedHg2vBooleanDevice", "EmbedHg2vAlgDistDevice",
     "EmbedHg2vAdjJaccardDevice", "EmbedHg2vNeighborhoodWeightedJaccardDevice",
-    "EmbedNMFDevice", "NonNegativeFactorizationDevice",
+    "EmbedNMFDevice", "NonNegativeFactorizationDevice", "EmbedSVDDevice", "TruncatedSVDDevice",
     "AlphaScaleValues", "ComputeSpans", "DictToSparseRow", "OneMinusValues", "UniformWeight",
     "WeightByAlgebraicSpan", "WeightByDistance", "WeightByDistanceCluster", "WeightByNeighborhood",
     "WeightBySameTypeDistance", "ZeroOneScaleValues",

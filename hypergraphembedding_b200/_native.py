@@ -150,6 +150,15 @@ SIGNATURES = {
     "hge_nmf_fit": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int, c_vp, c_vp,
                                    ctypes.c_int, ctypes.c_double, ctypes.c_int, ctypes.POINTER(ctypes.c_int), c_vp,
                                    c_vp]),
+    "hge_svd_start": (ctypes.c_int, [c_vp, ctypes.c_int32, ctypes.c_int, ctypes.c_uint64, c_vp, ctypes.c_int]),
+    "hge_svd_half": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int, ctypes.c_int32, ctypes.c_int32, ctypes.c_int, c_vp,
+                                    c_vp, c_vp, ctypes.c_int, c_vp]),
+    "hge_svd_rowmat": (ctypes.c_int, [c_vp, ctypes.c_int64, ctypes.c_int, ctypes.c_int, c_vp, c_vp, c_vp,
+                                      ctypes.c_int]),
+    "hge_svd_flip": (ctypes.c_int, [c_vp, ctypes.c_int64, ctypes.c_int64, ctypes.c_int, ctypes.c_int, c_vp, c_vp,
+                                    ctypes.c_int]),
+    "hge_svd_residuals": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int, ctypes.c_int,
+                                         c_vp, c_vp, c_vp, c_vp, ctypes.c_int]),
     "hge_mt19937_random_raw":(ctypes.c_int, [c_vp, ctypes.c_int64, c_vp]),
     "hge_mt19937_interval": (ctypes.c_int, [c_vp, ctypes.c_uint32, ctypes.c_int64, c_vp]),
     "hge_spgemm_rows": (ctypes.c_int, [ctypes.c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
@@ -975,6 +984,77 @@ def nmf_fit(ctx, inc, W, Ht, max_iter, tol, phase_ms=None):
                             int(max_iter), float(tol), mem, ctypes.byref(n_iter), ptr(viol), ptr(phase_ms)),
         "hge_nmf_fit")
   return n_iter.value, viol[:n_iter.value].copy()
+
+
+def svd_ld(l):
+  """Row stride of the truncated SVD's dense arrays: l rounded up to a multiple of 4."""
+  return (int(l) + 3) & ~3
+
+
+def _svd_dense(*arrays):
+  mem = _mem(*arrays)
+  for a in arrays:
+    if mem == MEM_HOST:
+      assert isinstance(a, np.ndarray) and a.dtype == np.float32, "host arrays must be float32 numpy arrays"
+    else:
+      import torch
+      assert a.dtype == torch.float32, "device arrays must be float32 tensors"
+    assert a.ndim == 2, "dense arrays must be [rows, ld]"
+  return mem
+
+
+def svd_start(ctx, num_edges, l, seed, omega):
+  """hge_svd_start into fp32 omega [num_edges, svd_ld(l)] (numpy, or a CUDA tensor)."""
+  mem = _svd_dense(omega)
+  assert tuple(omega.shape) == (int(num_edges), svd_ld(l)), "omega must be [E, ld]"
+  check(ctx.lib.hge_svd_start(ctx.handle, int(num_edges), int(l), int(seed) & 0xFFFFFFFFFFFFFFFF, ptr(omega), mem),
+        "hge_svd_start")
+  return omega
+
+
+def svd_half(ctx, inc, side, l, x, y, phase_ms=None):
+  """hge_svd_half: y = A x (side 0) or A^T x (side 1) in place, returns the f64 Gram matrix
+  y^T y [l, l] (numpy).  x, y: fp32 [rows, svd_ld(l)], both numpy or both CUDA tensors.  phase_ms:
+  optional float64 [2] numpy array (product, Gram milliseconds)."""
+  mem = _svd_dense(x, y)
+  nodes, edges = (y.shape[0], x.shape[0]) if side == 0 else (x.shape[0], y.shape[0])
+  gram = np.empty((int(l), int(l)), dtype=np.float64)
+  if phase_ms is not None:
+    assert phase_ms.dtype == np.float64 and phase_ms.shape == (2,)
+  check(ctx.lib.hge_svd_half(ctx.handle, inc.handle, int(side), int(nodes), int(edges), int(l), ptr(x), ptr(y),
+                             ptr(gram), mem, ptr(phase_ms)), "hge_svd_half")
+  return gram
+
+
+def svd_rowmat(ctx, l, y, m, out):
+  """hge_svd_rowmat: out = y m in place; y, out fp32 [rows, svd_ld(l)] (numpy or CUDA tensors),
+  m fp32 [l, cols] numpy."""
+  mem = _svd_dense(y, out)
+  m = np.ascontiguousarray(m, dtype=np.float32)
+  assert m.ndim == 2 and m.shape[0] == int(l), "m must be [l, cols]"
+  assert y.shape[0] == out.shape[0], "y and out must have the same rows"
+  check(ctx.lib.hge_svd_rowmat(ctx.handle, int(y.shape[0]), int(l), int(m.shape[1]), ptr(y), ptr(m), ptr(out), mem),
+        "hge_svd_rowmat")
+  return out
+
+
+def svd_flip(ctx, l, k, u, v):
+  """hge_svd_flip in place on fp32 u [N, svd_ld(l)] and v [E, svd_ld(l)]."""
+  mem = _svd_dense(u, v)
+  check(ctx.lib.hge_svd_flip(ctx.handle, int(u.shape[0]), int(v.shape[0]), int(l), int(k), ptr(u), ptr(v), mem),
+        "hge_svd_flip")
+  return u, v
+
+
+def svd_residuals(ctx, inc, l, k, u, v, sigma):
+  """hge_svd_residuals: ||A v_i - sigma_i u_i|| / sigma_0 for i < k as a float64 numpy array."""
+  mem = _svd_dense(u, v)
+  sigma = np.ascontiguousarray(sigma, dtype=np.float64)
+  assert sigma.shape == (int(k),)
+  resid = np.zeros(int(k), dtype=np.float64)
+  check(ctx.lib.hge_svd_residuals(ctx.handle, inc.handle, int(u.shape[0]), int(v.shape[0]), int(l), int(k), ptr(u),
+                                  ptr(v), ptr(sigma), ptr(resid), mem), "hge_svd_residuals")
+  return resid
 
 
 class PeerArena(object):

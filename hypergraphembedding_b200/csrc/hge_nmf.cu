@@ -3,7 +3,8 @@
 // loss, no regularization and no shuffling, for the 0/1 incidence A [N, E] ~ W [N, k] H [k, E].
 //
 // One iteration, both halves with the same three steps (W with H^T, then H^T with the new W):
-//   k_nmf_spmm  P = A Ht (node rows) or A^T W (edge rows): each row adds its neighbours' rows in
+//   k_nmf_spmm  (csrc/hge_factor.cuh, shared with the truncated SVD of csrc/hge_svd.cu)
+//               P = A Ht (node rows) or A^T W (edge rows): each row adds its neighbours' rows in
 //               ascending incidence order, one fp32 add per neighbour -- scipy's order, so P equals
 //               scipy's float32 product bit for bit.  A sub-warp of LPR lanes owns a row, a lane
 //               LPR-strided float4 columns (as the gathers of csrc/hge_weighting.cu).  Long rows are
@@ -27,6 +28,7 @@
 
 #include <algorithm>
 
+#include "hge_factor.cuh"
 #include "hge_incidence.cuh"
 #include "hge_philox.cuh"
 #include "hge_seeded_table.cuh"
@@ -39,19 +41,8 @@ constexpr int kGramChunk = 4096;   // rows per Gram partial
 constexpr int kGramTile = 32;      // rows per shared-memory tile of k_nmf_gram
 constexpr int kGramPer = 8;        // Gram entries per thread
 constexpr int kCdRows = 64;        // rows (threads) per block of k_nmf_cd
-constexpr int kSpmmUnroll = 8;     // neighbour rows in flight per sub-warp
 
-// ---- dense layout -----------------------------------------------------------------------------
-
-// [rows, k] -> [rows, ld] with zero columns k .. ld - 1
-__global__ void k_nmf_pad(int64_t rows, int k, int ld, const float* __restrict__ x, float* __restrict__ y) {
-  const int64_t total = rows * ld;
-  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
-    const int64_t r = i / ld;
-    const int c = (int)(i - r * ld);
-    y[i] = c < k ? x[r * k + c] : 0.f;
-  }
-}
+// ---- dense layout (k_nmf_pad and the product k_nmf_spmm are in csrc/hge_factor.cuh) ---------------
 
 __global__ void k_nmf_unpad(int64_t rows, int k, int ld, const float* __restrict__ y, float* __restrict__ x) {
   const int64_t total = rows * k;
@@ -73,59 +64,6 @@ __global__ void k_nmf_check(int64_t n, const float* __restrict__ x, int nonzero,
   }
   f = __reduce_or_sync(0xffffffffu, f);
   if ((threadIdx.x & 31) == 0 && f) atomicOr(flags, f);
-}
-
-// ---- SpMM ---------------------------------------------------------------------------------------
-
-template <int LPR, int S>
-__global__ void __launch_bounds__(kBlock) k_nmf_spmm(int32_t rows, const int64_t* __restrict__ ptr,
-                                                      const int32_t* __restrict__ idx, const float4* __restrict__ y,
-                                                      int ld4, float4* __restrict__ p) {
-  const int gl = threadIdx.x & (LPR - 1);
-  const int64_t sub = ((int64_t)blockIdx.x * kBlock + threadIdx.x) / LPR;
-  const int64_t nsub = (int64_t)gridDim.x * kBlock / LPR;
-  for (int64_t row = sub; row < rows; row += nsub) {
-    const int64_t b = ptr[row], e = ptr[row + 1];
-    float4 acc[S];
-#pragma unroll
-    for (int s = 0; s < S; ++s) acc[s] = hge_f4_zero();
-    for (int64_t q = b; q < e; q += kSpmmUnroll) {
-      int32_t id[kSpmmUnroll];
-#pragma unroll
-      for (int u = 0; u < kSpmmUnroll; ++u) id[u] = q + u < e ? __ldg(idx + q + u) : -1;
-      float4 v[kSpmmUnroll][S];
-#pragma unroll
-      for (int u = 0; u < kSpmmUnroll; ++u)
-#pragma unroll
-        for (int s = 0; s < S; ++s) {
-          const int c = s * LPR + gl;
-          v[u][s] = (id[u] >= 0 && c < ld4) ? __ldg(y + (size_t)id[u] * ld4 + c) : hge_f4_zero();
-        }
-#pragma unroll
-      for (int u = 0; u < kSpmmUnroll; ++u)
-        if (id[u] >= 0)
-#pragma unroll
-          for (int s = 0; s < S; ++s) hge_f4_add(acc[s], v[u][s]);
-    }
-#pragma unroll
-    for (int s = 0; s < S; ++s) {
-      const int c = s * LPR + gl;
-      if (c < ld4) p[(size_t)row * ld4 + c] = acc[s];
-    }
-  }
-}
-
-typedef void (*SpmmKernel)(int32_t, const int64_t*, const int32_t*, const float4*, int, float4*);
-
-// sub-warp width: next power of two of ld / 4, at most 32; two column slabs above 128 columns
-SpmmKernel spmm_kernel(int ld4) {
-  if (ld4 <= 1) return k_nmf_spmm<1, 1>;
-  if (ld4 <= 2) return k_nmf_spmm<2, 1>;
-  if (ld4 <= 4) return k_nmf_spmm<4, 1>;
-  if (ld4 <= 8) return k_nmf_spmm<8, 1>;
-  if (ld4 <= 16) return k_nmf_spmm<16, 1>;
-  if (ld4 <= 32) return k_nmf_spmm<32, 1>;
-  return k_nmf_spmm<32, 2>;
 }
 
 // ---- Gram -----------------------------------------------------------------------------------------
@@ -222,8 +160,6 @@ __global__ void k_nmf_viol(int64_t nw, const double* __restrict__ pw, int64_t nh
   *out = sw + sh;
 }
 
-int ld_of(int k) { return (k + 3) & ~3; }
-
 // Workspace and phase timing of one fit.
 struct Fit {
   hge_ctx* ctx;
@@ -236,7 +172,7 @@ struct Fit {
   int spmm_grid = 0;
   cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
   explicit Fit(hge_ctx* c, hge_incidence* i, int k_)
-      : ctx(c), inc(i), k(k_), ld(ld_of(k_)), w(c), h(c), p(c), part(c), g(c), vpart(c), viol(c) {}
+      : ctx(c), inc(i), k(k_), ld(factor_ld(k_)), w(c), h(c), p(c), part(c), g(c), vpart(c), viol(c) {}
   ~Fit() {
     for (cudaEvent_t e : ev)
       if (e) cudaEventDestroy(e);
@@ -372,9 +308,7 @@ int hge_nmf_fit(hge_ctx* ctx, hge_incidence* inc, int32_t num_nodes, int32_t num
   HGE_TRY(f.viol.alloc((size_t)max_iter));
   f.cd_smem = sizeof(float) * ((size_t)kCdRows * (ld + 1) + k);
   HGE_CUDA(cudaFuncSetAttribute(k_nmf_cd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)f.cd_smem));
-  const int per_sm = ctx->blocks_per_sm > 0 ? ctx->blocks_per_sm : 8;
-  f.spmm_grid = (int)std::max<int64_t>(1, std::min<int64_t>((rmax * 32 + kBlock - 1) / kBlock,
-                                                            (int64_t)ctx->num_sms * per_sm));
+  f.spmm_grid = spmm_grid(ctx, rmax);
   if (phase_ms) {
     for (cudaEvent_t& e : f.ev) HGE_CUDA(cudaEventCreate(&e));
     phase_ms[0] = phase_ms[1] = phase_ms[2] = 0.0;

@@ -3,7 +3,8 @@
 // device_sampler_ref.py restates everything in this file in numpy; oracle/seeded_training_ref.py
 // restates the training phases (epoch order, initial tables), oracle/lp_svm_ref.py the negatives of
 // the link-prediction classifiers, oracle/lp_node_edge_ref.py the training set, epoch orders and
-// initial weights of the node-edge classifier, oracle/nmf_ref.py the factorization's start.
+// initial weights of the node-edge classifier, oracle/nmf_ref.py the factorization's start, oracle/svd_ref.py
+// the truncated SVD's start.
 //
 // Layout.  Every item owns one stream of 32-bit words:
 //   key     = { (uint32)seed, (uint32)(seed >> 32) }
@@ -57,6 +58,9 @@ enum HgePhase : uint32_t {
   // of H^T (edge), word c is column c
   HGE_PHASE_NMF_W = 20,
   HGE_PHASE_NMF_H = 21,
+  // seeded start of the truncated SVD (csrc/hge_svd.cu): item = row of the start block Omega
+  // (edge), word c is column c
+  HGE_PHASE_SVD = 22,
 };
 
 #ifdef __CUDACC__

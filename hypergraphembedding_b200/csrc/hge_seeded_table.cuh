@@ -1,5 +1,6 @@
 // The seeded dense tables of the library: the hypergraph2vec embedding tables
-// (csrc/hge_hg2v_train.cu) and the start of the non-negative factorization (csrc/hge_nmf.cu).
+// (csrc/hge_hg2v_train.cu), the start of the non-negative factorization (csrc/hge_nmf.cu) and the
+// start block of the truncated SVD (csrc/hge_svd.cu).
 #pragma once
 
 #include "hge_philox.cuh"
@@ -9,7 +10,7 @@ namespace {
 // Seeded dense table [rows, dim]: element (r, c) = offset + scale * ((word c of the stream of row
 // r in `phase`) >> 8) * 2^-24, each operation rounded on its own (no contraction), so that the
 // float32 numpy restatement gives the same bits.  The hypergraph2vec tables and the
-// factorization's start are drawn with it.
+// factorizations' starts are drawn with it.
 __global__ void k_init_table(int64_t rows, int dim, uint64_t seed, uint32_t phase, float offset, float scale,
                              float* __restrict__ t) {
   const int blocks = (dim + 3) / 4;

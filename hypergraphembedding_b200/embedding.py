@@ -23,6 +23,7 @@ from .hypergraph_pb2 import HypergraphEmbedding
 from .hypergraph_util import (CompressRange, ToCsrMatrix, ToEdgeCsrMatrix, compressed_incidence,
                               embedding_to_wire)
 from .nmf import NonNegativeFactorizationDevice
+from .svd import TruncatedSVDDevice
 
 log = logging.getLogger()
 
@@ -238,6 +239,21 @@ def EmbedNMFDevice(hypergraph, dimension, max_iter=200, tol=1e-4, seed=0):
   embedding = HypergraphEmbedding()
   embedding.ParseFromString(embedding_to_wire(node_ids, W, edge_ids, np.ascontiguousarray(H.T), dimension,
                                               "NMF"))
+  return embedding
+
+
+def EmbedSVDDevice(hypergraph, dimension, n_iter=5, oversamples=10, seed=0):
+  """The SVD baseline (embedding.py:110-261 of the reference) on the GPU: the compressed incidence
+  A ~ U diag(s) V^T by TruncatedSVDDevice (randomized subspace iteration from the seeded start of
+  `seed`); node vectors are the rows of U, edge vectors the rows of V, keyed by the original ids,
+  method_name "SVD".  Triplets beyond the incidence's numerical rank give zero columns.  numpy's
+  global RNG is neither read nor advanced, so this is not the reference's call and not in
+  EMBEDDING_OPTIONS."""
+  node_ids, edge_ids, A = compressed_incidence(hypergraph)
+  U, _, Vt, _ = TruncatedSVDDevice(A, dimension, n_iter=n_iter, oversamples=oversamples, seed=seed)
+  embedding = HypergraphEmbedding()
+  embedding.ParseFromString(embedding_to_wire(node_ids, U, edge_ids, np.ascontiguousarray(Vt.T), dimension,
+                                              "SVD"))
   return embedding
 
 

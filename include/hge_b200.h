@@ -552,6 +552,46 @@ int hge_nmf_init(hge_ctx* ctx, int32_t num_nodes, int32_t num_edges, int k, uint
 int hge_nmf_fit(hge_ctx* ctx, hge_incidence* inc, int32_t num_nodes, int32_t num_edges, int k, float* W, float* Ht,
                 int max_iter, double tol, int mem, int* n_iter, double* violations, double* phase_ms);
 
+/* ---- truncated SVD of the incidence (csrc/hge_svd.cu) ---------------------------------------
+ * The SVD baseline embedder (embedding.py:110-261 of the reference): A [N, E] (the 0/1 incidence
+ * of `inc`) ~ U diag(s) V^T by randomized subspace iteration with Rayleigh-Ritz (DESIGN.md section
+ * 9.11).  The host drives the loop and does the l x l steps in f64; these entry points do the
+ * work of size N or E.  Every dense array is fp32 row-major [rows, ld], ld = l rounded up to a
+ * multiple of 4, with columns l .. ld - 1 zero; 1 <= l <= 256.  `mem` applies to the dense arrays;
+ * gram, m, sigma and resid are host arrays.  Every sum has one fixed order, so every result is
+ * bit-identical from run to run and for every launch setting.  The host loop, per iteration:
+ *   hge_svd_half(side 0, X = Omega -> Y), M from eigh(G), hge_svd_rowmat(Y, M -> Q),
+ *   hge_svd_half(side 1, Q -> Z),         M from eigh(G), hge_svd_rowmat(Z, M -> Omega)
+ * with M = U~ diag(1 / sigma) (1 / sigma = 0 where sigma <= 1e-6 sigma_1), rounded to fp32.
+ *
+ * hge_svd_start: omega [num_edges, ld], element (r, c < l) = -1 + 2 ((w >> 8) 2^-24) in fp32, each
+ *   operation rounded on its own, w = word c of the Philox stream (csrc/hge_philox.cuh) of item r
+ *   in phase HGE_PHASE_SVD (22).
+ * hge_svd_half: side 0: y [N, ld] = A x (x [E, ld]); side 1: y [E, ld] = A^T x (x [N, ld]); then
+ *   gram [l, l] (f64) = y^T y over the first l columns: per entry an f64 fma chain in ascending row
+ *   order within chunks of 4096 rows, the chunk partials added in ascending order.  phase_ms
+ *   (optional, [2]): milliseconds of the product and of the Gram matrix (CUDA events).
+ * hge_svd_rowmat: out [rows, ld] = y [rows, ld] (first l columns) times m [l, cols] (fp32, host),
+ *   1 <= cols <= l; each entry one fp32 fma chain over r = 0 .. l - 1 ascending from +0; columns
+ *   cols .. ld - 1 of out are 0.  out must not alias y.
+ * hge_svd_flip: scikit-learn's svd_flip on the first k <= l columns of u [num_u_rows, ld] and
+ *   v [num_v_rows, ld]: where the entry of largest magnitude of column i of u (lowest row on a
+ *   tie) is negative, columns i of u and of v are negated.
+ * hge_svd_residuals: resid[i] = || A v_i - sigma_i u_i ||_2 / sigma_0 for i < k (sigma [k], f64),
+ *   with u [N, ld], v [E, ld]: the product A v, then per column d = (A v)[j,i] - sigma_i u[j,i] and
+ *   sum d d in f64, each operation rounded on its own, in ascending row order within chunks of
+ *   4096 rows, the chunk sums in ascending order; sigma_0 = 0 gives the unscaled norm.
+ * Refused with HGE_ERR_INVALID before anything is written: l outside [1, 256], k or cols outside
+ * [1, l], a sharded incidence, num_nodes / num_edges different from the incidence's, y == out. */
+int hge_svd_start(hge_ctx* ctx, int32_t num_edges, int l, uint64_t seed, float* omega, int mem);
+int hge_svd_half(hge_ctx* ctx, hge_incidence* inc, int side, int32_t num_nodes, int32_t num_edges, int l,
+                 const float* x, float* y, double* gram, int mem, double* phase_ms);
+int hge_svd_rowmat(hge_ctx* ctx, int64_t rows, int l, int cols, const float* y, const float* m, float* out,
+                   int mem);
+int hge_svd_flip(hge_ctx* ctx, int64_t num_u_rows, int64_t num_v_rows, int l, int k, float* u, float* v, int mem);
+int hge_svd_residuals(hge_ctx* ctx, hge_incidence* inc, int32_t num_nodes, int32_t num_edges, int l, int k,
+                      const float* u, const float* v, const double* sigma, double* resid, int mem);
+
 /* ---- hypergraph.proto wire format (host code; all pointers are host pointers) --------------
  * The data formats either side of the path: a serialized Hypergraph (hypergraph.proto:6-23) is
  * read straight into arrays, replacing the per-incidence Python loops of ToCsrMatrix /

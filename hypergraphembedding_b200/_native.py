@@ -159,6 +159,17 @@ SIGNATURES = {
                                     ctypes.c_int]),
     "hge_svd_residuals": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int, ctypes.c_int,
                                          c_vp, c_vp, c_vp, c_vp, ctypes.c_int]),
+    "hge_n2v_walks": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int, ctypes.c_int, ctypes.c_double, ctypes.c_double,
+                                     ctypes.c_uint64, c_vp, c_vp]),
+    "hge_n2v_pairs": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_uint64, c_vp,
+                                     ctypes.c_int64, ctypes.POINTER(ctypes.c_int64)]),
+    "hge_n2v_negatives": (ctypes.c_int, [c_vp, ctypes.c_int64, c_vp, ctypes.c_int32, ctypes.c_int, ctypes.c_uint64,
+                                         ctypes.c_int, c_vp]),
+    "hge_n2v_init": (ctypes.c_int, [c_vp, ctypes.c_int32, ctypes.c_int, ctypes.c_uint64, c_vp, c_vp]),
+    "hge_n2v_train_epoch": (ctypes.c_int, [c_vp, ctypes.c_int32, ctypes.c_int, c_vp, c_vp, c_vp, ctypes.c_int64,
+                                           c_vp, ctypes.c_int, ctypes.c_uint64, ctypes.c_int, ctypes.c_int,
+                                           ctypes.c_int, ctypes.c_double, ctypes.c_double, ctypes.c_int64,
+                                           ctypes.POINTER(ctypes.c_double)]),
     "hge_mt19937_random_raw":(ctypes.c_int, [c_vp, ctypes.c_int64, c_vp]),
     "hge_mt19937_interval": (ctypes.c_int, [c_vp, ctypes.c_uint32, ctypes.c_int64, c_vp]),
     "hge_spgemm_rows": (ctypes.c_int, [ctypes.c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
@@ -1099,3 +1110,56 @@ class PeerArena(object):
     if getattr(self, "handle", None):
       self.ctx.lib.hge_p2p_destroy(self.handle)
       self.handle = None
+
+
+# ---- node2vec (csrc/hge_n2v.cu); every array is a CUDA tensor -------------------------------------
+
+def _cuda(*arrays):
+  assert all(is_device(a) and a.is_contiguous() for a in arrays), "node2vec arrays must be contiguous CUDA tensors"
+
+
+def n2v_walks(ctx, inc, num_walks, walk_length, p, q, seed, walks, counts):
+  """hge_n2v_walks into int32 walks [num_walks V, walk_length] and int64 counts [V]."""
+  _cuda(walks, counts)
+  check(ctx.lib.hge_n2v_walks(ctx.handle, inc.handle, int(num_walks), int(walk_length), float(p), float(q),
+                              int(seed) & 0xFFFFFFFFFFFFFFFF, ptr(walks), ptr(counts)), "hge_n2v_walks")
+
+
+def n2v_pairs(ctx, walks, window, seed, pairs=None):
+  """hge_n2v_pairs: the pair count, and with `pairs` (int32 [P, 2]) the pairs themselves."""
+  _cuda(walks)
+  n = ctypes.c_int64()
+  cap = 0
+  if pairs is not None:
+    _cuda(pairs)
+    cap = int(pairs.shape[0])
+  check(ctx.lib.hge_n2v_pairs(ctx.handle, ptr(walks), int(walks.shape[0]), int(walks.shape[1]), int(window),
+                              int(seed) & 0xFFFFFFFFFFFFFFFF, ptr(pairs), cap, ctypes.byref(n)), "hge_n2v_pairs")
+  return int(n.value)
+
+
+def n2v_negatives(ctx, num_pairs, cum, negative, seed, epoch, out):
+  """hge_n2v_negatives into int32 out [num_pairs, negative]; cum is the int64 noise table [V + 1]."""
+  _cuda(cum, out)
+  check(ctx.lib.hge_n2v_negatives(ctx.handle, int(num_pairs), ptr(cum), int(cum.shape[0]) - 1, int(negative),
+                                  int(seed) & 0xFFFFFFFFFFFFFFFF, int(epoch), ptr(out)), "hge_n2v_negatives")
+
+
+def n2v_init(ctx, seed, tin, tout):
+  """hge_n2v_init on fp32 tables [V, dim]."""
+  _cuda(tin, tout)
+  check(ctx.lib.hge_n2v_init(ctx.handle, int(tin.shape[0]), int(tin.shape[1]), int(seed) & 0xFFFFFFFFFFFFFFFF,
+                             ptr(tin), ptr(tout)), "hge_n2v_init")
+
+
+def n2v_train_epoch(ctx, tin, tout, pairs, cum, negative, seed, epoch, epochs, batch_pairs, alpha, min_alpha,
+                    plan_bytes=0):
+  """hge_n2v_train_epoch in place on tin / tout; returns the epoch loss."""
+  _cuda(tin, tout, pairs, cum)
+  loss = ctypes.c_double()
+  check(ctx.lib.hge_n2v_train_epoch(ctx.handle, int(tin.shape[0]), int(tin.shape[1]), ptr(tin), ptr(tout),
+                                    ptr(pairs), int(pairs.shape[0]), ptr(cum), int(negative),
+                                    int(seed) & 0xFFFFFFFFFFFFFFFF, int(epoch), int(epochs), int(batch_pairs),
+                                    float(alpha), float(min_alpha), int(plan_bytes), ctypes.byref(loss)),
+        "hge_n2v_train_epoch")
+  return float(loss.value)

@@ -4,7 +4,8 @@
 // restates the training phases (epoch order, initial tables), oracle/lp_svm_ref.py the negatives of
 // the link-prediction classifiers, oracle/lp_node_edge_ref.py the training set, epoch orders and
 // initial weights of the node-edge classifier, oracle/nmf_ref.py the factorization's start, oracle/svd_ref.py
-// the truncated SVD's start.
+// the truncated SVD's start, oracle/node2vec_ref.py the walks, windows, negatives, epoch orders and
+// initial table of node2vec.
 //
 // Layout.  Every item owns one stream of 32-bit words:
 //   key     = { (uint32)seed, (uint32)(seed >> 32) }
@@ -61,6 +62,17 @@ enum HgePhase : uint32_t {
   // seeded start of the truncated SVD (csrc/hge_svd.cu): item = row of the start block Omega
   // (edge), word c is column c
   HGE_PHASE_SVD = 22,
+  // node2vec (csrc/hge_n2v.cu): walk w (item = w) reads its words in step order, one below(d) for
+  // the first step, then per step of a vertex of degree >= 2 one Bernoulli word and, when it does
+  // not return, below(d - 1); token g = w L + i of the walks draws its window (item = g, one
+  // below(window)); the epoch orders (item = pair index, as HGE_PHASE_SHUFFLE); negatives of pair i
+  // in epoch e (item = e P + i, per sample two words (high, low) per 64-bit rejection round); the
+  // initial input table (item = vertex, word c is column c)
+  HGE_PHASE_N2V_WALK = 23,
+  HGE_PHASE_N2V_WINDOW = 24,
+  HGE_PHASE_N2V_SHUFFLE = 25,
+  HGE_PHASE_N2V_NEG = 26,
+  HGE_PHASE_N2V_INIT = 27,
 };
 
 #ifdef __CUDACC__

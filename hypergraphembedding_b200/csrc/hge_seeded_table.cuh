@@ -1,6 +1,6 @@
 // The seeded dense tables of the library: the hypergraph2vec embedding tables
 // (csrc/hge_hg2v_train.cu), the start of the non-negative factorization (csrc/hge_nmf.cu) and the
-// start block of the truncated SVD (csrc/hge_svd.cu).
+// start block of the truncated SVD (csrc/hge_svd.cu) and node2vec's input table (csrc/hge_n2v.cu).
 #pragma once
 
 #include "hge_philox.cuh"

@@ -23,6 +23,7 @@ from .hypergraph_pb2 import HypergraphEmbedding
 from .hypergraph_util import (CompressRange, ToCsrMatrix, ToEdgeCsrMatrix, compressed_incidence,
                               embedding_to_wire)
 from .nmf import NonNegativeFactorizationDevice
+from .node2vec import DEFAULT_BATCH_PAIRS, Node2VecDevice
 from .svd import TruncatedSVDDevice
 
 log = logging.getLogger()
@@ -254,6 +255,24 @@ def EmbedSVDDevice(hypergraph, dimension, n_iter=5, oversamples=10, seed=0):
   embedding = HypergraphEmbedding()
   embedding.ParseFromString(embedding_to_wire(node_ids, U, edge_ids, np.ascontiguousarray(Vt.T), dimension,
                                               "SVD"))
+  return embedding
+
+
+def EmbedNode2VecDevice(hypergraph, dimension, walk_length=80, num_walks=10, p=1.0, q=1.0, window=10, negative=5,
+                        epochs=5, alpha=0.025, min_alpha=1e-4, batch_pairs=DEFAULT_BATCH_PAIRS, seed=0):
+  """The node2vec baseline (embedding.py:110-261 of the reference) on the GPU: Node2VecDevice on the
+  node-edge bipartite graph of the compressed incidence; node vectors are the input-table rows of
+  the nodes, edge vectors those of the edges, keyed by the original ids, method_name "N2V".  numpy's
+  global RNG and Python's ``random`` are neither read nor advanced, so this is not the reference's
+  call and not in EMBEDDING_OPTIONS."""
+  node_ids, edge_ids, A = compressed_incidence(hypergraph)
+  X, _ = Node2VecDevice(A, dimension, walk_length=walk_length, num_walks=num_walks, p=p, q=q, window=window,
+                        negative=negative, epochs=epochs, alpha=alpha, min_alpha=min_alpha, batch_pairs=batch_pairs,
+                        seed=seed)
+  N = len(node_ids)
+  embedding = HypergraphEmbedding()
+  embedding.ParseFromString(embedding_to_wire(node_ids, np.ascontiguousarray(X[:N]), edge_ids,
+                                              np.ascontiguousarray(X[N:]), dimension, "N2V"))
   return embedding
 
 

@@ -592,6 +592,47 @@ int hge_svd_flip(hge_ctx* ctx, int64_t num_u_rows, int64_t num_v_rows, int l, in
 int hge_svd_residuals(hge_ctx* ctx, hge_incidence* inc, int32_t num_nodes, int32_t num_edges, int l, int k,
                       const float* u, const float* v, const double* sigma, double* resid, int mem);
 
+/* ---- node2vec on the node-edge bipartite graph (csrc/hge_n2v.cu) ----------------------------
+ * The node2vec baseline embedder (embedding.py:110-261 of the reference) on the bipartite graph of
+ * V = N + E vertices (node r is vertex r, edge c is vertex N + c); DESIGN.md section 9.12.  Every
+ * array argument is a DEVICE pointer.  The host loop:
+ *   hge_n2v_walks -> walks, counts; hge_n2v_pairs twice (count, then emit); noise table cum from
+ *   counts^0.75 (host); hge_n2v_init; hge_n2v_train_epoch for epoch = 0 .. epochs - 1.
+ *
+ * hge_n2v_walks: walks [num_walks V, walk_length] int32 (walk w starts at vertex w mod V; a walk
+ *   from a vertex of degree 0 is that vertex followed by -1), counts [V] int64 the occurrences of
+ *   every vertex in the walks.  Draws from Philox phase HGE_PHASE_N2V_WALK (23), item = walk.
+ * hge_n2v_pairs: (center, context) int32 pairs [*num_pairs, 2] of word2vec's shrunk windows (phase
+ *   HGE_PHASE_N2V_WINDOW (24), item = token), in ascending (token, context position) order.
+ *   pairs = NULL only counts.  2^31 pairs or more, or capacity < the count, is HGE_ERR_INVALID
+ *   (*num_pairs still receives the count).
+ * hge_n2v_negatives: out [num_pairs, negative] int32, the negatives pair i draws in `epoch`
+ *   (phase HGE_PHASE_N2V_NEG (26), item = epoch num_pairs + i) from the cumulative noise table cum
+ *   [num_vertices + 1] int64 (cum[0] = 0, cum[V] > 0): vertex v with cum[v] <= r < cum[v + 1] for
+ *   r uniform on [0, cum[V]).  Draws equal to the pair's context are included (training skips them).
+ * hge_n2v_init: tin [V, dim] uniform on [-0.5 / dim, 0.5 / dim) (phase HGE_PHASE_N2V_INIT (27)),
+ *   tout [V, dim] zero; 1 <= dim <= 256.
+ * hge_n2v_train_epoch: one epoch of mini-batch skip-gram with negative sampling over pairs [num_pairs,
+ *   2] in the order of hge_shuffle_order in phase HGE_PHASE_N2V_SHUFFLE (25), batches of
+ *   batch_pairs pairs.  Within a batch every coefficient g = lr (label - sigmoid(in[c] . out[x])) is
+ *   computed from the tables at the batch start; then in[c] += sum g out[x] and out[x] += sum g in[c]
+ *   over each row's contributions in ascending (pair position, slot) order.  lr of global batch t of
+ *   T = epochs ceil(num_pairs / batch_pairs) is (float)(alpha - (alpha - min_alpha) (t / T)) in f64.
+ *   *loss receives the epoch's sum of -log sigmoid(s+) - sum log sigmoid(-s-), in a fixed f64
+ *   order.  plan_bytes bounds the per-chunk plan (0: 512 MiB); results do not depend on it.  The
+ *   tables, *loss and the launch sequence are bit-identical from run to run.  Per epoch:
+ *   1 + (radix passes) launches for the order, 3 per chunk (plan, two sorts) and 3 per batch. */
+int hge_n2v_walks(hge_ctx* ctx, hge_incidence* inc, int num_walks, int walk_length, double p, double q,
+                  uint64_t seed, int32_t* walks, int64_t* counts);
+int hge_n2v_pairs(hge_ctx* ctx, const int32_t* walks, int64_t num_walk_items, int walk_length, int window,
+                  uint64_t seed, int32_t* pairs, int64_t capacity, int64_t* num_pairs);
+int hge_n2v_negatives(hge_ctx* ctx, int64_t num_pairs, const int64_t* cum, int32_t num_vertices, int negative,
+                      uint64_t seed, int epoch, int32_t* out);
+int hge_n2v_init(hge_ctx* ctx, int32_t num_vertices, int dim, uint64_t seed, float* tin, float* tout);
+int hge_n2v_train_epoch(hge_ctx* ctx, int32_t num_vertices, int dim, float* tin, float* tout, const int32_t* pairs,
+                        int64_t num_pairs, const int64_t* cum, int negative, uint64_t seed, int epoch, int epochs,
+                        int batch_pairs, double alpha, double min_alpha, int64_t plan_bytes, double* loss);
+
 /* ---- hypergraph.proto wire format (host code; all pointers are host pointers) --------------
  * The data formats either side of the path: a serialized Hypergraph (hypergraph.proto:6-23) is
  * read straight into arrays, replacing the per-incidence Python loops of ToCsrMatrix /

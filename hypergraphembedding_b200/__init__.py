@@ -20,10 +20,10 @@ from .hg2v_model import BooleanModel, KerasModelToEmbedding, UnweightedFloatMode
 from .embedding import (EMBEDDING_OPTIONS, EmbedHg2vAdjJaccard, EmbedHg2vAdjJaccardDevice,
                         EmbedHg2vAlgDist, EmbedHg2vAlgDistDevice, EmbedHg2vBoolean,
                         EmbedHg2vBooleanDevice, EmbedHg2vNeighborhoodWeightedJaccard,
-                        EmbedHg2vNeighborhoodWeightedJaccardDevice, EmbedNMFDevice, EmbedNode2VecDevice,
-                        EmbedSVDDevice)
+                        EmbedHg2vNeighborhoodWeightedJaccardDevice, EmbedNMFDevice, EmbedNode2VecCliqueDevice,
+                        EmbedNode2VecDevice, EmbedSVDDevice)
 from .nmf import NonNegativeFactorizationDevice
-from .node2vec import Node2VecDevice
+from .node2vec import Node2VecCliqueDevice, Node2VecDevice
 from .svd import TruncatedSVDDevice
 from .hg2v_weighting import (AlphaScaleValues, ComputeSpans, DictToSparseRow, OneMinusValues,
                              UniformWeight, WeightByAlgebraicSpan, WeightByDistance,
@@ -44,7 +44,7 @@ __all__ = [
     "EmbedHg2vAlgDist", "EmbedHg2vBooleanDevice", "EmbedHg2vAlgDistDevice",
     "EmbedHg2vAdjJaccardDevice", "EmbedHg2vNeighborhoodWeightedJaccardDevice",
     "EmbedNMFDevice", "NonNegativeFactorizationDevice", "EmbedSVDDevice", "TruncatedSVDDevice",
-    "EmbedNode2VecDevice", "Node2VecDevice",
+    "EmbedNode2VecDevice", "Node2VecDevice", "EmbedNode2VecCliqueDevice", "Node2VecCliqueDevice",
     "AlphaScaleValues", "ComputeSpans", "DictToSparseRow", "OneMinusValues", "UniformWeight",
     "WeightByAlgebraicSpan", "WeightByDistance", "WeightByDistanceCluster", "WeightByNeighborhood",
     "WeightBySameTypeDistance", "ZeroOneScaleValues",

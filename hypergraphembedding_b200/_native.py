@@ -170,6 +170,8 @@ SIGNATURES = {
                                            c_vp, ctypes.c_int, ctypes.c_uint64, ctypes.c_int, ctypes.c_int,
                                            ctypes.c_int, ctypes.c_double, ctypes.c_double, ctypes.c_int64,
                                            ctypes.POINTER(ctypes.c_double)]),
+    "hge_n2v_clique_walks": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_double,
+                                            ctypes.c_double, ctypes.c_uint64, c_vp, c_vp]),
     "hge_mt19937_random_raw":(ctypes.c_int, [c_vp, ctypes.c_int64, c_vp]),
     "hge_mt19937_interval": (ctypes.c_int, [c_vp, ctypes.c_uint32, ctypes.c_int64, c_vp]),
     "hge_spgemm_rows": (ctypes.c_int, [ctypes.c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
@@ -1163,3 +1165,12 @@ def n2v_train_epoch(ctx, tin, tout, pairs, cum, negative, seed, epoch, epochs, b
                                     float(alpha), float(min_alpha), int(plan_bytes), ctypes.byref(loss)),
         "hge_n2v_train_epoch")
   return float(loss.value)
+
+
+def n2v_clique_walks(ctx, inc, side, num_walks, walk_length, p, q, seed, walks, counts):
+  """hge_n2v_clique_walks on side 0 (nodes) or 1 (edges) into int32 walks [num_walks V,
+  walk_length] and int64 counts [V]."""
+  _cuda(walks, counts)
+  check(ctx.lib.hge_n2v_clique_walks(ctx.handle, inc.handle, int(side), int(num_walks), int(walk_length), float(p),
+                                     float(q), int(seed) & 0xFFFFFFFFFFFFFFFF, ptr(walks), ptr(counts)),
+        "hge_n2v_clique_walks")

@@ -5,7 +5,7 @@
 // the link-prediction classifiers, oracle/lp_node_edge_ref.py the training set, epoch orders and
 // initial weights of the node-edge classifier, oracle/nmf_ref.py the factorization's start, oracle/svd_ref.py
 // the truncated SVD's start, oracle/node2vec_ref.py the walks, windows, negatives, epoch orders and
-// initial table of node2vec.
+// initial table of node2vec, tests/n2v_clique_ref.py node2vec's walks on a clique expansion.
 //
 // Layout.  Every item owns one stream of 32-bit words:
 //   key     = { (uint32)seed, (uint32)(seed >> 32) }
@@ -73,6 +73,10 @@ enum HgePhase : uint32_t {
   HGE_PHASE_N2V_SHUFFLE = 25,
   HGE_PHASE_N2V_NEG = 26,
   HGE_PHASE_N2V_INIT = 27,
+  // node2vec on a clique expansion (csrc/hge_n2v_clique.cu): walk w (item = w) reads its words in
+  // proposal order, per proposal two words (high, low) per 64-bit rejection round for the position
+  // r in [0, S(v)), one below(|e| - 1) for the member, then one acceptance word when a' < m
+  HGE_PHASE_N2V_CLIQUE_WALK = 28,
 };
 
 #ifdef __CUDACC__

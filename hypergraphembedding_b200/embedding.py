@@ -23,7 +23,7 @@ from .hypergraph_pb2 import HypergraphEmbedding
 from .hypergraph_util import (CompressRange, ToCsrMatrix, ToEdgeCsrMatrix, compressed_incidence,
                               embedding_to_wire)
 from .nmf import NonNegativeFactorizationDevice
-from .node2vec import DEFAULT_BATCH_PAIRS, Node2VecDevice
+from .node2vec import DEFAULT_BATCH_PAIRS, Node2VecCliqueDevice, Node2VecDevice, clique_edge_seed
 from .svd import TruncatedSVDDevice
 
 log = logging.getLogger()
@@ -273,6 +273,25 @@ def EmbedNode2VecDevice(hypergraph, dimension, walk_length=80, num_walks=10, p=1
   embedding = HypergraphEmbedding()
   embedding.ParseFromString(embedding_to_wire(node_ids, np.ascontiguousarray(X[:N]), edge_ids,
                                               np.ascontiguousarray(X[N:]), dimension, "N2V"))
+  return embedding
+
+
+def EmbedNode2VecCliqueDevice(hypergraph, dimension, walk_length=80, num_walks=10, p=1.0, q=1.0, window=10,
+                              negative=5, epochs=5, alpha=0.025, min_alpha=1e-4, batch_pairs=DEFAULT_BATCH_PAIRS,
+                              seed=0):
+  """node2vec on the weighted clique expansions of the compressed incidence on the GPU
+  (Node2VecCliqueDevice): node vectors from the node-side expansion with `seed`, edge vectors from
+  the edge-side expansion with clique_edge_seed(seed), keyed by the original ids, method_name
+  "N2V_CLIQUE".  The two tables are trained apart, so node and edge vectors do not share a space.
+  numpy's global RNG and Python's ``random`` are neither read nor advanced; not in
+  EMBEDDING_OPTIONS."""
+  node_ids, edge_ids, A = compressed_incidence(hypergraph)
+  kw = dict(walk_length=walk_length, num_walks=num_walks, p=p, q=q, window=window, negative=negative, epochs=epochs,
+            alpha=alpha, min_alpha=min_alpha, batch_pairs=batch_pairs)
+  Xn, _ = Node2VecCliqueDevice(A, dimension, side="node", seed=seed, **kw)
+  Xe, _ = Node2VecCliqueDevice(A, dimension, side="edge", seed=clique_edge_seed(seed), **kw)
+  embedding = HypergraphEmbedding()
+  embedding.ParseFromString(embedding_to_wire(node_ids, Xn, edge_ids, Xe, dimension, "N2V_CLIQUE"))
   return embedding
 
 

@@ -633,6 +633,23 @@ int hge_n2v_train_epoch(hge_ctx* ctx, int32_t num_vertices, int dim, float* tin,
                         int64_t num_pairs, const int64_t* cum, int negative, uint64_t seed, int epoch, int epochs,
                         int batch_pairs, double alpha, double min_alpha, int64_t plan_bytes, double* loss);
 
+/* ---- node2vec on a weighted clique expansion (csrc/hge_n2v_clique.cu) -----------------------
+ * Walks of node2vec on one weighted clique expansion of the incidence, drawn from the incidence
+ * without building the expansion; DESIGN.md section 9.13.  side 0: V = N node vertices, w(u, x) =
+ * number of edges holding both; side 1: V = E edge vertices, w(c, y) = number of shared members
+ * (the side convention of hge_row_span).  Every array argument is a DEVICE pointer, with the
+ * contract of hge_n2v_walks: walks [num_walks V, walk_length] int32, walk w starting at vertex
+ * w mod V; a vertex with S(v) = sum over its edges e of (|e| - 1) = 0 gives that vertex followed
+ * by -1; counts [V] int64 the occurrences of every vertex.  Draws from Philox phase
+ * HGE_PHASE_N2V_CLIQUE_WALK (28), item = walk.  One int64 per incidence of the side is allocated
+ * for the call.  The pairs, noise table and training of the bipartite walker apply unchanged
+ * (hge_n2v_pairs, hge_n2v_init, hge_n2v_train_epoch with num_vertices = V).
+ * Refused with HGE_ERR_INVALID before anything runs: NULL pointers, a sharded incidence, side not
+ * 0 or 1, num_walks or walk_length < 1, p or q not positive and finite, max / min of (q, p q, p)
+ * above 65536 (the bound on the expected proposals per step), a side without vertices. */
+int hge_n2v_clique_walks(hge_ctx* ctx, hge_incidence* inc, int side, int num_walks, int walk_length, double p,
+                         double q, uint64_t seed, int32_t* walks, int64_t* counts);
+
 /* ---- hypergraph.proto wire format (host code; all pointers are host pointers) --------------
  * The data formats either side of the path: a serialized Hypergraph (hypergraph.proto:6-23) is
  * read straight into arrays, replacing the per-incidence Python loops of ToCsrMatrix /
